@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the detect-orfs scoring path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" is one pass of the hot path over one synthetic Ribo-seq library:
 K1 bin P-sites -> K2+K3 gather+score every candidate ORF -> clear of the resident
@@ -68,7 +68,14 @@ def parse_args():
                          "buffer, the step has no clear) or rt_bin_stream into a buffer the step clears (A/B)")
     ap.add_argument("--layout", default="compact", choices=["compact", "dense"],
                     help="coverage layout: exon union of the index (default) or genome-wide planes")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the result columns of the last step as DIR/<name>.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm keeps no per-ORF results")
+    return args
 
 
 # --------------------------------------------------------------------------- clocks
@@ -239,6 +246,27 @@ def cpu_closed_form_run(config_name: str, n_orf: int = 200_000):
             "sample": f"{idx.n_orf} ORFs of synthetic {config_name} at scale {scale:.2e}, contigs shrunk to fit host RAM"}
 
 
+# --------------------------------------------------------------------------- --dump-outputs
+DUMP_ROWS = 1_000_000   # ORFs written at most: six float64 files of this length stay under 64 MB
+
+
+def dump_outputs(out_dir: str, cols: dict, rows: np.ndarray, n_total: int, suffix: str = ""):
+    """Write the per-ORF result columns (score, valid, count, length, status) of the last timed step as float64
+    ``out_dir/<name><suffix>.npy``, with ``orf_index`` = the index row of each value.  ``rows`` are the index rows of
+    ``cols``.  An index of more than DUMP_ROWS ORFs is sampled: the same rows (seed 0) for every build and rank count,
+    so that two builds can be compared value for value."""
+    os.makedirs(out_dir, exist_ok=True)
+    if n_total > DUMP_ROWS:
+        keep = np.sort(np.random.default_rng(0).choice(n_total, DUMP_ROWS, replace=False))
+        pick = np.flatnonzero(np.isin(rows, keep))
+    else:
+        pick = np.arange(len(rows))
+    arrays = {k: cols[k] for k in ("score", "valid", "count", "length", "status")}
+    arrays["orf_index"] = rows
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), np.asarray(a)[pick].astype(np.float64))
+
+
 # --------------------------------------------------------------------------- reference arm
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
@@ -399,13 +427,16 @@ def run_ours(args):
     unbin_ms = float(np.mean([e[2].elapsed_time(e[3]) for e in per_step_events]))
     if not use_fresh:
         assert int(cov.abs().max().item()) == 0, "coverage did not return to zero after the sparse clear"
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: v.cpu().numpy() for k, v in out.items()}, np.asarray(shard.rows), n_orf_total,
+                     f".rank{rank}" if world > 1 else "")
 
     # ---- e2e: host buffers in, host buffers out, through the host-buffer C-ABI calls
     # From the decoder's host columns nothing is prepared outside the timed region: rt_bin_reads_host delta-codes every
     # chunk into the 4 B/read record stream on host threads while other chunks are on the wire and K1 runs on the stream.
     del dreads, dstream
     torch.cuda.empty_cache()
-    e2e_steps = max(3, min(args.steps, 5))
+    e2e_steps = args.steps
     hout = eng.new_host_score_columns(n_orf)      # pinned result columns, like the pinned read columns
     for _ in range(2):
         eng.clear_touched(cov)
@@ -588,7 +619,13 @@ def run_batch(args):
     n_lib_total = args.libraries
     mine = list(range(rank, n_lib_total, world))
     results = []
-    pipe = LibraryPipeline(eng, "forward", lambda tag, st, rlc, cols, cov: results.append((tag, st["valid"], int(cols["status"].sum()))))
+    last_cols = {}
+
+    def on_result(tag, st, rlc, cols, cov):
+        results.append((tag, st["valid"], int(cols["status"].sum())))
+        last_cols["cols"] = cols      # the pipeline's host buffer: valid after drain() for the last library
+
+    pipe = LibraryPipeline(eng, "forward", on_result)
 
     def barrier():
         if world > 1:
@@ -609,6 +646,8 @@ def run_batch(args):
         torch.cuda.synchronize()
         dt_local = time.perf_counter() - t0
         barrier()
+    if args.dump_outputs and last_cols:
+        dump_outputs(args.dump_outputs, last_cols["cols"], np.arange(idx.n_orf), idx.n_orf, f".rank{rank}" if world > 1 else "")
     t = torch.tensor([dt_local], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
