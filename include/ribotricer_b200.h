@@ -401,6 +401,67 @@ int rt_metagene_sums(const int32_t* flat, const int64_t* ptr, int64_t n_rows, in
 int rt_inflate_raw(const uint8_t* src, int64_t n_src, uint8_t* dst, int64_t n_dst);
 uint32_t rt_crc32(const uint8_t* p, int64_t n);
 
+/*
+ * ---- prepare-orfs: the candidate-ORF index from a GTF and a genome FASTA (DESIGN.md section 9) ----------------
+ * Host side (no GPU involved; errors in rt_io_last_error):
+ * rt_gtf_load parses the exon and CDS lines of a plain-text GTF in chunks on all cores (RT_GTF_THREADS overrides the
+ * number of chunks).  Comment and blank lines are skipped; any other line must have 9 tab-separated columns and
+ * integer start <= end, else RT_EINVAL with the line number.  Per kept line: 1-based line number, feature (0 exon,
+ * 1 CDS), chrom, start, end, strand (0 '+', 1 '-', 2 other) and 5 attribute string ids (gene_id, transcript_id,
+ * gene_name or else gene_id, gene_type or else gene_biotype, transcript_type or else transcript_biotype; -1 absent).
+ * Strings are NUL-terminated, back to back, in order of first appearance (rt_gtf_string_bytes bytes in all).
+ */
+typedef struct rt_gtf rt_gtf;
+int rt_gtf_load(const char* path, rt_gtf** out);
+void rt_gtf_free(rt_gtf* g);
+int64_t rt_gtf_n_lines(const rt_gtf* g);
+int64_t rt_gtf_n_strings(const rt_gtf* g);
+int64_t rt_gtf_string_bytes(const rt_gtf* g);
+int rt_gtf_copy(const rt_gtf* g, int64_t* line_no, uint8_t* feature, int32_t* chrom, int32_t* start, int32_t* end,
+                uint8_t* strand, int32_t* attr, char* strings);   /* any pointer may be NULL; attr: 5 per line */
+/* rt_fasta_load reads and indexes a plain-text FASTA on all cores (contig name = header up to the first blank; '\n' and
+ * '\r' are dropped; a duplicate name is RT_EINVAL).  rt_fasta_codes writes the listed contigs back to back as 1-byte
+ * codes (A C G T in either case -> 0-3, anything else -> 4).  Nothing is written next to the input. */
+typedef struct rt_fasta rt_fasta;
+int rt_fasta_load(const char* path, rt_fasta** out);
+void rt_fasta_free(rt_fasta* fa);
+int rt_fasta_n_contig(const rt_fasta* fa);
+const char* rt_fasta_contig_name(const rt_fasta* fa, int i);
+int64_t rt_fasta_contig_len(const rt_fasta* fa, int i);
+int rt_fasta_codes(const rt_fasta* fa, int n_sel, const int32_t* contigs, uint8_t* out);
+/* rt_orf_write writes {prefix}_candidate_orfs.tsv: the header, then one row per entry.  tx_text[tx_text_off[t],
+ * tx_text_off[t+1]) is "transcript_id\ttranscript_type\tgene_id\tgene_name\tgene_type\tchrom\tstrand" of transcript t,
+ * whose first tx_id_len[t] bytes are the transcript id.  row_type: 0 annotated, 1 uORF, 2 overlap_uORF, 3 super_uORF,
+ * 4 overlap_dORF, 5 dORF, 6 novel; row_codon: 6-bit codon code (16 b0 + 4 b1 + b2); intervals CSR, 1-based closed. */
+int rt_orf_write(const char* path, int64_t n_tx, const char* tx_text, const int64_t* tx_text_off, const int32_t* tx_id_len,
+                 int64_t n_rows, const int32_t* row_tx, const uint8_t* row_type, const uint8_t* row_codon,
+                 const int64_t* iv_ptr, const int32_t* iv_start, const int32_t* iv_end);
+/* Device side: rt_orf_search uploads the contig codes and the transcript table (merged exons, strand, oriented CDS
+ * bounds), splices and orients every transcript (orf_splice_kernel), counts and fills its candidate rows
+ * (orf_walk_kernel<false> / <true>: codon masks over the 6-bit codes, nearest in-frame stop, min length, longest, type;
+ * annotated and internal ORFs are not rows) and their genomic intervals (orf_interval_kernel<true> / <false>).  Rows are
+ * ordered by transcript, then start.  Returns the row and interval counts; the columns stay on the device until
+ * rt_orf_fetch copies them (any pointer may be NULL; iv_ptr has n_rows + 1 entries).  stage_ms (optional) receives the
+ * device time of RT_ORF_STAGES stages: upload, splice, count, row scan, fill, interval count + scan, interval fill. */
+#define RT_ORF_STAGES 7
+typedef struct rt_orf_query {
+    int64_t n_tx;
+    const int64_t* exon_ptr;        /* n_tx + 1 */
+    const int32_t* exon_start;      /* merged exons, 1-based closed, ascending within a transcript */
+    const int32_t* exon_end;
+    const int64_t* tx_base;         /* offset of the transcript's contig in codes */
+    const uint8_t* tx_strand;       /* 0 '+', 1 '-' */
+    const int32_t* tx_cds;          /* 2 per transcript: oriented first / last CDS nt, or -1 -1 */
+    const uint8_t* codes;           /* contig codes (rt_fasta_codes) */
+    int64_t n_codes;
+    uint64_t start_mask, stop_mask; /* bit c set: 6-bit codon code c is a start / stop codon */
+    int32_t min_orf_length;
+    int32_t longest;                /* of the starts that share a stop, keep the first only */
+} rt_orf_query;
+int rt_orf_search(rt_ctx* ctx, const rt_orf_query* q, int64_t* n_rows, int64_t* n_iv, float* stage_ms);
+int rt_orf_fetch(rt_ctx* ctx, int32_t* row_tx, int32_t* row_start, int32_t* row_stop, uint8_t* row_type, uint8_t* row_codon,
+                 int64_t* iv_ptr, int32_t* iv_start, int32_t* iv_end);
+
 /* number of kernel launches issued through this ctx so far (bench.py's gpu_launches) */
 int64_t rt_launch_count(const rt_ctx* ctx);
 /* bytes of read data the host-buffer entry points (rt_bin_reads_host, rt_bin_stream_host, rt_bin_reads_packed_host) have

@@ -31,7 +31,11 @@ EXPORTS = (
     "rt_repr_double", "rt_wig_open", "rt_wig_block", "rt_wig_close", "rt_bam_last_error", "rt_bam_load", "rt_bam_free", "rt_bam_n_reads", "rt_bam_n_ref",
     "rt_bam_ref_name", "rt_bam_ref_len", "rt_bam_sorted", "rt_bam_copy", "rt_bam_copy_span", "rt_bam_pack", "rt_bam_stream",
     "rt_inflate_raw", "rt_crc32", "rt_metagene_sums",
+    "rt_gtf_load", "rt_gtf_free", "rt_gtf_n_lines", "rt_gtf_n_strings", "rt_gtf_string_bytes", "rt_gtf_copy",
+    "rt_fasta_load", "rt_fasta_free", "rt_fasta_n_contig", "rt_fasta_contig_name", "rt_fasta_contig_len", "rt_fasta_codes",
+    "rt_orf_write", "rt_orf_search", "rt_orf_fetch",
 )
+RT_ORF_STAGES = 7
 
 
 class ScoreParams(C.Structure):
@@ -44,6 +48,13 @@ class ScoreOut(C.Structure):
     _fields_ = [("score", C.c_void_p), ("valid", C.c_void_p), ("count", C.c_void_p),
                 ("length", C.c_void_p), ("min_codon", C.c_void_p), ("status", C.c_void_p),
                 ("frame_K", C.c_void_p), ("frame_s", C.c_void_p)]
+
+
+class OrfQuery(C.Structure):
+    _fields_ = [("n_tx", C.c_int64), ("exon_ptr", C.c_void_p), ("exon_start", C.c_void_p), ("exon_end", C.c_void_p),
+                ("tx_base", C.c_void_p), ("tx_strand", C.c_void_p), ("tx_cds", C.c_void_p), ("codes", C.c_void_p),
+                ("n_codes", C.c_int64), ("start_mask", C.c_uint64), ("stop_mask", C.c_uint64),
+                ("min_orf_length", C.c_int32), ("longest", C.c_int32)]
 
 
 class RtError(RuntimeError):
@@ -153,6 +164,25 @@ def load():
     lib.rt_launch_count.restype = i64
     lib.rt_h2d_bytes.argtypes = [vp]
     lib.rt_h2d_bytes.restype = i64
+    lib.rt_gtf_load.argtypes = [C.c_char_p, C.POINTER(vp)]
+    lib.rt_gtf_free.argtypes = [vp]
+    lib.rt_gtf_free.restype = None
+    for name in ("rt_gtf_n_lines", "rt_gtf_n_strings", "rt_gtf_string_bytes"):
+        getattr(lib, name).argtypes = [vp]
+        getattr(lib, name).restype = i64
+    lib.rt_gtf_copy.argtypes = [vp] * 9
+    lib.rt_fasta_load.argtypes = [C.c_char_p, C.POINTER(vp)]
+    lib.rt_fasta_free.argtypes = [vp]
+    lib.rt_fasta_free.restype = None
+    lib.rt_fasta_n_contig.argtypes = [vp]
+    lib.rt_fasta_contig_name.argtypes = [vp, i32]
+    lib.rt_fasta_contig_name.restype = C.c_char_p
+    lib.rt_fasta_contig_len.argtypes = [vp, i32]
+    lib.rt_fasta_contig_len.restype = i64
+    lib.rt_fasta_codes.argtypes = [vp, i32, vp, vp]
+    lib.rt_orf_write.argtypes = [C.c_char_p, i64, vp, vp, vp, i64, vp, vp, vp, vp, vp, vp]
+    lib.rt_orf_search.argtypes = [vp, C.POINTER(OrfQuery), C.POINTER(i64), C.POINTER(i64), vp]
+    lib.rt_orf_fetch.argtypes = [vp] * 9
     if lib.rt_abi_version() != 3:
         raise RtError(f"ABI mismatch: library reports {lib.rt_abi_version()}, binding expects 3")
     _lib = lib

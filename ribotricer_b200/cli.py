@@ -1,8 +1,9 @@
-"""Command line of the B200 path: ``detect-orfs``, ``count-orfs`` and ``learn-cutoff``.
+"""Command line of the B200 path: ``prepare-orfs``, ``detect-orfs``, ``count-orfs`` and ``learn-cutoff``.
 
 The flag names, defaults, flag -> argument renames (``--min_read_density`` -> ``min_density_over_orf``,
 ``--stranded yes`` -> ``forward``, ``--meta-min-reads``) and every validation message are those of the
 reference command line (ribotricer/cli.py:127-289, 292-339, 435-560), so existing invocations keep working.
+``prepare-orfs`` takes the reference's flags (ribotricer/cli.py) and reads plain-text GTF and FASTA files only.
 The commands are assembled from option tables below.  ``--bam`` also accepts a ``.npz`` of decoded columns.
 """
 from __future__ import annotations
@@ -29,7 +30,7 @@ except ImportError:
 @click.group(**_GROUP_KW)
 @click.version_option(version=__version__)
 def cli() -> None:
-    """ribotricer: Tool for detecting translating ORF from Ribo-seq data (B200-native detect-orfs)"""
+    """ribotricer: Tool for detecting translating ORF from Ribo-seq data (B200-native prepare-orfs and detect-orfs)"""
 
 
 def _register(name: str, summary: str, options, handler) -> None:
@@ -60,6 +61,47 @@ def _int_list(text, name: str):
         return [int(item.strip()) for item in text.strip().split(",")]
     except Exception:
         _fail(f"cannot convert {name} into integers")
+
+
+# ------------------------------------------------------------------------------------ prepare-orfs
+def _codons(text: str, name: str) -> set:
+    """Comma separated codons, stripped and upper-cased; each must be three letters of ACGT."""
+    items = [item.strip().upper() for item in text.split(",")]
+    items = [item for item in items if item]
+    if not items:
+        _fail(f"{name} must list at least one codon")
+    for item in items:
+        if len(item) != 3 or any(b not in "ACGT" for b in item):
+            _fail(f"{name}: {item!r} is not a codon of three letters of ACGT")
+    return set(items)
+
+
+def _prepare(gtf, fasta, prefix, min_orf_length, start_codons, stop_codons, longest) -> None:
+    from .prepare_orfs import prepare_orfs
+
+    _need_file(gtf, "GTF file")
+    _need_file(fasta, "FASTA file")
+    for path, what in ((gtf, "GTF"), (fasta, "FASTA")):
+        if path.endswith((".gz", ".bgz")):
+            _fail(f"{what} file {path} is compressed; prepare-orfs reads plain text only (decompress it first)")
+    if min_orf_length < 0:
+        _fail("min_orf_length must be >= 0")
+    starts, stops = _codons(start_codons, "start_codons"), _codons(stop_codons, "stop_codons")
+    try:
+        prepare_orfs(gtf, fasta, prefix, min_orf_length, starts, stops, longest)
+    except ValueError as exc:
+        _fail(str(exc))
+
+
+_register("prepare-orfs", "Extract candidate ORFs based on GTF and FASTA files", [
+    ("--gtf", dict(help="Path to GTF file", required=True)),
+    ("--fasta", dict(help="Path to FASTA file", required=True)),
+    ("--prefix", dict(help="Prefix to output file", required=True)),
+    ("--min_orf_length", dict(type=int, default=60, show_default=True, help="The minimum length (nts) of ORF to include")),
+    ("--start_codons", dict(default="ATG", show_default=True, help="Comma separated list of start codons")),
+    ("--stop_codons", dict(default="TAG,TAA,TGA", show_default=True, help="Comma separated list of stop codons")),
+    ("--longest", dict(is_flag=True, help="Choose the most upstream start codon if multiple in frame ones exist")),
+], _prepare)
 
 
 # ------------------------------------------------------------------------------------ detect-orfs

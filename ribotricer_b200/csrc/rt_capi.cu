@@ -148,6 +148,11 @@ struct rt_ctx {
     DevBuf touched_buf;
     unsigned long long* d_n_touched = nullptr;
     int64_t touched_reserved = 0;    // reads binned (weight +1) since the last clear
+
+    // prepare-orfs (rt_orf_search / rt_orf_fetch): the last search's tables and rows stay on the device until fetched
+    DevBuf orf_buf[32];
+    std::vector<int64_t> orf_iv_ptr;                 // n_rows + 1: interval offsets of the last search
+    int64_t orf_rows = 0;
 };
 
 namespace {
@@ -420,6 +425,7 @@ int rt_create(int device, rt_ctx** out) {
 void rt_destroy(rt_ctx* ctx) {
     if (!ctx) return;
     DeviceGuard guard(ctx->device);
+    for (auto& b : ctx->orf_buf) b.release();
     cudaFree(ctx->d_contig_tab);
     cudaFree(ctx->d_uv_table);
     cudaFree(ctx->d_len_table);
@@ -1967,6 +1973,200 @@ int rt_bootstrap_medians(rt_ctx* ctx, const double* h_values, int64_t n, const i
     if (e == cudaSuccess) e = cudaMemcpy(h_out, outb.p, sizeof(double) * (size_t)reps, cudaMemcpyDeviceToHost);
     cleanup();
     if (e != cudaSuccess) return fail(ctx, e == cudaErrorMemoryAllocation ? RT_ENOMEM : RT_ECUDA, "rt_bootstrap_medians: %s", cudaGetErrorString(e));
+    return RT_OK;
+}
+
+// ------------------------------------------------------------------------------------------------ prepare-orfs
+namespace {
+enum OrfBuf { kCodes, kExSrc, kExDst, kExLen, kExRev, kTxSeq, kTxCds, kTxExon, kTxRev, kExStart, kExEnd, kExBefore, kSeq,
+              kTxRows, kRowOff, kRowTx, kRowStart, kRowStop, kRowType, kRowCodon, kIvCount, kIvOff, kIvStart, kIvEnd,
+              kClaim, kOrfBufs };
+static_assert(kOrfBufs <= 32, "rt_ctx::orf_buf is too small");
+}  // namespace
+
+int rt_orf_search(rt_ctx* ctx, const rt_orf_query* q, int64_t* n_rows, int64_t* n_iv, float* stage_ms) {
+    if (!ctx) return fail(nullptr, RT_EINVAL, "rt_orf_search: ctx is NULL");
+    if (!q || !n_rows || !n_iv || q->n_tx < 0 || q->n_codes < 0 || q->min_orf_length < 0 ||
+        (q->n_tx && (!q->exon_ptr || !q->exon_start || !q->exon_end || !q->tx_base || !q->tx_strand || !q->tx_cds)) ||
+        (q->n_codes && !q->codes))
+        return fail(ctx, RT_EINVAL, "rt_orf_search: NULL or negative argument");
+    if (q->n_tx > 0x7fffffff) return fail(ctx, RT_EINVAL, "rt_orf_search: more than 2^31 - 1 transcripts");
+    const int64_t n_tx = q->n_tx;
+    const int64_t n_ex = n_tx ? q->exon_ptr[n_tx] : 0;
+    // host side of the transcript table: per exon its source in codes, its place in the spliced buffer, its offset
+    // within the transcript's ascending concatenation
+    std::vector<int64_t> ex_src((size_t)n_ex), ex_dst((size_t)n_ex), tx_seq((size_t)n_tx + 1, 0);
+    std::vector<int32_t> ex_len((size_t)n_ex), ex_before((size_t)n_ex);
+    std::vector<uint8_t> ex_rev((size_t)n_ex);
+    for (int64_t t = 0; t < n_tx; ++t) {
+        const int64_t a = q->exon_ptr[t], b = q->exon_ptr[t + 1];
+        if (a < 0 || b <= a || b > n_ex) return fail(ctx, RT_EINVAL, "rt_orf_search: transcript %lld has no exon", (long long)t);
+        if (q->tx_strand[t] > 1) return fail(ctx, RT_EINVAL, "rt_orf_search: transcript %lld has no strand", (long long)t);
+        int64_t n = 0;
+        for (int64_t e = a; e < b; ++e) {
+            if (q->exon_start[e] < 1 || q->exon_end[e] < q->exon_start[e] || (e > a && q->exon_start[e] <= q->exon_end[e - 1]) ||
+                q->tx_base[t] < 0 || q->tx_base[t] + q->exon_end[e] > q->n_codes)
+                return fail(ctx, RT_EINVAL, "rt_orf_search: exon %lld of transcript %lld is unsorted or outside the codes",
+                            (long long)(e - a), (long long)t);
+            ex_before[(size_t)e] = (int32_t)n;
+            ex_len[(size_t)e] = q->exon_end[e] - q->exon_start[e] + 1;
+            ex_src[(size_t)e] = q->tx_base[t] + q->exon_start[e] - 1;
+            ex_rev[(size_t)e] = q->tx_strand[t];
+            n += ex_len[(size_t)e];
+            if (n > 0x7fffffff) return fail(ctx, RT_EINVAL, "rt_orf_search: transcript %lld is longer than 2^31 - 1", (long long)t);
+        }
+        for (int64_t e = a; e < b; ++e)
+            ex_dst[(size_t)e] = tx_seq[(size_t)t] + (q->tx_strand[t] ? n - ex_before[(size_t)e] - ex_len[(size_t)e] : ex_before[(size_t)e]);
+        tx_seq[(size_t)t + 1] = tx_seq[(size_t)t] + n;
+    }
+    const int64_t n_seq = tx_seq[(size_t)n_tx];
+    DeviceGuard guard(ctx->device);
+    DevBuf* B = ctx->orf_buf;
+    auto reserve = [&](int k, size_t bytes) { return B[k].reserve(std::max<size_t>(bytes, 16)); };
+    RT_CUDA(ctx, reserve(kCodes, (size_t)q->n_codes));
+    RT_CUDA(ctx, reserve(kExSrc, 8 * (size_t)n_ex));
+    RT_CUDA(ctx, reserve(kExDst, 8 * (size_t)n_ex));
+    RT_CUDA(ctx, reserve(kExLen, 4 * (size_t)n_ex));
+    RT_CUDA(ctx, reserve(kExRev, (size_t)n_ex));
+    RT_CUDA(ctx, reserve(kTxSeq, 8 * (size_t)(n_tx + 1)));
+    RT_CUDA(ctx, reserve(kTxCds, 8 * (size_t)n_tx));
+    RT_CUDA(ctx, reserve(kTxExon, 8 * (size_t)(n_tx + 1)));
+    RT_CUDA(ctx, reserve(kTxRev, (size_t)n_tx));
+    RT_CUDA(ctx, reserve(kExStart, 4 * (size_t)n_ex));
+    RT_CUDA(ctx, reserve(kExEnd, 4 * (size_t)n_ex));
+    RT_CUDA(ctx, reserve(kExBefore, 4 * (size_t)n_ex));
+    RT_CUDA(ctx, reserve(kSeq, (size_t)n_seq + 4));
+    RT_CUDA(ctx, reserve(kTxRows, 8 * (size_t)n_tx));
+    RT_CUDA(ctx, reserve(kRowOff, 8 * (size_t)n_tx));
+    RT_CUDA(ctx, reserve(kClaim, 4));
+    cudaStream_t st = 0;
+    cudaEvent_t ev[RT_ORF_STAGES + 1];
+    for (auto& e : ev) RT_CUDA(ctx, cudaEventCreate(&e));
+    struct EvGuard { cudaEvent_t* ev; ~EvGuard() { for (int i = 0; i <= RT_ORF_STAGES; ++i) cudaEventDestroy(ev[i]); } } evg{ev};
+    auto up = [&](int k, const void* src, size_t bytes) { return bytes ? cudaMemcpyAsync(B[k].p, src, bytes, cudaMemcpyHostToDevice, st) : cudaSuccess; };
+    RT_CUDA(ctx, cudaEventRecord(ev[0], st));
+    // 1. upload: contig codes, the transcript and exon tables
+    RT_CUDA(ctx, up(kCodes, q->codes, (size_t)q->n_codes));
+    RT_CUDA(ctx, up(kExSrc, ex_src.data(), 8 * (size_t)n_ex));
+    RT_CUDA(ctx, up(kExDst, ex_dst.data(), 8 * (size_t)n_ex));
+    RT_CUDA(ctx, up(kExLen, ex_len.data(), 4 * (size_t)n_ex));
+    RT_CUDA(ctx, up(kExRev, ex_rev.data(), (size_t)n_ex));
+    RT_CUDA(ctx, up(kTxSeq, tx_seq.data(), 8 * (size_t)(n_tx + 1)));
+    RT_CUDA(ctx, up(kTxCds, q->tx_cds, 8 * (size_t)n_tx));
+    RT_CUDA(ctx, up(kTxExon, q->exon_ptr, 8 * (size_t)(n_tx + 1)));
+    RT_CUDA(ctx, up(kTxRev, q->tx_strand, (size_t)n_tx));
+    RT_CUDA(ctx, up(kExStart, q->exon_start, 4 * (size_t)n_ex));
+    RT_CUDA(ctx, up(kExEnd, q->exon_end, 4 * (size_t)n_ex));
+    RT_CUDA(ctx, up(kExBefore, ex_before.data(), 4 * (size_t)n_ex));
+    RT_CUDA(ctx, cudaEventRecord(ev[1], st));
+    const unsigned big = (unsigned)std::max(1, ctx->n_sm * 8);
+    // 2. spliced, oriented sequences
+    if (n_ex) {
+        rt::orf_splice_kernel<<<(unsigned)std::min<int64_t>((n_ex + 7) / 8, big), 256, 0, st>>>(
+            (const uint8_t*)B[kCodes].p, (const long long*)B[kExSrc].p, (const long long*)B[kExDst].p, (const int*)B[kExLen].p,
+            (const uint8_t*)B[kExRev].p, n_ex, (uint8_t*)B[kSeq].p);
+        ctx->launches++;
+        RT_CUDA(ctx, cudaGetLastError());
+    }
+    RT_CUDA(ctx, cudaEventRecord(ev[2], st));
+    // 3. rows per transcript
+    rt::OrfArgs A{(const long long*)B[kTxSeq].p, (const int2*)B[kTxCds].p, (uint8_t*)B[kSeq].p, q->start_mask, q->stop_mask,
+                  (int)n_tx, q->min_orf_length, q->longest ? 1 : 0, (unsigned*)B[kClaim].p};
+    const unsigned walk_grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((n_tx + 7) / 8, big));
+    if (n_tx) {
+        RT_CUDA(ctx, cudaMemsetAsync(B[kClaim].p, 0, 4, st));
+        rt::orf_walk_kernel<false><<<walk_grid, 256, 0, st>>>(A, (long long*)B[kTxRows].p, nullptr, nullptr, nullptr, nullptr,
+                                                                nullptr, nullptr);
+        ctx->launches++;
+        RT_CUDA(ctx, cudaGetLastError());
+    }
+    RT_CUDA(ctx, cudaEventRecord(ev[3], st));
+    // 4. exclusive scan of the row counts (host: one int64 per transcript)
+    std::vector<int64_t> cnt((size_t)n_tx), off((size_t)n_tx + 1, 0);
+    if (n_tx) RT_CUDA(ctx, cudaMemcpyAsync(cnt.data(), B[kTxRows].p, 8 * (size_t)n_tx, cudaMemcpyDeviceToHost, st));
+    RT_CUDA(ctx, cudaStreamSynchronize(st));
+    for (int64_t t = 0; t < n_tx; ++t) off[(size_t)t + 1] = off[(size_t)t] + cnt[(size_t)t];
+    const int64_t rows = off[(size_t)n_tx];
+    RT_CUDA(ctx, reserve(kRowTx, 4 * (size_t)rows));
+    RT_CUDA(ctx, reserve(kRowStart, 4 * (size_t)rows));
+    RT_CUDA(ctx, reserve(kRowStop, 4 * (size_t)rows));
+    RT_CUDA(ctx, reserve(kRowType, (size_t)rows));
+    RT_CUDA(ctx, reserve(kRowCodon, (size_t)rows));
+    RT_CUDA(ctx, reserve(kIvCount, 8 * (size_t)rows));
+    RT_CUDA(ctx, reserve(kIvOff, 8 * (size_t)rows));
+    RT_CUDA(ctx, up(kRowOff, off.data(), 8 * (size_t)n_tx));
+    RT_CUDA(ctx, cudaEventRecord(ev[4], st));
+    // 5. the rows
+    if (rows) {
+        RT_CUDA(ctx, cudaMemsetAsync(B[kClaim].p, 0, 4, st));
+        rt::orf_walk_kernel<true><<<walk_grid, 256, 0, st>>>(A, (long long*)B[kTxRows].p, (const long long*)B[kRowOff].p,
+                                                               (int*)B[kRowTx].p, (int*)B[kRowStart].p, (int*)B[kRowStop].p,
+                                                               (uint8_t*)B[kRowType].p, (uint8_t*)B[kRowCodon].p);
+        ctx->launches++;
+        RT_CUDA(ctx, cudaGetLastError());
+    }
+    RT_CUDA(ctx, cudaEventRecord(ev[5], st));
+    // 6. intervals per row, their exclusive scan (host)
+    const unsigned row_grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((rows + 255) / 256, (int64_t)big * 4));
+    auto intervals = [&](bool count) {
+        if (count)
+            rt::orf_interval_kernel<true><<<row_grid, 256, 0, st>>>(
+                rows, (const int*)B[kRowTx].p, (const int*)B[kRowStart].p, (const int*)B[kRowStop].p, (const long long*)B[kTxExon].p,
+                (const long long*)B[kTxSeq].p, (const uint8_t*)B[kTxRev].p, (const int*)B[kExStart].p, (const int*)B[kExEnd].p,
+                (const int*)B[kExBefore].p, (long long*)B[kIvCount].p, nullptr, nullptr, nullptr);
+        else
+            rt::orf_interval_kernel<false><<<row_grid, 256, 0, st>>>(
+                rows, (const int*)B[kRowTx].p, (const int*)B[kRowStart].p, (const int*)B[kRowStop].p, (const long long*)B[kTxExon].p,
+                (const long long*)B[kTxSeq].p, (const uint8_t*)B[kTxRev].p, (const int*)B[kExStart].p, (const int*)B[kExEnd].p,
+                (const int*)B[kExBefore].p, nullptr, (const long long*)B[kIvOff].p, (int*)B[kIvStart].p, (int*)B[kIvEnd].p);
+        ctx->launches++;
+        return cudaGetLastError();
+    };
+    std::vector<int64_t>& ivp = ctx->orf_iv_ptr;
+    ivp.assign((size_t)rows + 1, 0);
+    if (rows) {
+        RT_CUDA(ctx, intervals(true));
+        std::vector<int64_t> ivc((size_t)rows);
+        RT_CUDA(ctx, cudaMemcpyAsync(ivc.data(), B[kIvCount].p, 8 * (size_t)rows, cudaMemcpyDeviceToHost, st));
+        RT_CUDA(ctx, cudaStreamSynchronize(st));
+        for (int64_t r = 0; r < rows; ++r) ivp[(size_t)r + 1] = ivp[(size_t)r] + ivc[(size_t)r];
+    }
+    const int64_t ivs = ivp.back();
+    RT_CUDA(ctx, reserve(kIvStart, 4 * (size_t)ivs));
+    RT_CUDA(ctx, reserve(kIvEnd, 4 * (size_t)ivs));
+    RT_CUDA(ctx, up(kIvOff, ivp.data(), 8 * (size_t)rows));
+    RT_CUDA(ctx, cudaEventRecord(ev[6], st));
+    // 7. the intervals
+    if (rows) RT_CUDA(ctx, intervals(false));
+    RT_CUDA(ctx, cudaEventRecord(ev[7], st));
+    RT_CUDA(ctx, cudaStreamSynchronize(st));
+    if (stage_ms)
+        for (int i = 0; i < RT_ORF_STAGES; ++i) RT_CUDA(ctx, cudaEventElapsedTime(&stage_ms[i], ev[i], ev[i + 1]));
+    ctx->orf_rows = rows;
+    *n_rows = rows;
+    *n_iv = ivs;
+    return RT_OK;
+}
+
+int rt_orf_fetch(rt_ctx* ctx, int32_t* row_tx, int32_t* row_start, int32_t* row_stop, uint8_t* row_type, uint8_t* row_codon,
+                 int64_t* iv_ptr, int32_t* iv_start, int32_t* iv_end) {
+    if (!ctx) return fail(nullptr, RT_EINVAL, "rt_orf_fetch: ctx is NULL");
+    const int64_t rows = ctx->orf_rows;
+    if ((int64_t)ctx->orf_iv_ptr.size() != rows + 1) return fail(ctx, RT_ESTATE, "rt_orf_fetch: call rt_orf_search first");
+    const int64_t ivs = ctx->orf_iv_ptr.back();
+    DeviceGuard guard(ctx->device);
+    DevBuf* B = ctx->orf_buf;
+    cudaStream_t st = 0;
+    auto down = [&](void* dst, int k, size_t bytes) { return dst && bytes ? cudaMemcpyAsync(dst, B[k].p, bytes, cudaMemcpyDeviceToHost, st) : cudaSuccess; };
+    RT_CUDA(ctx, down(row_tx, kRowTx, 4 * (size_t)rows));
+    RT_CUDA(ctx, down(row_start, kRowStart, 4 * (size_t)rows));
+    RT_CUDA(ctx, down(row_stop, kRowStop, 4 * (size_t)rows));
+    RT_CUDA(ctx, down(row_type, kRowType, (size_t)rows));
+    RT_CUDA(ctx, down(row_codon, kRowCodon, (size_t)rows));
+    RT_CUDA(ctx, down(iv_start, kIvStart, 4 * (size_t)ivs));
+    RT_CUDA(ctx, down(iv_end, kIvEnd, 4 * (size_t)ivs));
+    if (iv_ptr) memcpy(iv_ptr, ctx->orf_iv_ptr.data(), 8 * (size_t)(rows + 1));
+    RT_CUDA(ctx, cudaStreamSynchronize(st));
     return RT_OK;
 }
 

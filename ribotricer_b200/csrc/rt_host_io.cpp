@@ -239,6 +239,12 @@ extern "C" {
 
 const char* rt_io_last_error(void) { return g_io_error.c_str(); }
 
+}  // extern "C"
+
+void rt_io_set_error(const std::string& msg) { g_io_error = msg; }   // rt_prepare.cpp reports through the same slot
+
+extern "C" {
+
 int rt_index_load(const char* path, rt_index** out) {
     if (!path || !out) return RT_EINVAL;
     *out = nullptr;

@@ -3169,4 +3169,187 @@ __global__ void __launch_bounds__(32) phasescore_values_kernel(const double* __r
     }
 }
 
+
+// ------------------------------------------------------------------------------------------------- prepare-orfs
+// Candidate ORFs of every transcript (DESIGN.md section 9).  orf_splice_kernel writes each transcript's spliced,
+// strand-oriented sequence (codes 0-3 = ACGT, 4 = anything else; '-' transcripts reverse-complemented).  The count and
+// fill kernels give one warp to a transcript, claimed dynamically (lengths run from 100 nt to more than 100 knt), and
+// walk it in windows of 32 codon positions, one per lane: ballots of the start and stop positions, and per frame the
+// nearest stop to the right carried from window to window (3' -> 5').  With `longest`, a 5' -> 3' walk first marks the
+// first start of every stop segment (bit 7 of its code byte).  Rows come out in ascending start order per transcript.
+enum : uint8_t { kOrfAnnotated = 0, kOrfU = 1, kOrfOverlapU = 2, kOrfSuperU = 3, kOrfOverlapD = 4, kOrfD = 5,
+                 kOrfNovel = 6, kOrfInternal = 7 };
+
+struct OrfArgs {
+    const long long* tx_seq;          // n_tx + 1: offset of each transcript's spliced sequence
+    const int2* tx_cds;               // oriented first / last CDS nt, (-1, -1) without a CDS
+    uint8_t* seq;                     // spliced sequences (bit 7: first start of its stop segment, longest only)
+    unsigned long long start_mask, stop_mask;
+    int n_tx, min_len, longest;
+    unsigned* claim;                  // work counter, zeroed before the launch
+};
+
+__global__ void orf_splice_kernel(const uint8_t* __restrict__ codes, const long long* __restrict__ ex_src,
+                                  const long long* __restrict__ ex_dst, const int* __restrict__ ex_len,
+                                  const uint8_t* __restrict__ ex_rev, long long n_exon, uint8_t* __restrict__ seq) {
+    const int lane = threadIdx.x & 31;
+    const long long warps = (long long)gridDim.x * (blockDim.x >> 5);
+    for (long long e = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; e < n_exon; e += warps) {
+        const uint8_t* src = codes + ex_src[e];
+        const int len = ex_len[e];
+        if (ex_rev[e]) {            // '-': ex_dst is the oriented position of the exon's last genomic nt
+            uint8_t* dst = seq + ex_dst[e];
+            for (int k = lane; k < len; k += 32) {
+                const uint8_t c = src[k];
+                dst[len - 1 - k] = c < 4 ? (uint8_t)(3 - c) : (uint8_t)4;
+            }
+        } else {
+            uint8_t* dst = seq + ex_dst[e];
+            for (int k = lane; k < len; k += 32) dst[k] = src[k];
+        }
+    }
+}
+
+__device__ __forceinline__ uint8_t orf_classify(int a, int b, int2 cds) {
+    const int c = cds.x, d = cds.y;
+    if (c < 0) return kOrfNovel;
+    if (b < c) return kOrfU;
+    if (a < c) return b < d ? kOrfOverlapU : kOrfSuperU;
+    if (a > d) return kOrfD;
+    if (b > d) return kOrfOverlapD;
+    return (a == c && b == d) ? kOrfAnnotated : kOrfInternal;
+}
+
+// 6-bit codon code at i (16 c0 + 4 c1 + c2), or -1 when a base is not ACGT
+__device__ __forceinline__ int orf_codon(const uint8_t* s, long long i) {
+    const int a = s[i] & 7, b = s[i + 1] & 7, c = s[i + 2] & 7;
+    return (a | b | c) & 4 ? -1 : (a << 4) | (b << 2) | c;
+}
+
+template <bool FILL>
+__global__ void __launch_bounds__(256) orf_walk_kernel(OrfArgs A, long long* __restrict__ tx_rows,
+                                                       const long long* __restrict__ row_off, int* __restrict__ row_tx,
+                                                       int* __restrict__ row_start, int* __restrict__ row_stop,
+                                                       uint8_t* __restrict__ row_type, uint8_t* __restrict__ row_codon) {
+    const int lane = threadIdx.x & 31;
+    const unsigned full = 0xffffffffu;
+    const unsigned below = (1u << lane) - 1u, above = lane == 31 ? 0u : ~0u << (lane + 1);
+    for (;;) {
+        int t = 0;
+        if (lane == 0) t = (int)atomicAdd(A.claim, 1u);
+        t = __shfl_sync(full, t, 0);
+        if (t >= A.n_tx) return;
+        uint8_t* s = A.seq + A.tx_seq[t];
+        const long long n = A.tx_seq[t + 1] - A.tx_seq[t];
+        if (n < 3) { if (!FILL && lane == 0) tx_rows[t] = 0; continue; }
+        const long long last = n - 3;                   // last codon position
+        const int2 cds = A.tx_cds[t];
+        if (!FILL && A.longest) {                       // 5' -> 3': mark the first start of every stop segment
+            unsigned open = 0;                          // bit g: frame g has a start since its last stop
+            for (long long base = 0; base <= last; base += 32) {
+                const long long i = base + lane;
+                const int cc = i <= last ? orf_codon(s, i) : -1;
+                const bool st = cc >= 0 && ((A.stop_mask >> cc) & 1ull), sa = cc >= 0 && ((A.start_mask >> cc) & 1ull);
+                const unsigned bst = __ballot_sync(full, st), bsa = __ballot_sync(full, sa);
+                const int f = (int)(i % 3);
+                const unsigned fm0 = __ballot_sync(full, f == 0), fm1 = __ballot_sync(full, f == 1), fm2 = ~(fm0 | fm1);
+                if (sa) {
+                    const unsigned fm = f == 0 ? fm0 : f == 1 ? fm1 : fm2;
+                    const unsigned stops_le = bst & fm & (below | (1u << lane));
+                    bool first;
+                    if (stops_le) {
+                        const int lst = 31 - __clz(stops_le);
+                        first = (bsa & fm & below & ~((1u << lst) - 1u)) == 0u;   // a start at the stop itself opens the segment
+                    } else {
+                        first = (bsa & fm & below) == 0u && !((open >> f) & 1u);
+                    }
+                    if (first) s[i] |= 0x80;
+                }
+#pragma unroll
+                for (int g = 0; g < 3; ++g) {
+                    const unsigned fm = g == 0 ? fm0 : g == 1 ? fm1 : fm2;
+                    const unsigned ms = bst & fm, ma = bsa & fm;
+                    const bool o = ms ? (ma >> (31 - __clz(ms))) != 0u : (((open >> g) & 1u) || ma != 0u);
+                    open = (open & ~(1u << g)) | ((unsigned)o << g);
+                }
+            }
+            __syncwarp();
+        }
+        // 3' -> 5': the nearest in-frame stop of every start, the rules, the rows
+        int next0 = -1, next1 = -1, next2 = -1;           // per frame: nearest stop right of the window
+        long long done = 0;                             // rows of this transcript at positions right of the window
+        const long long total = FILL ? tx_rows[t] : 0;
+        const long long out0 = FILL ? row_off[t] : 0;
+        for (long long base = (last / 32) * 32; base >= 0; base -= 32) {
+            const long long i = base + lane;
+            const int cc = i <= last ? orf_codon(s, i) : -1;
+            const bool st = cc >= 0 && ((A.stop_mask >> cc) & 1ull), sa = cc >= 0 && ((A.start_mask >> cc) & 1ull);
+            const unsigned bst = __ballot_sync(full, st);
+            const int f = (int)(i % 3);
+            const unsigned fm0 = __ballot_sync(full, f == 0), fm1 = __ballot_sync(full, f == 1), fm2 = ~(fm0 | fm1);
+            bool keep = false;
+            int p = -1;
+            uint8_t type = 0;
+            if (sa) {
+                const unsigned right = bst & (f == 0 ? fm0 : f == 1 ? fm1 : fm2) & above;
+                p = right ? (int)base + __ffs(right) - 1 : f == 0 ? next0 : f == 1 ? next1 : next2;
+                if (p >= 0 && p - (int)i >= A.min_len && (!A.longest || (s[i] & 0x80))) {
+                    type = orf_classify((int)i, p - 1, cds);
+                    keep = type != kOrfAnnotated && type != kOrfInternal;
+                }
+            }
+            const unsigned bkeep = __ballot_sync(full, keep);
+            if (FILL && keep) {
+                const long long r = out0 + total - 1 - (done + __popc(bkeep & above));
+                row_tx[r] = t;
+                row_start[r] = (int)i;
+                row_stop[r] = p;
+                row_type[r] = type;
+                row_codon[r] = (uint8_t)cc;
+            }
+            done += __popc(bkeep);
+            if (bst & fm0) next0 = (int)base + __ffs(bst & fm0) - 1;
+            if (bst & fm1) next1 = (int)base + __ffs(bst & fm1) - 1;
+            if (bst & fm2) next2 = (int)base + __ffs(bst & fm2) - 1;
+        }
+        if (!FILL && lane == 0) tx_rows[t] = done;
+    }
+}
+
+// Genomic intervals of every row: the oriented range [start, stop) of transcript t as ascending 1-based closed
+// intervals of its merged exons.  COUNT writes the number per row, otherwise the intervals at iv_off[row].
+template <bool COUNT>
+__global__ void orf_interval_kernel(long long n_rows, const int* __restrict__ row_tx, const int* __restrict__ row_start,
+                                    const int* __restrict__ row_stop, const long long* __restrict__ tx_exon,
+                                    const long long* __restrict__ tx_seq, const uint8_t* __restrict__ tx_rev,
+                                    const int* __restrict__ ex_start, const int* __restrict__ ex_end,
+                                    const int* __restrict__ ex_before, long long* __restrict__ iv_count,
+                                    const long long* __restrict__ iv_off, int* __restrict__ iv_start, int* __restrict__ iv_end) {
+    for (long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x; r < n_rows; r += (long long)gridDim.x * blockDim.x) {
+        const int t = row_tx[r];
+        const int n = (int)(tx_seq[t + 1] - tx_seq[t]);
+        const int lo = tx_rev[t] ? n - row_stop[r] : row_start[r];
+        const int hi = tx_rev[t] ? n - row_start[r] : row_stop[r];
+        const long long e0 = tx_exon[t], e1 = tx_exon[t + 1];
+        auto find = [&](int x) {                        // last exon whose first nt is at or before x
+            long long a = e0, b = e1 - 1;
+            while (a < b) {
+                const long long m = (a + b + 1) >> 1;
+                if (ex_before[m] <= x) a = m; else b = m - 1;
+            }
+            return a;
+        };
+        const long long ea = find(lo), eb = find(hi - 1);
+        if (COUNT) {
+            iv_count[r] = eb - ea + 1;
+        } else {
+            long long o = iv_off[r];
+            for (long long e = ea; e <= eb; ++e, ++o) {
+                iv_start[o] = e == ea ? ex_start[e] + (lo - ex_before[e]) : ex_start[e];
+                iv_end[o] = e == eb ? ex_start[e] + (hi - 1 - ex_before[e]) : ex_end[e];
+            }
+        }
+    }
+}
+
 }  // namespace rt

@@ -522,3 +522,29 @@ class Engine:
                                                 C.c_void_p(d_ids.data_ptr()), C.c_void_p(d_ptr.data_ptr()),
                                                 C.c_void_p(d_out.data_ptr()), self._stream()))
         return out_ptr, d_out[:total].cpu().numpy()
+
+    # --------------------------------------------------------------- prepare-orfs
+    def orf_search(self, codes, tx_base, exon_ptr, exon_start, exon_end, tx_strand, tx_cds, start_mask: int,
+                   stop_mask: int, min_orf_length: int, longest: bool, stage_ms: np.ndarray | None = None) -> dict:
+        """Candidate ORFs of every transcript (``rt_orf_search`` + ``rt_orf_fetch``): HOST columns ``row_tx``,
+        ``row_start`` / ``row_stop`` (the oriented range [start, stop) in the transcript), ``row_type``, ``row_codon``
+        and the genomic intervals as CSR ``iv_ptr`` / ``iv_start`` / ``iv_end``, rows by transcript, then start."""
+        arr = lambda a, dt: np.ascontiguousarray(a, dt)  # noqa: E731
+        codes, tx_base, exon_ptr = arr(codes, np.uint8), arr(tx_base, np.int64), arr(exon_ptr, np.int64)
+        exon_start, exon_end = arr(exon_start, np.int32), arr(exon_end, np.int32)
+        tx_strand, tx_cds = arr(tx_strand, np.uint8), arr(tx_cds, np.int32)
+        q = _lib.OrfQuery(len(tx_base), _np_ptr(exon_ptr), _np_ptr(exon_start), _np_ptr(exon_end), _np_ptr(tx_base),
+                          _np_ptr(tx_strand), _np_ptr(tx_cds), _np_ptr(codes), len(codes), int(start_mask),
+                          int(stop_mask), int(min_orf_length), int(bool(longest)))
+        n_rows, n_iv = C.c_int64(0), C.c_int64(0)
+        ms = np.zeros(_lib.RT_ORF_STAGES, np.float32)
+        self._check(self.lib.rt_orf_search(self.ctx, C.byref(q), C.byref(n_rows), C.byref(n_iv), _np_ptr(ms)))
+        if stage_ms is not None:
+            stage_ms[:] = ms
+        n, m = int(n_rows.value), int(n_iv.value)
+        out = dict(row_tx=np.empty(n, np.int32), row_start=np.empty(n, np.int32), row_stop=np.empty(n, np.int32),
+                   row_type=np.empty(n, np.uint8), row_codon=np.empty(n, np.uint8), iv_ptr=np.empty(n + 1, np.int64),
+                   iv_start=np.empty(m, np.int32), iv_end=np.empty(m, np.int32))
+        self._check(self.lib.rt_orf_fetch(self.ctx, *[_np_ptr(out[k]) for k in (
+            "row_tx", "row_start", "row_stop", "row_type", "row_codon", "iv_ptr", "iv_start", "iv_end")]))
+        return out

@@ -344,3 +344,171 @@ def reads_to_numpy(cols: dict) -> dict:
             a = a.view(np.uint16)
         out[k] = a
     return out
+
+
+# --------------------------------------------------------------------------------------------------------------
+# Annotation + genome for prepare-orfs: a seeded FASTA and GTF with planted coding sequences.
+# --------------------------------------------------------------------------------------------------------------
+_STOPS = (b"TAA", b"TAG", b"TGA")
+_COMPLEMENT = np.frombuffer(bytes.maketrans(b"ACGTNacgtn", b"TGCANtgcan"), np.uint8)
+
+
+def _sense_codons(rng, k: int) -> bytes:
+    """k random codons, none of them a stop."""
+    out = rng.choice(np.frombuffer(b"ACGT", np.uint8), 3 * k + 96).tobytes()
+    codons = [out[i:i + 3] for i in range(0, len(out) - 2, 3)]
+    codons = [c for c in codons if c not in _STOPS]
+    while len(codons) < k:
+        codons.append(b"GCT")
+    return b"".join(codons[:k])
+
+
+def make_annotation(out_dir: str, n_genes: int = 40, tx_per_gene: float = 2.0, genome_size: int = 400_000,
+                    seed: int = 11, contigs: list | None = None, edge_cases: bool = True) -> dict:
+    """Write ``genome.fa`` and ``annotation.gtf`` under ``out_dir``.
+
+    Every gene sits in its own slot of a contig (``contigs`` or ``genome_size`` split over three contigs), on a random
+    strand, with 1-12 exons.  Its first transcript carries a planted CDS (ATG, sense codons, a stop that the CDS lines
+    exclude); the other isoforms skip inner exons and carry the same CDS when they keep every exon it touches, or none.
+    ``edge_cases`` (the small test configurations) adds: non-ATG CDS, lowercase and N bases, CRLF line ends,
+    overlapping and book-ended exon lines, shuffled attribute order, Ensembl ``*_biotype`` keys, missing
+    ``gene_name``, start / stop codons split across an exon junction, a uORF with a nested in-frame start, and
+    transcripts that must be skipped (contig absent from the FASTA, past a contig end, exons on both strands).
+    Returns the two paths, the contig table and the planted CDS per transcript id."""
+    import os
+
+    rng = np.random.default_rng(seed)
+    if contigs is None:
+        contigs = [(f"chr{k + 1}", int(genome_size * w)) for k, w in enumerate((0.5, 0.3, 0.2))]
+    acgt = np.frombuffer(b"ACGT", np.uint8)
+    seqs = {name: acgt[rng.integers(0, 4, length, dtype=np.uint8)] for name, length in contigs}
+    clen = np.array([length for _, length in contigs], np.int64)
+    gene_contig = rng.choice(len(contigs), n_genes, p=clen / clen.sum())
+    lines, planted = [], {}
+    crlf = edge_cases
+    slot_of = {}
+    for g in range(n_genes):
+        ci = int(gene_contig[g])
+        slot_of.setdefault(ci, []).append(g)
+    for ci, genes in slot_of.items():
+        name, length = contigs[ci]
+        seq = seqs[name]
+        slot = length // len(genes)
+        for k, g in enumerate(genes):
+            lo = k * slot + 1
+            span = slot - 2
+            if span < 400:
+                continue
+            strand = "+" if rng.random() < 0.5 else "-"
+            n_ex = int(rng.integers(1, 13))
+            ex_len = rng.integers(60, 700, n_ex)
+            intron = rng.integers(60, 3000, n_ex)
+            total = int(ex_len.sum() + intron[:-1].sum())
+            while total > span and n_ex > 1:
+                n_ex -= 1
+                ex_len, intron = ex_len[:n_ex], intron[:n_ex]
+                total = int(ex_len.sum() + intron[:-1].sum())
+            if total > span:
+                ex_len = np.array([span // 2])
+                total = int(ex_len[0])
+            start = lo + int(rng.integers(0, span - total + 1))
+            exons, at = [], start
+            for e in range(n_ex):
+                exons.append((at, at + int(ex_len[e]) - 1))
+                at += int(ex_len[e]) + int(intron[e])
+            # genomic position (0-based) of every transcript nt, in transcript (oriented) order
+            pos = np.concatenate([np.arange(s - 1, e) for s, e in exons])
+            if strand == "-":
+                pos = pos[::-1]
+            n = len(pos)
+            # plant the CDS: [c0, c0 + 3k) is ATG + sense codons, the stop follows and is not part of the CDS
+            k_cod = int(rng.integers(2, max(3, (n - 6) // 3)))
+            c0 = int(rng.integers(0, n - 3 * k_cod - 3 + 1))
+            if edge_cases and g % 7 == 3 and n_ex >= 3:     # start and stop codons split across exon junctions
+                j0 = int(ex_len[0]) if strand == "+" else int(ex_len[-1])
+                j1 = n - (int(ex_len[-1]) if strand == "+" else int(ex_len[0]))
+                for a, b in ((j0 - 1, j1 - 1), (j0 - 1, j1 - 2), (j0 - 2, j1 - 1), (j0 - 2, j1 - 2)):
+                    if (b - a) % 3 == 0 and b - a >= 6:
+                        c0, k_cod = a, (b - a) // 3
+                        break
+            body = bytearray(_sense_codons(rng, k_cod))
+            body[:3] = b"CTG" if edge_cases and g % 5 == 2 else b"ATG"
+            body += _STOPS[int(rng.integers(0, 3))]
+            codes = np.frombuffer(bytes(body), np.uint8)
+            if strand == "-":
+                codes = _COMPLEMENT[codes]
+            seq[pos[c0:c0 + len(codes)]] = codes
+            if edge_cases and g % 6 == 1 and c0 >= 100:     # uORF with a nested in-frame start sharing its stop
+                u = bytearray(b"ATG" + _sense_codons(rng, 4) + b"ATG" + _sense_codons(rng, 18) + b"TAA")
+                ucodes = np.frombuffer(bytes(u), np.uint8)
+                seq[pos[2:2 + len(ucodes)]] = _COMPLEMENT[ucodes] if strand == "-" else ucodes
+            cds_lo, cds_hi = sorted((int(pos[c0]) + 1, int(pos[c0 + 3 * k_cod - 1]) + 1))
+            gid, gname = f"G{seed}_{g:06d}", f"GENE{g}"
+            style = int(rng.integers(0, 3)) if edge_cases else 0
+            n_tx = max(1, int(rng.poisson(tx_per_gene - 1)) + 1)
+            for t in range(n_tx):
+                tid = f"T{seed}_{g:06d}_{t}"
+                keep = [True] * n_ex
+                if t > 0 and n_ex > 2:
+                    keep = [e in (0, n_ex - 1) or rng.random() < 0.6 for e in range(n_ex)]
+                tex = [ex for ex, kp in zip(exons, keep) if kp]
+                coding = all(kp for (s0, e0), kp in zip(exons, keep) if e0 >= cds_lo and s0 <= cds_hi)
+                ttype = "protein_coding" if coding else "processed_transcript"
+                attrs = [("gene_id", gid), ("transcript_id", tid), ("gene_name", gname),
+                         ("gene_type", "protein_coding"), ("transcript_type", ttype)]
+                if style == 1:                                          # Ensembl keys, shuffled order
+                    attrs = [(kk.replace("_type", "_biotype"), v) for kk, v in attrs]
+                    attrs = [attrs[i] for i in rng.permutation(len(attrs))]
+                elif style == 2:                                        # no gene_name
+                    attrs = [a for a in attrs if a[0] != "gene_name"] + [("tag", "basic"), ("tag", "CCDS")]
+                attr = " ".join(f'{kk} "{v}";' for kk, v in attrs)
+                rows = [(s, e, "exon") for s, e in tex]
+                if edge_cases and t == 0 and g % 4 == 0 and tex[0][1] - tex[0][0] > 20:
+                    s, e = tex[0]                                       # one exon as overlapping + book-ended pieces
+                    m = (s + e) // 2
+                    rows[0:1] = [(s, m, "exon"), (m - 5, m + 3, "exon"), (m + 1, e, "exon")]
+                if coding:
+                    cds_iv = [(max(s, cds_lo), min(e, cds_hi)) for s, e in tex if s <= cds_hi and e >= cds_lo]
+                    rows += [(s, e, "CDS") for s, e in cds_iv]
+                    planted[tid] = dict(gene_id=gid, chrom=name, strand=strand, cds=cds_iv)
+                for s, e, feat in rows:
+                    lines.append(f"{name}\tsynth\t{feat}\t{s}\t{e}\t.\t{strand}\t{'.' if feat == 'exon' else '0'}\t{attr}")
+    if edge_cases:
+        name0, len0 = contigs[0]
+        base = f'gene_type "protein_coding"; transcript_type "protein_coding";'
+        lines += [f"chrAbsent\tsynth\texon\t100\t400\t.\t+\t.\tgene_id \"GX1\"; transcript_id \"TX_absent\"; {base}",
+                  f"{name0}\tsynth\texon\t{len0 - 50}\t{len0 + 20}\t.\t+\t.\tgene_id \"GX2\"; transcript_id \"TX_pastend\"; {base}",
+                  f"{name0}\tsynth\texon\t100\t200\t.\t+\t.\tgene_id \"GX3\"; transcript_id \"TX_twostrands\"; {base}",
+                  f"{name0}\tsynth\texon\t300\t400\t.\t-\t.\tgene_id \"GX3\"; transcript_id \"TX_twostrands\"; {base}",
+                  f"{name0}\tsynth\tgene\t100\t400\t.\t+\t.\tgene_id \"GX3\";",
+                  f"{name0}\tsynth\texon\t500\t600\t.\t+\t.\ttranscript_id \"TX_nogene\";"]
+        for name, _ in contigs:                                         # soft-masked stretches and N runs
+            seq = seqs[name]
+            for _ in range(max(1, len(seq) // 20_000)):
+                a = int(rng.integers(0, len(seq) - 200))
+                seq[a:a + int(rng.integers(20, 200))] += 32
+                b = int(rng.integers(0, len(seq) - 50))
+                seq[b:b + int(rng.integers(1, 50))] = ord("N") + (32 if rng.random() < 0.3 else 0)
+    os.makedirs(out_dir, exist_ok=True)
+    eol = "\r\n" if crlf else "\n"
+    gtf = os.path.join(out_dir, "annotation.gtf")
+    with open(gtf, "w", newline="") as fh:
+        fh.write("#!genome-build synthetic" + eol + "##seed " + str(seed) + "\n")
+        for i, line in enumerate(lines):
+            fh.write(line + (eol if i % 2 else "\n"))
+        fh.write("\n")
+    fasta = os.path.join(out_dir, "genome.fa")
+    with open(fasta, "wb") as fh:
+        for name, length in contigs:
+            fh.write(f">{name} synthetic contig{eol}".encode())
+            seq = seqs[name]
+            width = 60 if not crlf else 61
+            full = (length // width) * width
+            if full:
+                block = np.empty((full // width, width + len(eol)), np.uint8)
+                block[:, :width] = seq[:full].reshape(-1, width)
+                block[:, width:] = np.frombuffer(eol.encode(), np.uint8)
+                fh.write(block.tobytes())
+            if full < length:
+                fh.write(seq[full:].tobytes() + eol.encode())
+    return dict(fasta=fasta, gtf=gtf, contigs=list(contigs), planted=planted)
