@@ -33,31 +33,28 @@ def check(rc, ctx):
 p = lambda a: a.ctypes.data_as(vp)
 cases = [("tiny", 1.0, 1.0), ("C1", 0.3, 1.0), ("C5", 0.02, 0.05), ("C2", 0.5, 0.5)]
 for name, scale, cscale in cases:
-    for env in ({}, {"RT_SCORE_PATH": "scan"}) if name in ("tiny", "C5") else ({},):
-        for k in ("RT_SCORE_PATH",): os.environ.pop(k, None)
-        os.environ.update(env)
-        cfg = synth.config(name, scale, cscale); idx = synth.make_index(cfg); d = idx.as_dict()
-        ctx = vp(); check(lib.rt_create(0, C.byref(ctx)), None)
-        lens = np.ascontiguousarray(idx.contig_len, np.int64)
-        check(lib.rt_set_genome(ctx, len(lens), p(lens), 256), ctx)
-        cols = [np.ascontiguousarray(d[k], dt) for k, dt in (("exon_ptr", np.int64), ("exon_start", np.int32), ("exon_end", np.int32), ("orf_contig", np.int32), ("orf_strand", np.uint8))]
-        check(lib.rt_set_index(ctx, idx.n_orf, *[p(c) for c in cols]), ctx)
-        digest(f"{name} {env} set_index ({idx.n_orf} ORFs)")
-        for layout in (1, 0):          # compact, dense
-            check(lib.rt_set_layout(ctx, layout), ctx)
-            digest(f"{name} {env} set_layout {layout}")
-            n = idx.n_orf; elems = lib.rt_coverage_elems(ctx)
-            cov = np.zeros(elems + 64, np.int32)
-            cols_out = dict(score=np.zeros(n), valid=np.zeros(n, np.int32), count=np.zeros(n, np.int64), length=np.zeros(n, np.int32),
-                            min_codon=np.zeros(n, np.int32), status=np.zeros(n, np.uint8))
-            out = Out(p(cols_out["score"]), p(cols_out["valid"]), p(cols_out["count"]), p(cols_out["length"]), p(cols_out["min_codon"]), p(cols_out["status"]), None, None)
-            prm = Params(0.428571428571, 5, 0, 0, 0.0)
-            for lo, hi in ((0, n), (n // 3, n - n // 5), (0, min(n, 1000))):
-                check(lib.rt_score(ctx, p(cov), lo, hi, C.byref(prm), C.byref(out), None), ctx)
-                digest(f"{name} {env} layout {layout} rt_score [{lo}, {hi})")
-            for parts in ("1", "3", "4", "16"):
-                os.environ["RT_SCORE_HOST_PARTS"] = parts
-                check(lib.rt_score_host(ctx, p(cov), 7, n - 3, C.byref(prm), C.byref(out)), ctx)
-                digest(f"{name} {env} layout {layout} rt_score_host parts {parts}")
-            os.environ.pop("RT_SCORE_HOST_PARTS", None)
-        lib.rt_destroy(ctx)
+    cfg = synth.config(name, scale, cscale); idx = synth.make_index(cfg); d = idx.as_dict()
+    ctx = vp(); check(lib.rt_create(0, C.byref(ctx)), None)
+    lens = np.ascontiguousarray(idx.contig_len, np.int64)
+    check(lib.rt_set_genome(ctx, len(lens), p(lens), 256), ctx)
+    cols = [np.ascontiguousarray(d[k], dt) for k, dt in (("exon_ptr", np.int64), ("exon_start", np.int32), ("exon_end", np.int32), ("orf_contig", np.int32), ("orf_strand", np.uint8))]
+    check(lib.rt_set_index(ctx, idx.n_orf, *[p(c) for c in cols]), ctx)
+    digest(f"{name} set_index ({idx.n_orf} ORFs)")
+    for layout in (1, 0):          # compact, dense
+        check(lib.rt_set_layout(ctx, layout), ctx)
+        digest(f"{name} set_layout {layout}")
+        n = idx.n_orf; elems = lib.rt_coverage_elems(ctx)
+        cov = np.zeros(elems + 64, np.int32)
+        cols_out = dict(score=np.zeros(n), valid=np.zeros(n, np.int32), count=np.zeros(n, np.int64), length=np.zeros(n, np.int32),
+                        min_codon=np.zeros(n, np.int32), status=np.zeros(n, np.uint8))
+        out = Out(p(cols_out["score"]), p(cols_out["valid"]), p(cols_out["count"]), p(cols_out["length"]), p(cols_out["min_codon"]), p(cols_out["status"]), None, None)
+        prm = Params(0.428571428571, 5, 0, 0, 0.0)
+        for lo, hi in ((0, n), (n // 3, n - n // 5), (0, min(n, 1000))):
+            check(lib.rt_score(ctx, p(cov), lo, hi, C.byref(prm), C.byref(out), None), ctx)
+            digest(f"{name} layout {layout} rt_score [{lo}, {hi})")
+        for parts in ("1", "3", "4", "16"):
+            os.environ["RT_SCORE_HOST_PARTS"] = parts
+            check(lib.rt_score_host(ctx, p(cov), 7, n - 3, C.byref(prm), C.byref(out)), ctx)
+            digest(f"{name} layout {layout} rt_score_host parts {parts}")
+        os.environ.pop("RT_SCORE_HOST_PARTS", None)
+    lib.rt_destroy(ctx)

@@ -23,7 +23,9 @@ unsigned __cudaPushCallConfiguration(dim3, dim3, size_t, cudaStream_t) { return 
 cudaError_t __cudaPopCallConfiguration(dim3*, dim3*, size_t*, void*) { return cudaSuccess; }
 cudaError_t cudaLaunchKernel(const void*, dim3, dim3, void**, size_t, cudaStream_t) { return cudaSuccess; }
 cudaError_t cudaDeviceSynchronize() { return cudaSuccess; }
+cudaError_t cudaEventCreate(cudaEvent_t* e) { *e = (cudaEvent_t)malloc(8); return cudaSuccess; }
 cudaError_t cudaEventCreateWithFlags(cudaEvent_t* e, unsigned) { *e = (cudaEvent_t)malloc(8); return cudaSuccess; }
+cudaError_t cudaEventElapsedTime(float* ms, cudaEvent_t, cudaEvent_t) { *ms = 0.f; return cudaSuccess; }
 cudaError_t cudaEventDestroy(cudaEvent_t e) { free(e); return cudaSuccess; }
 cudaError_t cudaEventRecord(cudaEvent_t, cudaStream_t) { return cudaSuccess; }
 cudaError_t cudaEventSynchronize(cudaEvent_t) { return cudaSuccess; }

@@ -72,26 +72,15 @@ struct rt_ctx {
     int64_t n_orf = 0;
     uint64_t* d_orf_desc = nullptr;
     int32_t* d_orf_len = nullptr;
-    cudaStream_t aux_stream = nullptr;               // long ORFs run beside the packed kernel
-    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     cudaEvent_t ev_scored = nullptr;                 // rt_score_host: a part's columns are ready for their copy
     uint64_t* d_exon_entries = nullptr;
     std::vector<int64_t> bytes_prefix;  // n_orf + 1: prefix of 4L + 8E + 42
     std::vector<int64_t> nt_prefix;     // n_orf + 1: prefix of L
-    unsigned long long* d_work_counter = nullptr;   // 4 x u64: work counters of the 3 score launches + fallback count
-    int pack_lpo = 8;                                // lanes per ORF of the packed kernel (RT_PACK_LPO)
-    int atom_lpo = 4;                                // lanes per atom in phase A (RT_ATOM_LPO)
-    bool use_ref_kernel = true;                      // phase B with one lane per atom reference (RT_PHASE_B=thread: one thread per ORF)
-    bool use_pass_kernel = true;                     // compact layout: streamed phase A (RT_PHASE_A=atoms selects the per-atom kernel)
-    int pass_warps = 16, pass_stages = 2;            // RT_PASS_WARPS (1..16), RT_PASS_STAGES (1..3)
-    bool use_atoms = true;                           // two-phase scoring (RT_SCORE_PATH=scan selects the scan kernel)
+    unsigned long long* d_work_counter = nullptr;   // 4 x u64: work counters of phase A (0) and the fallback (2), fallback count (3)
 
     // two-phase scoring: atoms (coverage intervals no ORF exon boundary splits) and per-ORF atom refs
     int64_t n_atoms = 0;
     uint64_t* d_atoms = nullptr;                     // (slot offset << 24) | len
-    uint64_t* d_orf_refs_desc = nullptr;             // per ORF: ref begin | n_refs << 40 | reverse << 63
-    uint64_t* d_ref_ent = nullptr;                   // refs in profile order
-    uint32_t* d_ref_atom = nullptr;
     rt::AtomSummary* d_summaries = nullptr;          // per-library scratch, written by phase A
     uint8_t* d_atom_nonzero = nullptr;               // per-library scratch: atom holds at least one read
     // compact layout: the coverage buffer holds the exon union only (atoms back to back, genome order)
@@ -102,25 +91,18 @@ struct rt_ctx {
     DevBuf zone_buf, spill_buf;                      // rt_bin_stream_fresh: zone boundaries, spill list + its counter
     uint2* d_cmap = nullptr;                         // per 32 dense slots: member mask | compact index after the last member
     uint64_t* d_atoms_c = nullptr;                   // the same tables with compact slot offsets
-    uint64_t* d_ref_ent_c = nullptr;
     uint64_t* d_exon_entries_c = nullptr;
     std::vector<uint64_t> h_atoms;                   // host copies used to build per-range atom lists
     std::vector<uint64_t> h_atoms_c;                 // ... with compact slot offsets
-    std::vector<uint64_t> h_orf_refs_desc;
-    std::vector<uint32_t> h_ref_atom;
-    std::vector<uint64_t> h_ref_ent;
+    std::vector<uint64_t> h_orf_refs_desc;           // per ORF: ref begin | n_refs << 40 | reverse << 63
+    std::vector<uint32_t> h_ref_atom;                // atom id of every ref (0xffffffff: reads as zeros)
+    std::vector<uint64_t> h_ref_ent;                 // refs in profile order
 
-    // score plan: ORFs of a range sorted by length (longest first), split by kernel
+    // score plan: the work lists of the three scoring launches for one ORF range
     struct ScorePlan {
         int64_t lo = -1, hi = -1;
-        int32_t* d_list = nullptr;      // [n_long | n_short] absolute ORF ids
-        int32_t* d_fallback = nullptr;  // capacity n_short
-        int64_t n_long = 0, n_short = 0;
+        int32_t* d_fallback = nullptr;  // ORFs redone by score_orfs_kernel; capacity hi - lo
         int32_t* d_atom_list = nullptr; // atoms the range touches, similar lengths adjacent
-        rt::RefSegment* d_segs = nullptr;      // segments of the ORFs with more than kSegRefs refs
-        rt::ComposeAcc* d_partials = nullptr;  // one per segment
-        unsigned* d_seg_done = nullptr;        // one per long ORF
-        int64_t n_segs = 0;
         int64_t n_atom_list = 0;
         rt::PassDesc* d_passes = nullptr;      // compact layout: runs of adjacent atoms for atom_pass_kernel
         int64_t n_passes = 0;
@@ -309,7 +291,7 @@ int build_atoms(rt_ctx* ctx, const std::vector<uint64_t>& desc, const std::vecto
     // compact layout: atom i starts at the sum of the lengths of the atoms before it
     std::vector<uint64_t>& atoms_c = ctx->h_atoms_c;
     atoms_c.assign(ctx->h_atoms.size(), 0);
-    std::vector<uint64_t> ref_ent_c(ctx->h_ref_ent.size()), entries_c(entries.size());
+    std::vector<uint64_t> entries_c(entries.size());
     uint64_t cat = 0;
     for (size_t i = 0; i < atoms_c.size(); ++i) {
         const uint64_t len = ctx->h_atoms[i] & rt::kLenMask;
@@ -324,8 +306,6 @@ int build_atoms(rt_ctx* ctx, const std::vector<uint64_t>& desc, const std::vecto
             ctx->compact_plus_end = (unsigned)(atoms_c[i] >> rt::kLenBits);
             break;
         }
-    for (size_t k = 0; k < ref_ent_c.size(); ++k)
-        ref_ent_c[k] = ctx->h_ref_atom[k] == 0xffffffffu ? ctx->h_ref_ent[k] : atoms_c[ctx->h_ref_atom[k]];
     for (size_t k = 0; k < entries.size(); ++k) {
         const uint64_t off = entries[k] >> rt::kLenBits, len = entries[k] & rt::kLenMask;
         entries_c[k] = off == kZero ? entries[k] : ((atoms_c[atom_begin[ilo[k]]] >> rt::kLenBits) << rt::kLenBits) | len;
@@ -337,15 +317,20 @@ int build_atoms(rt_ctx* ctx, const std::vector<uint64_t>& desc, const std::vecto
         return e;
     };
     RT_CUDA(ctx, upload(&ctx->d_atoms, ctx->h_atoms));
-    RT_CUDA(ctx, upload(&ctx->d_orf_refs_desc, ctx->h_orf_refs_desc));
-    RT_CUDA(ctx, upload(&ctx->d_ref_ent, ctx->h_ref_ent));
-    RT_CUDA(ctx, upload(&ctx->d_ref_atom, ctx->h_ref_atom));
     RT_CUDA(ctx, upload(&ctx->d_atoms_c, atoms_c));
-    RT_CUDA(ctx, upload(&ctx->d_ref_ent_c, ref_ent_c));
     RT_CUDA(ctx, upload(&ctx->d_exon_entries_c, entries_c));
     RT_CUDA(ctx, cudaMalloc(&ctx->d_summaries, sizeof(rt::AtomSummary) * std::max<size_t>(1, ctx->h_atoms.size())));
     RT_CUDA(ctx, cudaMalloc(&ctx->d_atom_nonzero, std::max<size_t>(1, ctx->h_atoms.size())));
-    return RT_OK;   // h_ref_ent stays: get_plan needs the ref lengths to cut long ORFs into segments
+    return RT_OK;   // the host copies stay: build_plan_host makes the atom lists and the families from them
+}
+
+void free_plan(rt_ctx::ScorePlan& p) {
+    cudaFree(p.d_fallback);
+    cudaFree(p.d_atom_list);
+    cudaFree(p.d_passes);
+    cudaFree(p.d_refs);
+    cudaFree(p.d_ref_warps);
+    cudaFree(p.d_long_acc);
 }
 
 constexpr size_t kReadBytes = 4 + 4 + 4 + 2 + 2 + 1 + 1;
@@ -405,19 +390,6 @@ int rt_create(int device, rt_ctx** out) {
         delete ctx;
         return fail(nullptr, RT_ECUDA, "rt_create: %s", cudaGetErrorString(cudaGetLastError()));
     }
-    if (const char* e = getenv("RT_SCORE_PATH")) ctx->use_atoms = strcmp(e, "scan") != 0;
-    if (const char* e = getenv("RT_ATOM_LPO")) {
-        const int v = atoi(e);
-        if (v == 2 || v == 4 || v == 8) ctx->atom_lpo = v;
-    }
-    if (const char* e = getenv("RT_PHASE_A")) ctx->use_pass_kernel = strcmp(e, "atoms") != 0;
-    if (const char* e = getenv("RT_PHASE_B")) ctx->use_ref_kernel = strcmp(e, "thread") != 0;
-    if (const char* e = getenv("RT_PASS_WARPS")) ctx->pass_warps = std::min(16, std::max(1, atoi(e)));
-    if (const char* e = getenv("RT_PASS_STAGES")) ctx->pass_stages = std::min(3, std::max(1, atoi(e)));
-    if (const char* e = getenv("RT_PACK_LPO")) {
-        const int v = atoi(e);
-        if (v == 8 || v == 16 || v == 32) ctx->pack_lpo = v;
-    }
     *out = ctx;
     return RT_OK;
 }
@@ -433,33 +405,15 @@ void rt_destroy(rt_ctx* ctx) {
     cudaFree(ctx->d_orf_len);
     cudaFree(ctx->d_exon_entries);
     cudaFree(ctx->d_atoms);
-    cudaFree(ctx->d_orf_refs_desc);
-    cudaFree(ctx->d_ref_ent);
-    cudaFree(ctx->d_ref_atom);
     cudaFree(ctx->d_summaries);
     cudaFree(ctx->d_atom_nonzero);
     cudaFree(ctx->d_cmap);
     cudaFree(ctx->d_cbits);
     cudaFree(ctx->d_atoms_c);
-    cudaFree(ctx->d_ref_ent_c);
     cudaFree(ctx->d_exon_entries_c);
     cudaFree(ctx->d_work_counter);
-    if (ctx->aux_stream) cudaStreamDestroy(ctx->aux_stream);
-    if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
-    if (ctx->ev_join) cudaEventDestroy(ctx->ev_join);
     if (ctx->ev_scored) cudaEventDestroy(ctx->ev_scored);
-    for (auto& p : ctx->plans) {
-        cudaFree(p.d_list);
-        cudaFree(p.d_fallback);
-        cudaFree(p.d_atom_list);
-        cudaFree(p.d_segs);
-        cudaFree(p.d_partials);
-        cudaFree(p.d_seg_done);
-        cudaFree(p.d_passes);
-        cudaFree(p.d_refs);
-        cudaFree(p.d_ref_warps);
-        cudaFree(p.d_long_acc);
-    }
+    for (auto& p : ctx->plans) free_plan(p);
     for (int s = 0; s < 16; ++s) {
         if (ctx->host_stage[s].rec) cudaFreeHost(ctx->host_stage[s].rec);
         if (ctx->host_stage[s].hdr) cudaFreeHost(ctx->host_stage[s].hdr);
@@ -1127,38 +1081,22 @@ int rt_set_index(rt_ctx* ctx, int64_t n_orf, const int64_t* h_exon_ptr, const in
     ctx->d_orf_desc = ctx->d_exon_entries = nullptr;
     ctx->d_orf_len = nullptr;
     ctx->n_orf = 0;
-    for (auto& p : ctx->plans) {
-        cudaFree(p.d_list);
-        cudaFree(p.d_fallback);
-        cudaFree(p.d_atom_list);
-        cudaFree(p.d_segs);
-        cudaFree(p.d_partials);
-        cudaFree(p.d_seg_done);
-        cudaFree(p.d_passes);
-        cudaFree(p.d_refs);
-        cudaFree(p.d_ref_warps);
-        cudaFree(p.d_long_acc);
-    }
+    for (auto& p : ctx->plans) free_plan(p);
     ctx->plans.clear();
     cudaFree(ctx->d_atoms);
-    cudaFree(ctx->d_orf_refs_desc);
-    cudaFree(ctx->d_ref_ent);
-    cudaFree(ctx->d_ref_atom);
     cudaFree(ctx->d_summaries);
     cudaFree(ctx->d_atom_nonzero);
     ctx->d_atom_nonzero = nullptr;
     cudaFree(ctx->d_cmap);
     cudaFree(ctx->d_cbits);
     cudaFree(ctx->d_atoms_c);
-    cudaFree(ctx->d_ref_ent_c);
     cudaFree(ctx->d_exon_entries_c);
     ctx->d_cmap = nullptr;
     ctx->d_cbits = nullptr;
-    ctx->d_atoms_c = ctx->d_ref_ent_c = ctx->d_exon_entries_c = nullptr;
+    ctx->d_atoms_c = ctx->d_exon_entries_c = nullptr;
     ctx->layout = RT_LAYOUT_DENSE;
     ctx->compact_elems = 0;
-    ctx->d_atoms = ctx->d_orf_refs_desc = ctx->d_ref_ent = nullptr;
-    ctx->d_ref_atom = nullptr;
+    ctx->d_atoms = nullptr;
     ctx->d_summaries = nullptr;
     ctx->n_atoms = 0;
     {
@@ -1219,16 +1157,10 @@ int rt_shard_bounds(const rt_ctx* ctx, int n_shards, int64_t* h_bounds) {
 
 namespace {
 
-// Work lists of the ORF range [lo, hi), cached per range: the ORF order for the scoring kernel and the
-// atoms the range touches for phase A.
 // What get_plan works out on the host for the ORFs [lo, hi) before anything touches the device: pure functions of the
 // index arrays of the ctx, so the part plans of rt_score_host can be built side by side.
 struct PlanHost {
     int64_t lo = 0, hi = 0;
-    std::vector<int32_t> ids;                 // scoring order (two-phase path: windows sorted by reference count)
-    std::vector<rt::RefSegment> segs;         // segments of the ORFs with more than kSegRefs references
-    int n_long_orfs = 0;                      // ORFs cut into segments
-    int64_t n_long = 0;                       // scan path: ORFs above kPackMaxNt
     std::vector<rt::PassDesc> passes;         // phase A
     std::vector<int32_t> alist;               // atoms of the range, similar lengths adjacent
     std::vector<rt::RefRec> refs;             // phase B slots
@@ -1241,70 +1173,6 @@ void build_plan_host(const rt_ctx* ctx, int64_t lo, int64_t hi, PlanHost& ph) {
     const auto t_plan = std::chrono::steady_clock::now();
     ph.lo = lo;
     ph.hi = hi;
-    const int64_t* np = ctx->nt_prefix.data();
-    auto len_of = [np](int32_t x) { return np[x + 1] - np[x]; };
-    std::vector<int32_t>& ids = ph.ids;
-    ids.reserve((size_t)n);
-    std::vector<rt::RefSegment>& segs = ph.segs;
-    int& n_long_orfs = ph.n_long_orfs;
-    int64_t& n_long = ph.n_long;
-    if (ctx->use_atoms) {
-        // two-phase path: one thread per ORF walks its atom refs, so the ORFs sharing a warp should hold
-        // similar numbers of refs; sort by that inside windows of the index (neighbours share atoms)
-        auto refs_of = [&](int32_t x) { return (ctx->h_orf_refs_desc[x] >> 40) & (uint64_t)rt::kMaxEntriesPerOrf; };
-        // ORFs with more than kSegRefs refs (giant transcripts) would be long serial chains for one thread:
-        // they are cut into segments of about kSegRefs refs, each scored by its own thread (cuts only after a
-        // ref of >= 2 values, so that a segment can start from that ref's last two values)
-        constexpr int64_t kPlanWindow = 2048;
-        for (int64_t w0 = lo; w0 < hi; w0 += kPlanWindow) {
-            const size_t begin = ids.size();
-            for (int64_t o = w0; o < std::min(hi, w0 + kPlanWindow); ++o) {
-                const uint64_t n_refs = refs_of((int32_t)o);
-                if (n_refs <= (uint64_t)rt::kSegRefs) {
-                    ids.push_back((int32_t)o);
-                    continue;
-                }
-                const uint64_t rb = ctx->h_orf_refs_desc[o] & rt::kBeginMask;
-                const size_t first_slot = segs.size();
-                int P = 0, seg_P0 = 0;
-                uint64_t seg_begin = 0;
-                for (uint64_t k = 0; k < n_refs; ++k) {
-                    const int len = (int)(ctx->h_ref_ent[rb + k] & rt::kLenMask);
-                    const bool cut_here = k > seg_begin && k - seg_begin >= (uint64_t)rt::kSegRefs &&
-                                          (int)(ctx->h_ref_ent[rb + k - 1] & rt::kLenMask) >= 2;
-                    if (cut_here) {
-                        segs.push_back({(int)o, (unsigned)(rb + seg_begin), (int)(k - seg_begin), seg_P0, (int)segs.size(), 0, 0, n_long_orfs});
-                        seg_begin = k;
-                        seg_P0 = P;
-                    }
-                    P += len;
-                }
-                segs.push_back({(int)o, (unsigned)(rb + seg_begin), (int)(n_refs - seg_begin), seg_P0, (int)segs.size(), 0, 0, n_long_orfs});
-                for (size_t q = first_slot; q < segs.size(); ++q) {
-                    segs[q].first_slot = (int)first_slot;
-                    segs[q].n_seg = (int)(segs.size() - first_slot);
-                }
-                ++n_long_orfs;
-            }
-            std::stable_sort(ids.begin() + begin, ids.end(), [&](int32_t x, int32_t y) { return refs_of(x) > refs_of(y); });
-        }
-    } else {
-        // scan path.  Long ORFs: all of them, longest first (they start first and run beside the packed kernel)
-        for (int64_t o = lo; o < hi; ++o)
-            if (len_of((int32_t)o) > rt::kPackMaxNt) ids.push_back((int32_t)o);
-        std::stable_sort(ids.begin(), ids.end(), [&](int32_t x, int32_t y) { return len_of(x) > len_of(y); });
-        n_long = (int64_t)ids.size();
-        // the rest: sorted by length inside windows of kPlanWindow consecutive index rows, so that the
-        // ORFs sharing a warp have similar lengths while neighbours in the index (nested ORFs, isoforms:
-        // same exons) are still scored close in time and meet in L2
-        constexpr int64_t kPlanWindow = 2048;
-        for (int64_t w0 = lo; w0 < hi; w0 += kPlanWindow) {
-            const size_t begin = ids.size();
-            for (int64_t o = w0; o < std::min(hi, w0 + kPlanWindow); ++o)
-                if (len_of((int32_t)o) <= rt::kPackMaxNt) ids.push_back((int32_t)o);
-            std::stable_sort(ids.begin() + begin, ids.end(), [&](int32_t x, int32_t y) { return len_of(x) > len_of(y); });
-        }
-    }
     const bool plan_timing = getenv("RT_HOST_TIMING") != nullptr;
     auto t_mark = std::chrono::steady_clock::now();
     auto lap = [&](const char* what) {
@@ -1313,7 +1181,6 @@ void build_plan_host(const rt_ctx* ctx, int64_t lo, int64_t hi, PlanHost& ph) {
         fprintf(stderr, "  get_plan: %-28s %.1f ms\n", what, std::chrono::duration<double, std::milli>(now - t_mark).count());
         t_mark = now;
     };
-    lap("ORF order");
     {   // atoms the ORFs of the range refer to; sorted by length inside windows so that the four atoms of
         // a warp are balanced while genomic neighbours stay close in time
         std::vector<uint8_t> used((size_t)ctx->n_atoms, 0);
@@ -1355,7 +1222,7 @@ void build_plan_host(const rt_ctx* ctx, int64_t lo, int64_t hi, PlanHost& ph) {
         }
     }
     lap("atom list + passes");
-    if (ctx->use_atoms) {
+    {
         // Phase B work list.  FAMILIES: candidate ORFs of one transcript that share their stop are suffixes of the
         // longest one -- same atoms from some reference on (the index is cut into atoms at every ORF start).  The
         // longest ORF of a family (the parent) lays its references out, one per slot; an ORF whose reference list is a
@@ -1481,39 +1348,14 @@ void build_plan_host(const rt_ctx* ctx, int64_t lo, int64_t hi, PlanHost& ph) {
 // The device side of a plan: the host arrays of `ph` uploaded, the plan entered into the (bounded) cache of the ctx.
 int upload_plan(rt_ctx* ctx, PlanHost& ph, rt_ctx::ScorePlan** out) {
     const int64_t lo = ph.lo, hi = ph.hi, n = hi - lo;
-    const std::vector<int32_t>& ids = ph.ids;
-    const std::vector<rt::RefSegment>& segs = ph.segs;
-    const int n_long_orfs = ph.n_long_orfs;
     if (ctx->plans.size() >= 24) {   // bounded cache (rt_score_host keeps four part plans per range it is asked for)
-        cudaFree(ctx->plans.front().d_list);
-        cudaFree(ctx->plans.front().d_fallback);
-        cudaFree(ctx->plans.front().d_atom_list);
-        cudaFree(ctx->plans.front().d_segs);
-        cudaFree(ctx->plans.front().d_partials);
-        cudaFree(ctx->plans.front().d_seg_done);
-        cudaFree(ctx->plans.front().d_passes);
-        cudaFree(ctx->plans.front().d_refs);
-        cudaFree(ctx->plans.front().d_ref_warps);
-        cudaFree(ctx->plans.front().d_long_acc);
+        free_plan(ctx->plans.front());
         ctx->plans.erase(ctx->plans.begin());
     }
     rt_ctx::ScorePlan p;
     p.lo = lo;
     p.hi = hi;
-    p.n_long = ph.n_long;
-    p.n_short = (int64_t)ids.size() - ph.n_long;
-    p.n_segs = (int64_t)segs.size();
-    if (!segs.empty()) {
-        if (ctx->h_ref_ent.size() >= 0xffffffffull) return fail(ctx, RT_EINVAL, "rt_score: too many atom references for 32-bit segment offsets");
-        RT_CUDA(ctx, cudaMalloc(&p.d_segs, sizeof(rt::RefSegment) * segs.size()));
-        RT_CUDA(ctx, cudaMemcpy(p.d_segs, segs.data(), sizeof(rt::RefSegment) * segs.size(), cudaMemcpyHostToDevice));
-        RT_CUDA(ctx, cudaMalloc(&p.d_partials, sizeof(rt::ComposeAcc) * segs.size()));
-        RT_CUDA(ctx, cudaMalloc(&p.d_seg_done, sizeof(unsigned) * (size_t)n_long_orfs));
-        RT_CUDA(ctx, cudaMemset(p.d_seg_done, 0, sizeof(unsigned) * (size_t)n_long_orfs));
-    }
-    RT_CUDA(ctx, cudaMalloc(&p.d_list, sizeof(int32_t) * std::max<int64_t>(1, n)));
     RT_CUDA(ctx, cudaMalloc(&p.d_fallback, sizeof(int32_t) * std::max<int64_t>(1, n)));
-    if (!ids.empty()) RT_CUDA(ctx, cudaMemcpy(p.d_list, ids.data(), sizeof(int32_t) * ids.size(), cudaMemcpyHostToDevice));
     p.n_passes = (int64_t)ph.passes.size();
     RT_CUDA(ctx, cudaMalloc(&p.d_passes, sizeof(rt::PassDesc) * std::max<size_t>(1, ph.passes.size())));
     if (!ph.passes.empty())
@@ -1522,23 +1364,20 @@ int upload_plan(rt_ctx* ctx, PlanHost& ph, rt_ctx::ScorePlan** out) {
     RT_CUDA(ctx, cudaMalloc(&p.d_atom_list, sizeof(int32_t) * std::max<size_t>(1, ph.alist.size())));
     if (!ph.alist.empty())
         RT_CUDA(ctx, cudaMemcpy(p.d_atom_list, ph.alist.data(), sizeof(int32_t) * ph.alist.size(), cudaMemcpyHostToDevice));
-    if (ctx->use_atoms) {
-        const std::vector<rt::RefRec>& refs = ph.refs;
-        const std::vector<rt::RefWarp>& warps = ph.warps;
-        const int n_long = ph.n_long_b;
-        p.n_ref_warps = (int64_t)warps.size();
-        RT_CUDA(ctx, cudaMalloc(&p.d_refs, sizeof(rt::RefRec) * std::max<size_t>(1, refs.size())));
-        RT_CUDA(ctx, cudaMalloc(&p.d_ref_warps, sizeof(rt::RefWarp) * std::max<size_t>(1, warps.size())));
-        if (!refs.empty()) {
-            RT_CUDA(ctx, cudaMemcpy(p.d_refs, refs.data(), sizeof(rt::RefRec) * refs.size(), cudaMemcpyHostToDevice));
-            RT_CUDA(ctx, cudaMemcpy(p.d_ref_warps, warps.data(), sizeof(rt::RefWarp) * warps.size(), cudaMemcpyHostToDevice));
-        }
-        std::vector<rt::LongAcc> acc((size_t)std::max(1, n_long));
-        memset(acc.data(), 0, sizeof(rt::LongAcc) * acc.size());
-        for (auto& a : acc) a.mn = 0xffffffffu;
-        RT_CUDA(ctx, cudaMalloc(&p.d_long_acc, sizeof(rt::LongAcc) * acc.size()));
-        RT_CUDA(ctx, cudaMemcpy(p.d_long_acc, acc.data(), sizeof(rt::LongAcc) * acc.size(), cudaMemcpyHostToDevice));
+    const std::vector<rt::RefRec>& refs = ph.refs;
+    const std::vector<rt::RefWarp>& warps = ph.warps;
+    p.n_ref_warps = (int64_t)warps.size();
+    RT_CUDA(ctx, cudaMalloc(&p.d_refs, sizeof(rt::RefRec) * std::max<size_t>(1, refs.size())));
+    RT_CUDA(ctx, cudaMalloc(&p.d_ref_warps, sizeof(rt::RefWarp) * std::max<size_t>(1, warps.size())));
+    if (!refs.empty()) {
+        RT_CUDA(ctx, cudaMemcpy(p.d_refs, refs.data(), sizeof(rt::RefRec) * refs.size(), cudaMemcpyHostToDevice));
+        RT_CUDA(ctx, cudaMemcpy(p.d_ref_warps, warps.data(), sizeof(rt::RefWarp) * warps.size(), cudaMemcpyHostToDevice));
     }
+    std::vector<rt::LongAcc> acc((size_t)std::max(1, ph.n_long_b));
+    memset(acc.data(), 0, sizeof(rt::LongAcc) * acc.size());
+    for (auto& a : acc) a.mn = 0xffffffffu;
+    RT_CUDA(ctx, cudaMalloc(&p.d_long_acc, sizeof(rt::LongAcc) * acc.size()));
+    RT_CUDA(ctx, cudaMemcpy(p.d_long_acc, acc.data(), sizeof(rt::LongAcc) * acc.size(), cudaMemcpyHostToDevice));
     ctx->plans.push_back(p);
     *out = &ctx->plans.back();
     return RT_OK;
@@ -1621,145 +1460,72 @@ int rt_score(rt_ctx* ctx, const int32_t* d_cov, int64_t orf_lo, int64_t orf_hi, 
     a.exon_entries = compact ? ctx->d_exon_entries_c : ctx->d_exon_entries;
     a.orf_len = ctx->d_orf_len;
     a.orf_lo = orf_lo;
-    a.fallback = plan->d_fallback;
     a.n_fallback = reinterpret_cast<unsigned*>(ctx->d_work_counter + 3);
     a.prm = *params;
     a.out = *d_out;
     const int threads = rt::kScoreWarps * 32;
-    if (ctx->use_atoms) {
-        // phase A: every atom the range touches is scanned once
-        if (plan->n_atom_list > 0) {
+    // the per-frame minima only matter for --min_reads_per_codon > 0 or when the caller asks for min_codon
+    const bool want_min = d_out->min_codon != nullptr || params->min_reads_per_codon > 0.0;
+    // phase A: every atom the range touches is scanned once
+    if (plan->n_atom_list > 0) {
+        if (compact) {
+            // streamed phase A: the compact buffer is read once, front to back, through TMA into shared memory
+            rt::PassArgs pa;
+            pa.cov = d_cov;
+            pa.atoms = ctx->d_atoms_c;
+            pa.passes = plan->d_passes;
+            pa.n_passes = (unsigned)plan->n_passes;
+            pa.out = ctx->d_summaries;
+            pa.nonzero = ctx->d_atom_nonzero;
+            const size_t smem = rt::kUvEntries * sizeof(double2) + (size_t)rt::kPassWarps * rt::kPassStages * rt::kPassStageBytes;
+            const auto kern = want_min ? rt::atom_pass_kernel<true> : rt::atom_pass_kernel<false>;
+            RT_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            const int64_t want = (plan->n_passes + rt::kPassWarps - 1) / rt::kPassWarps;
+            const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(want, ctx->n_sm));
+            kern<<<grid, rt::kPassWarps * 32, smem, st>>>(pa);
+        } else {
             rt::AtomArgs aa;
             aa.cov = d_cov;
-            aa.atoms = compact ? ctx->d_atoms_c : ctx->d_atoms;
+            aa.atoms = ctx->d_atoms;
             aa.list = plan->d_atom_list;
             aa.n_list = plan->n_atom_list;
             aa.work_counter = ctx->d_work_counter + 0;
             aa.out = ctx->d_summaries;
             aa.nonzero = ctx->d_atom_nonzero;
-            // the per-frame minima only matter for --min_reads_per_codon > 0 or when the caller asks for min_codon
-            const bool want_min = d_out->min_codon != nullptr || params->min_reads_per_codon > 0.0;
-            if (compact && ctx->use_pass_kernel) {
-                // streamed phase A: the compact buffer is read once, front to back, through TMA into shared memory
-                rt::PassArgs pa;
-                pa.cov = d_cov;
-                pa.atoms = ctx->d_atoms_c;
-                pa.passes = plan->d_passes;
-                pa.n_passes = (unsigned)plan->n_passes;
-                pa.out = ctx->d_summaries;
-                pa.nonzero = ctx->d_atom_nonzero;
-                const int warps = ctx->pass_warps, stages = ctx->pass_stages;
-                const size_t smem = rt::kUvEntries * sizeof(double2) + (size_t)warps * stages * rt::kPassStageBytes;
-                auto go = [&](auto kern) -> cudaError_t {
-                    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-                    if (e != cudaSuccess) return e;
-                    const int64_t want = (plan->n_passes + warps - 1) / warps;
-                    const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(want, ctx->n_sm));
-                    kern<<<grid, warps * 32, smem, st>>>(pa);
-                    return cudaSuccess;
-                };
-                cudaError_t e;
-                // 16 warps x 2 stages measured best on C2 (profiles/README.md): more warps need the 64-register build, which
-                // spills, and a third stage buys nothing -- the kernel is bound by the shared-memory pipe, not by the copies
-                if (stages == 1) e = want_min ? go(rt::atom_pass_kernel<1, true>) : go(rt::atom_pass_kernel<1, false>);
-                else if (stages == 2) e = want_min ? go(rt::atom_pass_kernel<2, true>) : go(rt::atom_pass_kernel<2, false>);
-                else e = want_min ? go(rt::atom_pass_kernel<3, true>) : go(rt::atom_pass_kernel<3, false>);
-                RT_CUDA(ctx, e);
-            } else {
-            auto launch = [&](auto kmin, auto knomin, int lpo) {
-                const int g = 32 / lpo;
-                const unsigned grid = persistent_grid(ctx, kmin, (plan->n_atom_list + g - 1) / g);
-                if (want_min) kmin<<<grid, threads, 0, st>>>(aa);
-                else knomin<<<grid, threads, 0, st>>>(aa);
-            };
-            if (ctx->atom_lpo == 2) launch(rt::atom_summary_kernel<2, true>, rt::atom_summary_kernel<2, false>, 2);
-            else if (ctx->atom_lpo == 4) launch(rt::atom_summary_kernel<4, true>, rt::atom_summary_kernel<4, false>, 4);
-            else launch(rt::atom_summary_kernel<8, true>, rt::atom_summary_kernel<8, false>, 8);
-            }
-            ctx->launches++;
+            const auto kern = want_min ? rt::atom_summary_kernel<true> : rt::atom_summary_kernel<false>;
+            const int g = 32 / rt::kAtomLPO;
+            kern<<<persistent_grid(ctx, kern, (plan->n_atom_list + g - 1) / g), threads, 0, st>>>(aa);
         }
-        // phase B: one thread per ORF composes its atoms
-        rt::ComposeArgs ca;
-        ca.cov = d_cov;
-        ca.orf_refs_desc = ctx->d_orf_refs_desc;
-        ca.ref_ent = compact ? ctx->d_ref_ent_c : ctx->d_ref_ent;
-        ca.ref_atom = ctx->d_ref_atom;
-        ca.summaries = ctx->d_summaries;
-        ca.atom_nonzero = ctx->d_atom_nonzero;
-        ca.want_min = (d_out->min_codon != nullptr || params->min_reads_per_codon > 0.0) ? 1 : 0;
-        ca.orf_len = ctx->d_orf_len;
-        ca.orf_lo = orf_lo;
-        ca.list = plan->d_list;
-        ca.n_list = plan->n_long + plan->n_short;
-        ca.fallback = plan->d_fallback;
-        ca.n_fallback = a.n_fallback;
-        ca.prm = *params;
-        ca.out = *d_out;
-        ca.segs = plan->d_segs;
-        ca.n_segs = plan->n_segs;
-        ca.partials = plan->d_partials;
-        ca.seg_done = plan->d_seg_done;
-        if (ctx->use_ref_kernel) {
-            rt::RefComposeArgs ra;
-            ra.refs = plan->d_refs;
-            ra.warps = plan->d_ref_warps;
-            ra.n_warps = plan->n_ref_warps;
-            ra.summaries = ctx->d_summaries;
-            ra.atom_nonzero = ctx->d_atom_nonzero;
-            ra.uv_table = ctx->d_uv_table;
-            ra.want_min = ca.want_min;
-            ra.orf_len = ctx->d_orf_len;
-            ra.orf_lo = orf_lo;
-            ra.fallback = plan->d_fallback;
-            ra.n_fallback = a.n_fallback;
-            ra.long_acc = plan->d_long_acc;
-            ra.prm = *params;
-            ra.out = *d_out;
-            if (ra.n_warps > 0) {
-                if (ra.want_min) rt::compose_refs_kernel<true><<<(unsigned)((ra.n_warps + 7) / 8), 256, 0, st>>>(ra);
-                else rt::compose_refs_kernel<false><<<(unsigned)((ra.n_warps + 7) / 8), 256, 0, st>>>(ra);
-            }
-        } else {
-            rt::score_from_atoms_kernel<<<(unsigned)((ca.n_segs + ca.n_list + 255) / 256), 256, 0, st>>>(ca);
-        }
-        ctx->launches++;
-        // ORFs holding counts >= 2^20: redone by the generic kernel (normally none)
-        a.list = plan->d_fallback;
-        a.n_list = 0;
-        a.n_long = 0;
-        a.n_list_dev = a.n_fallback;
-        a.work_counter = ctx->d_work_counter + 2;
-        rt::score_orfs_kernel<<<(unsigned)ctx->n_sm, threads, 0, st>>>(a);
-        ctx->launches++;
-    } else {
-    // 1. fused gather+score: long ORFs first (one warp each), then packs of short ORFs
-    {
-        a.list = plan->d_list;
-        a.n_list = plan->n_long + plan->n_short;
-        a.n_long = plan->n_long;
-        a.n_list_dev = nullptr;
-        a.work_counter = ctx->d_work_counter + 1;
-        if (ctx->pack_lpo == 8) {
-            const int64_t work = plan->n_long + (plan->n_short + 3) / 4;
-            rt::score_orfs_packed_kernel<8><<<persistent_grid(ctx, rt::score_orfs_packed_kernel<8>, work), threads, 0, st>>>(a);
-        } else if (ctx->pack_lpo == 16) {
-            const int64_t work = plan->n_long + (plan->n_short + 1) / 2;
-            rt::score_orfs_packed_kernel<16><<<persistent_grid(ctx, rt::score_orfs_packed_kernel<16>, work), threads, 0, st>>>(a);
-        } else {
-            const int64_t work = plan->n_long + plan->n_short;
-            rt::score_orfs_packed_kernel<32><<<persistent_grid(ctx, rt::score_orfs_packed_kernel<32>, work), threads, 0, st>>>(a);
-        }
-        ctx->launches++;
-        // 2. ORFs the fused kernel handed over (counts >= 2^20): normally none
-        a.list = plan->d_fallback;
-        a.n_list = 0;
-        a.n_long = 0;
-        a.n_list_dev = a.n_fallback;
-        a.work_counter = ctx->d_work_counter + 2;
-        rt::score_orfs_kernel<<<(unsigned)ctx->n_sm, threads, 0, st>>>(a);
         ctx->launches++;
     }
+    // phase B: the ORFs of every family from the summaries of their atoms
+    rt::RefComposeArgs ra;
+    ra.refs = plan->d_refs;
+    ra.warps = plan->d_ref_warps;
+    ra.n_warps = plan->n_ref_warps;
+    ra.summaries = ctx->d_summaries;
+    ra.atom_nonzero = ctx->d_atom_nonzero;
+    ra.uv_table = ctx->d_uv_table;
+    ra.want_min = want_min ? 1 : 0;
+    ra.orf_len = ctx->d_orf_len;
+    ra.orf_lo = orf_lo;
+    ra.fallback = plan->d_fallback;
+    ra.n_fallback = a.n_fallback;
+    ra.long_acc = plan->d_long_acc;
+    ra.prm = *params;
+    ra.out = *d_out;
+    if (ra.n_warps > 0) {
+        if (want_min) rt::compose_refs_kernel<true><<<(unsigned)((ra.n_warps + 7) / 8), 256, 0, st>>>(ra);
+        else rt::compose_refs_kernel<false><<<(unsigned)((ra.n_warps + 7) / 8), 256, 0, st>>>(ra);
     }
+    ctx->launches++;
+    // ORFs holding counts >= 2^20: redone by the generic kernel (normally none)
+    a.list = plan->d_fallback;
+    a.n_list = 0;
+    a.n_list_dev = a.n_fallback;
+    a.work_counter = ctx->d_work_counter + 2;
+    rt::score_orfs_kernel<<<(unsigned)ctx->n_sm, threads, 0, st>>>(a);
+    ctx->launches++;
     RT_CUDA(ctx, cudaGetLastError());
     return RT_OK;
 }

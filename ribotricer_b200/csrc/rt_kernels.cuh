@@ -4,11 +4,11 @@
 //                             library (persistent, per-warp cp.async.bulk rings; <Zoned>: every block writes its zone
 //                             of the compact buffer before it adds into it), with zone_bounds / zone_carry / zone_spill
 //      bin_psites_kernel      the same loop on the decoder's columns (any read order, dense planes with the sparse clear)
-//   K2+K3 atom_pass_kernel    detect_orfs.py:134-203 + statistics.py:48-115 per atom of the exon union, streamed by
-//                             cp.async.bulk (compact layout); atom_summary_kernel for the dense planes
-//      compose_refs_kernel    per-ORF columns from the atom summaries (families of nested ORFs, suffix scan),
-//                             detect_orfs.py:274-299 + common.py:164-180; score_from_atoms_kernel (A/B)
-//      score_orfs_kernel      the whole per-ORF loop in one kernel: fallback for counts >= 2^20, A/B (RT_SCORE_PATH=scan)
+//   K2+K3 atom_pass_kernel    phase A: detect_orfs.py:134-203 + statistics.py:48-115 per atom of the exon union,
+//                             streamed by cp.async.bulk (compact layout); atom_summary_kernel for the dense planes
+//      compose_refs_kernel    phase B: per-ORF columns from the atom summaries (families of nested ORFs, suffix scan),
+//                             detect_orfs.py:274-299 + common.py:164-180
+//      score_orfs_kernel      the whole per-ORF loop in one kernel: fallback for counts >= 2^20
 //   K4 gather_profiles_kernel detect_orfs.py:134-203 for the reported ORFs (:322)
 //
 // All "file:line" citations are relative to the reference tree.
@@ -198,12 +198,10 @@ struct ScoreArgs {
     const uint64_t* exon_entries;
     const int32_t* orf_len;     // profile length per ORF (absolute ORF id)
     long long orf_lo;           // output element k <-> ORF orf_lo + k
-    const int32_t* list;        // ORF ids to score (absolute), longest first
+    const int32_t* list;        // ORF ids to score (absolute)
     long long n_list;           // entries of `list` ...
-    long long n_long;           // fused kernel: the first n_long entries take a whole warp each
     const unsigned* n_list_dev; // ... or, when not NULL, read from the device (fallback queue)
     unsigned long long* work_counter;
-    int32_t* fallback;          // packed kernel only: ORFs handed over to the generic kernel
     unsigned* n_fallback;
     rt_score_params prm;
     rt_score_out out;
@@ -400,23 +398,6 @@ score_orfs_kernel(const ScoreArgs args) {
     }
 }
 
-// ---- K3, fused gather + score: LPO lanes per ORF, 32/LPO ORFs per warp in lock step -----------
-// The per-ORF overhead (cursor, reductions, epilogue) is paid once per 32/LPO ORFs.  The host sorts
-// ORFs by length inside windows of the index, which keeps the groups of a warp balanced and
-// neighbouring ORFs (which share exons) close in time.  No shared memory: every lane owns one
-// codon per round, loads its three values straight from the coverage plane and gets the two
-// values after them from its right-hand neighbour by shuffle; rounds are software pipelined.
-// ORFs longer than kPackMaxNt take a whole warp each (LPO = 32) and are started first.
-// An ORF that turns out to hold a count >= 2^kBigShift is appended to the fallback queue and
-// redone by the generic kernel (64-bit sums).
-constexpr int kPackMaxNt = 3045;      // <= 127 rounds of 8 lanes: the 7-bit per-lane fields never overflow
-constexpr int kShortLPO = 8;          // lanes per short ORF
-constexpr int kLongFlushRounds = 31;  // whole-warp ORFs: flush the 10-bit fields every 31 rounds
-#ifndef RT_DEFER_LANES
-#define RT_DEFER_LANES 0
-#endif
-constexpr int kDeferLanes = RT_DEFER_LANES;   // general codons wait until this many lanes hold one (0: no parking)
-
 template <int LPO>
 __device__ __forceinline__ unsigned group_sum_u32(unsigned v) {
 #pragma unroll
@@ -430,423 +411,21 @@ __device__ __forceinline__ double group_sum_f64(double v) {
     return v;
 }
 
-// Group-uniform cursor over the exon entries of one ORF in profile coordinates.  It keeps the
-// current entry and the one after it, so that a round that crosses one exon junction needs no
-// divergent code: coverage slot of profile position p = org + dir * p.
-struct ProfileCursor {
-    const uint64_t* entries;
-    int n_ent;
-    int dir;               // +1 '+', -1 '-' (entries are then walked last to first)
-    int e = -1;            // index of the current entry
-    int p1 = 0;            // the current entry covers profile positions [.., p1)
-    long long org = 0;
-    bool zero = true;
-    int q1 = 0;            // the next entry covers [p1, q1); q1 == p1 when there is none
-    long long qorg = 0;
-    bool qzero = true;
-
-    __device__ __forceinline__ void fetch_next() {      // decode entry e + 1 into the q-fields
-        if (e + 1 < n_ent) {
-            const uint64_t ent = __ldg(entries + (dir < 0 ? n_ent - 2 - e : e + 1));
-            const int len = (int)(ent & kLenMask);
-            const uint64_t off = ent >> kLenBits;
-            qzero = off == kZeroOff;
-            const long long first = dir < 0 ? (long long)off + len - 1 : (long long)off;
-            qorg = first - (long long)dir * p1;
-            q1 = p1 + len;
-        } else {
-            qzero = true;
-            q1 = p1;
-        }
-    }
-    __device__ __forceinline__ void advance() {
-        ++e;
-        p1 = q1;
-        org = qorg;
-        zero = qzero;
-        fetch_next();
-    }
-    __device__ __forceinline__ void init() {
-        fetch_next();   // entry 0 -> q
-        advance();      // q -> current, entry 1 -> q
-    }
-};
-
-// The three coverage values of codon (round r, sub-lane sl): profile positions P + 3 sl + {0,1,2}.
-template <int LPO>
-__device__ __forceinline__ void load_round(const int32_t* cov, ProfileCursor& cur, int P, int L, int sl,
-                                           int& v0, int& v1, int& v2) {
-    constexpr int RNT = 3 * LPO;
-    v0 = v1 = v2 = 0;
-    const bool live = P < L;                             // groups past their end only take part in the vote
-    if (live)
-        while (P >= cur.p1) cur.advance();               // group-uniform
-    const int p = P + 3 * sl;
-    const bool inside = !live || P + RNT <= cur.p1;
-    if (__all_sync(kFull, inside)) {                     // every group is inside one entry
-        if (live && !cur.zero) {
-            const int32_t* s = cov + cur.org + (long long)cur.dir * p;
-            v0 = ld_cov(s);
-            v1 = ld_cov(s + cur.dir);
-            v2 = ld_cov(s + 2 * cur.dir);
-        }
-        return;
-    }
-    if (!live) return;
-    if (P + RNT <= cur.q1 || cur.e + 2 >= cur.n_ent) {   // at most one junction in this round
-        const bool c0 = p < cur.p1, c1 = p + 1 < cur.p1, c2 = p + 2 < cur.p1;
-        const bool k0 = c0 ? !cur.zero : (p < cur.q1 && !cur.qzero);
-        const bool k1 = c1 ? !cur.zero : (p + 1 < cur.q1 && !cur.qzero);
-        const bool k2 = c2 ? !cur.zero : (p + 2 < cur.q1 && !cur.qzero);
-        const long long d = cur.dir;
-        if (k0) v0 = ld_cov(cov + (c0 ? cur.org : cur.qorg) + d * p);
-        if (k1) v1 = ld_cov(cov + (c1 ? cur.org : cur.qorg) + d * (p + 1));
-        if (k2) v2 = ld_cov(cov + (c2 ? cur.org : cur.qorg) + d * (p + 2));
-        return;
-    }
-    // several junctions inside one round (exons shorter than a round): position by position
-    const int end = min(P + RNT, L);
-    int lo = 0;
-    for (;;) {
-        // current entry covers [lo', p1) with lo' = start of entry; positions below were handled
-        if (!cur.zero) {
-            const long long d = cur.dir;
-            if (p >= lo && p < cur.p1) v0 = ld_cov(cov + cur.org + d * p);
-            if (p + 1 >= lo && p + 1 < cur.p1) v1 = ld_cov(cov + cur.org + d * (p + 1));
-            if (p + 2 >= lo && p + 2 < cur.p1) v2 = ld_cov(cov + cur.org + d * (p + 2));
-        }
-        if (cur.p1 >= end) break;
-        lo = cur.p1;
-        cur.advance();
-    }
-}
-
-// General codons are parked (one slot per frame and lane) and turned into unit vectors when
-// enough lanes hold one, so that the fp64 sequence runs with most lanes active.
-struct Deferred {
-    int A0 = 0, B0 = 0, A1 = 0, B1 = 0, A2 = 0, B2 = 0;
-    unsigned has = 0;
-};
-__device__ __forceinline__ void unit_vector_add(int A, int B, FrameLane& f) {
-    // |A|, |B| < 2^22: D is exact; MUFU seed (2^-22) + one Newton step -> ~1e-13 relative
-    const double dA = (double)A, dB = (double)B;
-    const double D = fma(dA, dA, (3.0 * dB) * dB);
-    const double r0 = (double)rsqrt_approx((float)D);
-    const double e = fma(-D * r0, r0, 1.0);
-    const double r = fma(0.5 * r0, e, r0);
-    f.sre = fma(dA, r, f.sre);
-    f.sim = fma(dB, r, f.sim);
-}
-__device__ __forceinline__ void flush_deferred(Deferred& d, FrameLane& f0, FrameLane& f1, FrameLane& f2) {
-    if (d.has & 1u) unit_vector_add(d.A0, d.B0, f0);
-    if (d.has & 2u) unit_vector_add(d.A1, d.B1, f1);
-    if (d.has & 4u) unit_vector_add(d.A2, d.B2, f2);
-    d.has = 0;
-}
-// statistics.py:72-90 for one complete codon of frame F (see accumulate_codon above).
-template <int F>
-__device__ __forceinline__ void classify_codon(int a, int b, int c, FrameLane& f, Deferred& d) {
-    if ((a | b | c) == 0) return;                       // statistics.py:72-73
-    if ((b | c) == 0) f.w1 += 1u;
-    else if ((a | c) == 0) f.w1 += 1u << 10;
-    else if ((a | b) == 0) f.w1 += 1u << 20;
-    else if (a == b && b == c) f.w2 += 1u << 10;        // uniform: counts in K only
-    else {
-        f.w2 += 1u;
-        int& A = F == 0 ? d.A0 : F == 1 ? d.A1 : d.A2;
-        int& B = F == 0 ? d.B0 : F == 1 ? d.B1 : d.B2;
-        if (d.has & (1u << F)) unit_vector_add(A, B, f);   // slot taken: settle the older codon now
-        A = 2 * a - b - c;
-        B = b - c;
-        d.has |= 1u << F;
-    }
-}
-
-// Single-non-zero codons by table: m5 = non-zero mask of the lane's five values (bit j <-> value j).
-// Window f sees bits f..f+2; when exactly one of them is set the codon is (a,0,0), (0,b,0) or
-// (0,0,c) and maps to a constant unit vector, so it only bumps the 7-bit counter 3 f + kind of
-// the packed 64-bit accumulator.  One table lookup and one 64-bit add settle all three frames.
-__device__ __forceinline__ unsigned long long single_codon_lut_entry(unsigned m5) {
-    unsigned long long e = 0;
-    for (int f = 0; f < 3; ++f) {
-        const unsigned wm = (m5 >> f) & 7u;
-        if (wm == 1u) e += 1ull << (7 * (3 * f + 0));
-        else if (wm == 2u) e += 1ull << (7 * (3 * f + 1));
-        else if (wm == 4u) e += 1ull << (7 * (3 * f + 2));
-    }
-    return e;
-}
-// A codon with at least two non-zero counts: uniform (K only) or general (parked for the fp64 pass).
-// acc2 packs 7-bit counters: 2 F = general, 2 F + 1 = uniform.
-template <int F>
-__device__ __forceinline__ void multi_codon(int a, int b, int c, unsigned long long& acc2, FrameLane& f, Deferred& d) {
-    if (a == b && b == c) {
-        acc2 += 1ull << (7 * (2 * F + 1));
-    } else {
-        acc2 += 1ull << (7 * (2 * F));
-        if (kDeferLanes == 0) {
-            unit_vector_add(2 * a - b - c, b - c, f);
-            return;
-        }
-        int& A = F == 0 ? d.A0 : F == 1 ? d.A1 : d.A2;
-        int& B = F == 0 ? d.B0 : F == 1 ? d.B1 : d.B2;
-        if (d.has & (1u << F)) unit_vector_add(A, B, f);   // slot taken: settle the older codon now
-        A = 2 * a - b - c;
-        B = b - c;
-        d.has |= 1u << F;
-    }
-}
-// 7-bit packed accumulators -> the 10-bit words the reductions use (w1 = na | nb<<10 | nc<<20, w2 = ng | nu<<10).
-__device__ __forceinline__ void unpack_acc(unsigned long long& acc1, unsigned long long& acc2, FrameLane& f0,
-                                           FrameLane& f1, FrameLane& f2) {
-    auto w1 = [&](int f) {
-        const unsigned x = (unsigned)(acc1 >> (21 * f));
-        return (x & 127u) | (((x >> 7) & 127u) << 10) | (((x >> 14) & 127u) << 20);
-    };
-    auto w2 = [&](int f) {
-        const unsigned x = (unsigned)(acc2 >> (14 * f));
-        return (x & 127u) | (((x >> 7) & 127u) << 10);
-    };
-    f0.w1 += w1(0); f1.w1 += w1(1); f2.w1 += w1(2);
-    f0.w2 += w2(0); f1.w2 += w2(1); f2.w2 += w2(2);
-    acc1 = acc2 = 0;
-}
-
-// Warp-uniform totals of one frame (whole-warp ORFs only).
-struct FrameTotals {
-    int na = 0, nb = 0, nc = 0, ng = 0, nu = 0;
-    __device__ __forceinline__ void flush(FrameLane& f) {
-        const unsigned t1 = __reduce_add_sync(kFull, f.w1);
-        const unsigned t2 = __reduce_add_sync(kFull, f.w2);
-        na += t1 & 1023;
-        nb += (t1 >> 10) & 1023;
-        nc += t1 >> 20;
-        ng += t2 & 1023;
-        nu += t2 >> 10;
-        f.w1 = f.w2 = 0;
-    }
-};
-
-template <int LPO, bool Long>
-__device__ __forceinline__ void score_pack(const ScoreArgs& args, const unsigned long long* lut, long long item0,
-                                           long long item_end, int lane) {
-    const int sl = lane % LPO;                     // lane within the group
-    const int gb = lane - sl;                      // first lane of the group
-    const int nbr = sl + 1 == LPO ? gb : lane + 1; // right-hand neighbour (wraps to the next round)
-    const double kSqrt3 = 1.7320508075688772;
-    const double kNaN = __longlong_as_double(0x7ff8000000000000ll);
-
-    const long long item = item0 + lane / LPO;
-    const bool active = item < item_end;
-    int orf = 0, L = 0;
-    uint64_t desc = 0;
-    if (active) {
-        orf = __ldg(args.list + item);
-        desc = __ldg(args.orf_desc + orf);
-        L = __ldg(args.orf_len + orf);
-    }
-    ProfileCursor cur;
-    cur.entries = args.exon_entries + (desc & kBeginMask);
-    cur.n_ent = (int)((desc >> 40) & kMaxEntriesPerOrf);
-    cur.dir = (desc >> 63) != 0 ? -1 : 1;
-    cur.init();
-
-    FrameLane f0, f1, f2;
-    unsigned long long acc1 = 0, acc2 = 0;        // 7-bit packed codon counters (see single_codon_lut_entry)
-    Deferred dfr;
-    FrameTotals t0, t1, t2;                       // Long only
-    long long count64 = 0;                        // Long only
-    unsigned cnt32 = 0, mn32 = 0xffffffffu;
-    int ormask = 0;
-    const int ncod = (L + 2) / 3;                 // codons incl. a trailing partial one
-    const int rounds = __reduce_max_sync(kFull, (ncod + LPO - 1) / LPO);
-
-    int c0, c1, c2;
-    load_round<LPO>(args.cov, cur, 0, L, sl, c0, c1, c2);
-    for (int r = 0; r < rounds; ++r) {
-        int n0, n1, n2;
-        load_round<LPO>(args.cov, cur, (r + 1) * 3 * LPO, L, sl, n0, n1, n2);
-        // values 3 and 4 of this lane's five come from the neighbour's codon
-        const int v3 = __shfl_sync(kFull, sl == 0 ? n0 : c0, nbr);
-        const int v4 = __shfl_sync(kFull, sl == 0 ? n1 : c1, nbr);
-        const int p = 3 * (r * LPO + sl);
-        if (p < L) {
-            const unsigned cs = (unsigned)c0 + (unsigned)c1 + (unsigned)c2;   // common.py:177-179
-            cnt32 += cs;                                                        // detect_orfs.py:278
-            mn32 = min(mn32, cs);
-            ormask |= c0 | c1 | c2;
-            if ((c0 | c1 | c2 | v3 | v4) != 0) {
-                if (p + 4 < L) {
-                    const unsigned m5 = min((unsigned)c0, 1u) | (min((unsigned)c1, 1u) << 1) | (min((unsigned)c2, 1u) << 2) |
-                                        (min((unsigned)v3, 1u) << 3) | (min((unsigned)v4, 1u) << 4);
-                    acc1 += lut[m5];
-                    const unsigned multi = ((m5 & (m5 >> 1)) | (m5 & (m5 >> 2)) | ((m5 >> 1) & (m5 >> 2))) & 7u;
-                    if (multi) {
-                        if (multi & 1u) multi_codon<0>(c0, c1, c2, acc2, f0, dfr);
-                        if (multi & 2u) multi_codon<1>(c1, c2, v3, acc2, f1, dfr);
-                        if (multi & 4u) multi_codon<2>(c2, v3, v4, acc2, f2, dfr);
-                    }
-                } else {                                                        // ragged end (statistics.py:71)
-                    if (p + 2 < L) classify_codon<0>(c0, c1, c2, f0, dfr);
-                    if (p + 3 < L) classify_codon<1>(c1, c2, v3, f1, dfr);
-                }
-            }
-        }
-        if (kDeferLanes > 0 && __popc(__ballot_sync(kFull, dfr.has != 0)) >= kDeferLanes) flush_deferred(dfr, f0, f1, f2);
-        if (Long && (r % kLongFlushRounds) == kLongFlushRounds - 1) {
-            unpack_acc(acc1, acc2, f0, f1, f2);
-            t0.flush(f0); t1.flush(f1); t2.flush(f2);
-            count64 += __reduce_add_sync(kFull, cnt32);
-            cnt32 = 0;
-        }
-        c0 = n0; c1 = n1; c2 = n2;
-    }
-    flush_deferred(dfr, f0, f1, f2);
-    unpack_acc(acc1, acc2, f0, f1, f2);
-
-    // ---- reductions (all lanes converged) ----
-    int na0, nb0, nc0, ng0, nu0, na1, nb1, nc1, ng1, nu1, na2, nb2, nc2, ng2, nu2;
-    long long count;
-    if (Long) {
-        t0.flush(f0); t1.flush(f1); t2.flush(f2);
-        count = count64 + __reduce_add_sync(kFull, cnt32);
-        na0 = t0.na; nb0 = t0.nb; nc0 = t0.nc; ng0 = t0.ng; nu0 = t0.nu;
-        na1 = t1.na; nb1 = t1.nb; nc1 = t1.nc; ng1 = t1.ng; nu1 = t1.nu;
-        na2 = t2.na; nb2 = t2.nb; nc2 = t2.nc; ng2 = t2.ng; nu2 = t2.nu;
-        mn32 = __reduce_min_sync(kFull, mn32);
-        ormask = (int)__reduce_or_sync(kFull, (unsigned)ormask);
-    } else {
-        const unsigned a1_0 = group_sum_u32<LPO>(f0.w1), a2_0 = group_sum_u32<LPO>(f0.w2);
-        const unsigned a1_1 = group_sum_u32<LPO>(f1.w1), a2_1 = group_sum_u32<LPO>(f1.w2);
-        const unsigned a1_2 = group_sum_u32<LPO>(f2.w1), a2_2 = group_sum_u32<LPO>(f2.w2);
-        count = (long long)group_sum_u32<LPO>(cnt32);
-#pragma unroll
-        for (int o = LPO / 2; o > 0; o >>= 1) {
-            mn32 = min(mn32, __shfl_xor_sync(kFull, mn32, o));
-            ormask |= __shfl_xor_sync(kFull, ormask, o);
-        }
-        na0 = a1_0 & 1023; nb0 = (a1_0 >> 10) & 1023; nc0 = a1_0 >> 20; ng0 = a2_0 & 1023; nu0 = a2_0 >> 10;
-        na1 = a1_1 & 1023; nb1 = (a1_1 >> 10) & 1023; nc1 = a1_1 >> 20; ng1 = a2_1 & 1023; nu1 = a2_1 >> 10;
-        na2 = a1_2 & 1023; nb2 = (a1_2 >> 10) & 1023; nc2 = a1_2 >> 20; ng2 = a2_2 & 1023; nu2 = a2_2 >> 10;
-    }
-    const bool any_general = __any_sync(kFull, (ng0 | ng1 | ng2) != 0);
-    double re0 = 0.0, im0 = 0.0, re1 = 0.0, im1 = 0.0, re2 = 0.0, im2 = 0.0;
-    if (any_general) {
-        re0 = group_sum_f64<LPO>(f0.sre); im0 = group_sum_f64<LPO>(f0.sim);
-        re1 = group_sum_f64<LPO>(f1.sre); im1 = group_sum_f64<LPO>(f1.sim);
-        re2 = group_sum_f64<LPO>(f2.sre); im2 = group_sum_f64<LPO>(f2.sim);
-    }
-
-    // ---- epilogue: statistics.py:92-115 + detect_orfs.py:278-299, once for all groups ----
-    const int n_codons = L / 3 > 1 ? L / 3 : 1;                        // detect_orfs.py:281
-    const int K0 = na0 + nb0 + nc0 + ng0 + nu0;
-    const int K1 = na1 + nb1 + nc1 + ng1 + nu1;
-    const int K2 = na2 + nb2 + nc2 + ng2 + nu2;
-    re0 += 0.5 * (double)(2 * na0 - nb0 - nc0); im0 = kSqrt3 * (im0 + 0.5 * (double)(nb0 - nc0));
-    re1 += 0.5 * (double)(2 * na1 - nb1 - nc1); im1 = kSqrt3 * (im1 + 0.5 * (double)(nb1 - nc1));
-    re2 += 0.5 * (double)(2 * na2 - nb2 - nc2); im2 = kSqrt3 * (im2 + 0.5 * (double)(nb2 - nc2));
-    // one fp64 division sequence for all seven quotients of every group: sub-lanes 0-2 the
-    // coherences |sum u|^2 / (K * M), sub-lane 3 the density, sub-lanes 4-6 K_f / n_codons
-    double nn, dd = (double)n_codons;
-    if (sl == 0) { nn = re0 * re0 + im0 * im0; dd = (double)K0 * (double)(K0 - nu0); }
-    else if (sl == 1) { nn = re1 * re1 + im1 * im1; dd = (double)K1 * (double)(K1 - nu1); }
-    else if (sl == 2) { nn = re2 * re2 + im2 * im2; dd = (double)K2 * (double)(K2 - nu2); }
-    else if (sl == 3) nn = (double)count;                              // detect_orfs.py:287
-    else if (sl == 4) nn = (double)K0;                                 // detect_orfs.py:285
-    else if (sl == 5) nn = (double)K1;
-    else nn = (double)K2;
-    const double q = nn / dd;                                          // 0/0 -> NaN never wins
-    double s0 = __shfl_sync(kFull, q, gb + 0);
-    double s1 = __shfl_sync(kFull, q, gb + 1);
-    double s2 = __shfl_sync(kFull, q, gb + 2);
-    const double density = __shfl_sync(kFull, q, gb + 3);
-    // statistics.py:64-66,92-115: running maximum with the K==0 reset quirk
-    double coh = 0.0;
-    int vf = -1;          // frame whose K is `valid`; -1: valid = 0
-    bool unset = true;    // valid == -1 in the reference
-    if (K0 == 0) { coh = 0.0; vf = -1; unset = false; s0 = kNaN; }
-    else { if (s0 > coh) { coh = s0; vf = 0; unset = false; } if (unset) { vf = 0; unset = false; } }
-    if (K1 == 0) { coh = 0.0; vf = -1; unset = false; s1 = kNaN; }
-    else { if (s1 > coh) { coh = s1; vf = 1; unset = false; } if (unset) { vf = 1; unset = false; } }
-    if (K2 == 0) { coh = 0.0; vf = -1; unset = false; s2 = kNaN; }
-    else { if (s2 > coh) { coh = s2; vf = 2; unset = false; } if (unset) { vf = 2; unset = false; } }
-    const double score = sqrt(coh);                                    // statistics.py:115
-    const int valid = vf == 0 ? K0 : vf == 1 ? K1 : vf == 2 ? K2 : 0;
-    double ratio = __shfl_sync(kFull, q, gb + (vf >= 0 ? 4 + vf : 4));
-    if (vf < 0) ratio = 0.0;
-
-    if (active && sl == 0) {
-        if ((ormask >> kBigShift) != 0) {
-            // a huge count: 32-bit sums may have wrapped -> hand over to the generic kernel
-            args.fallback[atomicAdd(args.n_fallback, 1u)] = orf;
-        } else {
-            const long long k_out = (long long)orf - args.orf_lo;
-            const unsigned min_codon = L == 0 ? 0u : mn32;
-            const bool ok = score >= args.prm.phase_score_cutoff &&
-                            (double)valid >= args.prm.min_valid_codons &&
-                            (L == 0 || (double)min_codon >= args.prm.min_reads_per_codon) &&
-                            ratio >= args.prm.min_valid_codons_ratio &&
-                            density >= args.prm.min_density_over_orf;   // detect_orfs.py:289-299
-            args.out.score[k_out] = score;
-            args.out.valid[k_out] = valid;
-            args.out.count[k_out] = count;
-            args.out.length[k_out] = L;
-            if (args.out.min_codon) args.out.min_codon[k_out] = (int32_t)min_codon;
-            if (args.out.status) args.out.status[k_out] = ok ? 1 : 0;
-            if (args.out.frame_K) {
-                args.out.frame_K[3 * k_out + 0] = K0;
-                args.out.frame_K[3 * k_out + 1] = K1;
-                args.out.frame_K[3 * k_out + 2] = K2;
-            }
-            if (args.out.frame_s) {
-                args.out.frame_s[3 * k_out + 0] = s0;
-                args.out.frame_s[3 * k_out + 1] = s1;
-                args.out.frame_s[3 * k_out + 2] = s2;
-            }
-        }
-    }
-    __syncwarp();
-}
-
-// Work items: [0, n_long) one long ORF per warp, then packs of 32/LPO short ORFs.
-template <int LPO>
-__global__ void __launch_bounds__(kScoreWarps * 32, 4)
-score_orfs_packed_kernel(const ScoreArgs args) {
-    constexpr int G = 32 / LPO;
-    __shared__ unsigned long long s_lut[32];
-    if (threadIdx.x < 32) s_lut[threadIdx.x] = single_codon_lut_entry(threadIdx.x);
-    __syncthreads();
-    const int lane = threadIdx.x & 31;
-    const long long n_short = args.n_list - args.n_long;
-    const long long n_work = args.n_long + (n_short + G - 1) / G;
-    for (;;) {
-        unsigned long long w = 0;
-        if (lane == 0) w = atomicAdd(args.work_counter, 1ull);
-        w = __shfl_sync(kFull, w, 0);
-        if ((long long)w >= n_work) break;
-        if ((long long)w < args.n_long) {
-            score_pack<32, true>(args, s_lut, (long long)w, (long long)w + 1, lane);
-        } else {
-            score_pack<LPO, false>(args, s_lut, args.n_long + ((long long)w - args.n_long) * G, args.n_list, lane);
-        }
-    }
-}
-
 // ---- K3, two-phase: atom summaries + per-ORF composition -----------------------------------------
 // Candidate ORFs overlap massively (nested ORFs share their 3' exons, isoforms share exons), so the
 // index is cut at every exon boundary of every ORF into ATOMS: maximal coverage intervals that no
 // ORF exon boundary splits.  Every ORF is a sequence of atoms (plus "reads-as-zero" stretches).
-//   phase A (atom_summary_kernel): every atom is scanned ONCE per library -- windows that lie fully
-//            inside the atom are classified exactly like the scan kernel does and summed by local
-//            frame (window start offset mod 3);
-//   phase B (score_from_atoms_kernel): one thread per ORF adds the summaries of its atoms with the
-//            frame rotation that the atom's profile offset implies, evaluates the two windows that
-//            straddle every seam between consecutive atoms from the raw coverage, and runs the
-//            epilogue (statistics.py:92-115, detect_orfs.py:278-299).
+//   phase A (atom_pass_kernel on the compact layout, atom_summary_kernel on the dense planes): every
+//            atom is scanned ONCE per library -- windows that lie fully inside the atom are classified
+//            and summed by local frame (window start offset mod 3) into the atom's summary;
+//   phase B (compose_refs_kernel): the summaries of an ORF's atoms are added with the frame rotation
+//            that the atom's profile offset implies, the two windows that straddle every seam between
+//            consecutive atoms are rebuilt from the edge values of the summaries, and the epilogue
+//            runs (statistics.py:92-115, detect_orfs.py:278-299).
 // The work per library is proportional to the UNION of the exons instead of the sum over ORFs.
 // '-' strand: a profile window (v0,v1,v2) is the reversed genomic triple and u(v0,v1,v2) =
 // w^2 conj(u(v2,v1,v0)), so |sum u| is what the '+'-oriented sums give; only the frame mapping of
-// a local frame differs (see score_from_atoms_kernel).
+// a local frame differs (see compose_refs_kernel).
 constexpr int kPieceNt = 33;           // values per lane and pass of atom_pass_kernel (odd multiple of 3: frames stay
                                        //   static per window and consecutive pieces fall into distinct banks)
 constexpr int kPassPieces = 32;        // pieces (= lanes) per pass
@@ -925,22 +504,17 @@ __device__ __forceinline__ void slow_window(int x, int y, int z, unsigned& accK,
     f.sim += u.y;
 }
 
-#ifndef RT_ATOM_MINBLOCKS
-#define RT_ATOM_MINBLOCKS 4
-#endif
+constexpr int kAtomLPO = 4;            // lanes per atom of atom_summary_kernel
 // Packs of G atoms are handed out through an atomic counter (the atoms of a plan window are sorted
 // by length, so a static split leaves warps idle).  The chain counter -> list[] -> atoms[] ->
 // coverage is four dependent memory round trips; it is software pipelined ACROSS packs: while pack k
 // is scanned the warp already holds the atom id of pack k+1, fetches its descriptor and the atom id
 // of pack k+2, and has the counter bump for pack k+3 in flight; the first coverage loads of pack
 // k+1 are issued before the reductions and the summary store of pack k.
-#ifndef RT_ATOM_PF_DIST
-#define RT_ATOM_PF_DIST 0
-#endif
-constexpr unsigned kPfDist = RT_ATOM_PF_DIST;          // packs of look-ahead of the cooperative L2 prefetch (0: off)
-template <int LPO, bool WantMin>
-__global__ void __launch_bounds__(kScoreWarps * 32, RT_ATOM_MINBLOCKS)
+template <bool WantMin>
+__global__ void __launch_bounds__(kScoreWarps * 32, 4)
 atom_summary_kernel(const AtomArgs args) {
+    constexpr int LPO = kAtomLPO;
     constexpr int G = 32 / LPO;
     constexpr int RNT = 3 * LPO;
     __shared__ double2 s_uv[kUvEntries];
@@ -977,10 +551,6 @@ atom_summary_kernel(const AtomArgs args) {
     unsigned raw2 = pack + 2;                             // lane 0's copy is the one that is read
     int atom = load_atom(pack);
     int atom1 = load_atom(pack1);
-    // cooperative L2 prefetch: packs are handed out in order, so the atoms of pack id + kPfDist will be
-    // scanned soon by SOME warp; every warp requests their lines now (two table lookups, one per turn)
-    int pf_atom = -1;
-    uint64_t pf_ent = 0;
     int len = 0;
     const int32_t* src = args.cov;
     if (atom >= 0) {
@@ -999,17 +569,6 @@ atom_summary_kernel(const AtomArgs args) {
     load3(c0, c1, c2);
 
     while (pack < n_packs) {
-        if (kPfDist > 0) {
-            const int pf_len = (int)(pf_ent & kLenMask);
-            const int32_t* pf_src = args.cov + (pf_ent >> kLenBits);
-#pragma unroll
-            for (int q = 0; q < 3; ++q) {                 // 128-byte lines 0..3 LPO-1 of the atom; longer atoms pipeline by themselves
-                const int o = 32 * (sl + q * LPO);
-                if (o < pf_len) asm volatile("prefetch.global.L2 [%0];" ::"l"(pf_src + o));
-            }
-            pf_ent = pf_atom >= 0 ? __ldg(args.atoms + pf_atom) : 0ull;
-            pf_atom = load_atom(pack + kPfDist);
-        }
         // ---- descriptor of pack k+1, atom id of pack k+2, counter bump for pack k+3 ----
         uint64_t ent1 = 0;
         if (atom1 >= 0) ent1 = __ldg(args.atoms + atom1);
@@ -1162,6 +721,9 @@ constexpr int kPassStageBytes = kPassBufSlots * 4 + kPassEntSlots * 8 + 16 + 16;
 static_assert(kPassStageBytes % 16 == 0 && (kPassBufSlots * 4) % 16 == 0, "stage layout");
 constexpr int kGroupNt = kPieceNt / 3;                               // a lane settles its piece in three groups of 11 windows
 static_assert(kGroupNt * 3 == kPieceNt, "piece = three groups");
+// 16 warps x 2 stages measured best on C2 (profiles/README.md): more warps need the 64-register build, which spills, and
+// a third stage buys nothing -- the kernel is bound by the shared-memory pipe, not by the copies
+constexpr int kPassWarps = 16, kPassStages = 2;
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint64_t* bar, unsigned count) {
@@ -1193,8 +755,9 @@ __device__ __forceinline__ void count_nonzero(unsigned& n, int x) {
     asm("{\n.reg .pred p;\nsetp.ne.s32 p, %1, 0;\n@p add.u32 %0, %0, 1;\n}" : "+r"(n) : "r"(x));
 }
 
-template <int STAGES, bool WantMin>
-__global__ void __launch_bounds__(512, 1) atom_pass_kernel(const PassArgs args) {
+template <bool WantMin>
+__global__ void __launch_bounds__(kPassWarps * 32, 1) atom_pass_kernel(const PassArgs args) {
+    constexpr int STAGES = kPassStages;
     extern __shared__ __align__(16) unsigned char s_raw[];
     double2* s_uv = reinterpret_cast<double2*>(s_raw);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, n_warps = blockDim.x >> 5;
@@ -1419,271 +982,6 @@ __global__ void __launch_bounds__(512, 1) atom_pass_kernel(const PassArgs args) 
     }
 }
 
-struct ComposeArgs {
-    const int32_t* cov;
-    const uint64_t* orf_refs_desc;     // per ORF: ref begin (40 bits) | n_refs (23 bits) << 40 | reverse << 63
-    const uint64_t* ref_ent;           // (slot offset << 24) | len in PROFILE order; offset kZeroOff: zeros
-    const uint32_t* ref_atom;          // atom id of the ref (unused for zero refs)
-    const AtomSummary* summaries;
-    const uint8_t* atom_nonzero;       // written by phase A: 0 = the atom reads as zeros, its summary is stale
-    int want_min;                      // per-frame minima needed (min_codon column or --min_reads_per_codon > 0)
-    const int32_t* orf_len;
-    long long orf_lo;
-    const int32_t* list;               // ORF ids to score
-    long long n_list;
-    int32_t* fallback;                 // ORFs holding counts >= 2^kBigShift: redone by the generic kernel
-    unsigned* n_fallback;
-    // ORFs with more than kSegRefs refs are cut into segments that run in parallel
-    const struct RefSegment* segs;     // work items [0, n_segs) of the launch; the ORFs of `list` follow
-    long long n_segs;
-    struct ComposeAcc* partials;       // one per segment
-    unsigned* seg_done;                // per long ORF: segments finished so far (self-resetting)
-    rt_score_params prm;
-    rt_score_out out;
-};
-constexpr int kSegRefs = 48;           // refs per segment of a long ORF
-
-// ---- phase B ----------------------------------------------------------------------------------
-// Per-frame sums of one ORF (or of one segment of a long ORF) in PROFILE frames.
-struct ComposeAcc {
-    unsigned K[3], U[3];
-    long long RE[3], IM[3];            // sums of unit vectors in units of 2^-42 (uv_grid): exact
-    unsigned mn;
-    int big;
-    long long count;
-};
-static_assert(sizeof(ComposeAcc) == 88, "ComposeAcc layout");
-
-// A slice of the atom references of a long ORF (more than kSegRefs refs), scored by its own thread.
-struct RefSegment {
-    int orf;
-    unsigned ref_begin;        // absolute index of the segment's first ref
-    int n_refs;
-    int P0;                    // profile offset of that ref
-    int slot;                  // where the partial sums go (ComposeArgs::partials)
-    int first_slot, n_seg;     // the ORF's segments occupy partial slots [first_slot, first_slot + n_seg)
-    int long_idx;              // index of the ORF among the long ORFs (ComposeArgs::seg_done)
-};
-
-// statistics.py:92-115 + detect_orfs.py:278-299 on the finished sums of one ORF.
-template <typename Args>
-__device__ __forceinline__ void finish_orf(const Args& args, int orf, int L, const unsigned* K, const unsigned* U,
-                                           const long long* RE, const long long* IM, unsigned mn, long long count) {
-    const double kSqrt3 = 1.7320508075688772;
-    const double kNaN = __longlong_as_double(0x7ff8000000000000ll);
-    const int n_codons = L / 3 > 1 ? L / 3 : 1;                          // detect_orfs.py:281
-    double s3[3];
-    double coh = 0.0;
-    int valid = -1;
-#pragma unroll
-    for (int f = 0; f < 3; ++f) {
-        if (K[f] == 0) { s3[f] = kNaN; coh = 0.0; valid = 0; continue; }   // statistics.py:94-95
-        const double re = (double)RE[f] * (1.0 / kUvGridScale);               // the sums are exact integers (units of 2^-42)
-        const double im = kSqrt3 * ((double)IM[f] * (1.0 / kUvGridScale));
-        const double s = (re * re + im * im) / ((double)K[f] * (double)(K[f] - U[f]));   // 0/0 -> NaN never wins
-        s3[f] = s;
-        if (s > coh) { coh = s; valid = (int)K[f]; }                     // statistics.py:109-111
-        if (valid == -1) valid = (int)K[f];                              // statistics.py:112-113
-    }
-    const double score = sqrt(coh);                                      // statistics.py:115
-    const double ratio = (double)valid / (double)n_codons;               // detect_orfs.py:285
-    const double density = (double)count / (double)n_codons;             // detect_orfs.py:287
-    const unsigned min_codon = L == 0 ? 0u : mn;
-    const bool ok = score >= args.prm.phase_score_cutoff && (double)valid >= args.prm.min_valid_codons &&
-                    (L == 0 || (double)min_codon >= args.prm.min_reads_per_codon) &&
-                    ratio >= args.prm.min_valid_codons_ratio && density >= args.prm.min_density_over_orf;
-    const long long k_out = (long long)orf - args.orf_lo;
-    args.out.score[k_out] = score;
-    args.out.valid[k_out] = valid;
-    args.out.count[k_out] = count;
-    args.out.length[k_out] = L;
-    if (args.out.min_codon) args.out.min_codon[k_out] = (int32_t)min_codon;
-    if (args.out.status) args.out.status[k_out] = ok ? 1 : 0;
-    if (args.out.frame_K) {
-        args.out.frame_K[3 * k_out + 0] = (int)K[0];
-        args.out.frame_K[3 * k_out + 1] = (int)K[1];
-        args.out.frame_K[3 * k_out + 2] = (int)K[2];
-    }
-    if (args.out.frame_s) {
-        args.out.frame_s[3 * k_out + 0] = s3[0];
-        args.out.frame_s[3 * k_out + 1] = s3[1];
-        args.out.frame_s[3 * k_out + 2] = s3[2];
-    }
-}
-
-// One thread per ORF -- or per segment of a long ORF; the segments are the first work items of the launch --
-// streams the summaries of its atoms: no raw coverage is read any more.  The windows that straddle atom
-// seams are rebuilt from the edge values kept in the summaries: while the profile streams by, (x, y) are
-// its last two values, and every value that enters a new atom completes one window that is not interior to
-// any atom.  A segment starts from the last two values of the ref before it (the host only cuts after refs
-// of >= 2 values) and leaves its sums in `partials`; the thread that finishes an ORF's last outstanding
-// segment adds the partial sums up in segment order and scores the ORF.
-__global__ void __launch_bounds__(256) score_from_atoms_kernel(const ComposeArgs args) {
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= args.n_segs + args.n_list) return;
-    const bool Seg = i < args.n_segs;
-    RefSegment seg{};
-    if (Seg) seg = args.segs[i];
-    const int orf = Seg ? seg.orf : __ldg(args.list + (i - args.n_segs));
-    const uint64_t desc = __ldg(args.orf_refs_desc + orf);
-    const uint64_t begin = Seg ? (uint64_t)seg.ref_begin : (desc & kBeginMask);
-    const int n_refs = Seg ? seg.n_refs : (int)((desc >> 40) & kMaxEntriesPerOrf);
-    const bool rev = (desc >> 63) != 0;
-    const int L = __ldg(args.orf_len + orf);
-
-    unsigned K[3] = {0, 0, 0}, U[3] = {0, 0, 0};
-    long long RE[3] = {0, 0, 0}, IM[3] = {0, 0, 0};          // units of 2^-42: integer sums, no rounding, any order
-    unsigned mn = 0xffffffffu;
-    long long count = 0;
-    int ormask = 0;
-    bool big = false;
-    constexpr long long kOne = 1ll << 42, kHalf = 1ll << 41;
-
-    // one seam window of the profile starting at position p = (values v0,v1,v2): statistics.py:72-90
-    auto window = [&](int p, int v0, int v1, int v2) {
-        const int f = p % 3;
-        ormask |= v0 | v1 | v2;
-        if (f == 0) mn = min(mn, (unsigned)v0 + (unsigned)v1 + (unsigned)v2);
-        if ((v0 | v1 | v2) == 0) return;
-        // '+'-oriented triple (a,b,c): the profile of a '-' ORF runs against the plane
-        const int a = rev ? v2 : v0, b = v1, c = rev ? v0 : v2;
-        long long re, im;
-        if ((b | c) == 0) { re = kOne; im = 0; }
-        else if ((a | c) == 0) { re = -kHalf; im = kHalf; }
-        else if ((a | b) == 0) { re = -kHalf; im = -kHalf; }
-        else if (a == b && b == c) { re = 0; im = 0; }
-        else {
-            const double2 u = uv_grid((double)(2ll * a - b - c), (double)((long long)b - c));
-            re = __double2ll_rn(u.x * kUvGridScale);
-            im = __double2ll_rn(u.y * kUvGridScale);
-        }
-        const bool uniform = a == b && b == c;
-#pragma unroll
-        for (int q = 0; q < 3; ++q)
-            if (q == f) { K[q] += 1u; U[q] += uniform ? 1u : 0u; RE[q] += re; IM[q] += im; }
-    };
-
-    int P = Seg ? seg.P0 : 0;   // profile offset of the current ref
-    int x = 0, y = 0;           // profile values at P - 2 and P - 1
-    if (Seg && seg.P0 > 0) {    // the ref before the segment holds >= 2 values: its last two in profile order
-        const uint64_t pe = __ldg(args.ref_ent + begin - 1);
-        if ((pe >> kLenBits) != kZeroOff) {
-            const unsigned pa = __ldg(args.ref_atom + begin - 1);
-            if (__ldg(args.atom_nonzero + pa) != 0) {
-                const int4 edge = __ldg(reinterpret_cast<const int4*>(args.summaries + pa) + 3);
-                if (rev) { x = edge.y; y = edge.x; }
-                else { x = edge.z; y = edge.w; }
-            }
-        }
-    }
-    // software pipeline: (entry, atom id) two refs ahead, the atom's non-zero flag one ref ahead
-    uint64_t ent = 0, ent_n = 0;
-    unsigned atom = 0, atom_n = 0;
-    bool nz = false;
-    if (n_refs > 0) {
-        ent = __ldg(args.ref_ent + begin);
-        atom = __ldg(args.ref_atom + begin);
-    }
-    if (n_refs > 1) {
-        ent_n = __ldg(args.ref_ent + begin + 1);
-        atom_n = __ldg(args.ref_atom + begin + 1);
-    }
-    if (n_refs > 0 && (ent >> kLenBits) != kZeroOff) nz = __ldg(args.atom_nonzero + atom) != 0;
-    for (int j = 0; j < n_refs; ++j) {
-        const int len = (int)(ent & kLenMask);
-        const bool zero = !nz;                  // reads-as-zero stretch or an atom without a single read
-        const AtomSummary* s = args.summaries + atom;
-        ent = ent_n;
-        atom = atom_n;
-        nz = false;
-        if (j + 1 < n_refs && (ent >> kLenBits) != kZeroOff) nz = __ldg(args.atom_nonzero + atom) != 0;
-        if (j + 2 < n_refs) {
-            ent_n = __ldg(args.ref_ent + begin + j + 2);
-            atom_n = __ldg(args.ref_atom + begin + j + 2);
-        }
-        int a0 = 0, a1 = 0, z0 = 0, z1 = 0;    // first two / last two values of the ref in profile order
-        if (!zero) {
-            const longlong2 r01 = __ldg(reinterpret_cast<const longlong2*>(s));          // re[0], re[1]
-            const longlong2 r2i0 = __ldg(reinterpret_cast<const longlong2*>(s) + 1);     // re[2], im[0]
-            const longlong2 i12 = __ldg(reinterpret_cast<const longlong2*>(s) + 2);      // im[1], im[2]
-            const int4 edge = __ldg(reinterpret_cast<const int4*>(s) + 3);
-            const uint4 ku = __ldg(reinterpret_cast<const uint4*>(s) + 4);           // kpack, upack, count
-            uint4 mc = make_uint4(0xffffffffu, 0xffffffffu, 0xffffffffu, 0u);
-            if (args.want_min) mc = __ldg(reinterpret_cast<const uint4*>(s) + 5);    // mn[0..2]
-            const long long sre[3] = {r01.x, r01.y, r2i0.x}, sim[3] = {r2i0.y, i12.x, i12.y};
-            const unsigned smn[3] = {mc.x, mc.y, mc.z};
-            const unsigned sK[3] = {ku.x & 1023u, (ku.x >> 10) & 1023u, (ku.x >> 20) & 1023u};
-            const unsigned sU[3] = {ku.y & 1023u, (ku.y >> 10) & 1023u, (ku.y >> 20) & 1023u};
-            big |= (ku.x >> 31) != 0;
-            count += ku.z;
-            if (rev) { a0 = edge.w; a1 = edge.z; z0 = edge.y; z1 = edge.x; }
-            else { a0 = edge.x; a1 = edge.y; z0 = edge.z; z1 = edge.w; }
-            // local frame fl (window start offset inside the atom, mod 3) -> profile frame f:
-            //   '+': f = (fl + P) mod 3          '-': f = (len + P - fl) mod 3
-            const int base = rev ? (len + P) % 3 : P % 3;
-#pragma unroll
-            for (int fl = 0; fl < 3; ++fl) {
-                const int f = rev ? (base - fl + 3) % 3 : (base + fl) % 3;
-#pragma unroll
-                for (int q = 0; q < 3; ++q)
-                    if (q == f) { K[q] += sK[fl]; U[q] += sU[fl]; RE[q] += sre[fl]; IM[q] += sim[fl]; }
-                if (f == 0) mn = min(mn, smn[fl]);
-            }
-        } else if (len >= 3 && (3 - P % 3) % 3 <= len - 3) {
-            mn = 0;     // a reads-as-zero stretch that holds a whole frame-0 codon
-        }
-        // seam windows: the ones that END on the first and on the second value of this ref
-        if (P >= 2) window(P - 2, x, y, a0);
-        if (len >= 2) {
-            if (P >= 1) window(P - 1, y, a0, a1);
-            x = z0;
-            y = z1;
-        } else {
-            x = y;
-            y = a0;
-        }
-        P += len;
-    }
-    if (!Seg || seg.slot == seg.first_slot + seg.n_seg - 1) {
-        // trailing partial codon (common.py:177-179): the last L % 3 values are x, y
-        if (L % 3 == 1) { mn = min(mn, (unsigned)y); ormask |= y; }
-        else if (L % 3 == 2) { mn = min(mn, (unsigned)x + (unsigned)y); ormask |= x | y; }
-    }
-    big |= (ormask >> kBigShift) != 0;
-    if (Seg) {
-        ComposeAcc acc;
-#pragma unroll
-        for (int f = 0; f < 3; ++f) { acc.K[f] = K[f]; acc.U[f] = U[f]; acc.RE[f] = RE[f]; acc.IM[f] = IM[f]; }
-        acc.mn = mn;
-        acc.big = big ? 1 : 0;
-        acc.count = count;
-        args.partials[seg.slot] = acc;
-        __threadfence();
-        if (atomicAdd(args.seg_done + seg.long_idx, 1u) != (unsigned)(seg.n_seg - 1)) return;
-        // this thread finished the ORF's last outstanding segment: add the partial sums in segment order
-        __threadfence();
-        args.seg_done[seg.long_idx] = 0;                    // ready for the next launch
-#pragma unroll
-        for (int f = 0; f < 3; ++f) { K[f] = 0; U[f] = 0; RE[f] = 0; IM[f] = 0; }
-        mn = 0xffffffffu;
-        count = 0;
-        big = false;
-        for (int sidx = seg.first_slot; sidx < seg.first_slot + seg.n_seg; ++sidx) {
-            const volatile ComposeAcc* pa = args.partials + sidx;
-#pragma unroll
-            for (int f = 0; f < 3; ++f) { K[f] += pa->K[f]; U[f] += pa->U[f]; RE[f] += pa->RE[f]; IM[f] += pa->IM[f]; }
-            mn = min(mn, pa->mn);
-            big |= pa->big != 0;
-            count += pa->count;
-        }
-    }
-    if (big) {
-        args.fallback[atomicAdd(args.n_fallback, 1u)] = orf;
-        return;
-    }
-    finish_orf(args, orf, L, K, U, RE, IM, mn, count);
-}
-
 // ---- phase B, one lane per atom reference of a FAMILY of ORFs: compose_refs_kernel ------------------------
 // Candidate ORFs that share their stop (nested ORFs of a transcript) are suffixes of the longest one: from some
 // reference on they consist of the same atoms.  The host groups such ORFs into families and lays the references of
@@ -1802,11 +1100,8 @@ __device__ __forceinline__ void finish_orf_lean(const Args& args, int orf, int L
     }
 }
 
-#ifndef RT_COMPOSE_MINBLOCKS
-#define RT_COMPOSE_MINBLOCKS 4
-#endif
 template <bool WantMin>
-__global__ void __launch_bounds__(256, RT_COMPOSE_MINBLOCKS) compose_refs_kernel(const RefComposeArgs args) {
+__global__ void __launch_bounds__(256, 4) compose_refs_kernel(const RefComposeArgs args) {
     const long long w = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (w >= args.n_warps) return;
     const int lane = threadIdx.x & 31;
