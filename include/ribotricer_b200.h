@@ -48,7 +48,7 @@
 extern "C" {
 #endif
 
-#define RT_ABI_VERSION 3
+#define RT_ABI_VERSION 4
 
 /* read-length table: one int32 per matched length = the P-site offset of that length (may be negative:
  * align_metagenes returns lag + 12 with lag in [-min(base, length), ...), metagene.py:319-324; |offset| <=
@@ -121,7 +121,7 @@ int rt_set_length_table(rt_ctx* ctx, const int32_t* h_len_table /* RT_LEN_TABLE 
  * Adds into d_cov (2*plane int32; clear it first for a fresh library),
  * accumulates into d_stats[RT_N_STATS] and d_len_counts[RT_LEN_TABLE] (int64).
  * `sorted_hint` != 0 promises reads grouped by reference (a coordinate-sorted BAM); the device-pointer
- * entry ignores it, the host-pointer entry uses it to ship packed records (below).  Results are identical
+ * entry ignores it, the host-pointer entry uses it to ship the record stream (below).  Results are identical
  * either way.
  * `weight` is +1 to add a library, or -1 to take the same reads out again
  * (coverage, stats and length counts all return to their previous values),
@@ -142,28 +142,6 @@ int rt_bin_reads_host(rt_ctx* ctx, int32_t* d_cov, int64_t n, const int32_t* h_r
                       const int32_t* h_first, const int32_t* h_last, const uint16_t* h_mlen,
                       const uint16_t* h_flag, const uint8_t* h_mapq, const uint8_t* h_nh,
                       int protocol, int sorted_hint, int64_t* h_stats, int64_t* h_len_counts);
-
-/*
- * ---- K1 on PACKED read records: 11 B/read over PCIe instead of 18.  `first`, `last`, `mlen` are the
- * columns above; `meta` (u8) replaces flag, mapq and nh -- bits 0-2 hold the outcome of the filter
- * cascade (bam.py:77-91 + common.py:33-69), decided on the host: 0 = passed, else RT_ST_QCFAIL ..
- * RT_ST_MULTI; bit 3 = is_reverse -- and ref_id is run-length coded: reads [run_start[r],
- * run_start[r+1]) belong to reference run_ref[r] (a coordinate-sorted BAM has one run per reference).
- * rt_pack_read_meta builds meta and the run table from the columns (RT_ESTATE if there are more than
- * run_cap runs: the input is not grouped by reference, use rt_bin_reads_host).  Results are identical
- * to rt_bin_reads on the same reads.  `read_base` = number of the launch's first read in the run table.
- */
-int rt_pack_read_meta(int64_t n, const int32_t* h_ref_id, const uint16_t* h_flag, const uint8_t* h_mapq,
-                      const uint8_t* h_nh, uint8_t* h_meta, int64_t run_cap, int64_t* h_run_start /* run_cap+1 */,
-                      int32_t* h_run_ref /* run_cap */, int64_t* n_runs);
-int rt_bin_reads_packed(rt_ctx* ctx, int32_t* d_cov, int64_t n, const int32_t* d_first, const int32_t* d_last,
-                        const uint16_t* d_mlen, const uint8_t* d_meta, int64_t read_base, int64_t n_runs,
-                        const int64_t* d_run_start, const int32_t* d_run_ref, int protocol, int weight,
-                        int64_t* d_stats, int64_t* d_len_counts, void* stream);
-int rt_bin_reads_packed_host(rt_ctx* ctx, int32_t* d_cov, int64_t n, const int32_t* h_first, const int32_t* h_last,
-                             const uint16_t* h_mlen, const uint8_t* h_meta, int64_t n_runs,
-                             const int64_t* h_run_start, const int32_t* h_run_ref, int protocol,
-                             int64_t* h_stats, int64_t* h_len_counts);
 
 /*
  * ---- K1 on a RECORD STREAM: a coordinate-sorted library as 4-byte delta-coded records (a quarter of the 18 B/read
@@ -379,9 +357,6 @@ int rt_bam_copy(const rt_bam* b, int32_t* ref_id, int32_t* first, int32_t* last,
 /* reference_start / reference_end of every record as infer_protocol.py:84-85 reads them (host-side protocol
  * inference only; ref_end = -1 where pysam gives None: unmapped flag or no CIGAR) */
 int rt_bam_copy_span(const rt_bam* b, int32_t* pos, int32_t* ref_end);
-/* the decoded reads as packed records (rt_pack_read_meta on the decoder's own columns): meta[n_reads] and the
- * run table; first / last / mlen come from rt_bam_copy */
-int rt_bam_pack(const rt_bam* b, uint8_t* meta, int64_t run_cap, int64_t* run_start, int32_t* run_ref, int64_t* n_runs);
 /* the decoded reads as a record stream (rt_stream_pack on the decoder's own columns; same arguments, same two-call
  * pattern: records == NULL counts the blocks).  RT_ESTATE when the BAM is not coordinate-sorted after all */
 int rt_bam_stream(const rt_bam* b, int n_threads, int64_t cap_blocks, uint32_t* records, int32_t* hdr, int64_t* n_blocks);
@@ -464,7 +439,7 @@ int rt_orf_fetch(rt_ctx* ctx, int32_t* row_tx, int32_t* row_start, int32_t* row_
 
 /* number of kernel launches issued through this ctx so far (bench.py's gpu_launches) */
 int64_t rt_launch_count(const rt_ctx* ctx);
-/* bytes of read data the host-buffer entry points (rt_bin_reads_host, rt_bin_stream_host, rt_bin_reads_packed_host) have
+/* bytes of read data the host-buffer entry points (rt_bin_reads_host, rt_bin_stream_host) have
  * copied to the device through this ctx so far (bench.py's e2e.h2d_bytes_per_step) */
 int64_t rt_h2d_bytes(const rt_ctx* ctx);
 

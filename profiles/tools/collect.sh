@@ -18,6 +18,6 @@ ncu --set full --import-source on --clock-control none -k regex:"bin_stream|atom
 python profiles/e2e_detect_orfs.py > $out/${tag}_e2e_detect_orfs.json 2> $out/${tag}_e2e_detect_orfs.err
 python profiles/e2e_probe.py > $out/${tag}_e2e_probe.txt 2>&1
 python profiles/tools/k1_time.py > $out/${tag}_k1_fresh_vs_red.txt 2>&1
-compute-sanitizer --tool memcheck python -m pytest tests/test_gpu_parity.py -x -q -m gpu -k "stream or edge or packed or golden_pipeline or sparse_clear" > $out/${tag}_sanitizer_memcheck.log 2>&1; tail -3 $out/${tag}_sanitizer_memcheck.log
+compute-sanitizer --tool memcheck python -m pytest tests/test_gpu_parity.py -x -q -m gpu -k "stream or edge or golden_pipeline or sparse_clear" > $out/${tag}_sanitizer_memcheck.log 2>&1; tail -3 $out/${tag}_sanitizer_memcheck.log
 compute-sanitizer --tool racecheck python -m pytest tests/test_gpu_parity.py -x -q -m gpu -k "stream or edge_cases_compact" > $out/${tag}_sanitizer_racecheck.log 2>&1; tail -3 $out/${tag}_sanitizer_racecheck.log
 ls $out | grep ${tag}_

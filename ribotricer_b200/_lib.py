@@ -23,13 +23,13 @@ RT_STREAM_BLOCK = 256
 EXPORTS = (
     "rt_abi_version", "rt_last_error", "rt_create", "rt_destroy", "rt_device_count",
     "rt_set_genome", "rt_plane_elems", "rt_get_contig_base", "rt_set_length_table",
-    "rt_bin_reads", "rt_bin_reads_host", "rt_pack_read_meta", "rt_bin_reads_packed", "rt_bin_reads_packed_host", "rt_stream_pack", "rt_bin_stream", "rt_bin_stream_host", "rt_bin_stream_fresh", "rt_clear_coverage", "rt_set_layout", "rt_coverage_elems", "rt_track_touched", "rt_clear_touched", "rt_set_index", "rt_index_orfs",
+    "rt_bin_reads", "rt_bin_reads_host", "rt_stream_pack", "rt_bin_stream", "rt_bin_stream_host", "rt_bin_stream_fresh", "rt_clear_coverage", "rt_set_layout", "rt_coverage_elems", "rt_track_touched", "rt_clear_touched", "rt_set_index", "rt_index_orfs",
     "rt_index_score_bytes", "rt_index_total_nt", "rt_shard_bounds", "rt_score", "rt_score_host",
     "rt_gather_profiles", "rt_compact_from_dense", "rt_wig_tiles", "rt_wig_count", "rt_wig_fill", "rt_interval_sums", "rt_bootstrap_medians", "rt_launch_count", "rt_h2d_bytes", "rt_phasescore_values", "rt_io_last_error", "rt_index_load",
     "rt_index_free", "rt_index_n_orf", "rt_index_n_exon", "rt_index_n_annotated_prefix", "rt_index_n_chrom",
     "rt_index_chrom_name", "rt_index_copy", "rt_index_field", "rt_tsv_open", "rt_tsv_write", "rt_tsv_close",
     "rt_repr_double", "rt_wig_open", "rt_wig_block", "rt_wig_close", "rt_bam_last_error", "rt_bam_load", "rt_bam_free", "rt_bam_n_reads", "rt_bam_n_ref",
-    "rt_bam_ref_name", "rt_bam_ref_len", "rt_bam_sorted", "rt_bam_copy", "rt_bam_copy_span", "rt_bam_pack", "rt_bam_stream",
+    "rt_bam_ref_name", "rt_bam_ref_len", "rt_bam_sorted", "rt_bam_copy", "rt_bam_copy_span", "rt_bam_stream",
     "rt_inflate_raw", "rt_crc32", "rt_metagene_sums",
     "rt_gtf_load", "rt_gtf_free", "rt_gtf_n_lines", "rt_gtf_n_strings", "rt_gtf_string_bytes", "rt_gtf_copy",
     "rt_fasta_load", "rt_fasta_free", "rt_fasta_n_contig", "rt_fasta_contig_name", "rt_fasta_contig_len", "rt_fasta_codes",
@@ -88,9 +88,6 @@ def load():
     lib.rt_set_length_table.argtypes = [vp, vp]
     lib.rt_bin_reads.argtypes = [vp, vp, i64, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, vp, vp, vp]
     lib.rt_bin_reads_host.argtypes = [vp, vp, i64, vp, vp, vp, vp, vp, vp, vp, i32, i32, vp, vp]
-    lib.rt_pack_read_meta.argtypes = [i64, vp, vp, vp, vp, vp, i64, vp, vp, C.POINTER(i64)]
-    lib.rt_bin_reads_packed.argtypes = [vp, vp, i64, vp, vp, vp, vp, i64, i64, vp, vp, i32, i32, vp, vp, vp]
-    lib.rt_bin_reads_packed_host.argtypes = [vp, vp, i64, vp, vp, vp, vp, i64, vp, vp, i32, vp, vp]
     lib.rt_stream_pack.argtypes = [i64, vp, vp, vp, vp, vp, vp, vp, i32, i64, vp, vp, C.POINTER(i64)]
     lib.rt_bin_stream.argtypes = [vp, vp, i64, vp, vp, i32, i32, vp, vp, vp]
     lib.rt_bin_stream_host.argtypes = [vp, vp, i64, vp, vp, i32, vp, vp]
@@ -155,7 +152,6 @@ def load():
     lib.rt_bam_sorted.argtypes = [vp]
     lib.rt_bam_copy.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp]
     lib.rt_bam_copy_span.argtypes = [vp, vp, vp]
-    lib.rt_bam_pack.argtypes = [vp, vp, i64, vp, vp, C.POINTER(i64)]
     lib.rt_bam_stream.argtypes = [vp, i32, i64, vp, vp, C.POINTER(i64)]
     lib.rt_inflate_raw.argtypes = [vp, i64, vp, i64]
     lib.rt_metagene_sums.argtypes = [vp, vp, i64, i64, vp, vp, vp, vp]
@@ -183,8 +179,8 @@ def load():
     lib.rt_orf_write.argtypes = [C.c_char_p, i64, vp, vp, vp, i64, vp, vp, vp, vp, vp, vp]
     lib.rt_orf_search.argtypes = [vp, C.POINTER(OrfQuery), C.POINTER(i64), C.POINTER(i64), vp]
     lib.rt_orf_fetch.argtypes = [vp] * 9
-    if lib.rt_abi_version() != 3:
-        raise RtError(f"ABI mismatch: library reports {lib.rt_abi_version()}, binding expects 3")
+    if lib.rt_abi_version() != 4:
+        raise RtError(f"ABI mismatch: library reports {lib.rt_abi_version()}, binding expects 4")
     _lib = lib
     return lib
 

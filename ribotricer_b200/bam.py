@@ -9,7 +9,6 @@ environment, the same columns can also be loaded from a ``.npz`` file
 """
 from __future__ import annotations
 
-import os
 from collections import Counter, defaultdict
 from dataclasses import dataclass
 
@@ -159,7 +158,7 @@ class Alignments:
         self.n = len(reads)
         self.sorted = reads.sorted_by_coordinate
         self.dcols = self.dstream = None
-        if self.sorted and self.n and os.environ.get("RT_READS_FORMAT", "stream") == "stream":
+        if self.sorted and self.n:
             try:
                 self.dstream = engine.upload_stream(engine.stream_reads(reads.cols))
             except _lib.RtError:       # "sorted" in the header, but the positions descend somewhere: plain columns

@@ -5,8 +5,9 @@ The index, its atoms and the compact slot map are set up once and stay on the GP
 ranks of a torchrun job round-robin; inside a rank they run through a three-stage software pipeline:
 
     stage(i)     decode / pack library i on the host, start its host-to-device copy on the copy stream
-    compute(i-1) K1 on the record stream (rt_bin_stream_fresh: overwrites a coverage buffer, no clear), phase A + B, start the device-to-host copy of the
-                 result columns -- all enqueued on the compute stream behind the copy of library i-1
+    compute(i-1) K1 on the record stream (rt_bin_stream_fresh: overwrites a coverage buffer, no clear) or, for a library
+                 that cannot be streamed, a clear and K1 on its read columns; phase A + B, start the device-to-host
+                 copy of the result columns -- all enqueued on the compute stream behind the copy of library i-1
     finalize(i-2) wait for library i-2, write its _bam_summary.txt and its TSV (K4 gathers the profiles of the
                  reported ORFs from the library's coverage buffer, which the pipeline keeps alive until then)
 
@@ -24,7 +25,7 @@ import numpy as np
 from .bam import bam_summary_text, load_reads
 from .const import (CUTOFF, DEFAULT_PAD, MINIMUM_DENSITY_OVER_ORF, MINIMUM_READS_PER_CODON, MINIMUM_VALID_CODONS,
                     MINIMUM_VALID_CODONS_RATIO)
-from .engine import ScoreParams
+from .engine import READ_COLUMNS, ScoreParams
 
 
 class LibraryPipeline:
@@ -57,13 +58,8 @@ class LibraryPipeline:
                 ev = t.cuda.Event()
                 ev.record(self.copy_stream)
                 return dict(tag=tag, dev=dev, copied=ev, keep=packed)
-            for k in ("first", "last", "mlen", "meta"):
-                a = packed[k]
-                a = a if hasattr(a, "data_ptr") else t.from_numpy(np.ascontiguousarray(a).view(np.int16) if a.dtype == np.uint16 else np.ascontiguousarray(a))
-                dev[k] = a.to(eng.device, non_blocking=True)
-            dev["run_start"] = t.from_numpy(np.ascontiguousarray(packed["run_start"])).to(eng.device, non_blocking=True)
-            dev["run_ref"] = t.from_numpy(np.ascontiguousarray(packed["run_ref"])).to(eng.device, non_blocking=True)
-            dev["n"] = int(packed["n"])
+            for name, _ in READ_COLUMNS:   # the read columns of _host_records: 18 B/read
+                dev[name] = packed[name].to(eng.device, non_blocking=True)
             ev = t.cuda.Event()
             ev.record(self.copy_stream)
         return dict(tag=tag, dev=dev, copied=ev, keep=packed)
@@ -81,7 +77,7 @@ class LibraryPipeline:
                 eng.bin_stream_device(cov, job["dev"], self.protocol, stats, len_counts, fresh=True)
             else:
                 eng.clear_coverage(cov)
-                eng.bin_reads_packed_device(cov, job["dev"], self.protocol, stats, len_counts)
+                eng.bin_reads_device(cov, job["dev"], self.protocol, stats, len_counts)
             out = eng.new_score_columns(n_orf, min_codon=self.want_min)
             eng.score_device(cov, out, 0, n_orf, self.params)
             if self._host_cols[slot] is None:
@@ -118,7 +114,8 @@ class LibraryPipeline:
     # -- driver ------------------------------------------------------------------------------------------------
     def submit(self, tag, packed):
         """``packed``: what ``Engine.stream_reads(cols, pinned=True)`` (a coordinate-sorted library as 4 B/read records)
-        or ``Engine.pack_reads(cols, pinned=True)`` (11 B/read, any order grouped by reference) returns for one library."""
+        returns for one library, or its seven read columns as page-locked tensors (18 B/read, any order; 16-bit
+        columns viewed as int16), as ``_host_records`` makes them."""
         nxt = self._stage(tag, packed)
         run = self._compute(self._staged) if self._staged is not None else None
         if self._running is not None:
@@ -137,7 +134,7 @@ class LibraryPipeline:
 
 def _host_records(eng, reads):
     """The library as page-locked host records: the 4 B/read record stream when it is coordinate-sorted (and codes),
-    else the 11 B/read packed records."""
+    else its 18 B/read columns."""
     from ._lib import RtError
 
     if reads.sorted_by_coordinate:
@@ -145,7 +142,13 @@ def _host_records(eng, reads):
             return eng.stream_reads(reads.cols, pinned=True)
         except RtError:
             pass
-    return eng.pack_reads(reads.cols, pinned=True, max_runs=max(64, len(reads) + 1) if not reads.sorted_by_coordinate else None)
+    t = eng.torch
+    cols = {}
+    for name, dt in READ_COLUMNS:
+        a = np.ascontiguousarray(reads.cols[name], dtype=dt)
+        # torch has no uint16 arithmetic but can hold the bytes; view as int16 for transport, as Engine.upload_reads does
+        cols[name] = t.from_numpy(a.view(np.int16) if dt == np.uint16 else a).pin_memory()
+    return cols
 
 
 def detect_orfs_batch(bams, ribotricer_index: str, prefixes, protocol: str, read_lengths, psite_offsets: dict,

@@ -540,12 +540,6 @@ int rt_bam_copy_span(const rt_bam* b, int32_t* pos, int32_t* ref_end) {
     return RT_OK;
 }
 
-int rt_bam_pack(const rt_bam* b, uint8_t* meta, int64_t run_cap, int64_t* run_start, int32_t* run_ref, int64_t* n_runs) {
-    if (!b) return RT_EINVAL;
-    return rt_pack_read_meta((int64_t)b->ref_id.size(), b->ref_id.data(), b->flag.data(), b->mapq.data(), b->nh.data(),
-                             meta, run_cap, run_start, run_ref, n_runs);
-}
-
 int rt_bam_stream(const rt_bam* b, int n_threads, int64_t cap_blocks, uint32_t* records, int32_t* hdr, int64_t* n_blocks) {
     if (!b) return RT_EINVAL;
     return rt_stream_pack((int64_t)b->ref_id.size(), b->ref_id.data(), b->first.data(), b->last.data(), b->mlen.data(), b->flag.data(),

@@ -15,9 +15,6 @@
 
 #include "rt_kernels.cuh"
 
-// rt_host_io.cpp: filter cascade + run-length code of ref_id for one chunk of host columns
-int64_t rt_pack_chunk(const int32_t* ref_id, const uint16_t* flag, const uint8_t* mapq, const uint8_t* nh, int64_t m, uint8_t* meta,
-                      int64_t* run_start, int32_t* run_ref, int64_t cap);
 // rt_host_io.cpp: one chunk of host columns as a run of record-stream blocks (-1: cannot be coded, -2: cap too small)
 int64_t rt_stream_pack_range(const int32_t* ref_id, const int32_t* first, const int32_t* last, const uint16_t* mlen, const uint16_t* flag,
                              const uint8_t* mapq, const uint8_t* nh, int64_t m, uint32_t* rec, int32_t* hdr, int64_t cap);
@@ -334,7 +331,6 @@ void free_plan(rt_ctx::ScorePlan& p) {
 }
 
 constexpr size_t kReadBytes = 4 + 4 + 4 + 2 + 2 + 1 + 1;
-constexpr size_t kPackedReadBytes = 4 + 4 + 2 + 1;
 constexpr int64_t kHostChunkReads = 4 << 20;
 constexpr int64_t kPackChunkReads = 1 << 20;      // reads per chunk of the packing pipelines
 // stream blocks a chunk may fill: 1.5 records per read (every second read spliced or far from its neighbour) + slack;
@@ -599,8 +595,8 @@ int rt_clear_touched(rt_ctx* ctx, int32_t* d_cov, void* stream) {
 
 namespace {
 
-// Common part of rt_bin_reads / rt_bin_reads_packed: `a` arrives with its read columns filled in.
-int launch_bin(rt_ctx* ctx, const char* who, rt::BinArgs& a, bool packed, int32_t* d_cov, int64_t n, int protocol,
+// Checks and launch of rt_bin_reads: `a` arrives with its read columns filled in.
+int launch_bin(rt_ctx* ctx, const char* who, rt::BinArgs& a, int32_t* d_cov, int64_t n, int protocol,
                int weight, int64_t* d_stats, int64_t* d_len_counts, void* stream) {
     if (weight != 1 && weight != -1) return fail(ctx, RT_EINVAL, "%s: weight must be +1 or -1", who);
     if (ctx->plane == 0) return fail(ctx, RT_ESTATE, "%s: call rt_set_genome first", who);
@@ -635,13 +631,8 @@ int launch_bin(rt_ctx* ctx, const char* who, rt::BinArgs& a, bool packed, int32_
     const int64_t blocks = (n + per_block - 1) / per_block;
     if (blocks > 0x7fffffff) return fail(ctx, RT_EINVAL, "%s: n too large for one launch", who);
     cudaStream_t st = (cudaStream_t)stream;
-    if (packed) {
-        if (a.cmap) rt::bin_psites_kernel<true, true><<<(unsigned)blocks, rt::kBinThreads, 0, st>>>(a);
-        else rt::bin_psites_kernel<false, true><<<(unsigned)blocks, rt::kBinThreads, 0, st>>>(a);
-    } else {
-        if (a.cmap) rt::bin_psites_kernel<true, false><<<(unsigned)blocks, rt::kBinThreads, 0, st>>>(a);
-        else rt::bin_psites_kernel<false, false><<<(unsigned)blocks, rt::kBinThreads, 0, st>>>(a);
-    }
+    if (a.cmap) rt::bin_psites_kernel<true><<<(unsigned)blocks, rt::kBinThreads, 0, st>>>(a);
+    else rt::bin_psites_kernel<false><<<(unsigned)blocks, rt::kBinThreads, 0, st>>>(a);
     ctx->launches++;
     RT_CUDA(ctx, cudaGetLastError());
     return RT_OK;
@@ -662,24 +653,7 @@ int rt_bin_reads(rt_ctx* ctx, int32_t* d_cov, int64_t n, const int32_t* d_ref_id
     rt::BinArgs a{};
     a.ref_id = d_ref_id; a.first = d_first; a.last = d_last; a.mlen = d_mlen; a.flag = d_flag;
     a.mapq = d_mapq; a.nh = d_nh;
-    return launch_bin(ctx, "rt_bin_reads", a, false, d_cov, n, protocol, weight, d_stats, d_len_counts, stream);
-}
-
-int rt_bin_reads_packed(rt_ctx* ctx, int32_t* d_cov, int64_t n, const int32_t* d_first, const int32_t* d_last,
-                        const uint16_t* d_mlen, const uint8_t* d_meta, int64_t read_base, int64_t n_runs,
-                        const int64_t* d_run_start, const int32_t* d_run_ref, int protocol, int weight,
-                        int64_t* d_stats, int64_t* d_len_counts, void* stream) {
-    if (!ctx) return fail(nullptr, RT_EINVAL, "rt_bin_reads_packed: ctx is NULL");
-    if (n > 0 && (!d_first || !d_last || !d_mlen || !d_meta || !d_run_start || !d_run_ref || n_runs < 1 ||
-                  n_runs > 0x7fffffff || read_base < 0))
-        return fail(ctx, RT_EINVAL, "rt_bin_reads_packed: NULL column or empty run table");
-    rt::BinArgs a{};
-    a.first = d_first; a.last = d_last; a.mlen = d_mlen; a.meta = d_meta;
-    a.run_start = reinterpret_cast<const long long*>(d_run_start);
-    a.run_ref = d_run_ref;
-    a.n_runs = (int)n_runs;
-    a.read_base = read_base;
-    return launch_bin(ctx, "rt_bin_reads_packed", a, true, d_cov, n, protocol, weight, d_stats, d_len_counts, stream);
+    return launch_bin(ctx, "rt_bin_reads", a, d_cov, n, protocol, weight, d_stats, d_len_counts, stream);
 }
 
 static int launch_stream(rt_ctx* ctx, const char* who, bool fresh, int32_t* d_cov, int64_t n_blocks, const uint32_t* d_records,
@@ -720,7 +694,7 @@ static int launch_stream(rt_ctx* ctx, const char* who, bool fresh, int32_t* d_co
     a.stats = reinterpret_cast<unsigned long long*>(d_stats);
     a.len_counts = reinterpret_cast<unsigned long long*>(d_len_counts);
     // persistent: a few CTAs per SM; every warp walks blocks with the next one in flight (cp.async.bulk)
-    const unsigned grid = (unsigned)std::min<int64_t>((n_blocks + rt::kStreamWarps - 1) / rt::kStreamWarps, (int64_t)ctx->n_sm * RT_STREAM_CTAS_PER_SM);
+    const unsigned grid = (unsigned)std::min<int64_t>((n_blocks + rt::kStreamWarps - 1) / rt::kStreamWarps, (int64_t)ctx->n_sm * rt::kStreamCtasPerSm);
     if (fresh) {
         // zone boundaries of the blocks (rank of the first position a read of the block can reach), made monotone
         const int64_t tiles = (n_blocks + 1 + rt::kZoneTile - 1) / rt::kZoneTile;
@@ -839,9 +813,7 @@ int rt_bin_reads_host(rt_ctx* ctx, int32_t* d_cov, int64_t n, const int32_t* h_r
     // into their own page-locked staging slot, start the copy on their own stream and launch K1 behind it -- so the
     // coding of some chunks, the copies of others and the kernels of yet others overlap.  A chunk that cannot be coded
     // (positions descend: not sorted after all) is sent as plain columns.
-    int64_t pack_chunk_reads = kPackChunkReads;
-    if (const char* e = getenv("RT_PACK_CHUNK")) pack_chunk_reads = std::min<int64_t>(kPackChunkReads, std::max(1 << 16, atoi(e)));
-    const int64_t chunk = use_stream ? std::min<int64_t>(pack_chunk_reads, std::max<int64_t>(n, 1))
+    const int64_t chunk = use_stream ? std::min<int64_t>(kPackChunkReads, std::max<int64_t>(n, 1))
                                       : std::min<int64_t>(kHostChunkReads, std::max<int64_t>(n, 1));
     const int64_t n_chunks = (n + chunk - 1) / chunk;
     // the delta coding is the bottleneck of this call (about 1.5 ns per read and thread): one pipeline per hardware thread
@@ -956,61 +928,6 @@ int rt_bin_reads_host(rt_ctx* ctx, int32_t* d_cov, int64_t n, const int32_t* h_r
                         "enqueueing %.2f\n", (long long)n, n_pipes, (long long)chunk, ms(t_issued - t_begin), ms(std::chrono::steady_clock::now() - t_issued),
                 pack_ns.load() / 1e6, wait_ns.load() / 1e6, issue_ns.load() / 1e6);
     }
-    RT_CUDA(ctx, cudaMemcpy(h_stats, d_stats, sizeof(int64_t) * RT_N_STATS, cudaMemcpyDeviceToHost));
-    RT_CUDA(ctx, cudaMemcpy(h_len_counts, d_len_counts, sizeof(int64_t) * RT_LEN_TABLE, cudaMemcpyDeviceToHost));
-    return RT_OK;
-}
-
-int rt_bin_reads_packed_host(rt_ctx* ctx, int32_t* d_cov, int64_t n, const int32_t* h_first, const int32_t* h_last,
-                             const uint16_t* h_mlen, const uint8_t* h_meta, int64_t n_runs, const int64_t* h_run_start,
-                             const int32_t* h_run_ref, int protocol, int64_t* h_stats, int64_t* h_len_counts) {
-    if (!ctx) return fail(nullptr, RT_EINVAL, "rt_bin_reads_packed_host: ctx is NULL");
-    if (!h_stats || !h_len_counts) return fail(ctx, RT_EINVAL, "rt_bin_reads_packed_host: NULL output");
-    if (n > 0 && (n_runs < 1 || !h_run_start || !h_run_ref || h_run_start[0] != 0 || h_run_start[n_runs] != n))
-        return fail(ctx, RT_EINVAL, "rt_bin_reads_packed_host: the run table must cover reads [0, n)");
-    DeviceGuard guard(ctx->device);
-    const size_t acc_bytes = sizeof(int64_t) * (RT_N_STATS + RT_LEN_TABLE);
-    const size_t run_bytes = n > 0 ? sizeof(int64_t) * (size_t)(n_runs + 1) + sizeof(int32_t) * (size_t)n_runs : 0;
-    RT_CUDA(ctx, ctx->stats_buf.reserve(acc_bytes + run_bytes + 16));
-    int64_t* d_stats = static_cast<int64_t*>(ctx->stats_buf.p);
-    int64_t* d_len_counts = d_stats + RT_N_STATS;
-    int64_t* d_run_start = d_len_counts + RT_LEN_TABLE;
-    int32_t* d_run_ref = reinterpret_cast<int32_t*>(d_run_start + (n > 0 ? n_runs + 1 : 0));
-    for (int s = 0; s < 2; ++s)
-        if (!ctx->slot_stream[s]) RT_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->slot_stream[s], cudaStreamNonBlocking));
-    RT_CUDA(ctx, cudaMemsetAsync(d_stats, 0, acc_bytes, ctx->slot_stream[0]));
-    if (n > 0) {
-        RT_CUDA(ctx, cudaMemcpyAsync(d_run_start, h_run_start, sizeof(int64_t) * (size_t)(n_runs + 1), cudaMemcpyHostToDevice, ctx->slot_stream[0]));
-        RT_CUDA(ctx, cudaMemcpyAsync(d_run_ref, h_run_ref, sizeof(int32_t) * (size_t)n_runs, cudaMemcpyHostToDevice, ctx->slot_stream[0]));
-    }
-    RT_CUDA(ctx, cudaStreamSynchronize(ctx->slot_stream[0]));
-    if (ctx->track_touched && ctx->layout != RT_LAYOUT_COMPACT) {
-        int rc = ensure_touched_capacity(ctx, ctx->touched_reserved + n);
-        if (rc != RT_OK) return rc;
-    }
-    const int64_t chunk = std::min<int64_t>(kHostChunkReads, std::max<int64_t>(n, 1));
-    const size_t slot_bytes = (size_t)chunk * kPackedReadBytes + 64;
-    int slot = 0;
-    for (int64_t at = 0; at < n; at += chunk, slot ^= 1) {
-        const int64_t m = std::min(chunk, n - at);
-        RT_CUDA(ctx, ctx->read_slot[slot].reserve(slot_bytes));
-        char* base = static_cast<char*>(ctx->read_slot[slot].p);
-        int32_t* d_first = reinterpret_cast<int32_t*>(base);
-        int32_t* d_last = d_first + chunk;
-        uint16_t* d_mlen = reinterpret_cast<uint16_t*>(d_last + chunk);
-        uint8_t* d_meta = reinterpret_cast<uint8_t*>(d_mlen + chunk);
-        cudaStream_t st = ctx->slot_stream[slot];   // stream order protects the slot's previous use
-        RT_CUDA(ctx, cudaMemcpyAsync(d_first, h_first + at, 4 * m, cudaMemcpyHostToDevice, st));
-        RT_CUDA(ctx, cudaMemcpyAsync(d_last, h_last + at, 4 * m, cudaMemcpyHostToDevice, st));
-        RT_CUDA(ctx, cudaMemcpyAsync(d_mlen, h_mlen + at, 2 * m, cudaMemcpyHostToDevice, st));
-        RT_CUDA(ctx, cudaMemcpyAsync(d_meta, h_meta + at, m, cudaMemcpyHostToDevice, st));
-        ctx->h2d_bytes += (int64_t)m * (int64_t)kPackedReadBytes;
-        int rc = rt_bin_reads_packed(ctx, d_cov, m, d_first, d_last, d_mlen, d_meta, at, n_runs, d_run_start, d_run_ref,
-                                     protocol, 1, d_stats, d_len_counts, st);
-        if (rc != RT_OK) return rc;
-    }
-    RT_CUDA(ctx, cudaStreamSynchronize(ctx->slot_stream[0]));
-    RT_CUDA(ctx, cudaStreamSynchronize(ctx->slot_stream[1]));
     RT_CUDA(ctx, cudaMemcpy(h_stats, d_stats, sizeof(int64_t) * RT_N_STATS, cudaMemcpyDeviceToHost));
     RT_CUDA(ctx, cudaMemcpy(h_len_counts, d_len_counts, sizeof(int64_t) * RT_LEN_TABLE, cudaMemcpyDeviceToHost));
     return RT_OK;

@@ -756,95 +756,6 @@ int rt_wig_close(rt_tsv* t) { return rt_tsv_close(t); }
 
 }  // extern "C"
 
-// ---- packed read records (11 B/read instead of 18): the filter cascade is decided here, on the host ----
-#include <thread>
-
-// bam.py:77-91 + common.py:33-69 for reads [0, m) of a chunk (same order as classify_read() in rt_kernels.cuh: the
-// EARLIER test wins, so the selects run from the last test to the first) and the run-length code of ref_id.  One
-// thread; branch-free and in blocks so that the compiler vectorises both loops (an AVX2 clone is picked at load time).
-// Returns the number of runs, or -1 when there are more than `cap` (the chunk is not grouped by reference).
-#if defined(__x86_64__) && defined(__GNUC__) && !defined(__clang__)
-__attribute__((target_clones("avx2", "default")))
-#endif
-int64_t rt_pack_chunk(const int32_t* __restrict__ ref_id, const uint16_t* __restrict__ flag, const uint8_t* __restrict__ mapq,
-                      const uint8_t* __restrict__ nh, int64_t m, uint8_t* __restrict__ meta, int64_t* run_start, int32_t* run_ref,
-                      int64_t cap) {
-    for (int64_t i = 0; i < m; ++i) {
-        const unsigned f = flag[i];
-        const unsigned nn = nh[i], qq = mapq[i];             // both loaded unconditionally: no control flow, the loop vectorises
-        const unsigned uniq = (nn == 1u) | ((nn == 0u) & (qq == 255u));
-        unsigned code = uniq ? 0u : (unsigned)RT_ST_MULTI;
-        code = (f & 0x4) ? (unsigned)RT_ST_UNMAPPED : code;
-        code = (f & 0x100) ? (unsigned)RT_ST_SECONDARY : code;
-        code = (f & 0x400) ? (unsigned)RT_ST_DUPLICATE : code;
-        code = (f & 0x200) ? (unsigned)RT_ST_QCFAIL : code;
-        meta[i] = (uint8_t)(code | ((f >> 1) & 8u));
-    }
-    int64_t r = 0;
-    if (m > 0) {
-        run_start[0] = 0;
-        run_ref[0] = ref_id[0];
-        r = 1;
-    }
-    constexpr int64_t kBlock = 256;
-    for (int64_t b = 1; b < m; b += kBlock) {
-        const int64_t e = b + kBlock < m ? b + kBlock : m;
-        int32_t diff = 0;
-        for (int64_t i = b; i < e; ++i) diff |= ref_id[i] ^ ref_id[i - 1];
-        if (diff == 0) continue;                    // the usual case: no reference changes inside the block
-        for (int64_t i = b; i < e; ++i)
-            if (ref_id[i] != ref_id[i - 1]) {
-                if (r >= cap) return -1;
-                run_start[r] = i;
-                run_ref[r] = ref_id[i];
-                ++r;
-            }
-    }
-    run_start[r] = m;
-    return r;
-}
-
-extern "C" {
-
-int rt_pack_read_meta(int64_t n, const int32_t* ref_id, const uint16_t* flag, const uint8_t* mapq, const uint8_t* nh,
-                      uint8_t* meta, int64_t run_cap, int64_t* run_start, int32_t* run_ref, int64_t* n_runs) {
-    if (n < 0 || !n_runs || (n > 0 && (!ref_id || !flag || !mapq || !nh || !meta || !run_start || !run_ref)))
-        return RT_EINVAL;
-    // bam.py:77-91 + common.py:33-69, same order as classify_read() in rt_kernels.cuh
-    auto work = [&](int64_t a, int64_t b) {
-        for (int64_t i = a; i < b; ++i) {
-            const unsigned f = flag[i];
-            unsigned code;
-            if (f & 0x200) code = RT_ST_QCFAIL;
-            else if (f & 0x400) code = RT_ST_DUPLICATE;
-            else if (f & 0x100) code = RT_ST_SECONDARY;
-            else if (f & 0x4) code = RT_ST_UNMAPPED;
-            else code = (nh[i] != 0 ? nh[i] == 1 : mapq[i] == 255) ? 0u : (unsigned)RT_ST_MULTI;
-            meta[i] = (uint8_t)(code | ((f & 0x10) ? 8u : 0u));
-        }
-    };
-    const int n_thr = (int)std::max<int64_t>(1, std::min<int64_t>(std::thread::hardware_concurrency(), n / (1 << 20)));
-    std::vector<std::thread> pool;
-    for (int t = 0; t < n_thr; ++t) pool.emplace_back(work, n * t / n_thr, n * (t + 1) / n_thr);
-    for (auto& th : pool) th.join();
-    int64_t r = 0;
-    for (int64_t i = 0; i < n; ++i)
-        if (i == 0 || ref_id[i] != ref_id[i - 1]) {
-            if (r >= run_cap) {
-                g_io_error = "rt_pack_read_meta: more reference runs than run_cap (input not grouped by reference?)";
-                return RT_ESTATE;
-            }
-            run_start[r] = i;
-            run_ref[r] = ref_id[i];
-            ++r;
-        }
-    if (n > 0) run_start[r] = n;
-    *n_runs = r;
-    return RT_OK;
-}
-
-}  // extern "C"
-
 // ---- record stream (4 B/read, format in ribotricer_b200.h): delta code of a coordinate-sorted library ----
 namespace {
 
@@ -943,13 +854,10 @@ int64_t rt_stream_pack_range(const int32_t* __restrict__ ref_id, const int32_t* 
     int64_t cur_pos = m > 0 ? first[0] : 0;
     int64_t i = 0;
     // A core streams only ~12 GB/s through its L1 miss buffers; prefetches into L2 run ahead of them (measured on the
-    // GPU box: 10 % off the coding time at 512 reads, nothing more further out).  RT_PACK_PREFETCH overrides, 0 = off.
-    static const int64_t ahead_reads = [] {
-        const char* e = getenv("RT_PACK_PREFETCH");
-        return e ? (int64_t)atoll(e) : (int64_t)512;
-    }();
+    // GPU box: 10 % off the coding time at 512 reads, nothing more further out).
+    constexpr int64_t ahead_reads = 512;
     while (i < m) {
-        if (ahead_reads > 0 && i + ahead_reads + kStreamGroup <= m) {   // one 64-read group of every column, `ahead_reads` further on
+        if (i + ahead_reads + kStreamGroup <= m) {   // one 64-read group of every column, `ahead_reads` further on
             const int64_t a = i + ahead_reads;
             for (int k = 0; k < 4; ++k) {
                 __builtin_prefetch(ref_id + a + 16 * k, 0, 2);

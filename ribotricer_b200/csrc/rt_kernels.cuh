@@ -67,11 +67,7 @@ __device__ __forceinline__ float rsqrt_approx(float x) {
     return r;
 }
 
-#ifdef RT_PLAIN_LD
-__device__ __forceinline__ int ld_cov(const int32_t* p) { return *p; }
-#else
 __device__ __forceinline__ int ld_cov(const int32_t* p) { return __ldg(p); }
-#endif
 
 // Per-lane accumulators of one frame.  w1 / w2 pack 10-bit counters and are flushed into the
 // warp-uniform totals every kFlushTiles tiles; the fp64 sums live for the whole ORF.
@@ -1474,13 +1470,6 @@ struct BinArgs {
     const uint16_t* flag;
     const uint8_t* mapq;
     const uint8_t* nh;
-    // packed records (Packed = true): `meta` replaces flag/mapq/nh (bits 0-2: RT_ST_QCFAIL..RT_ST_MULTI decided on the
-    // host, 0 = passed the cascade; bit 3: is_reverse) and ref_id is run-length coded over GLOBAL read numbers
-    const uint8_t* meta;
-    const long long* run_start;    // n_runs + 1
-    const int32_t* run_ref;        // n_runs
-    int n_runs;
-    long long read_base;           // global number of this launch's first read
     long long n;
     int protocol;
     int weight;                    // +1 bin, -1 un-bin
@@ -1498,14 +1487,8 @@ struct BinArgs {
     unsigned long long* len_counts;  // RT_LEN_TABLE
 };
 
-#ifndef RT_BIN_BATCH
-#define RT_BIN_BATCH 4
-#endif
 constexpr int kBinThreads = 256;
-#ifndef RT_BIN_RPT
-#define RT_BIN_RPT 8
-#endif
-constexpr int kBinReadsPerThread = RT_BIN_RPT;
+constexpr int kBinReadsPerThread = 8;
 constexpr int kLenHist = 512;   // read lengths below this are histogrammed in shared memory
 
 // Category of one read after the cascade of bam.py:77-91: one of RT_ST_QCFAIL .. RT_ST_VALID.
@@ -1532,25 +1515,13 @@ __device__ __forceinline__ int classify_read(unsigned fl, unsigned mapq, unsigne
     return cat ? cat : (uniq ? RT_ST_VALID : RT_ST_MULTI);
 }
 
-template <bool Compact, bool Packed>
+template <bool Compact>
 __global__ void __launch_bounds__(kBinThreads) bin_psites_kernel(const BinArgs a) {
     __shared__ unsigned int s_stats[RT_N_STATS];
     __shared__ unsigned int s_len[kLenHist];
     __shared__ unsigned long long s_touch[Compact ? 1 : kBinThreads * kBinReadsPerThread];
     __shared__ unsigned int s_ntouch;
     __shared__ unsigned long long s_touch_base;
-    __shared__ int s_run;          // Packed: run of the block's first read, and whether the block sits inside it
-    __shared__ int s_one_run;
-    if (Packed && threadIdx.x == 0) {
-        const long long g0 = a.read_base + (long long)blockIdx.x * (kBinThreads * kBinReadsPerThread);
-        int lo = 0, hi = a.n_runs - 1;                       // last run with run_start <= g0
-        while (lo < hi) {
-            const int mid = (lo + hi + 1) >> 1;
-            if (a.run_start[mid] <= g0) lo = mid; else hi = mid - 1;
-        }
-        s_run = lo;
-        s_one_run = g0 + kBinThreads * kBinReadsPerThread <= a.run_start[lo + 1];
-    }
     if (threadIdx.x == 0) s_ntouch = 0;
     for (int i = threadIdx.x; i < kLenHist; i += kBinThreads) s_len[i] = 0;
     if (threadIdx.x < RT_N_STATS) s_stats[threadIdx.x] = 0;
@@ -1563,10 +1534,7 @@ __global__ void __launch_bounds__(kBinThreads) bin_psites_kernel(const BinArgs a
     // per-thread 4-bit counters of categories RT_ST_QCFAIL..RT_ST_BADREF (<= 8 reads per thread)
     unsigned packed = 0;
     unsigned long long len_packed = 0;
-#ifdef RT_BIN_NO_RED
-    unsigned long long sink = 0;
-#endif
-    constexpr int kBatch = RT_BIN_BATCH;     // reads per thread whose columns are in flight together
+    constexpr int kBatch = 4;                // reads per thread whose columns are in flight together
 #pragma unroll 1
     for (int it0 = 0; it0 < kBinReadsPerThread; it0 += kBatch) {
         // ---- all column loads of the batch first (7 x kBatch independent, coalesced loads) ----
@@ -1576,16 +1544,10 @@ __global__ void __launch_bounds__(kBinThreads) bin_psites_kernel(const BinArgs a
         for (int j = 0; j < kBatch; ++j) {
             const long long i = block_base + (long long)(it0 + j) * kBinThreads + threadIdx.x;
             const bool in = i < a.n;
-            if (Packed) {
-                fl[j] = in ? a.meta[i] : 0u;
-                mq[j] = nh[j] = 0u;
-                rid[j] = 0;
-            } else {
-                fl[j] = in ? a.flag[i] : 0u;
-                mq[j] = in ? a.mapq[i] : 0u;
-                nh[j] = in ? a.nh[i] : 0u;
-                rid[j] = in ? a.ref_id[i] : 0;
-            }
+            fl[j] = in ? a.flag[i] : 0u;
+            mq[j] = in ? a.mapq[i] : 0u;
+            nh[j] = in ? a.nh[i] : 0u;
+            rid[j] = in ? a.ref_id[i] : 0;
             ml[j] = in ? a.mlen[i] : 0u;
             fi[j] = in ? a.first[i] : 0;
             la[j] = in ? a.last[i] : 0;
@@ -1596,15 +1558,8 @@ __global__ void __launch_bounds__(kBinThreads) bin_psites_kernel(const BinArgs a
             int len = -1;            // >= 0: counts in read_length_counts
             slot_t slot = kNone;     // coverage slot to bump
             if (i < a.n) {
-                int cat;
-                bool rev;
-                if (Packed) {
-                    cat = (fl[j] & 7u) ? (int)(fl[j] & 7u) : RT_ST_VALID;
-                    rev = (fl[j] & 8u) != 0;
-                } else {
-                    cat = classify_read(fl[j], mq[j], nh[j]);
-                    rev = (fl[j] & 0x10) != 0;                      // bam.py:94
-                }
+                int cat = classify_read(fl[j], mq[j], nh[j]);
+                const bool rev = (fl[j] & 0x10) != 0;               // bam.py:94
                 if (cat == RT_ST_VALID) {
                     const int l = (int)ml[j];                       // bam.py:99
                     const int mode = __ldg(a.len_table + l);
@@ -1612,15 +1567,7 @@ __global__ void __launch_bounds__(kBinThreads) bin_psites_kernel(const BinArgs a
                     // reverse protocol swaps the strand and takes the other end (bam.py:118-131)
                     const bool minus = rev == (a.protocol == RT_PROTOCOL_FORWARD);
                     const int pos = minus ? la[j] : fi[j];
-                    int c = rid[j];
-                    if (Packed) {
-                        int r = s_run;
-                        if (!s_one_run) {
-                            const long long g = a.read_base + i;
-                            while (r + 1 < a.n_runs && g >= __ldg(a.run_start + r + 1)) ++r;
-                        }
-                        c = __ldg(a.run_ref + r);
-                    }
+                    const int c = rid[j];
                     if (mode == RT_LEN_FILTERED || a.protocol > RT_PROTOCOL_REVERSE) {
                         cat = 0;                                    // bam.py:101 / no protocol branch: only `total`
                     } else if ((unsigned)c >= (unsigned)a.n_contig) {
@@ -1661,11 +1608,7 @@ __global__ void __launch_bounds__(kBinThreads) bin_psites_kernel(const BinArgs a
             if (head && slot != kNone) {
                 const unsigned after = lane == 31 ? 0u : heads >> (lane + 1);
                 const int run = after ? __ffs(after) : 32 - lane;
-#ifdef RT_BIN_NO_RED      // A/B build only: everything but the scatter itself (what no change to the atomics can go below)
-                sink += (unsigned long long)slot * (unsigned)run;
-#else
                 atomicAdd(a.cov + slot, a.weight * run);
-#endif
             }
             if (!Compact && a.touched) {   // remember the 32 B sector so the planes can be cleared sparsely afterwards
                 const long long sec = slot != kNone ? (long long)(slot >> 3) : -1;
@@ -1686,9 +1629,6 @@ __global__ void __launch_bounds__(kBinThreads) bin_psites_kernel(const BinArgs a
             }
         }
     }
-#ifdef RT_BIN_NO_RED
-    if (sink == 0x123456789abcdefull) a.cov[0] = 1;      // keeps the slot computation alive
-#endif
     {   // flush the register length counters: one REDUX per length, one shared atomic per lane
         unsigned mine_len = 0;
 #pragma unroll
@@ -1782,28 +1722,16 @@ __device__ __forceinline__ void stream_scatter(int32_t* cov, const slot_t (&slot
     constexpr slot_t kNone = (slot_t)-1;
     slot_t cur = kNone;
     int cnt = 0;
-#ifdef RT_BIN_NO_RED      // A/B build only: everything but the scatter itself
-    unsigned long long sink = 0;
-#define RT_STREAM_RED(p, v) sink += (unsigned long long)((p) - cov) * (unsigned)(v)
-#elif defined(RT_BIN_RED_L2ONLY)   // A/B build only: the same REDs folded into 256 KB that stay in L2 (wrong coverage)
-#define RT_STREAM_RED(p, v) atomicAdd(cov + (((p) - cov) & 0xffff), (v))
-#else
-#define RT_STREAM_RED(p, v) atomicAdd((p), (v))
-#endif
 #pragma unroll
     for (int j = 0; j < kStreamStrip; ++j) {
         if (slot[j] != cur) {
-            if (cur != kNone) RT_STREAM_RED(cov + cur, weight * cnt);
+            if (cur != kNone) atomicAdd(cov + cur, weight * cnt);
             cur = slot[j];
             cnt = 0;
         }
         ++cnt;
     }
-    if (cur != kNone) RT_STREAM_RED(cov + cur, weight * cnt);
-#ifdef RT_BIN_NO_RED
-    if (sink == 0x123456789abcdefull) cov[0] = 1;      // keeps the slot computation alive
-#endif
-#undef RT_STREAM_RED
+    if (cur != kNone) atomicAdd(cov + cur, weight * cnt);
 }
 
 // (word, bit) of the dense slot -> slot of the current layout (compact: through the member bitmap and the rank word)
@@ -1835,9 +1763,7 @@ __device__ __forceinline__ void stream_slots(const StreamArgs& a, unsigned live,
 }
 
 constexpr int kStreamContigs = 256;     // contig table entries kept in shared memory
-#ifndef RT_STREAM_CTAS_PER_SM
-#define RT_STREAM_CTAS_PER_SM 3
-#endif
+constexpr int kStreamCtasPerSm = 3;
 
 // Zero the compact slots [z0, z1): 16-byte stores where the range is aligned, single slots at its two ends.
 __device__ __forceinline__ void stream_zero_zone(int32_t* cov, unsigned z0, unsigned z1, int lane) {
@@ -1939,13 +1865,13 @@ __global__ void __launch_bounds__(256) zone_spill_kernel(int32_t* cov, const uns
         atomicAdd(cov + spill[i], 1);
 }
 
-// Persistent: RT_STREAM_CTAS_PER_SM CTAs per SM; every WARP walks blocks of the stream on its own (no CTA-wide barrier
+// Persistent: kStreamCtasPerSm CTAs per SM; every WARP walks blocks of the stream on its own (no CTA-wide barrier
 // after start-up, so the warps of an SM drift apart and cover each other's load latencies).  A warp owns a ring of two
 // shared-memory stages with one mbarrier each: an elected lane brings block i + 1 (1 KB of records and its header) in
 // with a cp.async.bulk pair while the warp works on block i.  The lookup tables are built once per CTA and the
 // per-thread 4-bit counters are drained into 8-bit ones every block.
 template <bool Compact, bool Zoned>
-__global__ void __launch_bounds__(kStreamThreads, RT_STREAM_CTAS_PER_SM) bin_stream_kernel(const StreamArgs a) {
+__global__ void __launch_bounds__(kStreamThreads, kStreamCtasPerSm) bin_stream_kernel(const StreamArgs a) {
     static_assert(Compact || !Zoned, "zones are ranges of the compact buffer");
     __shared__ __align__(128) unsigned int s_rec[kStreamWarps][2][RT_STREAM_BLOCK];
     __shared__ __align__(16) int4 s_hdr[kStreamWarps][2];

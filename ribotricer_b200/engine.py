@@ -262,77 +262,6 @@ class Engine:
                                                _np_ptr(len_counts)))
         return dict(zip(_lib.ST_NAMES, stats.tolist())), len_counts
 
-    def pack_reads(self, cols: dict, pinned: bool = False, max_runs: int | None = None) -> dict:
-        """Packed read records for ``bin_reads_packed_host`` (``rt_pack_read_meta``): 11 B/read instead of
-        18.  ``first/last/mlen`` are reused as they are; ``flag/mapq/nh`` collapse into one ``meta`` byte
-        (filter cascade decided on the host) and ``ref_id`` into a run table.  Raises when the reads are
-        not grouped by reference (more than ``max_runs`` runs)."""
-        t = self.torch
-        host = {}
-        for name, dt in READ_COLUMNS:
-            v = cols[name]
-            if hasattr(v, "cpu"):                       # torch tensor (16-bit columns are stored as int16)
-                v = v.cpu().numpy()
-                if v.dtype.itemsize == np.dtype(dt).itemsize and v.dtype != dt:
-                    v = v.view(dt)
-            host[name] = np.ascontiguousarray(v, dt)
-        n = len(host["ref_id"])
-        cap = int(max_runs if max_runs is not None else max(64, 4 * len(self.contig_len) + 8))
-        meta = np.empty(n, np.uint8)
-        run_start = np.zeros(cap + 1, np.int64)
-        run_ref = np.zeros(cap, np.int32)
-        n_runs = C.c_int64(0)
-        rc = self.lib.rt_pack_read_meta(n, _np_ptr(host["ref_id"]), _np_ptr(host["flag"]), _np_ptr(host["mapq"]),
-                                        _np_ptr(host["nh"]), _np_ptr(meta), cap, _np_ptr(run_start), _np_ptr(run_ref),
-                                        C.byref(n_runs))
-        if rc != 0:
-            raise _lib.RtError(self.lib.rt_io_last_error().decode() or f"rt_pack_read_meta failed ({rc})")
-        k = int(n_runs.value)
-        out = dict(first=host["first"], last=host["last"], mlen=host["mlen"], meta=meta)
-        if pinned:
-            out = {name: t.from_numpy(np.ascontiguousarray(a)).pin_memory() for name, a in out.items()}
-        out["run_start"] = np.ascontiguousarray(run_start[:k + 1])
-        out["run_ref"] = np.ascontiguousarray(run_ref[:k])
-        out["n"] = n
-        return out
-
-    def upload_packed(self, packed: dict) -> dict:
-        """Packed host records (``pack_reads``) -> device tensors, run table included (plumbing only)."""
-        t = self.torch
-
-        def dev(a):
-            if hasattr(a, "data_ptr"):
-                return a.to(self.device)
-            a = np.ascontiguousarray(a)
-            return t.from_numpy(a.view(np.int16) if a.dtype == np.uint16 else a).to(self.device)
-
-        out = {k: dev(packed[k]) for k in ("first", "last", "mlen", "meta", "run_start", "run_ref")}
-        out["n"] = int(packed["n"])
-        return out
-
-    def bin_reads_packed_device(self, cov, dpacked: dict, protocol, stats, len_counts, weight: int = 1):
-        """Enqueue K1 on device-resident PACKED records (11 B/read; no host sync)."""
-        p = lambda x: C.c_void_p(x.data_ptr())  # noqa: E731
-        self._check(self.lib.rt_bin_reads_packed(
-            self.ctx, p(cov), int(dpacked["n"]), p(dpacked["first"]), p(dpacked["last"]), p(dpacked["mlen"]),
-            p(dpacked["meta"]), 0, int(dpacked["run_ref"].numel()), p(dpacked["run_start"]), p(dpacked["run_ref"]),
-            protocol_code(protocol), int(weight), p(stats), p(len_counts), self._stream()))
-
-    def bin_reads_packed_host(self, cov, packed: dict, protocol):
-        """K1 on packed HOST records (see ``pack_reads``): chunked H2D of 11 B/read inside the call.
-        Returns ``(stats, read_length_counts)`` exactly like ``bin_reads_host``."""
-        def ptr(a):
-            return C.c_void_p(a.data_ptr()) if hasattr(a, "data_ptr") else _np_ptr(a)
-
-        stats = np.zeros(_lib.RT_N_STATS, np.int64)
-        len_counts = np.zeros(_lib.RT_LEN_TABLE, np.int64)
-        self.torch.cuda.current_stream(self.device).synchronize()
-        self._check(self.lib.rt_bin_reads_packed_host(
-            self.ctx, C.c_void_p(cov.data_ptr()), int(packed["n"]), ptr(packed["first"]), ptr(packed["last"]),
-            ptr(packed["mlen"]), ptr(packed["meta"]), len(packed["run_ref"]), _np_ptr(packed["run_start"]),
-            _np_ptr(packed["run_ref"]), protocol_code(protocol), _np_ptr(stats), _np_ptr(len_counts)))
-        return dict(zip(_lib.ST_NAMES, stats.tolist())), len_counts
-
     def stream_reads(self, cols: dict, pinned: bool = False, n_threads: int = 0) -> dict:
         """A coordinate-sorted library as the 4 B/read record stream of ``rt_stream_pack`` (blocks of 256 delta-coded
         records; the raw filter bits travel with every read and the cascade runs on the device).  Raises ``RtError``

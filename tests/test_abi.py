@@ -21,13 +21,13 @@ def test_header_declares_the_expected_surface():
     assert sorted(_lib.EXPORTS) == header_symbols()
 
 
-def test_library_exports_every_declared_symbol(built):
+def test_library_exports_every_declared_symbol_and_abi_version(built):
     from ribotricer_b200 import _lib
 
     lib = ctypes.CDLL(_lib.LIB_PATH)
     for name in header_symbols():
         assert hasattr(lib, name), name
-    assert _lib.load().rt_abi_version() == 3
+    assert _lib.load().rt_abi_version() == 4
 
 
 def test_no_cpu_fallback(built):

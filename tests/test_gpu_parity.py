@@ -603,59 +603,6 @@ def test_edge_cases_compact_layout(engine):
             engine.set_layout("dense")
 
 
-@pytest.mark.parametrize("layout", ["dense", "compact"])
-def test_packed_records_match_columns(engine, layout):
-    """rt_pack_read_meta + rt_bin_reads_packed_host (11 B/read) against rt_bin_reads_host (18 B/read) on
-    the same reads: stats, length totals and every coverage slot; reads of unknown references and all
-    filter categories included; several launches (chunks) and runs that end inside a block."""
-    from ribotricer_b200 import synth
-    from ribotricer_b200._lib import RtError
-
-    cfg = synth.config("tiny")
-    idx = synth.make_index(cfg)
-    reads = synth.reads_to_numpy(synth.make_reads(cfg, idx, n_reads=700_000))
-    rng = np.random.default_rng(3)
-    n = len(reads["ref_id"])
-    reads["flag"] = np.where(rng.random(n) < 0.1, rng.choice([4, 256, 512, 1024, 2048, 272], n), reads["flag"]).astype(np.uint16)
-    reads["nh"] = rng.choice([0, 1, 1, 1, 2], n).astype(np.uint8)
-    reads["mapq"] = rng.choice([255, 255, 3, 0], n).astype(np.uint8)
-    tail = slice(n - 5000, n)                      # a last run of reads without a reference, like unmapped BAM tails
-    reads["ref_id"][tail] = -1
-    _setup(engine, idx.contig_names, idx.contig_len, idx.as_dict(), synth.TRUE_OFFSETS, pad=64)
-    engine.set_layout(layout)
-    try:
-        for protocol in ("forward", "reverse"):
-            want = engine.new_coverage()
-            stats_w, len_w = engine.bin_reads_host(want, reads, protocol, sorted_hint=True)
-            packed = engine.pack_reads(reads)
-            assert len(packed["run_ref"]) <= len(idx.contig_names) + 1 and packed["run_start"][-1] == n
-            got = engine.new_coverage()
-            stats_g, len_g = engine.bin_reads_packed_host(got, packed, protocol)
-            assert stats_g == stats_w and (len_g == len_w).all()
-            assert engine.torch.equal(got, want)
-            dev = engine.new_coverage()                    # the same records resident on the device
-            st, lc = engine.new_bin_accumulators()
-            engine.bin_reads_packed_device(dev, engine.upload_packed(packed), protocol, st, lc)
-            assert engine.torch.equal(dev, want) and dict(zip(stats_w.keys(), st.cpu().tolist())) == stats_w
-        empty = engine.pack_reads({k: v[:0] for k, v in reads.items()})        # no reads at all
-        stats_e, len_e = engine.bin_reads_packed_host(engine.new_coverage(), empty, "forward")
-        assert stats_e["total"] == 0 and not len_e.any()
-        # unsorted input has one run per read, far more than the table holds: refused, not mis-binned
-        shuffled = {k: v[rng.permutation(n)] for k, v in reads.items()}
-        with pytest.raises(RtError, match="not grouped by reference"):
-            engine.pack_reads(shuffled)
-        # ... unless the caller sizes the run table for it; results are still the same
-        small = {k: v[:30_000] for k, v in shuffled.items()}
-        packed = engine.pack_reads(small, max_runs=30_000)
-        want = engine.new_coverage()
-        stats_w, _ = engine.bin_reads_host(want, small, "forward")
-        got = engine.new_coverage()
-        stats_g, _ = engine.bin_reads_packed_host(got, packed, "forward")
-        assert stats_g == stats_w and engine.torch.equal(got, want)
-    finally:
-        engine.set_layout("dense")
-
-
 def test_random_many_exon_orfs_both_layouts(engine):
     """Randomised soak (fixed seed): ORFs of up to 200 exons of 1-40 nt with gaps of 0-7 nt, nested ORFs that
     share their tails, both strands, coverage densities from 0.02 to 30 per nt (table path, slow path,

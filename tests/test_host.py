@@ -275,66 +275,6 @@ def test_native_bam_decoder(tmp_path, built):
         read_bam_columns_native(str(bad))
 
 
-def test_bam_pack_matches_pack_read_meta(tmp_path, built):
-    """rt_bam_pack (the decoder's packed records) == rt_pack_read_meta on the decoder's columns, and the
-    meta byte restates the cascade of bam.py:77-91 / common.py:33-69 (checked against oracle_py)."""
-    import base64
-    import ctypes as C
-
-    from helpers import load_golden
-    from oracle import oracle_py as O
-    from ribotricer_b200 import _lib
-    from ribotricer_b200.bam import read_bam_columns_native
-
-    case = load_golden("split_bam_case.json.gz")["case"]
-    path = tmp_path / "g.bam"
-    path.write_bytes(base64.b64decode(case["bam_b64"]))
-    rc = read_bam_columns_native(str(path), 2)
-    n = len(rc)
-    lib = _lib.load()
-    vp = C.c_void_p
-    p = lambda a: a.ctypes.data_as(vp)      # noqa: E731
-
-    def pack_cols():
-        meta = np.empty(n, np.uint8)
-        rs, rr, k = np.zeros(65, np.int64), np.zeros(64, np.int32), C.c_int64(0)
-        assert lib.rt_pack_read_meta(n, p(rc.cols["ref_id"]), p(rc.cols["flag"]), p(rc.cols["mapq"]), p(rc.cols["nh"]),
-                                     p(meta), 64, p(rs), p(rr), C.byref(k)) == 0
-        return meta, rs[:k.value + 1], rr[:k.value]
-
-    handle = vp()
-    assert lib.rt_bam_load(str(path).encode(), 2, C.byref(handle)) == 0
-    try:
-        meta2 = np.empty(n, np.uint8)
-        rs2, rr2, k2 = np.zeros(65, np.int64), np.zeros(64, np.int32), C.c_int64(0)
-        assert lib.rt_bam_pack(handle, p(meta2), 64, p(rs2), p(rr2), C.byref(k2)) == 0
-    finally:
-        lib.rt_bam_free(handle)
-    meta, rs, rr = pack_cols()
-    assert (meta == meta2).all() and (rs == rs2[:k2.value + 1]).all() and (rr == rr2[:k2.value]).all()
-    # runs reproduce ref_id; sorted BAM: one run per reference present (+ the unmapped tail)
-    assert (np.repeat(rr, np.diff(rs)) == rc.cols["ref_id"]).all() and len(rr) <= len(rc.contig_names) + 1
-    # meta against the oracle's cascade
-    codes = {"qcfail": 1, "duplicate": 2, "secondary": 3, "unmapped": 4, "multi": 5}
-    for i in range(n):
-        flag, mapq, nh = int(rc.cols["flag"][i]), int(rc.cols["mapq"][i]), int(rc.cols["nh"][i])
-        if flag & O.FLAG_QCFAIL:
-            want = codes["qcfail"]
-        elif flag & O.FLAG_DUPLICATE:
-            want = codes["duplicate"]
-        elif flag & O.FLAG_SECONDARY:
-            want = codes["secondary"]
-        elif flag & O.FLAG_UNMAPPED:
-            want = codes["unmapped"]
-        else:
-            want = 0 if O.is_read_uniq_mapping(flag, mapq, nh) else codes["multi"]
-        assert meta[i] == (want | (8 if flag & O.FLAG_REVERSE else 0)), i
-    # too few run slots: refused
-    k = C.c_int64(0)
-    assert lib.rt_pack_read_meta(n, p(rc.cols["ref_id"]), p(rc.cols["flag"]), p(rc.cols["mapq"]), p(rc.cols["nh"]),
-                                 p(meta), 1, p(np.zeros(2, np.int64)), p(np.zeros(1, np.int32)), C.byref(k)) != 0
-
-
 def test_count_orfs_text_matches_reference(tmp_path, built):
     """ribotricer_b200.count_orfs.count_orfs (same signature as count_orfs.py:28) on the golden TSVs."""
     from helpers import load_golden
