@@ -321,6 +321,9 @@ int rt_index_copy(const rt_index* ix, int64_t* exon_ptr, int32_t* exon_start, in
                   int32_t* orf_chrom, uint8_t* orf_strand);
 /* raw text of column k (1 = ORF_type .. 9 = start_codon) of row `orf`; not NUL terminated */
 const char* rt_index_field(const rt_index* ix, int64_t orf, int k, int* len);
+/* the first column (ORF_ID) of every row, byte for byte, back to back: row o is blob[off[o], off[o+1]).  With
+ * blob == NULL only off (n_orf + 1 entries) is filled, so a caller can size blob first. */
+int rt_index_ids(const rt_index* ix, int64_t* off, char* blob);
 int rt_tsv_open(const char* path, int write_header, rt_tsv** out);
 int rt_tsv_write(rt_tsv* t, const rt_index* ix, int64_t n_sel, const int64_t* orf_ids, int64_t orf_lo,
                  const double* score, const int32_t* valid, const int64_t* count, const int32_t* length,
@@ -436,6 +439,38 @@ typedef struct rt_orf_query {
 int rt_orf_search(rt_ctx* ctx, const rt_orf_query* q, int64_t* n_rows, int64_t* n_iv, float* stage_ms);
 int rt_orf_fetch(rt_ctx* ctx, int32_t* row_tx, int32_t* row_start, int32_t* row_stop, uint8_t* row_type, uint8_t* row_codon,
                  int64_t* iv_ptr, int32_t* iv_start, int32_t* iv_end);
+
+/*
+ * ---- orfs-seq: the sequence of every index row (DESIGN.md section 10) ----------------------------------------------
+ * rt_orf_seq_write writes `path`: the line "ORF_ID\tsequence", then per row its id, a tab, the sequence and a newline.
+ * The sequence is the row's intervals (ascending, 1-based closed) concatenated from `codes`, reverse-complemented when
+ * orf_strand is 1; letters A C G T, N for code 4.  With `protein` the codons from the first nt are translated with the
+ * standard genetic code (stops '*', a codon holding an N 'X', a trailing 1-2 nt dropped).  Every row is checked before
+ * the file is opened (RT_EINVAL naming the ORF_ID: an interval that ends before it starts, starts before 1 or ends past
+ * its contig).  The host cuts the rows into chunks of whole lines of at most chunk_bytes (0: 64 MiB; never less than the
+ * longest line); orf_seq_kernel<nt|protein> writes a chunk's lines into one of two device buffers while the previous
+ * chunk is copied back and the one before it is written by a writer thread.  On any error the file is removed.
+ * stage_ms (optional) receives RT_SEQ_STAGES device times: upload, kernels (summed), copy-back (summed).
+ */
+#define RT_SEQ_STAGES 3
+typedef struct rt_seq_query {
+    int64_t n_orf;
+    const int64_t* exon_ptr;        /* n_orf + 1 */
+    const int32_t* exon_start;      /* 1-based closed, ascending within a row */
+    const int32_t* exon_end;
+    const int32_t* orf_contig;      /* into the contig table below */
+    const uint8_t* orf_strand;      /* 1 reverse, anything else forward */
+    int32_t n_contig;
+    const int64_t* contig_base;     /* offset of each contig in codes */
+    const int64_t* contig_len;
+    const uint8_t* codes;           /* rt_fasta_codes of the contigs */
+    int64_t n_codes;
+    const int64_t* id_off;          /* n_orf + 1: row o's ORF_ID is ids[id_off[o], id_off[o+1]) */
+    const char* ids;
+    int32_t protein;
+    int64_t chunk_bytes;
+} rt_seq_query;
+int rt_orf_seq_write(rt_ctx* ctx, const rt_seq_query* q, const char* path, float* stage_ms);
 
 /* number of kernel launches issued through this ctx so far (bench.py's gpu_launches) */
 int64_t rt_launch_count(const rt_ctx* ctx);

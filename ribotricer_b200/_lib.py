@@ -33,9 +33,11 @@ EXPORTS = (
     "rt_inflate_raw", "rt_crc32", "rt_metagene_sums",
     "rt_gtf_load", "rt_gtf_free", "rt_gtf_n_lines", "rt_gtf_n_strings", "rt_gtf_string_bytes", "rt_gtf_copy",
     "rt_fasta_load", "rt_fasta_free", "rt_fasta_n_contig", "rt_fasta_contig_name", "rt_fasta_contig_len", "rt_fasta_codes",
-    "rt_orf_write", "rt_orf_search", "rt_orf_fetch",
+    "rt_orf_write", "rt_orf_search", "rt_orf_fetch", "rt_index_ids", "rt_orf_seq_write",
 )
+RT_EINVAL = -1
 RT_ORF_STAGES = 7
+RT_SEQ_STAGES = 3
 
 
 class ScoreParams(C.Structure):
@@ -55,6 +57,13 @@ class OrfQuery(C.Structure):
                 ("tx_base", C.c_void_p), ("tx_strand", C.c_void_p), ("tx_cds", C.c_void_p), ("codes", C.c_void_p),
                 ("n_codes", C.c_int64), ("start_mask", C.c_uint64), ("stop_mask", C.c_uint64),
                 ("min_orf_length", C.c_int32), ("longest", C.c_int32)]
+
+
+class SeqQuery(C.Structure):
+    _fields_ = [("n_orf", C.c_int64), ("exon_ptr", C.c_void_p), ("exon_start", C.c_void_p), ("exon_end", C.c_void_p),
+                ("orf_contig", C.c_void_p), ("orf_strand", C.c_void_p), ("n_contig", C.c_int32),
+                ("contig_base", C.c_void_p), ("contig_len", C.c_void_p), ("codes", C.c_void_p), ("n_codes", C.c_int64),
+                ("id_off", C.c_void_p), ("ids", C.c_void_p), ("protein", C.c_int32), ("chunk_bytes", C.c_int64)]
 
 
 class RtError(RuntimeError):
@@ -179,6 +188,8 @@ def load():
     lib.rt_orf_write.argtypes = [C.c_char_p, i64, vp, vp, vp, i64, vp, vp, vp, vp, vp, vp]
     lib.rt_orf_search.argtypes = [vp, C.POINTER(OrfQuery), C.POINTER(i64), C.POINTER(i64), vp]
     lib.rt_orf_fetch.argtypes = [vp] * 9
+    lib.rt_index_ids.argtypes = [vp, vp, vp]
+    lib.rt_orf_seq_write.argtypes = [vp, C.POINTER(SeqQuery), C.c_char_p, vp]
     if lib.rt_abi_version() != 4:
         raise RtError(f"ABI mismatch: library reports {lib.rt_abi_version()}, binding expects 4")
     _lib = lib

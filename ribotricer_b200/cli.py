@@ -1,9 +1,10 @@
-"""Command line of the B200 path: ``prepare-orfs``, ``detect-orfs``, ``count-orfs`` and ``learn-cutoff``.
+"""Command line of the B200 path: ``prepare-orfs``, ``detect-orfs``, ``count-orfs``, ``learn-cutoff`` and ``orfs-seq``.
 
 The flag names, defaults, flag -> argument renames (``--min_read_density`` -> ``min_density_over_orf``,
 ``--stranded yes`` -> ``forward``, ``--meta-min-reads``) and every validation message are those of the
 reference command line (ribotricer/cli.py:127-289, 292-339, 435-560), so existing invocations keep working.
-``prepare-orfs`` takes the reference's flags (ribotricer/cli.py) and reads plain-text GTF and FASTA files only.
+``prepare-orfs`` and ``orfs-seq`` take the reference's flags (ribotricer/cli.py) and read plain-text GTF and FASTA
+files only.
 The commands are assembled from option tables below.  ``--bam`` also accepts a ``.npz`` of decoded columns.
 """
 from __future__ import annotations
@@ -30,7 +31,8 @@ except ImportError:
 @click.group(**_GROUP_KW)
 @click.version_option(version=__version__)
 def cli() -> None:
-    """ribotricer: Tool for detecting translating ORF from Ribo-seq data (B200-native prepare-orfs and detect-orfs)"""
+    """ribotricer: Tool for detecting translating ORF from Ribo-seq data (B200-native prepare-orfs, detect-orfs and
+    orfs-seq)"""
 
 
 def _register(name: str, summary: str, options, handler) -> None:
@@ -230,6 +232,26 @@ _register("learn-cutoff", "Learn phase score cutoff from BAM/TSV file", [
                               help="Number of protein coding regions to sample per bootstrap")),
     ("--n_bootstraps", dict(type=int, default=20000, show_default=True, help="Number of bootstraps")),
 ], _learn)
+
+
+# ------------------------------------------------------------------------------------ orfs-seq
+def _seq(ribotricer_index, fasta, saveto, protein) -> None:
+    from .orf_seq import orf_seq
+
+    _need_file(ribotricer_index, "ribotricer index file")
+    _need_file(fasta, "FASTA file")
+    try:
+        orf_seq(ribotricer_index, fasta, saveto, protein)
+    except ValueError as exc:
+        _fail(str(exc))
+
+
+_register("orfs-seq", "Generate sequence for ORFs in ribotricer's index", [
+    ("--ribotricer_index", dict(help=_INDEX_HELP, required=True)),
+    ("--fasta", dict(help="Path to FASTA file", required=True)),
+    ("--saveto", dict(help="Path to output file", required=True)),
+    ("--protein", dict(is_flag=True, help="Output protein sequence instead of nucleotide sequence")),
+], _seq)
 
 
 if __name__ == "__main__":

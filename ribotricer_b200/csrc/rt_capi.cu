@@ -7,6 +7,8 @@
 #include <cstring>
 #include <atomic>
 #include <chrono>
+#include <condition_variable>
+#include <deque>
 #include <mutex>
 #include <string>
 #include <unordered_map>
@@ -132,6 +134,9 @@ struct rt_ctx {
     DevBuf orf_buf[32];
     std::vector<int64_t> orf_iv_ptr;                 // n_rows + 1: interval offsets of the last search
     int64_t orf_rows = 0;
+
+    // orfs-seq (rt_orf_seq_write): the uploaded tables and the two chunk buffers, kept for the next call
+    DevBuf seq_buf[16];
 };
 
 namespace {
@@ -394,6 +399,7 @@ void rt_destroy(rt_ctx* ctx) {
     if (!ctx) return;
     DeviceGuard guard(ctx->device);
     for (auto& b : ctx->orf_buf) b.release();
+    for (auto& b : ctx->seq_buf) b.release();
     cudaFree(ctx->d_contig_tab);
     cudaFree(ctx->d_uv_table);
     cudaFree(ctx->d_len_table);
@@ -1851,6 +1857,250 @@ int rt_orf_fetch(rt_ctx* ctx, int32_t* row_tx, int32_t* row_start, int32_t* row_
     if (iv_ptr) memcpy(iv_ptr, ctx->orf_iv_ptr.data(), 8 * (size_t)(rows + 1));
     RT_CUDA(ctx, cudaStreamSynchronize(st));
     return RT_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------- orfs-seq
+namespace {
+enum SeqBuf { kSqCodes, kSqExPtr, kSqExStart, kSqExEnd, kSqContig, kSqStrand, kSqBase, kSqIdOff, kSqIds, kSqLineOff,
+              kSqOut0, kSqOut1, kSqClaim, kSeqBufs };
+static_assert(kSeqBufs <= 16, "rt_ctx::seq_buf is too small");
+constexpr int64_t kSeqChunkDefault = int64_t(64) << 20;
+
+// Writes the chunks handed to it, in order, on its own thread; `written` counts the chunks it has finished.
+struct SeqWriter {
+    FILE* fh = nullptr;
+    std::mutex m;
+    std::condition_variable cv;
+    std::deque<std::pair<const char*, size_t>> todo;
+    int64_t written = 0;
+    bool stop = false, failed = false;
+    std::thread th;
+    void run() {
+        for (;;) {
+            std::pair<const char*, size_t> job;
+            {
+                std::unique_lock<std::mutex> lk(m);
+                cv.wait(lk, [&] { return stop || !todo.empty(); });
+                if (todo.empty()) return;
+                job = todo.front();
+                todo.pop_front();
+            }
+            const bool ok = fwrite(job.first, 1, job.second, fh) == job.second;
+            {
+                std::lock_guard<std::mutex> lk(m);
+                failed = failed || !ok;
+                ++written;
+            }
+            cv.notify_all();
+        }
+    }
+    void push(const char* p, size_t n) {
+        {
+            std::lock_guard<std::mutex> lk(m);
+            todo.emplace_back(p, n);
+        }
+        cv.notify_all();
+    }
+    bool wait_written(int64_t k) {   // false once a write has failed
+        std::unique_lock<std::mutex> lk(m);
+        cv.wait(lk, [&] { return written >= k || failed; });
+        return !failed;
+    }
+    void finish() {
+        {
+            std::lock_guard<std::mutex> lk(m);
+            stop = true;
+        }
+        cv.notify_all();
+        if (th.joinable()) th.join();
+    }
+};
+
+// Streams, events, page-locked buffers and the writer of one rt_orf_seq_write call; the destructor joins the writer and
+// waits for both streams before anything is freed, so every early return leaves nothing behind.
+struct SeqPipeline {
+    cudaStream_t ks = nullptr, cs = nullptr;   // kernels + uploads, copy-back
+    cudaEvent_t ev[10] = {};                   // upload begin / end, then per buffer b: kernel begin/end, copy begin/end
+    char* pinned[2] = {};
+    SeqWriter writer;
+    ~SeqPipeline() {
+        writer.finish();
+        if (ks) cudaStreamSynchronize(ks);
+        if (cs) cudaStreamSynchronize(cs);
+        for (char* p : pinned)
+            if (p) cudaFreeHost(p);
+        for (cudaEvent_t e : ev)
+            if (e) cudaEventDestroy(e);
+        if (ks) cudaStreamDestroy(ks);
+        if (cs) cudaStreamDestroy(cs);
+    }
+};
+
+int seq_emit(rt_ctx* ctx, const rt_seq_query* q, const std::vector<int64_t>& line_off, const std::vector<int64_t>& cut,
+             int64_t buf_bytes, FILE* fh, float* stage_ms) {
+    const int64_t n = q->n_orf, n_ex = n ? q->exon_ptr[n] : 0, n_ids = n ? q->id_off[n] : 0;
+    const int64_t n_chunks = (int64_t)cut.size() - 1;
+    DevBuf* B = ctx->seq_buf;
+    auto reserve = [&](int k, size_t bytes) { return B[k].reserve(std::max<size_t>(bytes, 16)); };
+    RT_CUDA(ctx, reserve(kSqCodes, (size_t)q->n_codes));
+    RT_CUDA(ctx, reserve(kSqExPtr, 8 * (size_t)(n + 1)));
+    RT_CUDA(ctx, reserve(kSqExStart, 4 * (size_t)n_ex));
+    RT_CUDA(ctx, reserve(kSqExEnd, 4 * (size_t)n_ex));
+    RT_CUDA(ctx, reserve(kSqContig, 4 * (size_t)n));
+    RT_CUDA(ctx, reserve(kSqStrand, (size_t)n));
+    RT_CUDA(ctx, reserve(kSqBase, 8 * (size_t)q->n_contig));
+    RT_CUDA(ctx, reserve(kSqIdOff, 8 * (size_t)(n + 1)));
+    RT_CUDA(ctx, reserve(kSqIds, (size_t)n_ids));
+    RT_CUDA(ctx, reserve(kSqLineOff, 8 * (size_t)(n + 1)));
+    RT_CUDA(ctx, reserve(kSqClaim, 4));
+    SeqPipeline P;
+    RT_CUDA(ctx, cudaStreamCreateWithFlags(&P.ks, cudaStreamNonBlocking));
+    RT_CUDA(ctx, cudaStreamCreateWithFlags(&P.cs, cudaStreamNonBlocking));
+    for (auto& e : P.ev) RT_CUDA(ctx, cudaEventCreate(&e));
+    cudaEvent_t *k_begin = P.ev + 2, *k_end = P.ev + 4, *c_begin = P.ev + 6, *c_end = P.ev + 8;
+    // 1. upload: the contig codes and the tables, once
+    auto up = [&](int k, const void* src, size_t bytes) {
+        return bytes ? cudaMemcpyAsync(B[k].p, src, bytes, cudaMemcpyHostToDevice, P.ks) : cudaSuccess;
+    };
+    RT_CUDA(ctx, cudaEventRecord(P.ev[0], P.ks));
+    RT_CUDA(ctx, up(kSqCodes, q->codes, (size_t)q->n_codes));
+    RT_CUDA(ctx, up(kSqExPtr, q->exon_ptr, 8 * (size_t)(n + 1)));
+    RT_CUDA(ctx, up(kSqExStart, q->exon_start, 4 * (size_t)n_ex));
+    RT_CUDA(ctx, up(kSqExEnd, q->exon_end, 4 * (size_t)n_ex));
+    RT_CUDA(ctx, up(kSqContig, q->orf_contig, 4 * (size_t)n));
+    RT_CUDA(ctx, up(kSqStrand, q->orf_strand, (size_t)n));
+    RT_CUDA(ctx, up(kSqBase, q->contig_base, 8 * (size_t)q->n_contig));
+    RT_CUDA(ctx, up(kSqIdOff, q->id_off, 8 * (size_t)(n + 1)));
+    RT_CUDA(ctx, up(kSqIds, q->ids, (size_t)n_ids));
+    RT_CUDA(ctx, up(kSqLineOff, line_off.data(), 8 * (size_t)(n + 1)));
+    RT_CUDA(ctx, cudaEventRecord(P.ev[1], P.ks));
+    if (stage_ms) stage_ms[1] = stage_ms[2] = 0.f;
+    if (n_chunks == 0) {
+        RT_CUDA(ctx, cudaStreamSynchronize(P.ks));
+        if (stage_ms) RT_CUDA(ctx, cudaEventElapsedTime(&stage_ms[0], P.ev[0], P.ev[1]));
+        return RT_OK;
+    }
+    // 2. the chunks: kernel k+1 runs while chunk k is copied back and chunk k-1 is written
+    for (int b = 0; b < 2 && b < n_chunks; ++b) {
+        RT_CUDA(ctx, reserve(kSqOut0 + b, (size_t)buf_bytes));
+        RT_CUDA(ctx, cudaHostAlloc((void**)&P.pinned[b], (size_t)buf_bytes, cudaHostAllocDefault));
+    }
+    P.writer.fh = fh;
+    P.writer.th = std::thread([&P] { P.writer.run(); });
+    const rt::SeqArgs A{(const uint8_t*)B[kSqCodes].p, (const long long*)B[kSqExPtr].p, (const int*)B[kSqExStart].p,
+                        (const int*)B[kSqExEnd].p, (const int*)B[kSqContig].p, (const uint8_t*)B[kSqStrand].p,
+                        (const long long*)B[kSqBase].p, (const long long*)B[kSqIdOff].p, (const char*)B[kSqIds].p,
+                        (const long long*)B[kSqLineOff].p, (unsigned*)B[kSqClaim].p};
+    const int64_t big = std::max(1, ctx->n_sm * 8);
+    auto bytes_of = [&](int64_t k) { return (size_t)(line_off[(size_t)cut[(size_t)k + 1]] - line_off[(size_t)cut[(size_t)k]]); };
+    // chunk k is on the host: add its times, hand it to the writer
+    auto collect = [&](int64_t k) -> int {
+        const int b = (int)(k & 1);
+        RT_CUDA(ctx, cudaEventSynchronize(c_end[b]));
+        if (stage_ms) {
+            float kms = 0.f, cms = 0.f;
+            RT_CUDA(ctx, cudaEventElapsedTime(&kms, k_begin[b], k_end[b]));
+            RT_CUDA(ctx, cudaEventElapsedTime(&cms, c_begin[b], c_end[b]));
+            stage_ms[1] += kms;
+            stage_ms[2] += cms;
+        }
+        P.writer.push(P.pinned[b], bytes_of(k));
+        return RT_OK;
+    };
+    for (int64_t k = 0; k < n_chunks; ++k) {
+        const int b = (int)(k & 1);
+        const int64_t r0 = cut[(size_t)k], rows = cut[(size_t)k + 1] - r0;
+        // device buffer b is free: chunk k-2's copy finished before collect(k-2) returned
+        RT_CUDA(ctx, cudaMemsetAsync(B[kSqClaim].p, 0, 4, P.ks));
+        RT_CUDA(ctx, cudaEventRecord(k_begin[b], P.ks));
+        const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((rows + rt::kSeqWarps - 1) / rt::kSeqWarps, big));
+        if (q->protein)
+            rt::orf_seq_kernel<true><<<grid, rt::kSeqWarps * 32, 0, P.ks>>>(A, r0, rows, (char*)B[kSqOut0 + b].p);
+        else
+            rt::orf_seq_kernel<false><<<grid, rt::kSeqWarps * 32, 0, P.ks>>>(A, r0, rows, (char*)B[kSqOut0 + b].p);
+        ctx->launches++;
+        RT_CUDA(ctx, cudaGetLastError());
+        RT_CUDA(ctx, cudaEventRecord(k_end[b], P.ks));
+        if (k >= 1) {
+            const int rc = collect(k - 1);
+            if (rc != RT_OK) return rc;
+        }
+        // page-locked buffer b is free once chunk k-2 has been written
+        if (k >= 2 && !P.writer.wait_written(k - 1)) return fail(ctx, RT_EINVAL, "rt_orf_seq_write: write error");
+        RT_CUDA(ctx, cudaStreamWaitEvent(P.cs, k_end[b], 0));
+        RT_CUDA(ctx, cudaEventRecord(c_begin[b], P.cs));
+        RT_CUDA(ctx, cudaMemcpyAsync(P.pinned[b], B[kSqOut0 + b].p, bytes_of(k), cudaMemcpyDeviceToHost, P.cs));
+        RT_CUDA(ctx, cudaEventRecord(c_end[b], P.cs));
+    }
+    const int rc = collect(n_chunks - 1);
+    if (rc != RT_OK) return rc;
+    if (!P.writer.wait_written(n_chunks)) return fail(ctx, RT_EINVAL, "rt_orf_seq_write: write error");
+    if (stage_ms) RT_CUDA(ctx, cudaEventElapsedTime(&stage_ms[0], P.ev[0], P.ev[1]));
+    return RT_OK;
+}
+}  // namespace
+
+int rt_orf_seq_write(rt_ctx* ctx, const rt_seq_query* q, const char* path, float* stage_ms) {
+    if (!ctx) return fail(nullptr, RT_EINVAL, "rt_orf_seq_write: ctx is NULL");
+    if (!q || !path || q->n_orf < 0 || q->n_contig < 0 || q->n_codes < 0 || q->chunk_bytes < 0 ||
+        (q->n_orf && (!q->exon_ptr || !q->orf_contig || !q->orf_strand || !q->id_off)) ||
+        (q->n_contig && (!q->contig_base || !q->contig_len)) || (q->n_codes && !q->codes))
+        return fail(ctx, RT_EINVAL, "rt_orf_seq_write: NULL or negative argument");
+    const int64_t n = q->n_orf;
+    const int64_t n_ex = n ? q->exon_ptr[n] : 0, n_ids = n ? q->id_off[n] : 0;
+    if ((n_ex && (!q->exon_start || !q->exon_end)) || (n_ids && !q->ids) || (n && (q->exon_ptr[0] != 0 || q->id_off[0] != 0)))
+        return fail(ctx, RT_EINVAL, "rt_orf_seq_write: NULL or negative argument");
+    for (int c = 0; c < q->n_contig; ++c)
+        if (q->contig_base[c] < 0 || q->contig_len[c] < 0 || q->contig_base[c] + q->contig_len[c] > q->n_codes)
+            return fail(ctx, RT_EINVAL, "rt_orf_seq_write: contig %d lies outside the codes", c);
+    // 1. host pass: every row checked, the length and offset of every line
+    std::vector<int64_t> line_off((size_t)n + 1, 0);
+    int64_t longest = 0;
+    for (int64_t r = 0; r < n; ++r) {
+        const int64_t a = q->exon_ptr[r], b = q->exon_ptr[r + 1], i0 = q->id_off[r], i1 = q->id_off[r + 1];
+        if (b < a || b > n_ex || i1 < i0 || i1 > n_ids)
+            return fail(ctx, RT_EINVAL, "rt_orf_seq_write: exon_ptr or id_off is not monotone at row %lld", (long long)r);
+        const int id_len = (int)std::min<int64_t>(i1 - i0, 200);
+        const int c = q->orf_contig[r];
+        if (c < 0 || c >= q->n_contig)
+            return fail(ctx, RT_EINVAL, "rt_orf_seq_write: ORF %.*s: contig %d is not in the contig table", id_len, q->ids + i0, c);
+        int64_t L = 0;
+        for (int64_t e = a; e < b; ++e) {
+            const int32_t s = q->exon_start[e], t = q->exon_end[e];
+            if (t < s)
+                return fail(ctx, RT_EINVAL, "rt_orf_seq_write: ORF %.*s: interval %d-%d ends before it starts", id_len, q->ids + i0, s, t);
+            if (s < 1 || t > q->contig_len[c])
+                return fail(ctx, RT_EINVAL, "rt_orf_seq_write: ORF %.*s: interval %d-%d is outside its contig of %lld nt", id_len,
+                            q->ids + i0, s, t, (long long)q->contig_len[c]);
+            L += (int64_t)t - s + 1;
+        }
+        const int64_t line = (i1 - i0) + 1 + (q->protein ? L / 3 : L) + 1;
+        line_off[(size_t)r + 1] = line_off[(size_t)r] + line;
+        longest = std::max(longest, line);
+    }
+    // 2. chunks of whole lines, none smaller than the longest line
+    const int64_t cap = std::max(q->chunk_bytes ? q->chunk_bytes : kSeqChunkDefault, longest);
+    std::vector<int64_t> cut{0};
+    int64_t buf_bytes = 0;
+    for (int64_t r = 0; r < n;) {
+        const int64_t limit = line_off[(size_t)r] + cap;
+        int64_t r1 = std::upper_bound(line_off.begin() + r + 1, line_off.end(), limit) - line_off.begin() - 1;
+        r1 = std::min<int64_t>(r1, r + 0x7fffffff);
+        buf_bytes = std::max(buf_bytes, line_off[(size_t)r1] - line_off[(size_t)r]);
+        cut.push_back(r1);
+        r = r1;
+    }
+    // 3. the header, then the lines
+    DeviceGuard guard(ctx->device);
+    FILE* fh = fopen(path, "wb");
+    if (!fh) return fail(ctx, RT_EINVAL, "rt_orf_seq_write: cannot open %s", path);
+    static const char kHeader[] = "ORF_ID\tsequence\n";
+    int rc = fwrite(kHeader, 1, sizeof kHeader - 1, fh) == sizeof kHeader - 1
+                 ? RT_OK : fail(ctx, RT_EINVAL, "rt_orf_seq_write: cannot write %s", path);
+    if (rc == RT_OK) rc = seq_emit(ctx, q, line_off, cut, buf_bytes, fh, stage_ms);
+    if (fclose(fh) != 0 && rc == RT_OK) rc = fail(ctx, RT_EINVAL, "rt_orf_seq_write: cannot write %s", path);
+    if (rc != RT_OK) remove(path);
+    return rc;
 }
 
 }  // extern "C"

@@ -498,6 +498,22 @@ const char* rt_index_field(const rt_index* ix, int64_t orf, int k, int* len) {
     return ix->text + off;
 }
 
+// Field 0 (ORF_ID) of every row.  A row's first field runs from the end of the previous line (the header's for row 0)
+// to the tab before field 1.
+int rt_index_ids(const rt_index* ix, int64_t* off, char* blob) {
+    if (!ix || !off) return RT_EINVAL;
+    const int64_t n = (int64_t)ix->orf_chrom.size();
+    off[0] = 0;
+    for (int64_t o = 0; o < n; ++o) {
+        const char* end = ix->text + ix->line_field[o] - 1;
+        const char* p = end;
+        while (p > ix->text && p[-1] != '\n') --p;
+        if (blob) memcpy(blob + off[o], p, (size_t)(end - p));
+        off[o + 1] = off[o] + (end - p);
+    }
+    return RT_OK;
+}
+
 int rt_tsv_open(const char* path, int write_header, rt_tsv** out) {
     if (!path || !out) return RT_EINVAL;
     FILE* fh = fopen(path, "wb");

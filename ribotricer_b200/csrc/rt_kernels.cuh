@@ -2573,4 +2573,116 @@ __global__ void orf_interval_kernel(long long n_rows, const int* __restrict__ ro
     }
 }
 
+// ----------------------------------------------------------------------------------------------------- orfs-seq
+// The output lines of index rows [row_lo, row_lo + n_rows) (DESIGN.md section 10): "ORF_ID\tsequence\n" at
+// line_off[row] - line_off[row_lo] of `out`.  One warp per row, claimed dynamically (rows run from 3 nt to more than
+// 100 knt).  Nucleotides go straight from the contig codes to their oriented place.  For protein the warp stages the
+// oriented codes in a shared-memory window of kSeqWindow nt (a multiple of 3, so a codon never straddles two windows)
+// and each lane translates codons of it through a 64-entry table.
+struct SeqArgs {
+    const uint8_t* codes;
+    const long long* exon_ptr;
+    const int* ex_start;
+    const int* ex_end;
+    const int* contig;
+    const uint8_t* strand;            // 1: reverse complement
+    const long long* contig_base;
+    const long long* id_off;
+    const char* ids;
+    const long long* line_off;        // n_orf + 1: offset of every line after the header
+    unsigned* claim;                  // work counter, zeroed before every launch
+};
+
+constexpr int kSeqWarps = 8;
+constexpr int kSeqWindow = 3 * 32 * 8;
+
+template <bool Protein>
+__global__ void __launch_bounds__(kSeqWarps * 32) orf_seq_kernel(SeqArgs A, long long row_lo, long long n_rows,
+                                                                 char* __restrict__ out) {
+    __shared__ uint8_t window[Protein ? kSeqWarps : 1][Protein ? kSeqWindow : 1];
+    __shared__ char amino[64];
+    const int lane = threadIdx.x & 31;
+    if (Protein) {
+        // NCBI table 1, codon code 16 b0 + 4 b1 + b2 with A C G T = 0 1 2 3
+        if (threadIdx.x < 64) amino[threadIdx.x] = "KNKNTTTTRSRSIIMIQHQHPPPPRRRRLLLLEDEDAAAAGGGGVVVV*Y*YSSSS*CWCLFLF"[threadIdx.x];
+        __syncthreads();
+    }
+    uint8_t* win = window[Protein ? threadIdx.x >> 5 : 0];
+    const long long base = A.line_off[row_lo];
+    for (;;) {
+        unsigned t = 0;
+        if (lane == 0) t = atomicAdd(A.claim, 1u);
+        t = __shfl_sync(kFull, t, 0);
+        if ((long long)t >= n_rows) return;
+        const long long r = row_lo + t;
+        char* o = out + (A.line_off[r] - base);
+        const long long i0 = A.id_off[r], n_id = A.id_off[r + 1] - i0;
+        for (long long k = lane; k < n_id; k += 32) o[k] = A.ids[i0 + k];
+        o += n_id;
+        if (lane == 0) *o = '\t';
+        ++o;
+        const long long e0 = A.exon_ptr[r], e1 = A.exon_ptr[r + 1];
+        const uint8_t* g = A.codes + A.contig_base[A.contig[r]];
+        const bool rev = A.strand[r] == 1;
+        long long n_out;
+        if (!Protein) {
+            long long L = 0;
+            for (long long e = e0; e < e1; ++e) L += A.ex_end[e] - A.ex_start[e] + 1;
+            long long before = 0;                     // nt of the row's intervals left of interval e
+            for (long long e = e0; e < e1; ++e) {
+                const uint8_t* src = g + A.ex_start[e] - 1;
+                const int len = A.ex_end[e] - A.ex_start[e] + 1;
+                if (rev) {
+                    char* dst = o + (L - 1 - before);
+                    for (int k = lane; k < len; k += 32) {
+                        const uint8_t c = src[k];
+                        dst[-k] = c < 4 ? "TGCA"[c] : 'N';
+                    }
+                } else {
+                    char* dst = o + before;
+                    for (int k = lane; k < len; k += 32) {
+                        const uint8_t c = src[k];
+                        dst[k] = c < 4 ? "ACGT"[c] : 'N';
+                    }
+                }
+                before += len;
+            }
+            n_out = L;
+        } else {
+            int fill = 0;                             // oriented nt staged in the window
+            long long done = 0;                       // amino acids written
+            auto emit = [&](int n_codon) {
+                __syncwarp();
+                for (int c = lane; c < n_codon; c += 32) {
+                    const int a = win[3 * c], b = win[3 * c + 1], d = win[3 * c + 2];
+                    o[done + c] = (a | b | d) & 4 ? 'X' : amino[(a << 4) | (b << 2) | d];
+                }
+                __syncwarp();
+                done += n_codon;
+            };
+            for (long long j = 0; j < e1 - e0; ++j) {
+                const long long e = rev ? e1 - 1 - j : e0 + j;
+                const uint8_t* src = g + A.ex_start[e] - 1;
+                const int len = A.ex_end[e] - A.ex_start[e] + 1;
+                for (int k0 = 0; k0 < len;) {
+                    const int n = min(len - k0, kSeqWindow - fill);
+                    for (int k = lane; k < n; k += 32) {
+                        const uint8_t c = rev ? src[len - 1 - (k0 + k)] : src[k0 + k];
+                        win[fill + k] = c < 4 ? (rev ? (uint8_t)(3 - c) : c) : (uint8_t)4;
+                    }
+                    fill += n;
+                    k0 += n;
+                    if (fill == kSeqWindow) {
+                        emit(kSeqWindow / 3);
+                        fill = 0;
+                    }
+                }
+            }
+            emit(fill / 3);
+            n_out = done;
+        }
+        if (lane == 0) o[n_out] = '\n';
+    }
+}
+
 }  // namespace rt

@@ -477,3 +477,26 @@ class Engine:
         self._check(self.lib.rt_orf_fetch(self.ctx, *[_np_ptr(out[k]) for k in (
             "row_tx", "row_start", "row_stop", "row_type", "row_codon", "iv_ptr", "iv_start", "iv_end")]))
         return out
+
+    # --------------------------------------------------------------- orfs-seq
+    def orf_seq_write(self, path: str, exon_ptr, exon_start, exon_end, orf_contig, orf_strand, contig_base, contig_len,
+                      codes, id_off, ids, protein: bool, chunk_bytes: int = 0, stage_ms: np.ndarray | None = None):
+        """Write the sequence file of DESIGN.md section 10 (``rt_orf_seq_write``).  ``orf_contig`` indexes the contig
+        table ``contig_base`` / ``contig_len`` (offsets and lengths in ``codes``), ``orf_strand`` 1 = reverse,
+        ``id_off`` / ``ids`` the ORF_ID column.  A row the rules refuse raises ValueError and leaves no file."""
+        arr = lambda a, dt: np.ascontiguousarray(a, dt)  # noqa: E731
+        exon_ptr, exon_start, exon_end = arr(exon_ptr, np.int64), arr(exon_start, np.int32), arr(exon_end, np.int32)
+        orf_contig, orf_strand = arr(orf_contig, np.int32), arr(orf_strand, np.uint8)
+        contig_base, contig_len = arr(contig_base, np.int64), arr(contig_len, np.int64)
+        codes, id_off, ids = arr(codes, np.uint8), arr(id_off, np.int64), arr(ids, np.uint8)
+        q = _lib.SeqQuery(len(exon_ptr) - 1, _np_ptr(exon_ptr), _np_ptr(exon_start), _np_ptr(exon_end),
+                          _np_ptr(orf_contig), _np_ptr(orf_strand), len(contig_base), _np_ptr(contig_base),
+                          _np_ptr(contig_len), _np_ptr(codes), len(codes), _np_ptr(id_off), _np_ptr(ids),
+                          int(bool(protein)), int(chunk_bytes))
+        ms = np.zeros(_lib.RT_SEQ_STAGES, np.float32)
+        rc = self.lib.rt_orf_seq_write(self.ctx, C.byref(q), str(path).encode(), _np_ptr(ms))
+        if rc == _lib.RT_EINVAL:
+            raise ValueError(self.lib.rt_last_error(self.ctx).decode())
+        self._check(rc)
+        if stage_ms is not None:
+            stage_ms[:] = ms

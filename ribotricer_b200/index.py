@@ -205,6 +205,17 @@ class NativeIndex:
         return (self.field(o, 1), self.field(o, 2), self.field(o, 3), self.field(o, 4), self.field(o, 5),
                 self.field(o, 6), self.field(o, 9))
 
+    def ids(self):
+        """The ORF_ID column byte for byte (``rt_index_ids``): row o is ``blob[off[o]:off[o + 1]]`` (uint8)."""
+        import ctypes as C
+
+        p = lambda a: a.ctypes.data_as(C.c_void_p)  # noqa: E731
+        off = np.empty(self._n + 1, np.int64)
+        self._lib.rt_index_ids(self.handle, p(off), None)
+        blob = np.empty(max(1, int(off[-1])), np.uint8)
+        self._lib.rt_index_ids(self.handle, p(off), p(blob))
+        return off, blob[:int(off[-1])]
+
     def lengths(self) -> np.ndarray:
         exlen = self.exon_end.astype(np.int64) - self.exon_start + 1
         cs = np.concatenate([[0], np.cumsum(exlen)])

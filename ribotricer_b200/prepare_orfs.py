@@ -38,10 +38,10 @@ def codon_mask(codons) -> int:
     return mask
 
 
-def _refuse_gzip(path: str) -> None:
+def _refuse_gzip(path: str, command: str = "prepare-orfs") -> None:
     with open(path, "rb") as fh:
         if fh.read(2) == b"\x1f\x8b":
-            raise ValueError(f"{path} is gzip-compressed; prepare-orfs reads plain text only")
+            raise ValueError(f"{path} is gzip-compressed; {command} reads plain text only")
 
 
 def _np_ptr(a: np.ndarray):
