@@ -31,39 +31,17 @@
 #include <memory>
 #include <mutex>
 #include <string>
-#include <thread>
 #include <vector>
 
 #include "ribotricer_b200.h"
-
-// A column of the decoded library: plain uninitialised storage, so that the pages of a large library are first
-// touched by the threads that fill them and not by one thread zero-filling a std::vector.
-template <class T>
-struct Col {
-    T* p = nullptr;
-    size_t n = 0;
-    Col() = default;
-    Col(const Col&) = delete;
-    Col& operator=(const Col&) = delete;
-    ~Col() { free(p); }
-    bool alloc(size_t m) {
-        free(p);
-        p = static_cast<T*>(malloc(std::max<size_t>(m, 1) * sizeof(T)));
-        n = p ? m : 0;
-        return p != nullptr;
-    }
-    T* data() const { return p; }
-    size_t size() const { return n; }
-    T* begin() const { return p; }
-    T* end() const { return p + n; }
-};
+#include "rt_host.h"
 
 struct rt_bam {
     std::vector<std::string> ref_names;
     std::vector<int64_t> ref_lens;
-    Col<int32_t> ref_id, first, last, pos, ref_end;
-    Col<uint16_t> mlen, flag;
-    Col<uint8_t> mapq, nh;
+    HostArr<int32_t> ref_id, first, last, pos, ref_end;   // uninitialised: first touched by the threads that fill them
+    HostArr<uint16_t> mlen, flag;
+    HostArr<uint8_t> mapq, nh;
     bool sorted = false;
 };
 
@@ -271,19 +249,7 @@ int parse_header(const uint8_t* d, size_t n, rt_bam& bam, size_t& used) {
 template <class F>
 void parallel_slices(size_t n, const F& fn) {
     const size_t slice = 1u << 20, n_slices = (n + slice - 1) / slice;
-    const size_t n_threads = std::min<size_t>({n_slices, 16, std::max(1u, std::thread::hardware_concurrency())});
-    if (n_threads <= 1) {
-        if (n) fn(0, n);
-        return;
-    }
-    std::atomic<size_t> next{0};
-    auto run = [&]() {
-        for (size_t k; (k = next.fetch_add(1)) < n_slices;) fn(k * slice, std::min(n, (k + 1) * slice));
-    };
-    std::vector<std::thread> th;
-    for (size_t t = 1; t < n_threads; ++t) th.emplace_back(run);
-    run();
-    for (auto& x : th) x.join();
+    claim_parallel(host_threads(n_slices, 16), n_slices, [&](size_t k) { fn(k * slice, std::min(n, (k + 1) * slice)); });
 }
 
 }  // namespace
@@ -295,7 +261,7 @@ const char* rt_bam_last_error(void) { return g_bam_error.c_str(); }
 int rt_bam_load(const char* path, int n_threads, rt_bam** out) {
     if (!path || !out) return RT_EINVAL;
     *out = nullptr;
-    if (n_threads <= 0) n_threads = (int)std::max(1u, std::thread::hardware_concurrency());
+    if (n_threads <= 0) n_threads = host_threads(SIZE_MAX, SIZE_MAX);    // every hardware thread
     const int fd = open(path, O_RDONLY);
     if (fd < 0) { g_bam_error = std::string("cannot open ") + path; return RT_EINVAL; }
     struct stat st;
@@ -461,12 +427,7 @@ int rt_bam_load(const char* path, int n_threads, rt_bam** out) {
             set_fail("out of memory while decoding");
         }
     };
-    {
-        std::vector<std::thread> th;
-        for (int t = 1; t < n_threads; ++t) th.emplace_back(guarded);
-        guarded();
-        for (auto& x : th) x.join();
-    }
+    run_parallel(n_threads, [&](int) { guarded(); });
     if (size) munmap((void*)base, size);
     if (failed) { g_bam_error = fail_msg; return RT_EINVAL; }
     if (!cur.header_done) { g_bam_error = "truncated BAM header"; return RT_EINVAL; }
@@ -481,25 +442,16 @@ int rt_bam_load(const char* path, int n_threads, rt_bam** out) {
         g_bam_error = "out of memory";
         return RT_ENOMEM;
     }
-    std::atomic<size_t> next_out{0};
-    auto gather = [&]() {
-        for (size_t j; (j = next_out.fetch_add(1)) < done.size();) {
-            BatchOut& bo = done[j];
-            const ColView v = bo.view();
-            const size_t o = bo.base, m = bo.n;
-            memcpy(B.ref_id.p + o, v.ref_id, 4 * m); memcpy(B.first.p + o, v.first, 4 * m); memcpy(B.last.p + o, v.last, 4 * m);
-            memcpy(B.pos.p + o, v.pos, 4 * m); memcpy(B.ref_end.p + o, v.ref_end, 4 * m);
-            memcpy(B.mlen.p + o, v.mlen, 2 * m); memcpy(B.flag.p + o, v.flag, 2 * m);
-            memcpy(B.mapq.p + o, v.mapq, m); memcpy(B.nh.p + o, v.nh, m);
-            bo.mem.reset();
-        }
-    };
-    {
-        std::vector<std::thread> th;
-        for (int t = 1; t < n_threads && (size_t)t < done.size(); ++t) th.emplace_back(gather);
-        gather();
-        for (auto& x : th) x.join();
-    }
+    claim_parallel((int)std::min<size_t>((size_t)n_threads, done.size()), done.size(), [&](size_t j) {
+        BatchOut& bo = done[j];
+        const ColView v = bo.view();
+        const size_t o = bo.base, m = bo.n;
+        memcpy(B.ref_id.p + o, v.ref_id, 4 * m); memcpy(B.first.p + o, v.first, 4 * m); memcpy(B.last.p + o, v.last, 4 * m);
+        memcpy(B.pos.p + o, v.pos, 4 * m); memcpy(B.ref_end.p + o, v.ref_end, 4 * m);
+        memcpy(B.mlen.p + o, v.mlen, 2 * m); memcpy(B.flag.p + o, v.flag, 2 * m);
+        memcpy(B.mapq.p + o, v.mapq, m); memcpy(B.nh.p + o, v.nh, m);
+        bo.mem.reset();
+    });
     *out = bam.release();
     return RT_OK;
 }

@@ -7,14 +7,12 @@
 #include <cstring>
 #include <atomic>
 #include <chrono>
-#include <condition_variable>
-#include <deque>
 #include <mutex>
 #include <string>
 #include <unordered_map>
-#include <thread>
 #include <vector>
 
+#include "rt_host.h"
 #include "rt_kernels.cuh"
 
 // rt_host_io.cpp: one chunk of host columns as a run of record-stream blocks (-1: cannot be coded, -2: cap too small)
@@ -202,24 +200,18 @@ int build_atoms(rt_ctx* ctx, const std::vector<uint64_t>& desc, const std::vecto
         pts.push_back(off + len);
     }
     // a human index has 10^7 boundaries: the sort (chunks, then a tree of merges) and the look-ups below run on all cores
-    const int n_thr = (int)std::max<size_t>(1, std::min<size_t>({(size_t)std::thread::hardware_concurrency(), (size_t)16, pts.size() >> 16}));
+    const int n_thr = host_threads(pts.size() >> 16, 16);
     auto parallel_for = [&](size_t n_items, auto&& body) {          // body(lo, hi) on slices of [0, n_items)
-        std::vector<std::thread> pool;
-        for (int k = 1; k < n_thr; ++k) pool.emplace_back([&, k]() { body(n_items * k / n_thr, n_items * (k + 1) / n_thr); });
-        body(0, n_items / n_thr);
-        for (auto& th : pool) th.join();
+        run_parallel(n_thr, [&](int k) { body(n_items * k / n_thr, n_items * (k + 1) / n_thr); });
     };
     parallel_for(pts.size(), [&](size_t lo, size_t hi) { std::sort(pts.begin() + lo, pts.begin() + hi); });
-    for (int width = 1; width < n_thr; width *= 2) {
-        std::vector<std::thread> pool;
-        for (int k = 0; k + width < n_thr; k += 2 * width)
-            pool.emplace_back([&, k, width]() {
-                const size_t a = pts.size() * k / n_thr, m = pts.size() * (k + width) / n_thr;
-                const size_t b = pts.size() * std::min(k + 2 * width, n_thr) / n_thr;
-                std::inplace_merge(pts.begin() + a, pts.begin() + m, pts.begin() + b);
-            });
-        for (auto& th : pool) th.join();
-    }
+    for (int width = 1; width < n_thr; width *= 2)   // merge k = 0, 2w, 4w, ...: the runs [k, k + w) and [k + w, k + 2w)
+        run_parallel((n_thr + width - 1) / (2 * width), [&](int j) {
+            const int k = 2 * width * j;
+            const size_t a = pts.size() * k / n_thr, m = pts.size() * (k + width) / n_thr;
+            const size_t b = pts.size() * std::min(k + 2 * width, n_thr) / n_thr;
+            std::inplace_merge(pts.begin() + a, pts.begin() + m, pts.begin() + b);
+        });
     pts.erase(std::unique(pts.begin(), pts.end()), pts.end());
     // which elementary intervals [pts[i], pts[i+1]) are covered by an entry
     std::vector<int32_t> diff(pts.size() + 1, 0);
@@ -823,9 +815,9 @@ int rt_bin_reads_host(rt_ctx* ctx, int32_t* d_cov, int64_t n, const int32_t* h_r
                                       : std::min<int64_t>(kHostChunkReads, std::max<int64_t>(n, 1));
     const int64_t n_chunks = (n + chunk - 1) / chunk;
     // the delta coding is the bottleneck of this call (about 1.5 ns per read and thread): one pipeline per hardware thread
-    int64_t want_pipes = std::min<int64_t>(kMaxPipes, (int64_t)std::thread::hardware_concurrency());
-    if (const char* e = getenv("RT_PACK_PIPES")) want_pipes = std::min<int64_t>(kMaxPipes, std::max(1, atoi(e)));
-    const int n_pipes = use_stream ? (int)std::max<int64_t>(1, std::min<int64_t>(want_pipes, n_chunks)) : 2;
+    const int n_pipes = use_stream ? (int)std::max<int64_t>(1, std::min<int64_t>({host_threads((size_t)n_chunks, kMaxPipes, "RT_PACK_PIPES"),
+                                                                                 kMaxPipes, n_chunks}))
+                                   : 2;
     const bool timing = getenv("RT_HOST_TIMING") != nullptr;
     std::atomic<long long> pack_ns{0}, wait_ns{0}, issue_ns{0};
     const auto t_begin = std::chrono::steady_clock::now();
@@ -916,12 +908,7 @@ int rt_bin_reads_host(rt_ctx* ctx, int32_t* d_cov, int64_t n, const int32_t* h_r
             }
         }
     };
-    {
-        std::vector<std::thread> pipes;
-        for (int s = 1; s < n_pipes; ++s) pipes.emplace_back(pipeline, s);
-        pipeline(0);
-        for (auto& th : pipes) th.join();
-    }
+    run_parallel(n_pipes, pipeline);
     if (status.load() != RT_OK) return first_error.empty() ? status.load() : fail(ctx, status.load(), "rt_bin_reads_host: %s", first_error.c_str());
     const auto t_issued = std::chrono::steady_clock::now();
     for (int s = 0; s < n_pipes; ++s) {
@@ -1332,13 +1319,7 @@ int prebuild_plans(rt_ctx* ctx, const std::vector<int64_t>& cut) {
         }
     }
     if (todo.size() < 2) return RT_OK;           // get_plan does a single one just as well
-    {
-        std::vector<std::thread> pool;
-        for (size_t k = 1; k < todo.size(); ++k)
-            pool.emplace_back([ctx, &todo, k]() { build_plan_host(ctx, todo[k].lo, todo[k].hi, todo[k]); });
-        build_plan_host(ctx, todo[0].lo, todo[0].hi, todo[0]);
-        for (auto& th : pool) th.join();
-    }
+    run_parallel((int)todo.size(), [&](int k) { build_plan_host(ctx, todo[(size_t)k].lo, todo[(size_t)k].hi, todo[(size_t)k]); });
     for (PlanHost& ph : todo) {
         rt_ctx::ScorePlan* unused = nullptr;
         const int rc = upload_plan(ctx, ph, &unused);
@@ -1866,65 +1847,16 @@ enum SeqBuf { kSqCodes, kSqExPtr, kSqExStart, kSqExEnd, kSqContig, kSqStrand, kS
 static_assert(kSeqBufs <= 16, "rt_ctx::seq_buf is too small");
 constexpr int64_t kSeqChunkDefault = int64_t(64) << 20;
 
-// Writes the chunks handed to it, in order, on its own thread; `written` counts the chunks it has finished.
-struct SeqWriter {
-    FILE* fh = nullptr;
-    std::mutex m;
-    std::condition_variable cv;
-    std::deque<std::pair<const char*, size_t>> todo;
-    int64_t written = 0;
-    bool stop = false, failed = false;
-    std::thread th;
-    void run() {
-        for (;;) {
-            std::pair<const char*, size_t> job;
-            {
-                std::unique_lock<std::mutex> lk(m);
-                cv.wait(lk, [&] { return stop || !todo.empty(); });
-                if (todo.empty()) return;
-                job = todo.front();
-                todo.pop_front();
-            }
-            const bool ok = fwrite(job.first, 1, job.second, fh) == job.second;
-            {
-                std::lock_guard<std::mutex> lk(m);
-                failed = failed || !ok;
-                ++written;
-            }
-            cv.notify_all();
-        }
-    }
-    void push(const char* p, size_t n) {
-        {
-            std::lock_guard<std::mutex> lk(m);
-            todo.emplace_back(p, n);
-        }
-        cv.notify_all();
-    }
-    bool wait_written(int64_t k) {   // false once a write has failed
-        std::unique_lock<std::mutex> lk(m);
-        cv.wait(lk, [&] { return written >= k || failed; });
-        return !failed;
-    }
-    void finish() {
-        {
-            std::lock_guard<std::mutex> lk(m);
-            stop = true;
-        }
-        cv.notify_all();
-        if (th.joinable()) th.join();
-    }
-};
-
 // Streams, events, page-locked buffers and the writer of one rt_orf_seq_write call; the destructor joins the writer and
 // waits for both streams before anything is freed, so every early return leaves nothing behind.
 struct SeqPipeline {
     cudaStream_t ks = nullptr, cs = nullptr;   // kernels + uploads, copy-back
     cudaEvent_t ev[10] = {};                   // upload begin / end, then per buffer b: kernel begin/end, copy begin/end
     char* pinned[2] = {};
-    SeqWriter writer;
+    WriteBehind writer;
+    explicit SeqPipeline(FILE* fh) : writer(fh) {}
     ~SeqPipeline() {
-        writer.finish();
+        writer.finish();                       // before the page-locked buffers it writes from are freed
         if (ks) cudaStreamSynchronize(ks);
         if (cs) cudaStreamSynchronize(cs);
         for (char* p : pinned)
@@ -1953,7 +1885,7 @@ int seq_emit(rt_ctx* ctx, const rt_seq_query* q, const std::vector<int64_t>& lin
     RT_CUDA(ctx, reserve(kSqIds, (size_t)n_ids));
     RT_CUDA(ctx, reserve(kSqLineOff, 8 * (size_t)(n + 1)));
     RT_CUDA(ctx, reserve(kSqClaim, 4));
-    SeqPipeline P;
+    SeqPipeline P(fh);
     RT_CUDA(ctx, cudaStreamCreateWithFlags(&P.ks, cudaStreamNonBlocking));
     RT_CUDA(ctx, cudaStreamCreateWithFlags(&P.cs, cudaStreamNonBlocking));
     for (auto& e : P.ev) RT_CUDA(ctx, cudaEventCreate(&e));
@@ -1985,8 +1917,6 @@ int seq_emit(rt_ctx* ctx, const rt_seq_query* q, const std::vector<int64_t>& lin
         RT_CUDA(ctx, reserve(kSqOut0 + b, (size_t)buf_bytes));
         RT_CUDA(ctx, cudaHostAlloc((void**)&P.pinned[b], (size_t)buf_bytes, cudaHostAllocDefault));
     }
-    P.writer.fh = fh;
-    P.writer.th = std::thread([&P] { P.writer.run(); });
     const rt::SeqArgs A{(const uint8_t*)B[kSqCodes].p, (const long long*)B[kSqExPtr].p, (const int*)B[kSqExStart].p,
                         (const int*)B[kSqExEnd].p, (const int*)B[kSqContig].p, (const uint8_t*)B[kSqStrand].p,
                         (const long long*)B[kSqBase].p, (const long long*)B[kSqIdOff].p, (const char*)B[kSqIds].p,
@@ -2004,7 +1934,7 @@ int seq_emit(rt_ctx* ctx, const rt_seq_query* q, const std::vector<int64_t>& lin
             stage_ms[1] += kms;
             stage_ms[2] += cms;
         }
-        P.writer.push(P.pinned[b], bytes_of(k));
+        if (!P.writer.put_view(P.pinned[b], bytes_of(k))) return fail(ctx, RT_EINVAL, "rt_orf_seq_write: write error");
         return RT_OK;
     };
     for (int64_t k = 0; k < n_chunks; ++k) {

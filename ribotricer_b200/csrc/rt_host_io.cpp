@@ -4,23 +4,15 @@
 //   * {prefix}_translating_ORFs.tsv writer: rows formatted exactly as detect_orfs.py:304-323 prints
 //     them (np.float64 / Python float shortest repr, str(list) profile).
 // No GPU is involved; these entry points also work on a CPU-only box.
-#include <fcntl.h>
-#include <sys/stat.h>
-#include <unistd.h>
-
 #include <algorithm>
 #include <atomic>
 #include <charconv>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
-#include <condition_variable>
 #include <cstring>
-#include <deque>
 #include <memory>
-#include <mutex>
 #include <string>
-#include <thread>
 #include <unordered_map>
 #include <vector>
 
@@ -29,130 +21,26 @@
 #endif
 
 #include "ribotricer_b200.h"
-
-// A column of the parsed index: plain uninitialised storage (the threads that fill a large array also touch its pages
-// first; a std::vector would have one thread zero-fill it)
-template <class T>
-struct Arr {
-    T* p = nullptr;
-    size_t n = 0;
-    Arr() = default;
-    Arr(const Arr&) = delete;
-    Arr& operator=(const Arr&) = delete;
-    ~Arr() { free(p); }
-    bool alloc(size_t m) {
-        free(p);
-        p = static_cast<T*>(malloc(std::max<size_t>(m, 1) * sizeof(T)));
-        n = p ? m : 0;
-        return p != nullptr;
-    }
-    T& operator[](size_t i) { return p[i]; }
-    const T& operator[](size_t i) const { return p[i]; }
-    T* data() const { return p; }
-    size_t size() const { return n; }
-    T* begin() const { return p; }
-    T* end() const { return p + n; }
-};
+#include "rt_host.h"
 
 struct rt_index {
-    char* text = nullptr;                // the whole file (malloc); fields point into it
-    size_t text_size = 0;
-    ~rt_index() { free(text); }
-    Arr<int64_t> exon_ptr;               // n_orf + 1
-    Arr<int32_t> exon_start, exon_end;
-    Arr<int32_t> orf_chrom;              // index into chrom_names
-    Arr<uint8_t> orf_strand;             // 0 '+', 1 '-', 2 anything else
-    Arr<uint32_t> field_len;             // 9 per ORF: lengths of fields 1..9
-    Arr<uint64_t> line_field;            // per ORF: offset of field 1 (64-bit, files > 4 GB)
+    HostArr<char> text;                  // the whole file; fields point into it
+    HostArr<int64_t> exon_ptr;           // n_orf + 1
+    HostArr<int32_t> exon_start, exon_end;
+    HostArr<int32_t> orf_chrom;          // index into chrom_names
+    HostArr<uint8_t> orf_strand;         // 0 '+', 1 '-', 2 anything else
+    HostArr<uint32_t> field_len;         // 9 per ORF: lengths of fields 1..9
+    HostArr<uint64_t> line_field;        // per ORF: offset of field 1 (64-bit, files > 4 GB)
     std::vector<std::string> chrom_names;
     int64_t n_annotated_prefix = 0;
     std::string error;
 };
 
-// Text under construction: a growable char buffer written through a raw pointer (no per-character capacity checks).
-struct TextBuf {
-    char* base = nullptr;
-    size_t len = 0, cap = 0;
-    TextBuf() = default;
-    TextBuf(TextBuf&& o) noexcept : base(o.base), len(o.len), cap(o.cap) { o.base = nullptr; o.len = o.cap = 0; }
-    TextBuf& operator=(TextBuf&& o) noexcept {
-        if (this != &o) { free(base); base = o.base; len = o.len; cap = o.cap; o.base = nullptr; o.len = o.cap = 0; }
-        return *this;
-    }
-    TextBuf(const TextBuf&) = delete;
-    TextBuf& operator=(const TextBuf&) = delete;
-    ~TextBuf() { free(base); }
-    // room for n more bytes; returns where to write them (nullptr: out of memory)
-    char* need(size_t n) {
-        if (cap - len < n) {
-            const size_t want = std::max(len + n, cap + cap / 2 + (1u << 16));
-            char* q = static_cast<char*>(realloc(base, want));
-            if (!q) return nullptr;
-            base = q;
-            cap = want;
-        }
-        return base + len;
-    }
-    void advance_to(char* p) { len = (size_t)(p - base); }
-    void append(const char* d, size_t n) {
-        if (char* p = need(n)) { memcpy(p, d, n); len += n; }
-    }
-};
-
-// An output file with a write-behind thread: formatted text is queued and written in order while the caller formats
-// the next piece (or waits for the GPU).  At most kPendingMax bytes wait in the queue.
+// An output file (TSV or WIG) with its write-behind thread.
 struct rt_tsv {
-    FILE* fh = nullptr;
-    std::thread writer;
-    std::mutex mu;
-    std::condition_variable cv;
-    std::deque<TextBuf> queue;
-    size_t pending = 0;
-    bool closing = false, failed = false;
-    static constexpr size_t kPendingMax = 1ull << 30;
-
-    void run() {
-        std::unique_lock<std::mutex> lk(mu);
-        for (;;) {
-            cv.wait(lk, [&] { return closing || !queue.empty(); });
-            if (queue.empty()) return;
-            TextBuf b = std::move(queue.front());
-            queue.pop_front();
-            lk.unlock();
-            const bool ok = b.len == 0 || fwrite(b.base, 1, b.len, fh) == b.len;
-            lk.lock();
-            pending -= b.len;
-            if (!ok) failed = true;
-            cv.notify_all();
-        }
-    }
-    // false when an earlier write has failed
-    bool put(TextBuf&& b) {
-        std::unique_lock<std::mutex> lk(mu);
-        if (failed) return false;
-        if (b.len == 0) return true;
-        if (!writer.joinable()) writer = std::thread([this] { run(); });
-        cv.wait(lk, [&] { return pending < kPendingMax || failed; });
-        pending += b.len;
-        queue.push_back(std::move(b));
-        cv.notify_all();
-        return !failed;
-    }
-    bool put(const std::string& s) {
-        TextBuf b;
-        b.append(s.data(), s.size());
-        return b.len == s.size() && put(std::move(b));
-    }
-    // drains the queue and stops the thread; false when any write failed
-    bool finish() {
-        {
-            std::lock_guard<std::mutex> lk(mu);
-            closing = true;
-        }
-        cv.notify_all();
-        if (writer.joinable()) writer.join();
-        return !failed;
-    }
+    FILE* fh;
+    WriteBehind out;
+    explicit rt_tsv(FILE* f) : fh(f), out(f) {}
 };
 
 namespace {
@@ -198,29 +86,6 @@ void append_repr(std::string& out, double x) {
     }
 }
 
-// Decimal digits of v at p; returns the end.  Coverage profiles are mostly one-digit numbers.
-inline char* put_int(char* p, long long v) {
-    static const char pairs[] =
-        "00010203040506070809101112131415161718192021222324252627282930313233343536373839404142434445464748495051525354555657585960616263"
-        "646566676869707172737475767778798081828384858687888990919293949596979899";
-    unsigned long long u = (unsigned long long)v;
-    if (v < 0) { *p++ = '-'; u = 0ull - u; }
-    if (u < 10) { *p++ = (char)('0' + u); return p; }
-    if (u < 100) { memcpy(p, pairs + 2 * u, 2); return p + 2; }
-    char tmp[24];
-    int k = 24;
-    while (u >= 100) {
-        const unsigned r = (unsigned)(u % 100);
-        u /= 100;
-        k -= 2;
-        memcpy(tmp + k, pairs + 2 * r, 2);
-    }
-    if (u >= 10) { k -= 2; memcpy(tmp + k, pairs + 2 * u, 2); }
-    else tmp[--k] = (char)('0' + u);
-    memcpy(p, tmp + k, (size_t)(24 - k));
-    return p + (24 - k);
-}
-
 bool parse_int(const char*& p, const char* end, long long& v) {   // Python int(): optional blanks and sign
     while (p < end && (*p == ' ')) ++p;
     bool neg = false;
@@ -248,41 +113,15 @@ extern "C" {
 int rt_index_load(const char* path, rt_index** out) {
     if (!path || !out) return RT_EINVAL;
     *out = nullptr;
-    const int fd = open(path, O_RDONLY);
-    if (fd < 0) { g_io_error = std::string("cannot open ") + path; return RT_EINVAL; }
-    struct stat st;
-    if (fstat(fd, &st) != 0) { close(fd); g_io_error = std::string("cannot stat ") + path; return RT_EINVAL; }
-    const size_t size = (size_t)st.st_size;
     std::unique_ptr<rt_index> ix(new rt_index());
-    ix->text = static_cast<char*>(malloc(size + 1));
-    if (!ix->text) { close(fd); g_io_error = "out of memory"; return RT_ENOMEM; }
-    ix->text_size = size;
-    int n_thr = (int)std::max<size_t>(1, std::min<size_t>({(size_t)std::thread::hardware_concurrency(), (size_t)16, size >> 22}));
-    if (const char* e = getenv("RT_INDEX_THREADS")) n_thr = std::max(1, std::min(64, atoi(e)));   // tests: chunked parse of a small file
-    // 1. the file, read in slices by all threads (the buffer's pages are first touched by the thread that fills them)
-    {
-        std::atomic<bool> ok{true};
-        auto read_slice = [&](int k) {
-            size_t at = size * (size_t)k / n_thr;
-            const size_t hi = size * (size_t)(k + 1) / n_thr;
-            while (at < hi) {
-                const ssize_t got = pread(fd, ix->text + at, hi - at, (off_t)at);
-                if (got <= 0) { ok = false; return; }
-                at += (size_t)got;
-            }
-        };
-        std::vector<std::thread> pool;
-        for (int k = 1; k < n_thr; ++k) pool.emplace_back(read_slice, k);
-        read_slice(0);
-        for (auto& th : pool) th.join();
-        close(fd);
-        if (!ok) { g_io_error = "short read"; return RT_EINVAL; }
-    }
-    ix->text[size] = '\0';
-    const char* base = ix->text;
+    // 1. the file, read in slices by all threads
+    if (const int rc = read_file(path, ix->text)) return rc;
+    const size_t size = ix->text.size();
+    const char* base = ix->text.data();
     const char* end = base + size;
     const char* body = (const char*)memchr(base, '\n', size);   // skip the header (detect_orfs.py:273)
     body = body ? body + 1 : end;
+    const int n_thr = host_threads(size >> 22, 16, "RT_INDEX_THREADS");   // tests: chunked parse of a small file
 
     // 2. the rows, parsed in chunks cut at line ends
     struct Chunk {
@@ -298,22 +137,8 @@ int rt_index_load(const char* path, rt_index** out) {
         int64_t err_row = 0;
     };
     std::vector<Chunk> chunks((size_t)n_thr);
-    {
-        const size_t span = (size_t)(end - body);
-        const char* lo = body;
-        for (int k = 0; k < n_thr; ++k) {
-            const char* hi = end;
-            if (k + 1 < n_thr) {
-                const char* guess = body + span * (size_t)(k + 1) / n_thr;
-                if (guess < lo) guess = lo;
-                const char* nl = guess < end ? (const char*)memchr(guess, '\n', (size_t)(end - guess)) : nullptr;
-                hi = nl ? nl + 1 : end;
-            }
-            chunks[(size_t)k].lo = lo;
-            chunks[(size_t)k].hi = hi;
-            lo = hi;
-        }
-    }
+    const std::vector<const char*> cut = cut_lines(body, end, n_thr);
+    for (int k = 0; k < n_thr; ++k) { chunks[(size_t)k].lo = cut[(size_t)k]; chunks[(size_t)k].hi = cut[(size_t)k + 1]; }
     auto parse_chunk = [&](Chunk& ck) {
         std::unordered_map<std::string, int> chrom_id;
         std::vector<std::pair<long long, long long>> ivs;
@@ -377,12 +202,7 @@ int rt_index_load(const char* path, rt_index** out) {
             p = line_end + 1;
         }
     };
-    {
-        std::vector<std::thread> pool;
-        for (int k = 1; k < n_thr; ++k) pool.emplace_back([&, k]() { parse_chunk(chunks[(size_t)k]); });
-        parse_chunk(chunks[0]);
-        for (auto& th : pool) th.join();
-    }
+    run_parallel(n_thr, [&](int k) { parse_chunk(chunks[(size_t)k]); });
     // 3. the first error in file order, as the row-by-row loop of the reference would meet it
     {
         int64_t rows_before = 0;
@@ -429,7 +249,8 @@ int rt_index_load(const char* path, rt_index** out) {
         return RT_ENOMEM;
     }
     ix->exon_ptr[0] = 0;
-    auto merge_chunk = [&](size_t k) {
+    run_parallel(n_thr, [&](int kk) {
+        const size_t k = (size_t)kk;
         Chunk& ck = chunks[k];
         const size_t r0 = row0[k], e0 = exon0[k], m = ck.n_exon.size();
         if (!ck.exon_start.empty()) {
@@ -450,13 +271,7 @@ int rt_index_load(const char* path, rt_index** out) {
         Chunk().exon_start.swap(ck.exon_start);        // give the chunk's memory back early
         Chunk().exon_end.swap(ck.exon_end);
         Chunk().field_len.swap(ck.field_len);
-    };
-    {
-        std::vector<std::thread> pool;
-        for (size_t k = 1; k < chunks.size(); ++k) pool.emplace_back(merge_chunk, k);
-        merge_chunk(0);
-        for (auto& th : pool) th.join();
-    }
+    });
     *out = ix.release();
     return RT_OK;
 }
@@ -474,18 +289,19 @@ int rt_index_copy(const rt_index* ix, int64_t* exon_ptr, int32_t* exon_start, in
                   uint8_t* orf_strand) {
     if (!ix) return RT_EINVAL;
     // one thread per column when the index is large (the destination is usually fresh memory)
-    std::vector<std::thread> pool;
+    struct Copy { void* dst; const void* src; size_t bytes; };
+    std::vector<Copy> big;
     auto copy = [&](void* dst, const void* src, size_t bytes) {
         if (!dst || !bytes) return;
         if (bytes < (1u << 22)) memcpy(dst, src, bytes);
-        else pool.emplace_back([=]() { memcpy(dst, src, bytes); });
+        else big.push_back({dst, src, bytes});
     };
     copy(exon_ptr, ix->exon_ptr.p, 8 * ix->exon_ptr.n);
     copy(exon_start, ix->exon_start.p, 4 * ix->exon_start.n);
     copy(exon_end, ix->exon_end.p, 4 * ix->exon_end.n);
     copy(orf_chrom, ix->orf_chrom.p, 4 * ix->orf_chrom.n);
     copy(orf_strand, ix->orf_strand.p, ix->orf_strand.n);
-    for (auto& th : pool) th.join();
+    run_parallel((int)big.size(), [&](int k) { memcpy(big[(size_t)k].dst, big[(size_t)k].src, big[(size_t)k].bytes); });
     return RT_OK;
 }
 
@@ -495,7 +311,7 @@ const char* rt_index_field(const rt_index* ix, int64_t orf, int k, int* len) {
     uint64_t off = ix->line_field[orf];
     for (int j = 1; j < k; ++j) off += ix->field_len[9 * orf + (j - 1)] + 1;
     if (len) *len = (int)ix->field_len[9 * orf + (k - 1)];
-    return ix->text + off;
+    return ix->text.data() + off;
 }
 
 // Field 0 (ORF_ID) of every row.  A row's first field runs from the end of the previous line (the header's for row 0)
@@ -505,9 +321,9 @@ int rt_index_ids(const rt_index* ix, int64_t* off, char* blob) {
     const int64_t n = (int64_t)ix->orf_chrom.size();
     off[0] = 0;
     for (int64_t o = 0; o < n; ++o) {
-        const char* end = ix->text + ix->line_field[o] - 1;
+        const char* end = ix->text.data() + ix->line_field[o] - 1;
         const char* p = end;
-        while (p > ix->text && p[-1] != '\n') --p;
+        while (p > ix->text.data() && p[-1] != '\n') --p;
         if (blob) memcpy(blob + off[o], p, (size_t)(end - p));
         off[o + 1] = off[o] + (end - p);
     }
@@ -518,8 +334,7 @@ int rt_tsv_open(const char* path, int write_header, rt_tsv** out) {
     if (!path || !out) return RT_EINVAL;
     FILE* fh = fopen(path, "wb");
     if (!fh) { g_io_error = std::string("cannot open ") + path; return RT_EINVAL; }
-    rt_tsv* t = new rt_tsv();
-    t->fh = fh;
+    rt_tsv* t = new rt_tsv(fh);
     if (write_header)   // detect_orfs.py:241-260
         fputs("ORF_ID\tORF_type\tstatus\tphase_score\tread_count\tlength\tvalid_codons\tvalid_codons_ratio\t"
               "read_density\ttranscript_id\ttranscript_type\tgene_id\tgene_name\tgene_type\tchrom\tstrand\t"
@@ -617,8 +432,7 @@ int rt_tsv_write(rt_tsv* t, const rt_index* ix, int64_t n_sel, const int64_t* or
     // the profile column is most of the text: rows are formatted by several threads in slices balanced by
     // profile length, and handed in order to the file's write-behind thread
     const int64_t total = n_sel ? prof_ptr[n_sel] - prof_ptr[0] : 0;
-    const int n_thr = (int)std::max<int64_t>(1, std::min<int64_t>({(int64_t)std::thread::hardware_concurrency(), (int64_t)16,
-                                                                  (total + n_sel * 40) / (1 << 21)}));
+    const int n_thr = host_threads((size_t)((total + n_sel * 40) / (1 << 21)), 16);
     std::vector<int64_t> cut(n_thr + 1, n_sel);
     cut[0] = 0;
     for (int k = 1; k < n_thr; ++k) {
@@ -628,23 +442,19 @@ int rt_tsv_write(rt_tsv* t, const rt_index* ix, int64_t n_sel, const int64_t* or
     }
     std::vector<TextBuf> parts(n_thr);
     std::vector<char> ok(n_thr, 1);
-    std::vector<std::thread> pool;
-    for (int k = 1; k < n_thr; ++k)
-        pool.emplace_back([&, k]() {
-            ok[k] = format_rows(parts[k], ix, cut[k], cut[k + 1], orf_ids, orf_lo, score, valid, count, length, status, prof_ptr, prof);
-        });
-    ok[0] = format_rows(parts[0], ix, cut[0], cut[1], orf_ids, orf_lo, score, valid, count, length, status, prof_ptr, prof);
-    for (auto& th : pool) th.join();
+    run_parallel(n_thr, [&](int k) {
+        ok[k] = format_rows(parts[k], ix, cut[k], cut[k + 1], orf_ids, orf_lo, score, valid, count, length, status, prof_ptr, prof);
+    });
     for (int k = 0; k < n_thr; ++k)
         if (!ok[k]) { g_io_error = "rt_tsv_write: ORF id outside the index or the result range, or out of memory"; return RT_EINVAL; }
     for (int k = 0; k < n_thr; ++k)
-        if (!t->put(std::move(parts[k]))) { g_io_error = "rt_tsv_write: write failed"; return RT_EINVAL; }
+        if (!t->out.put(std::move(parts[k]))) { g_io_error = "rt_tsv_write: write failed"; return RT_EINVAL; }
     return RT_OK;
 }
 
 int rt_tsv_close(rt_tsv* t) {
     if (!t) return RT_EINVAL;
-    const bool wrote = t->finish();
+    const bool wrote = t->out.finish();
     const int rc = fclose(t->fh);
     delete t;
     if (!wrote || rc != 0) g_io_error = "write failed (disk full?)";
@@ -677,39 +487,30 @@ extern "C" int rt_metagene_sums(const int32_t* flat, const int64_t* ptr, int64_t
     const int64_t kBlock = 2048, n_blocks = (n_rows + kBlock - 1) / kBlock, w = width;
     std::vector<double> sums((size_t)(n_blocks * 2 * w), 0.0);
     std::vector<int64_t> cnts((size_t)(n_blocks * 2 * w), 0);
-    std::atomic<int64_t> next{0};
-    auto run = [&]() {
-        for (int64_t b; (b = next.fetch_add(1)) < n_blocks;) {
-            double* s5 = sums.data() + (size_t)(b * 2 * w);
-            double* s3 = s5 + w;
-            int64_t* c5 = cnts.data() + (size_t)(b * 2 * w);
-            int64_t* c3 = c5 + w;
-            for (int64_t i = b * kBlock; i < std::min(n_rows, (b + 1) * kBlock); ++i) {
-                const int32_t* row = flat + ptr[i];
-                const int64_t len = ptr[i + 1] - ptr[i];
-                long long total = 0;
-                for (int64_t k = 0; k < len; ++k) total += row[k];
-                if (len == 0) continue;
-                const double mean = (double)total / (double)len;
-                if (!(mean > 0)) continue;                       // metagene.py:216: ORFs without reads are skipped
-                const int64_t shift = w - len;
-                for (int64_t k = 0; k < len; ++k) {
-                    const double v = (double)row[k] / mean;
-                    s5[k] += v;
-                    s3[shift + k] += v;
-                    c5[k]++;
-                    c3[shift + k]++;
-                }
+    claim_parallel(host_threads((size_t)n_blocks, 16), (size_t)n_blocks, [&](size_t bb) {
+        const int64_t b = (int64_t)bb;
+        double* s5 = sums.data() + (size_t)(b * 2 * w);
+        double* s3 = s5 + w;
+        int64_t* c5 = cnts.data() + (size_t)(b * 2 * w);
+        int64_t* c3 = c5 + w;
+        for (int64_t i = b * kBlock; i < std::min(n_rows, (b + 1) * kBlock); ++i) {
+            const int32_t* row = flat + ptr[i];
+            const int64_t len = ptr[i + 1] - ptr[i];
+            long long total = 0;
+            for (int64_t k = 0; k < len; ++k) total += row[k];
+            if (len == 0) continue;
+            const double mean = (double)total / (double)len;
+            if (!(mean > 0)) continue;                       // metagene.py:216: ORFs without reads are skipped
+            const int64_t shift = w - len;
+            for (int64_t k = 0; k < len; ++k) {
+                const double v = (double)row[k] / mean;
+                s5[k] += v;
+                s3[shift + k] += v;
+                c5[k]++;
+                c3[shift + k]++;
             }
         }
-    };
-    {
-        const int n_thr = (int)std::max<int64_t>(1, std::min<int64_t>({(int64_t)std::thread::hardware_concurrency(), (int64_t)16, n_blocks}));
-        std::vector<std::thread> pool;
-        for (int t = 1; t < n_thr; ++t) pool.emplace_back(run);
-        run();
-        for (auto& th : pool) th.join();
-    }
+    });
     for (int64_t k = 0; k < w; ++k) { start_sum[k] = stop_sum[k] = 0.0; start_cnt[k] = stop_cnt[k] = 0; }
     for (int64_t b = 0; b < n_blocks; ++b) {
         const double* s5 = sums.data() + (size_t)(b * 2 * w);
@@ -749,22 +550,19 @@ int rt_wig_block(rt_tsv* t, const char* chrom, int64_t n, const int64_t* pos, co
     head.append(title.data(), title.size());
     // a long block (a human chromosome holds millions of covered positions) is formatted by several threads, a slice of
     // the block each; the pieces go to the write-behind thread in order
-    const int n_thr = (int)std::max<int64_t>(1, std::min<int64_t>({(int64_t)std::thread::hardware_concurrency(), (int64_t)16, n >> 16}));
+    const int n_thr = host_threads((size_t)(n >> 16), 16);
     if (n_thr == 1) {
-        if (!lines(head, 0, n) || !t->put(std::move(head))) return RT_EINVAL;
+        if (!lines(head, 0, n) || !t->out.put(std::move(head))) return RT_EINVAL;
         return RT_OK;
     }
     std::vector<TextBuf> part((size_t)n_thr);
     std::vector<char> ok((size_t)n_thr, 1);
-    std::vector<std::thread> pool;
-    for (int k = 0; k < n_thr; ++k)
-        pool.emplace_back([&, k]() { ok[(size_t)k] = lines(part[(size_t)k], n * k / n_thr, n * (k + 1) / n_thr); });
-    for (auto& th : pool) th.join();
+    run_parallel(n_thr, [&](int k) { ok[(size_t)k] = lines(part[(size_t)k], n * k / n_thr, n * (k + 1) / n_thr); });
     for (char c : ok)
         if (!c) return RT_EINVAL;
-    if (!t->put(std::move(head))) return RT_EINVAL;
+    if (!t->out.put(std::move(head))) return RT_EINVAL;
     for (TextBuf& o : part)
-        if (!t->put(std::move(o))) return RT_EINVAL;
+        if (!t->out.put(std::move(o))) return RT_EINVAL;
     return RT_OK;
 }
 
@@ -954,34 +752,25 @@ int rt_stream_pack(int64_t n, const int32_t* ref_id, const int32_t* first, const
     if (n < 0 || !n_blocks || (n > 0 && (!ref_id || !first || !last || !mlen || !flag || !mapq || !nh)) || (records && !hdr))
         return RT_EINVAL;
     const int64_t n_ranges = (n + RT_STREAM_RANGE - 1) / RT_STREAM_RANGE;
-    if (n_threads <= 0) n_threads = (int)std::thread::hardware_concurrency();
-    n_threads = (int)std::max<int64_t>(1, std::min<int64_t>(n_threads, n_ranges));
+    n_threads = n_threads > 0 ? (int)std::max<int64_t>(1, std::min<int64_t>(n_threads, n_ranges)) : host_threads((size_t)n_ranges, SIZE_MAX);
     std::vector<int64_t> blocks(n_ranges + 1, 0);
     auto sweep = [&](bool write) {
-        std::atomic<int64_t> next{0};
         std::atomic<int64_t> worst{0};
-        auto work = [&]() {
-            for (;;) {
-                const int64_t r = next.fetch_add(1);
-                if (r >= n_ranges) break;
-                const int64_t at = r * RT_STREAM_RANGE, m = std::min<int64_t>(RT_STREAM_RANGE, n - at);
-                int64_t got;
-                if (write)
-                    got = rt_stream_pack_range(ref_id + at, first + at, last + at, mlen + at, flag + at, mapq + at, nh + at, m,
-                                               records + blocks[r] * RT_STREAM_BLOCK, hdr + 4 * blocks[r], blocks[r + 1] - blocks[r]);
-                else
-                    got = blocks[r + 1] = rt_stream_pack_range(ref_id + at, first + at, last + at, mlen + at, flag + at, mapq + at,
-                                                               nh + at, m, nullptr, nullptr, 0);
-                if (got < 0) {
-                    int64_t seen = worst.load();
-                    while (got < seen && !worst.compare_exchange_weak(seen, got)) {}
-                }
+        claim_parallel(n_threads, (size_t)n_ranges, [&](size_t rr) {
+            const int64_t r = (int64_t)rr;
+            const int64_t at = r * RT_STREAM_RANGE, m = std::min<int64_t>(RT_STREAM_RANGE, n - at);
+            int64_t got;
+            if (write)
+                got = rt_stream_pack_range(ref_id + at, first + at, last + at, mlen + at, flag + at, mapq + at, nh + at, m,
+                                           records + blocks[r] * RT_STREAM_BLOCK, hdr + 4 * blocks[r], blocks[r + 1] - blocks[r]);
+            else
+                got = blocks[r + 1] = rt_stream_pack_range(ref_id + at, first + at, last + at, mlen + at, flag + at, mapq + at,
+                                                           nh + at, m, nullptr, nullptr, 0);
+            if (got < 0) {
+                int64_t seen = worst.load();
+                while (got < seen && !worst.compare_exchange_weak(seen, got)) {}
             }
-        };
-        std::vector<std::thread> pool;
-        for (int t = 1; t < n_threads; ++t) pool.emplace_back(work);
-        work();
-        for (auto& th : pool) th.join();
+        });
         return worst.load();
     };
     if (sweep(false) < 0) {

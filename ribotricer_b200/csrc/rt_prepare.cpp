@@ -4,12 +4,7 @@
 //     else -> 4) straight into the caller's buffer; nothing is written next to the input;
 //   * candidate-ORF index writer: rows formatted on all cores, written in order by a write-behind thread.
 // No GPU is involved; these entry points also work on a CPU-only box.
-#include <fcntl.h>
-#include <sys/stat.h>
-#include <unistd.h>
-
 #include <algorithm>
-#include <atomic>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
@@ -17,70 +12,11 @@
 #include <memory>
 #include <string>
 #include <string_view>
-#include <thread>
 #include <unordered_map>
 #include <vector>
 
 #include "ribotricer_b200.h"
-
-const char* rt_io_last_error(void);
-void rt_io_set_error(const std::string& msg);   // rt_host_io.cpp
-
-namespace {
-
-int host_threads(const char* env, size_t bytes) {
-    int n = (int)std::max<size_t>(1, std::min<size_t>({(size_t)std::thread::hardware_concurrency(), (size_t)32, bytes >> 20}));
-    if (const char* e = getenv(env)) n = std::max(1, std::min(64, atoi(e)));
-    return n;
-}
-
-template <class F>
-void run_parallel(int n, F&& f) {
-    std::vector<std::thread> pool;
-    for (int k = 1; k < n; ++k) pool.emplace_back(f, k);
-    f(0);
-    for (auto& th : pool) th.join();
-}
-
-// The whole file in memory, read in slices by `n_thr` threads.  Returns false (error set) on failure.
-bool read_file(const char* path, int n_thr_max, std::vector<char>& buf) {
-    const int fd = open(path, O_RDONLY);
-    if (fd < 0) { rt_io_set_error(std::string("cannot open ") + path); return false; }
-    struct stat st;
-    if (fstat(fd, &st) != 0) { close(fd); rt_io_set_error(std::string("cannot stat ") + path); return false; }
-    const size_t size = (size_t)st.st_size;
-    buf.resize(size + 1);
-    const int n_thr = std::max(1, std::min<int>(n_thr_max, (int)std::max<size_t>(1, size >> 22)));
-    std::atomic<bool> ok{true};
-    run_parallel(n_thr, [&](int k) {
-        size_t at = size * (size_t)k / n_thr;
-        const size_t hi = size * (size_t)(k + 1) / n_thr;
-        while (at < hi) {
-            const ssize_t got = pread(fd, buf.data() + at, hi - at, (off_t)at);
-            if (got <= 0) { ok = false; return; }
-            at += (size_t)got;
-        }
-    });
-    close(fd);
-    buf[size] = '\0';
-    if (!ok) { rt_io_set_error(std::string("short read of ") + path); return false; }
-    buf.resize(size);
-    return true;
-}
-
-// Line boundaries of n_thr chunks of [lo, hi): every chunk but the last ends after a '\n'.
-std::vector<const char*> cut_lines(const char* lo, const char* hi, int n_thr) {
-    std::vector<const char*> cut{lo};
-    for (int k = 1; k < n_thr; ++k) {
-        const char* guess = std::max(cut.back(), lo + (size_t)(hi - lo) * (size_t)k / n_thr);
-        const char* nl = guess < hi ? (const char*)memchr(guess, '\n', (size_t)(hi - guess)) : nullptr;
-        cut.push_back(nl ? nl + 1 : hi);
-    }
-    cut.push_back(hi);
-    return cut;
-}
-
-}  // namespace
+#include "rt_host.h"
 
 // ------------------------------------------------------------------------------------------------------------ GTF
 enum { kGeneId, kTxId, kGeneName, kGeneType, kTxType, kAttrs };
@@ -201,9 +137,9 @@ extern "C" {
 int rt_gtf_load(const char* path, rt_gtf** out) {
     if (!path || !out) return RT_EINVAL;
     *out = nullptr;
-    std::vector<char> text;
-    if (!read_file(path, 16, text)) return RT_EINVAL;
-    const int n_thr = host_threads("RT_GTF_THREADS", text.size());
+    HostArr<char> text;
+    if (const int rc = read_file(path, text)) return rc;
+    const int n_thr = host_threads(text.size() >> 20, 32, "RT_GTF_THREADS");
     const char* base = text.data();
     std::vector<const char*> cut = cut_lines(base, base + text.size(), n_thr);
     std::vector<GtfChunk> chunks((size_t)n_thr);
@@ -291,7 +227,7 @@ int rt_gtf_copy(const rt_gtf* g, int64_t* line_no, uint8_t* feature, int32_t* ch
 
 // ---------------------------------------------------------------------------------------------------------- FASTA
 struct rt_fasta {
-    std::vector<char> text;
+    HostArr<char> text;
     std::vector<std::string> names;
     std::vector<int64_t> length;
     struct Piece { int contig; size_t lo, hi; int64_t out; };   // a slice of one contig's text, its first base's rank
@@ -306,10 +242,10 @@ int rt_fasta_load(const char* path, rt_fasta** out) {
     if (!path || !out) return RT_EINVAL;
     *out = nullptr;
     std::unique_ptr<rt_fasta> fa(new rt_fasta());
-    if (!read_file(path, 16, fa->text)) return RT_EINVAL;
+    if (const int rc = read_file(path, fa->text)) return rc;
     const char* base = fa->text.data();
     const size_t size = fa->text.size();
-    fa->n_thr = host_threads("RT_FASTA_THREADS", size);
+    fa->n_thr = host_threads(size >> 20, 32, "RT_FASTA_THREADS");
     // 1. header lines: a '>' at the start of a line, found by all threads in slices of the file
     std::vector<std::vector<size_t>> found((size_t)fa->n_thr);
     run_parallel(fa->n_thr, [&](int k) {
@@ -347,15 +283,12 @@ int rt_fasta_load(const char* path, rt_fasta** out) {
     }
     fa->piece0.push_back(fa->pieces.size());
     // 3. bases per piece (everything but '\n' and '\r'), then each piece's rank within its contig
-    std::atomic<size_t> next{0};
     std::vector<int64_t> count(fa->pieces.size());
-    run_parallel(fa->n_thr, [&](int) {
-        for (size_t i; (i = next++) < fa->pieces.size();) {
-            const auto& pc = fa->pieces[i];
-            int64_t skip = 0;
-            for (size_t j = pc.lo; j < pc.hi; ++j) skip += base[j] == '\n' || base[j] == '\r';
-            count[i] = (int64_t)(pc.hi - pc.lo) - skip;
-        }
+    claim_parallel(fa->n_thr, fa->pieces.size(), [&](size_t i) {
+        const auto& pc = fa->pieces[i];
+        int64_t skip = 0;
+        for (size_t j = pc.lo; j < pc.hi; ++j) skip += base[j] == '\n' || base[j] == '\r';
+        count[i] = (int64_t)(pc.hi - pc.lo) - skip;
     });
     fa->length.assign(fa->names.size(), 0);
     for (size_t i = 0; i < fa->pieces.size(); ++i) {
@@ -391,16 +324,13 @@ int rt_fasta_codes(const rt_fasta* fa, int n_sel, const int32_t* contigs, uint8_
         at += fa->length[(size_t)c];
     }
     const char* base = fa->text.data();
-    std::atomic<size_t> next{0};
-    run_parallel(fa->n_thr, [&](int) {
-        for (size_t j; (j = next++) < jobs.size();) {
-            const auto& pc = fa->pieces[jobs[j].piece];
-            uint8_t* o = out + jobs[j].at;
-            for (size_t i = pc.lo; i < pc.hi; ++i) {
-                const unsigned char ch = (unsigned char)base[i];
-                if (ch == '\n' || ch == '\r') continue;
-                *o++ = lut[ch];
-            }
+    claim_parallel(fa->n_thr, jobs.size(), [&](size_t j) {
+        const auto& pc = fa->pieces[jobs[j].piece];
+        uint8_t* o = out + jobs[j].at;
+        for (size_t i = pc.lo; i < pc.hi; ++i) {
+            const unsigned char ch = (unsigned char)base[i];
+            if (ch == '\n' || ch == '\r') continue;
+            *o++ = lut[ch];
         }
     });
     return RT_OK;
@@ -412,14 +342,6 @@ int rt_fasta_codes(const rt_fasta* fa, int n_sel, const int32_t* contigs, uint8_
 namespace {
 
 const char* const kTypeName[] = {"annotated", "uORF", "overlap_uORF", "super_uORF", "overlap_dORF", "dORF", "novel", "internal"};
-
-inline char* put_uint(char* p, uint64_t u) {
-    char tmp[24];
-    int k = 24;
-    do { tmp[--k] = (char)('0' + u % 10); u /= 10; } while (u);
-    memcpy(p, tmp + k, (size_t)(24 - k));
-    return p + (24 - k);
-}
 
 }  // namespace
 
@@ -442,26 +364,22 @@ int rt_orf_write(const char* path, int64_t n_tx, const char* tx_text, const int6
     if (!fh) { rt_io_set_error(std::string("cannot open ") + path); return RT_EINVAL; }
     static const char kHeader[] = "ORF_ID\tORF_type\ttranscript_id\ttranscript_type\tgene_id\tgene_name\tgene_type\t"
                                   "chrom\tstrand\tstart_codon\tcoordinate\n";
-    std::atomic<bool> ok{fwrite(kHeader, 1, sizeof kHeader - 1, fh) == sizeof kHeader - 1};
-    const int n_thr = host_threads("RT_WRITE_THREADS", (size_t)n_rows * 64);
+    const int n_thr = host_threads((size_t)n_rows * 64 >> 20, 32, "RT_WRITE_THREADS");
     constexpr int64_t kBatchRows = 1 << 16;
-    auto format = [&](int64_t r0, int64_t r1, std::string& s) {
-        s.clear();
+    auto format = [&](int64_t r0, int64_t r1, TextBuf& s) {
         for (int64_t r = r0; r < r1; ++r) {
             const int64_t t = row_tx[r], a = iv_ptr[r], b = iv_ptr[r + 1];
             const char* tt = tx_text + tx_text_off[t];
             const size_t tlen = (size_t)(tx_text_off[t + 1] - tx_text_off[t]);
             const char* type = kTypeName[row_type[r]];
-            const size_t need = tlen + (size_t)tx_id_len[t] + 96 + 24 * (size_t)(b - a);
-            const size_t old = s.size();
-            s.resize(old + need);
-            char* p = &s[old];
+            char* p = s.need(tlen + (size_t)tx_id_len[t] + 96 + 24 * (size_t)(b - a));
+            if (!p) return false;
             int64_t length = 0;
             for (int64_t i = a; i < b; ++i) length += (int64_t)iv_end[i] - iv_start[i] + 1;
             memcpy(p, tt, (size_t)tx_id_len[t]); p += tx_id_len[t];
-            *p++ = '_'; p = put_uint(p, (uint64_t)iv_start[a]);
-            *p++ = '_'; p = put_uint(p, (uint64_t)iv_end[b - 1]);
-            *p++ = '_'; p = put_uint(p, (uint64_t)length);
+            *p++ = '_'; p = put_int(p, iv_start[a]);
+            *p++ = '_'; p = put_int(p, iv_end[b - 1]);
+            *p++ = '_'; p = put_int(p, length);
             *p++ = '\t';
             const size_t tl = strlen(type);
             memcpy(p, type, tl); p += tl;
@@ -473,31 +391,36 @@ int rt_orf_write(const char* path, int64_t n_tx, const char* tx_text, const int6
             *p++ = '\t';
             for (int64_t i = a; i < b; ++i) {
                 if (i > a) *p++ = ',';
-                p = put_uint(p, (uint64_t)iv_start[i]);
+                p = put_int(p, iv_start[i]);
                 *p++ = '-';
-                p = put_uint(p, (uint64_t)iv_end[i]);
+                p = put_int(p, iv_end[i]);
             }
             *p++ = '\n';
-            s.resize((size_t)(p - s.data()));
+            s.advance_to(p);
         }
+        return true;
     };
-    // rounds of n_thr batches: formatted by all threads while the previous round is written behind
-    std::vector<std::string> cur((size_t)n_thr), prev((size_t)n_thr);
-    std::thread writer;
-    for (int64_t r0 = 0; r0 < n_rows && ok; r0 += kBatchRows * n_thr) {
-        run_parallel(n_thr, [&](int k) {
-            const int64_t lo = std::min(n_rows, r0 + k * kBatchRows), hi = std::min(n_rows, lo + kBatchRows);
-            format(lo, hi, cur[(size_t)k]);
-        });
-        if (writer.joinable()) writer.join();
-        std::swap(cur, prev);
-        writer = std::thread([&]() {
-            for (const std::string& s : prev)
-                if (!s.empty() && fwrite(s.data(), 1, s.size(), fh) != s.size()) ok = false;
-        });
+    // rounds of n_thr batches: formatted by all threads while the earlier rounds are written behind
+    bool ok, formatted = true;
+    {
+        WriteBehind out(fh);
+        ok = out.put_view(kHeader, sizeof kHeader - 1);
+        std::vector<TextBuf> part((size_t)n_thr);
+        std::vector<char> part_ok((size_t)n_thr);
+        for (int64_t r0 = 0; r0 < n_rows && ok && formatted; r0 += kBatchRows * n_thr) {
+            run_parallel(n_thr, [&](int k) {
+                const int64_t lo = std::min(n_rows, r0 + k * kBatchRows), hi = std::min(n_rows, lo + kBatchRows);
+                part_ok[(size_t)k] = format(lo, hi, part[(size_t)k]);
+            });
+            for (int k = 0; k < n_thr && ok && formatted; ++k) {
+                formatted = part_ok[(size_t)k];
+                if (formatted) ok = out.put(std::move(part[(size_t)k]));
+            }
+        }
+        ok = out.finish() && ok;
     }
-    if (writer.joinable()) writer.join();
     if (fclose(fh) != 0) ok = false;
+    if (!formatted) { rt_io_set_error("rt_orf_write: out of memory"); return RT_ENOMEM; }
     if (!ok) { rt_io_set_error(std::string("write failed: ") + path); return RT_EINVAL; }
     return RT_OK;
 }

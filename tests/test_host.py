@@ -2,6 +2,7 @@
 import os
 
 import numpy as np
+import pytest
 
 
 def test_cli_validation(tmp_path):
@@ -185,6 +186,41 @@ def test_native_tsv_writer_matches_reference_formatting(tmp_path, built):
                                     p(status), p(ptr), p(prof)) == 0
             assert lib.rt_tsv_close(h) == 0
             assert out.read_text() == run["text"]
+
+
+@pytest.mark.parametrize("rows", [0, 3000])
+def test_tsv_writer_reports_a_refused_write(tmp_path, built, rows):
+    """A disk that refuses the text: with no rows the header fails when the file is closed, with megabytes of rows
+    the write-behind thread meets the failure; either way the caller gets an error code and a message, and the
+    close returns (the writer thread is not left waiting)."""
+    import ctypes as C
+
+    from helpers import load_golden
+    from ribotricer_b200 import _lib
+    from ribotricer_b200.index import NativeIndex
+
+    if not os.path.exists("/dev/full"):
+        pytest.skip("no /dev/full")
+    lib = _lib.load()
+    p = lambda a: a.ctypes.data_as(C.c_void_p)  # noqa: E731
+    path = tmp_path / "idx.tsv"
+    path.write_text("\n".join(load_golden("pipeline_cases.json.gz")["cases"][0]["index"]) + "\n")
+    idx = NativeIndex(str(path))
+    n = idx.n_orf
+    sel = np.zeros(rows, np.int64)                      # one ORF, many times, with a long profile each
+    score, valid = np.full(n, 0.5), np.ones(n, np.int32)
+    count, length, status = np.full(n, 7, np.int64), np.full(n, 30, np.int32), np.ones(n, np.uint8)
+    ptr = np.arange(rows + 1, dtype=np.int64) * 1000
+    prof = np.full(rows * 1000, 12, np.int32)
+    assert lib.rt_tsv_open(str(tmp_path / "missing" / "x.tsv").encode(), 1, C.byref(C.c_void_p())) != 0
+    assert lib.rt_io_last_error().decode().startswith("cannot open")
+    h = C.c_void_p()
+    assert lib.rt_tsv_open(b"/dev/full", 1, C.byref(h)) == 0
+    for _ in range(3):                                  # a write may or may not see the failure yet: it is asynchronous
+        lib.rt_tsv_write(h, idx.handle, rows, p(sel), 0, p(score), p(valid), p(count), p(length), p(status), p(ptr), p(prof))
+    rc = lib.rt_tsv_close(h)
+    assert rc != 0                                      # the close reports it whatever the writes returned
+    assert "write failed" in lib.rt_io_last_error().decode()
 
 
 def test_repr_double_is_python_repr(built):

@@ -169,6 +169,92 @@ def test_fasta_loader_matches_the_statement(annotation, built):
     assert not os.path.exists(annotation["fasta"] + ".fai")
 
 
+@pytest.fixture(scope="module")
+def big_fasta(tmp_path_factory):
+    """Contigs of a few bases up to one of 9 Mb (several 8 MB pieces), 60- and 61-column lines, one with CRLF ends."""
+    rng = np.random.default_rng(5)
+    path = tmp_path_factory.mktemp("fa") / "g.fa"
+    parts = []
+    for i, (n, width, eol) in enumerate([(5, 60, "\n"), (9_000_000, 60, "\n"), (130_001, 61, "\r\n"), (1, 60, "\n")]):
+        seq = np.frombuffer(b"ACGTNacgt", np.uint8)[rng.integers(0, 9, n)].tobytes().decode()
+        parts.append(f">c{i} contig {i}{eol}" + "".join(seq[j:j + width] + eol for j in range(0, n, width)))
+    path.write_text("".join(parts), newline="")
+    return str(path)
+
+
+@pytest.mark.parametrize("threads", ["1", "2", "7"])
+def test_fasta_loader_thread_count_does_not_change_the_codes(big_fasta, built, monkeypatch, threads):
+    from ribotricer_b200.prepare_orfs import Genome
+
+    ref = P.parse_fasta(big_fasta)
+    monkeypatch.setenv("RT_FASTA_THREADS", threads)
+    g = Genome(big_fasta)
+    assert g.names == list(ref) and g.lengths.tolist() == [len(v) for v in ref.values()]
+    codes = g.codes(np.arange(len(g.names))[::-1].copy())
+    assert np.frombuffer(b"ACGTN", np.uint8)[codes].tobytes().decode() == "".join(reversed(ref.values()))
+
+
+def _orf_rows(n_rows, seed=9):
+    """Arguments of rt_orf_write for n_rows rows of two transcripts, and the text the rows must become."""
+    rng = np.random.default_rng(seed)
+    tx = ["T1\tpc\tGA\tA\tpc\tk1\t+", "TX22\tNA\tGB\tGB\tlnc\tk2\t-"]
+    tx_text = "".join(tx).encode()
+    tx_off = np.array([0, len(tx[0]), len(tx[0]) + len(tx[1])], np.int64)
+    tx_id_len = np.array([2, 4], np.int32)
+    row_tx = rng.integers(0, 2, n_rows).astype(np.int32)
+    row_type = rng.integers(0, 8, n_rows).astype(np.uint8)
+    row_codon = rng.integers(0, 64, n_rows).astype(np.uint8)
+    n_iv = rng.integers(1, 4, n_rows)
+    iv_ptr = np.zeros(n_rows + 1, np.int64)
+    np.cumsum(n_iv, out=iv_ptr[1:])
+    iv_start = rng.integers(1, 10**9, iv_ptr[-1]).astype(np.int32)
+    iv_end = (iv_start + rng.integers(0, 5000, iv_ptr[-1])).astype(np.int32)
+    args = (len(tx), tx_text, tx_off, tx_id_len, n_rows, row_tx, row_type, row_codon, iv_ptr, iv_start, iv_end)
+    acgt = "ACGT"
+    lines = [P.HEADER]
+    for r in range(n_rows):
+        t, a, b = int(row_tx[r]), int(iv_ptr[r]), int(iv_ptr[r + 1])
+        ivs = list(zip(iv_start[a:b].tolist(), iv_end[a:b].tolist()))
+        c = int(row_codon[r])
+        lines.append(f"{tx[t][:tx_id_len[t]]}_{ivs[0][0]}_{ivs[-1][1]}_{sum(e - s + 1 for s, e in ivs)}\t"
+                     f"{P.TYPES[row_type[r]]}\t{tx[t]}\t{acgt[c >> 4 & 3]}{acgt[c >> 2 & 3]}{acgt[c & 3]}\t"
+                     + ",".join(f"{s}-{e}" for s, e in ivs) + "\n")
+    return args, "".join(lines)
+
+
+def _orf_write(path, args):
+    import ctypes as C
+
+    from ribotricer_b200 import _lib
+
+    p = lambda a: a.ctypes.data_as(C.c_void_p)  # noqa: E731
+    n_tx, tx_text, tx_off, tx_id_len, n_rows, *cols = args
+    return _lib.load().rt_orf_write(str(path).encode(), n_tx, tx_text, p(tx_off), p(tx_id_len), n_rows, *map(p, cols))
+
+
+@pytest.mark.parametrize("threads", ["1", "3"])
+def test_index_writer_thread_count_does_not_change_the_bytes(tmp_path, built, monkeypatch, threads):
+    args, want = _orf_rows(450_000)                     # 7 rounds of 64 Ki rows on one thread, 3 on three
+    monkeypatch.setenv("RT_WRITE_THREADS", threads)
+    assert _orf_write(tmp_path / "idx.tsv", args) == 0
+    assert (tmp_path / "idx.tsv").read_text() == want
+
+
+@pytest.mark.parametrize("n_rows", [0, 200_000])
+def test_index_writer_reports_a_refused_write(tmp_path, built, n_rows):
+    """The header alone fails when the file is closed; megabytes of rows fail in the write-behind thread."""
+    from ribotricer_b200 import _lib
+
+    if not os.path.exists("/dev/full"):
+        pytest.skip("no /dev/full")
+    lib = _lib.load()
+    args, _ = _orf_rows(n_rows)
+    assert _orf_write(tmp_path / "missing" / "idx.tsv", args) != 0
+    assert lib.rt_io_last_error().decode().startswith("cannot open")
+    assert _orf_write("/dev/full", args) != 0
+    assert lib.rt_io_last_error().decode() == "write failed: /dev/full"
+
+
 @pytest.mark.parametrize("text,message", [
     ("c\tt\texon\t1\t10\t.\t+\t.\n", "GTF line 2: expected 9 tab-separated columns, found 8"),
     ("c\tt\texon\tx1\t10\t.\t+\t.\tgene_id \"g\";\n", "GTF line 2: start is not a positive integer"),
