@@ -472,6 +472,72 @@ typedef struct rt_seq_query {
 } rt_seq_query;
 int rt_orf_seq_write(rt_ctx* ctx, const rt_seq_query* q, const char* path, float* stage_ms);
 
+/*
+ * ---- count-orfs-codon: per-gene and pooled codon tables of detected ORFs (DESIGN.md section 11) --------------------
+ * Host side (no GPU involved; errors in rt_io_last_error, naming the file and line):
+ * rt_codon_load_tsv reads a detected-ORFs TSV in line-aligned chunks on all cores (RT_CODON_THREADS overrides the number
+ * of chunks).  The first line is skipped; every other line, stripped of ASCII blanks at both ends, must have 18
+ * tab-separated fields.  A line is selected when its ORF_type is one of `features` and, unless report_all, its status is
+ * not "nontranslating"; its ORF_ID must then be the re-derived id tid_start_end_len of an index row whose ORF_type is one
+ * of `features` (a later duplicate replaces an earlier one).  Per selected line: index row, gene id ((gene_id,
+ * gene_name) in order of first appearance), (gene, chrom, strand) id, 1-based line number and the span of the profile
+ * field in the file text.
+ * rt_codon_load_seq checks the orfs-seq nucleotide file against the index: the header "ORF_ID\tsequence", then per index
+ * row, in order, its ORF_ID byte for byte, a tab and as many letters of ACGTN as the row has nt.  seq_off gives, per
+ * index row, where its letters start in the file text.
+ * rt_codon_write formats the two tables the device computed and writes them; on any error neither file is left.
+ */
+typedef struct rt_codon rt_codon;
+int rt_codon_load_tsv(const rt_index* ix, const char* path, int n_features, const char* const* features, int report_all,
+                      rt_codon** out);
+int rt_codon_load_seq(rt_codon* h, const rt_index* ix, const char* path);
+void rt_codon_free(rt_codon* h);
+/* sizes[4]: selected lines, genes, (gene, chrom, strand) groups, data lines of the TSV */
+int rt_codon_sizes(const rt_codon* h, int64_t* sizes);
+/* any pointer may be NULL; seq_off has n_orf entries (after rt_codon_load_seq) */
+int rt_codon_copy(const rt_codon* h, int64_t* row, int32_t* gene, int32_t* gseq, int64_t* line, int64_t* prof_off,
+                  int64_t* prof_len, int64_t* seq_off);
+/* gene g as "gene_id\tgene_name" in the TSV text (not NUL terminated) */
+const char* rt_codon_gene(const rt_codon* h, int64_t g, int* id_len, int* name_len);
+/* the whole text of the TSV (which = 0) or of the sequence file (which = 1) */
+const char* rt_codon_text(const rt_codon* h, int which, int64_t* len);
+/* gene_tab: RT_CODON_CELL values per (gene, codon) cell, cell = gene * 64 + codon; pooled_tab: the same per codon */
+int rt_codon_write(const rt_codon* h, const uint64_t* gene_tab, const uint64_t* pooled_tab, const char* gene_path,
+                   const char* pooled_path);
+/* Device side: rt_codon_counts gathers the profile text and the letters of the selected rows on all cores and uploads
+ * them with the index intervals.  codon_emit_kernel parses every profile (one warp per row, claimed dynamically),
+ * folds it into codons, names them and places each on the genome; a stable radix sort on ((gene, chrom, strand),
+ * first nt) keeps the first row's codon at every place; radix sorts on (gene, codon, count) and (codon, count) put
+ * every cell's counts in order, and codon_stats_kernel (one warp per cell) gives its cell values:
+ * n, S1 = sum x, S2 = sum x^2 as two 64-bit halves (low first), and x[n/2 - 1] + x[n/2] (n even) or 2 x[n/2] (n odd)
+ * over the counts x in ascending order.  summary[6]: codons named, codons with N, duplicates skipped, codons kept, the
+ * first selected row whose profile is refused (-1: none) and its reasons (1 malformed, 2 a value above 2^31 - 1, 4 a
+ * codon count above 2^32 - 1); when a row is refused the tables are not computed.  At most 2^26 genes and 2^32 - 1
+ * codon slots (sum of floor(length / 3)).  stage_ms (optional) receives RT_CODON_STAGES times: host gather (host
+ * clock), upload, codon_emit_kernel, dedup sort + keep, count sorts, codon_stats_kernel, copy-back. */
+#define RT_CODON_STAGES 7
+#define RT_CODON_CELL 5
+typedef struct rt_codon_query {
+    int64_t n_sel;
+    const int64_t* row;             /* index row of each selected TSV line */
+    const int32_t* gene;            /* gene id, < n_gene */
+    const int32_t* gseq;            /* (gene, chrom, strand) id, < n_gseq */
+    const int64_t* prof_off;        /* profile field of each in `tsv` */
+    const int64_t* prof_len;
+    const char* tsv;
+    const int64_t* seq_off;         /* n_orf: letters of each index row in `seq` */
+    const char* seq;
+    int64_t n_orf;
+    const int64_t* exon_ptr;        /* n_orf + 1 */
+    const int32_t* exon_start;      /* 1-based closed, ascending within a row */
+    const int32_t* exon_end;
+    const uint8_t* orf_strand;      /* 1 reverse, anything else forward */
+    int32_t n_gene;
+    int32_t n_gseq;
+} rt_codon_query;
+int rt_codon_counts(rt_ctx* ctx, const rt_codon_query* q, uint64_t* gene_tab, uint64_t* pooled_tab, int64_t* summary,
+                    float* stage_ms);
+
 /* number of kernel launches issued through this ctx so far (bench.py's gpu_launches) */
 int64_t rt_launch_count(const rt_ctx* ctx);
 /* bytes of read data the host-buffer entry points (rt_bin_reads_host, rt_bin_stream_host) have

@@ -34,10 +34,14 @@ EXPORTS = (
     "rt_gtf_load", "rt_gtf_free", "rt_gtf_n_lines", "rt_gtf_n_strings", "rt_gtf_string_bytes", "rt_gtf_copy",
     "rt_fasta_load", "rt_fasta_free", "rt_fasta_n_contig", "rt_fasta_contig_name", "rt_fasta_contig_len", "rt_fasta_codes",
     "rt_orf_write", "rt_orf_search", "rt_orf_fetch", "rt_index_ids", "rt_orf_seq_write",
+    "rt_codon_load_tsv", "rt_codon_load_seq", "rt_codon_free", "rt_codon_sizes", "rt_codon_copy", "rt_codon_gene",
+    "rt_codon_text", "rt_codon_write", "rt_codon_counts",
 )
 RT_EINVAL = -1
 RT_ORF_STAGES = 7
 RT_SEQ_STAGES = 3
+RT_CODON_STAGES = 7
+RT_CODON_CELL = 5
 
 
 class ScoreParams(C.Structure):
@@ -64,6 +68,13 @@ class SeqQuery(C.Structure):
                 ("orf_contig", C.c_void_p), ("orf_strand", C.c_void_p), ("n_contig", C.c_int32),
                 ("contig_base", C.c_void_p), ("contig_len", C.c_void_p), ("codes", C.c_void_p), ("n_codes", C.c_int64),
                 ("id_off", C.c_void_p), ("ids", C.c_void_p), ("protein", C.c_int32), ("chunk_bytes", C.c_int64)]
+
+
+class CodonQuery(C.Structure):
+    _fields_ = [("n_sel", C.c_int64), ("row", C.c_void_p), ("gene", C.c_void_p), ("gseq", C.c_void_p),
+                ("prof_off", C.c_void_p), ("prof_len", C.c_void_p), ("tsv", C.c_void_p), ("seq_off", C.c_void_p),
+                ("seq", C.c_void_p), ("n_orf", C.c_int64), ("exon_ptr", C.c_void_p), ("exon_start", C.c_void_p),
+                ("exon_end", C.c_void_p), ("orf_strand", C.c_void_p), ("n_gene", C.c_int32), ("n_gseq", C.c_int32)]
 
 
 class RtError(RuntimeError):
@@ -190,6 +201,18 @@ def load():
     lib.rt_orf_fetch.argtypes = [vp] * 9
     lib.rt_index_ids.argtypes = [vp, vp, vp]
     lib.rt_orf_seq_write.argtypes = [vp, C.POINTER(SeqQuery), C.c_char_p, vp]
+    lib.rt_codon_load_tsv.argtypes = [vp, C.c_char_p, i32, C.POINTER(C.c_char_p), i32, C.POINTER(vp)]
+    lib.rt_codon_load_seq.argtypes = [vp, vp, C.c_char_p]
+    lib.rt_codon_free.argtypes = [vp]
+    lib.rt_codon_free.restype = None
+    lib.rt_codon_sizes.argtypes = [vp, vp]
+    lib.rt_codon_copy.argtypes = [vp] * 8
+    lib.rt_codon_gene.argtypes = [vp, i64, C.POINTER(C.c_int), C.POINTER(C.c_int)]
+    lib.rt_codon_gene.restype = vp
+    lib.rt_codon_text.argtypes = [vp, i32, C.POINTER(i64)]
+    lib.rt_codon_text.restype = vp
+    lib.rt_codon_write.argtypes = [vp, vp, vp, C.c_char_p, C.c_char_p]
+    lib.rt_codon_counts.argtypes = [vp, C.POINTER(CodonQuery), vp, vp, vp, vp]
     if lib.rt_abi_version() != 4:
         raise RtError(f"ABI mismatch: library reports {lib.rt_abi_version()}, binding expects 4")
     _lib = lib

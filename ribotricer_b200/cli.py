@@ -1,10 +1,11 @@
-"""Command line of the B200 path: ``prepare-orfs``, ``detect-orfs``, ``count-orfs``, ``learn-cutoff`` and ``orfs-seq``.
+"""Command line of the B200 path: ``prepare-orfs``, ``detect-orfs``, ``count-orfs``, ``learn-cutoff``, ``orfs-seq`` and
+``count-orfs-codon``.
 
 The flag names, defaults, flag -> argument renames (``--min_read_density`` -> ``min_density_over_orf``,
 ``--stranded yes`` -> ``forward``, ``--meta-min-reads``) and every validation message are those of the
 reference command line (ribotricer/cli.py:127-289, 292-339, 435-560), so existing invocations keep working.
-``prepare-orfs`` and ``orfs-seq`` take the reference's flags (ribotricer/cli.py) and read plain-text GTF and FASTA
-files only.
+``prepare-orfs``, ``orfs-seq`` and ``count-orfs-codon`` take the reference's flags (ribotricer/cli.py) and read
+plain-text files only.
 The commands are assembled from option tables below.  ``--bam`` also accepts a ``.npz`` of decoded columns.
 """
 from __future__ import annotations
@@ -31,8 +32,8 @@ except ImportError:
 @click.group(**_GROUP_KW)
 @click.version_option(version=__version__)
 def cli() -> None:
-    """ribotricer: Tool for detecting translating ORF from Ribo-seq data (B200-native prepare-orfs, detect-orfs and
-    orfs-seq)"""
+    """ribotricer: Tool for detecting translating ORF from Ribo-seq data (B200-native prepare-orfs, detect-orfs,
+    orfs-seq and count-orfs-codon)"""
 
 
 def _register(name: str, summary: str, options, handler) -> None:
@@ -252,6 +253,32 @@ _register("orfs-seq", "Generate sequence for ORFs in ribotricer's index", [
     ("--saveto", dict(help="Path to output file", required=True)),
     ("--protein", dict(is_flag=True, help="Output protein sequence instead of nucleotide sequence")),
 ], _seq)
+
+
+# ------------------------------------------------------------------------------------ count-orfs-codon
+def _count_codon(ribotricer_index, detected_orfs, features, ribotricer_index_fasta, prefix, report_all) -> None:
+    from .count_orfs import count_orfs_codon
+
+    _need_file(ribotricer_index, "ribotricer index file")
+    _need_file(detected_orfs, "detected orfs file")
+    _need_file(ribotricer_index_fasta, "ribotricer index fasta file")
+    try:
+        count_orfs_codon(ribotricer_index, detected_orfs, {item.strip() for item in features.strip().split(",")},
+                         ribotricer_index_fasta, prefix, report_all)
+    except ValueError as exc:
+        _fail(str(exc))
+
+
+_register("count-orfs-codon", "Count reads for detected ORFs at codon level", [
+    ("--ribotricer_index", dict(help=_INDEX_HELP, required=True)),
+    ("--detected_orfs", dict(required=True, help="Path to the detected orfs file\nThis file should be generated "
+                                                 "using ribotricer detect-orfs")),
+    ("--features", dict(help="ORF types separated with comma", required=True)),
+    ("--ribotricer_index_fasta", dict(required=True, help="Path to the nucleotide sequence file of the index\nThis "
+                                                          "file should be generated using ribotricer orfs-seq")),
+    ("--prefix", dict(help="Prefix to output file", required=True)),
+    ("--report_all", dict(is_flag=True, help=_REPORT_ALL_HELP)),
+], _count_codon)
 
 
 if __name__ == "__main__":

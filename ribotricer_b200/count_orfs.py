@@ -9,14 +9,27 @@ points give the same table:
   packed index and the status column -- so no profile is ever turned into text: the union intervals of every
   gene are merged on the host (a sort over exon intervals) and summed by ``rt_interval_sums``;
 * ``count_orfs``         keeps the reference's signature (index path, TSV path) for existing pipelines.
+
+``count_orfs_codon`` gives the same selection at codon level (DESIGN.md section 11): per gene and pooled over all
+genes, the occurrences, total, mean, median and variance of the read count of every codon.
+
+    TSV            rt_codon_load_tsv (all cores): fields, selection, ORF_ID -> index row, gene keys
+    sequences      rt_codon_load_seq (all cores): the orfs-seq nucleotide file checked against the index
+    codons         Engine.codon_counts: codon_emit_kernel, radix sorts (place dedup, counts in order),
+                   codon_stats_kernel
+    tables         rt_codon_write: formatted on all cores, written by a write-behind thread
 """
 from __future__ import annotations
 
 import ctypes as C
+import os
+import pathlib
+import time
 from collections import defaultdict
 
 import numpy as np
 
+from . import _lib
 from .index import load_native_index
 
 _POS_BITS = 33          # positions are int32: gene * 2^33 + (pos + 2^31) orders intervals by (gene, pos)
@@ -178,3 +191,123 @@ def count_orfs(ribotricer_index, detected_orfs, features, outfile, report_all=Fa
         _, first = np.unique(pos, return_index=True)              # first coverage seen at a position wins (:80-82)
         total[g], length[g] = cov[first].sum(), len(first)
     write_counts(outfile, keys, total, length)
+
+
+class CodonInput:
+    """The selected rows of a detected-ORFs TSV matched to the index (``rt_codon_load_tsv``) and, after
+    ``load_seq``, the checked orfs-seq nucleotide file (``rt_codon_load_seq``).  Rule violations raise ValueError."""
+
+    def __init__(self, idx, detected_orfs: str, features, report_all: bool = False):
+        self._lib = lib = _lib.load()
+        self.idx = idx
+        feats = [f.encode() for f in features]
+        arr = (C.c_char_p * max(1, len(feats)))(*feats)
+        handle = C.c_void_p()
+        if lib.rt_codon_load_tsv(idx.handle, str(detected_orfs).encode(), len(feats), arr, int(bool(report_all)),
+                                 C.byref(handle)) != 0:
+            raise ValueError(lib.rt_io_last_error().decode())
+        self.handle = handle
+        sizes = np.zeros(4, np.int64)
+        lib.rt_codon_sizes(handle, sizes.ctypes.data_as(C.c_void_p))
+        self.n_sel, self.n_gene, self.n_gseq, self.n_lines = (int(v) for v in sizes)
+        n = self.n_sel
+        self.sel = dict(row=np.empty(n, np.int64), gene=np.empty(n, np.int32), gseq=np.empty(n, np.int32),
+                        line=np.empty(n, np.int64), prof_off=np.empty(n, np.int64), prof_len=np.empty(n, np.int64),
+                        seq_off=np.zeros(idx.n_orf, np.int64))
+        self._copy()
+
+    def _copy(self):
+        p = lambda a: a.ctypes.data_as(C.c_void_p)  # noqa: E731
+        s = self.sel
+        self._lib.rt_codon_copy(self.handle, p(s["row"]), p(s["gene"]), p(s["gseq"]), p(s["line"]), p(s["prof_off"]),
+                                p(s["prof_len"]), p(s["seq_off"]))
+
+    def load_seq(self, path: str) -> None:
+        if self._lib.rt_codon_load_seq(self.handle, self.idx.handle, str(path).encode()) != 0:
+            raise ValueError(self._lib.rt_io_last_error().decode())
+        self._copy()
+
+    def text(self, which: int) -> np.ndarray:
+        """The TSV (0) or sequence file (1) text as a uint8 view of the native buffer."""
+        n = C.c_int64()
+        ptr = self._lib.rt_codon_text(self.handle, int(which), C.byref(n))
+        if not n.value:
+            return np.zeros(1, np.uint8)[:0]
+        return np.ctypeslib.as_array((C.c_uint8 * n.value).from_address(ptr))
+
+    def gene(self, g: int) -> tuple:
+        """(gene_id, gene_name) of gene g as bytes."""
+        il, nl = C.c_int(), C.c_int()
+        ptr = self._lib.rt_codon_gene(self.handle, int(g), C.byref(il), C.byref(nl))
+        raw = C.string_at(ptr, il.value + 1 + nl.value)
+        return raw[:il.value], raw[il.value + 1:]
+
+    def write(self, gene_tab, pooled_tab, gene_path: str, pooled_path: str) -> None:
+        p = lambda a: np.ascontiguousarray(a, np.uint64).ctypes.data_as(C.c_void_p)  # noqa: E731
+        gene_tab, pooled_tab = np.ascontiguousarray(gene_tab, np.uint64), np.ascontiguousarray(pooled_tab, np.uint64)
+        if self._lib.rt_codon_write(self.handle, p(gene_tab), p(pooled_tab), str(gene_path).encode(),
+                                    str(pooled_path).encode()) != 0:
+            raise ValueError(self._lib.rt_io_last_error().decode())
+
+    def __del__(self):
+        try:
+            if getattr(self, "handle", None):
+                self._lib.rt_codon_free(self.handle)
+                self.handle = None
+        except Exception:
+            pass
+
+
+_PROFILE_REFUSALS = ((1, "the profile is not a list of integers written as str(list) writes it"),
+                     (2, "a profile value lies outside 0..2147483647"),
+                     (4, "a codon count exceeds 4294967295"))
+
+
+def count_orfs_codon(ribotricer_index, detected_orfs, features, ribotricer_index_fasta, prefix, report_all=False,
+                     stage_ms: dict | None = None):
+    """Write ``{prefix}_codon_counts_by_gene.tsv`` and ``{prefix}_codon_counts.tsv`` (DESIGN.md section 11) from the
+    index, a detected-ORFs TSV and the orfs-seq nucleotide file of the same index.  ``features`` is a set of ORF types.
+    Every check runs before either file is opened.  ``stage_ms``, when given, receives the time of every stage in
+    milliseconds.  Returns a summary dict."""
+    from .detect_orfs import get_engine
+    from .prepare_orfs import _refuse_gzip
+
+    times = {} if stage_ms is None else stage_ms
+    clock = time.perf_counter()
+
+    def lap(name):
+        nonlocal clock
+        now = time.perf_counter()
+        times[name] = (now - clock) * 1e3
+        clock = now
+
+    for path in (ribotricer_index, detected_orfs, ribotricer_index_fasta):
+        _refuse_gzip(path, "count-orfs-codon")
+    idx = load_native_index(ribotricer_index)
+    lap("index_load")
+    inp = CodonInput(idx, detected_orfs, features, report_all)
+    lap("tsv_load")
+    inp.load_seq(ribotricer_index_fasta)
+    lap("seq_check")
+    dev_ms = np.zeros(_lib.RT_CODON_STAGES, np.float32)
+    gene_tab, pooled_tab, summary = get_engine().codon_counts(
+        inp.sel, inp.text(0), inp.text(1), idx.exon_ptr, idx.exon_start, idx.exon_end, idx.orf_strand_code,
+        inp.n_gene, inp.n_gseq, stage_ms=dev_ms)
+    lap("codon_counts")
+    for name, ms in zip(("host_gather", "upload", "codon_emit_kernel", "dedup", "count_sorts", "codon_stats_kernel",
+                         "copy_back"), dev_ms.tolist()):
+        times["device:" + name] = ms
+    bad = int(summary[4])
+    if bad >= 0:
+        reason = next(text for bit, text in _PROFILE_REFUSALS if int(summary[5]) & bit)
+        raise ValueError(f"{detected_orfs} line {int(inp.sel['line'][bad])}: {reason}")
+    gene_path, pooled_path = f"{prefix}_codon_counts_by_gene.tsv", f"{prefix}_codon_counts.tsv"
+    pathlib.Path(os.path.dirname(os.path.abspath(gene_path))).mkdir(parents=True, exist_ok=True)
+    inp.write(gene_tab, pooled_tab, gene_path, pooled_path)
+    lap("write")
+    genes = int(np.count_nonzero(gene_tab[:, 0].reshape(-1, 64).any(axis=1))) if inp.n_gene else 0
+    result = dict(rows=inp.n_sel, genes=genes, codons=int(summary[3]), duplicates=int(summary[2]),
+                  codons_with_n=int(summary[1]), gene_table=gene_path, codon_table=pooled_path)
+    print(f"count-orfs-codon: {inp.n_sel} rows selected, {genes} genes, {result['codons']} codons kept, "
+          f"{result['duplicates']} duplicates skipped, {result['codons_with_n']} codons with N")
+    return result

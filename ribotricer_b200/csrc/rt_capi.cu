@@ -12,6 +12,8 @@
 #include <unordered_map>
 #include <vector>
 
+#include <cub/device/device_radix_sort.cuh>
+
 #include "rt_host.h"
 #include "rt_kernels.cuh"
 
@@ -2031,6 +2033,218 @@ int rt_orf_seq_write(rt_ctx* ctx, const rt_seq_query* q, const char* path, float
     if (fclose(fh) != 0 && rc == RT_OK) rc = fail(ctx, RT_EINVAL, "rt_orf_seq_write: cannot write %s", path);
     if (rc != RT_OK) remove(path);
     return rc;
+}
+
+// ---------------------------------------------------------------------------------------------- count-orfs-codon
+}  // extern "C"
+
+namespace {
+enum CodonBuf { kCdProf, kCdSeq, kCdProfBase, kCdSeqBase, kCdSlotBase, kCdRow, kCdGene, kCdGseq, kCdExPtr, kCdExStart,
+                kCdExEnd, kCdStrand, kCdCnt, kCdKey, kCdVal, kCdKey2, kCdVal2, kCdCounters, kCdFlag, kCdClaim, kCdTemp,
+                kCdGeneTab, kCdPooledTab, kCodonBufs };
+
+// The device buffers and events of one rt_codon_counts call; everything is freed on every return.
+struct CodonScratch {
+    DevBuf b[kCodonBufs];
+    cudaStream_t st = nullptr;
+    cudaEvent_t ev[7] = {};
+    ~CodonScratch() {
+        if (st) cudaStreamSynchronize(st);
+        for (DevBuf& x : b) x.release();
+        for (cudaEvent_t e : ev)
+            if (e) cudaEventDestroy(e);
+        if (st) cudaStreamDestroy(st);
+    }
+};
+
+int bit_length(unsigned long long x) { return x ? 64 - __builtin_clzll(x) : 0; }
+}  // namespace
+
+extern "C" {
+
+int rt_codon_counts(rt_ctx* ctx, const rt_codon_query* q, uint64_t* gene_tab, uint64_t* pooled_tab, int64_t* summary,
+                    float* stage_ms) {
+    if (!ctx) return fail(nullptr, RT_EINVAL, "rt_codon_counts: ctx is NULL");
+    if (!q || !pooled_tab || !summary || q->n_sel < 0 || q->n_orf < 0 || q->n_gene < 0 || q->n_gseq < 0 ||
+        (q->n_sel && (!q->row || !q->gene || !q->gseq || !q->prof_off || !q->prof_len || !q->tsv || !q->seq_off || !q->seq ||
+                      !q->exon_ptr || !q->orf_strand)) || (q->n_gene && !gene_tab))
+        return fail(ctx, RT_EINVAL, "rt_codon_counts: NULL or negative argument");
+    if (q->n_gene > (1 << 26))
+        return fail(ctx, RT_EINVAL, "count-orfs-codon handles at most 2^26 genes; the selection has %d", q->n_gene);
+    const auto t_host = std::chrono::steady_clock::now();
+    const int64_t n = q->n_sel, n_ex = q->n_orf ? q->exon_ptr[q->n_orf] : 0;
+    // 1. host: per selected row its length, slots and the offsets of its profile text and letters
+    std::vector<int64_t> prof_base((size_t)n + 1, 0), seq_base((size_t)n + 1, 0), slot_base((size_t)n + 1, 0);
+    for (int64_t i = 0; i < n; ++i) {
+        const int64_t r = q->row[i];
+        if (r < 0 || r >= q->n_orf || q->gene[i] < 0 || q->gene[i] >= q->n_gene || q->gseq[i] < 0 || q->gseq[i] >= q->n_gseq)
+            return fail(ctx, RT_EINVAL, "rt_codon_counts: selected row %lld lies outside the index or the gene tables", (long long)i);
+        int64_t L = 0;
+        for (int64_t e = q->exon_ptr[r]; e < q->exon_ptr[r + 1]; ++e) L += (int64_t)q->exon_end[e] - q->exon_start[e] + 1;
+        prof_base[(size_t)i + 1] = prof_base[(size_t)i] + q->prof_len[i];
+        seq_base[(size_t)i + 1] = seq_base[(size_t)i] + L;
+        slot_base[(size_t)i + 1] = slot_base[(size_t)i] + L / 3;
+    }
+    const int64_t n_slot = slot_base[(size_t)n];
+    if (n_slot > (int64_t)0xffffffffll)
+        return fail(ctx, RT_EINVAL, "count-orfs-codon handles at most 2^32 - 1 codons; the selection has %lld", (long long)n_slot);
+    // the profile text and the letters of the selected rows, gathered by all cores
+    HostArr<char> prof, letters;
+    if (!prof.alloc((size_t)prof_base[(size_t)n]) || !letters.alloc((size_t)seq_base[(size_t)n]))
+        return fail(ctx, RT_ENOMEM, "rt_codon_counts: out of host memory");
+    const int64_t block = 1 << 10;
+    claim_parallel(host_threads((size_t)((prof_base[(size_t)n] + seq_base[(size_t)n]) >> 22) + 1, 32),
+                   (size_t)((n + block - 1) / block), [&](size_t bk) {
+        for (int64_t i = (int64_t)bk * block; i < std::min(n, (int64_t)(bk + 1) * block); ++i) {
+            memcpy(prof.p + prof_base[(size_t)i], q->tsv + q->prof_off[i], (size_t)q->prof_len[i]);
+            memcpy(letters.p + seq_base[(size_t)i], q->seq + q->seq_off[q->row[i]], (size_t)(seq_base[(size_t)i + 1] - seq_base[(size_t)i]));
+        }
+    });
+    if (stage_ms) {
+        for (int k = 0; k < RT_CODON_STAGES; ++k) stage_ms[k] = 0.f;
+        stage_ms[0] = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_host).count();
+    }
+    for (int k = 0; k < 6; ++k) summary[k] = 0;
+    summary[4] = -1;
+    // 2. uploads
+    DeviceGuard guard(ctx->device);
+    CodonScratch S;
+    DevBuf* B = S.b;
+    RT_CUDA(ctx, cudaStreamCreateWithFlags(&S.st, cudaStreamNonBlocking));
+    for (auto& e : S.ev) RT_CUDA(ctx, cudaEventCreate(&e));
+    auto reserve = [&](int k, size_t bytes) { return B[k].reserve(std::max<size_t>(bytes, 16)); };
+    auto up = [&](int k, const void* src, size_t bytes) {
+        return bytes ? cudaMemcpyAsync(B[k].p, src, bytes, cudaMemcpyHostToDevice, S.st) : cudaSuccess;
+    };
+    const size_t ns = (size_t)n_slot;
+    RT_CUDA(ctx, reserve(kCdProf, prof.size()));
+    RT_CUDA(ctx, reserve(kCdSeq, letters.size()));
+    RT_CUDA(ctx, reserve(kCdProfBase, 8 * ((size_t)n + 1)));
+    RT_CUDA(ctx, reserve(kCdSeqBase, 8 * ((size_t)n + 1)));
+    RT_CUDA(ctx, reserve(kCdSlotBase, 8 * ((size_t)n + 1)));
+    RT_CUDA(ctx, reserve(kCdRow, 8 * (size_t)n));
+    RT_CUDA(ctx, reserve(kCdGene, 4 * (size_t)n));
+    RT_CUDA(ctx, reserve(kCdGseq, 4 * (size_t)n));
+    RT_CUDA(ctx, reserve(kCdExPtr, 8 * ((size_t)q->n_orf + 1)));
+    RT_CUDA(ctx, reserve(kCdExStart, 4 * (size_t)n_ex));
+    RT_CUDA(ctx, reserve(kCdExEnd, 4 * (size_t)n_ex));
+    RT_CUDA(ctx, reserve(kCdStrand, (size_t)q->n_orf));
+    RT_CUDA(ctx, reserve(kCdCnt, 8 * ns));
+    RT_CUDA(ctx, reserve(kCdKey, 8 * ns));
+    RT_CUDA(ctx, reserve(kCdVal, 8 * ns));
+    RT_CUDA(ctx, reserve(kCdKey2, 8 * ns));
+    RT_CUDA(ctx, reserve(kCdVal2, 8 * ns));
+    RT_CUDA(ctx, reserve(kCdCounters, 8 * 4));
+    RT_CUDA(ctx, reserve(kCdFlag, (size_t)n));
+    RT_CUDA(ctx, reserve(kCdClaim, 4));
+    RT_CUDA(ctx, reserve(kCdGeneTab, 8 * RT_CODON_CELL * 64 * (size_t)q->n_gene));
+    RT_CUDA(ctx, reserve(kCdPooledTab, 8 * RT_CODON_CELL * 64));
+    RT_CUDA(ctx, cudaEventRecord(S.ev[0], S.st));
+    RT_CUDA(ctx, up(kCdProf, prof.p, prof.size()));
+    RT_CUDA(ctx, up(kCdSeq, letters.p, letters.size()));
+    RT_CUDA(ctx, up(kCdProfBase, prof_base.data(), 8 * ((size_t)n + 1)));
+    RT_CUDA(ctx, up(kCdSeqBase, seq_base.data(), 8 * ((size_t)n + 1)));
+    RT_CUDA(ctx, up(kCdSlotBase, slot_base.data(), 8 * ((size_t)n + 1)));
+    RT_CUDA(ctx, up(kCdRow, q->row, 8 * (size_t)n));
+    RT_CUDA(ctx, up(kCdGene, q->gene, 4 * (size_t)n));
+    RT_CUDA(ctx, up(kCdGseq, q->gseq, 4 * (size_t)n));
+    if (n) {
+        RT_CUDA(ctx, up(kCdExPtr, q->exon_ptr, 8 * ((size_t)q->n_orf + 1)));
+        RT_CUDA(ctx, up(kCdExStart, q->exon_start, 4 * (size_t)n_ex));
+        RT_CUDA(ctx, up(kCdExEnd, q->exon_end, 4 * (size_t)n_ex));
+        RT_CUDA(ctx, up(kCdStrand, q->orf_strand, (size_t)q->n_orf));
+    }
+    const unsigned long long counters0[4] = {0, 0, ~0ull, 0};
+    RT_CUDA(ctx, up(kCdCounters, counters0, sizeof counters0));
+    RT_CUDA(ctx, cudaMemsetAsync(B[kCdCnt].p, 0, 8 * ns, S.st));
+    RT_CUDA(ctx, cudaMemsetAsync(B[kCdClaim].p, 0, 4, S.st));
+    RT_CUDA(ctx, cudaEventRecord(S.ev[1], S.st));
+    // 3. codon_emit_kernel
+    auto* cnt = (unsigned long long*)B[kCdCnt].p;
+    auto* key = (unsigned long long*)B[kCdKey].p;
+    auto* val = (unsigned long long*)B[kCdVal].p;
+    auto* key2 = (unsigned long long*)B[kCdKey2].p;
+    auto* val2 = (unsigned long long*)B[kCdVal2].p;
+    auto* counters = (unsigned long long*)B[kCdCounters].p;
+    const rt::CodonArgs A{(const char*)B[kCdProf].p, (const long long*)B[kCdProfBase].p, (const char*)B[kCdSeq].p,
+                          (const long long*)B[kCdSeqBase].p, (const long long*)B[kCdSlotBase].p, (const long long*)B[kCdRow].p,
+                          (const long long*)B[kCdExPtr].p, (const int*)B[kCdExStart].p, (const int*)B[kCdExEnd].p,
+                          (const uint8_t*)B[kCdStrand].p, (const int*)B[kCdGene].p, (const int*)B[kCdGseq].p, cnt, key, val,
+                          counters, (uint8_t*)B[kCdFlag].p, (long long)n, (unsigned*)B[kCdClaim].p};
+    const int64_t big = std::max(1, ctx->n_sm * 8);
+    if (n) {
+        const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((n + rt::kCodonWarps - 1) / rt::kCodonWarps, big));
+        rt::codon_emit_kernel<<<grid, rt::kCodonWarps * 32, 0, S.st>>>(A);
+        ctx->launches++;
+        RT_CUDA(ctx, cudaGetLastError());
+    }
+    RT_CUDA(ctx, cudaEventRecord(S.ev[2], S.st));
+    unsigned long long h_counters[4];
+    RT_CUDA(ctx, cudaMemcpyAsync(h_counters, counters, sizeof h_counters, cudaMemcpyDeviceToHost, S.st));
+    RT_CUDA(ctx, cudaStreamSynchronize(S.st));
+    summary[0] = (int64_t)h_counters[0];
+    summary[1] = (int64_t)h_counters[1];
+    if (h_counters[2] != ~0ull) {                      // a refused profile: no tables
+        uint8_t f = 0;
+        RT_CUDA(ctx, cudaMemcpyAsync(&f, (uint8_t*)B[kCdFlag].p + h_counters[2], 1, cudaMemcpyDeviceToHost, S.st));
+        RT_CUDA(ctx, cudaStreamSynchronize(S.st));
+        summary[4] = (int64_t)h_counters[2];
+        summary[5] = f;
+        if (stage_ms) RT_CUDA(ctx, cudaEventElapsedTime(&stage_ms[1], S.ev[0], S.ev[1]));
+        return RT_OK;
+    }
+    // 4. dedup: stable sort by place, keep the first slot of every place
+    const unsigned items = (unsigned)ns;
+    const int place_bits = std::min(64, 32 + bit_length((unsigned long long)q->n_gseq));
+    const int gene_bits = 32 + bit_length(64ull * (unsigned long long)q->n_gene);
+    size_t t1 = 0, t2 = 0, t3 = 0;
+    RT_CUDA(ctx, cub::DeviceRadixSort::SortPairs(nullptr, t1, key, key2, val, val2, items, 0, place_bits, S.st));
+    RT_CUDA(ctx, cub::DeviceRadixSort::SortKeys(nullptr, t2, val, val2, items, 0, gene_bits, S.st));
+    RT_CUDA(ctx, cub::DeviceRadixSort::SortKeys(nullptr, t3, val, val2, items, 0, 38, S.st));
+    RT_CUDA(ctx, reserve(kCdTemp, std::max({t1, t2, t3})));
+    void* temp = B[kCdTemp].p;
+    if (items) RT_CUDA(ctx, cub::DeviceRadixSort::SortPairs(temp, t1, key, key2, val, val2, items, 0, place_bits, S.st));
+    // kept values -> cnt (free now), pooled keys -> key (free now)
+    const unsigned keep_grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((int64_t)(ns + 255) / 256, big));
+    if (items) {
+        rt::codon_keep_kernel<<<keep_grid, 256, 0, S.st>>>(key2, val2, (long long)ns, cnt, key, counters + 3);
+        ctx->launches++;
+        RT_CUDA(ctx, cudaGetLastError());
+    }
+    RT_CUDA(ctx, cudaEventRecord(S.ev[3], S.st));
+    RT_CUDA(ctx, cudaMemcpyAsync(h_counters + 3, counters + 3, 8, cudaMemcpyDeviceToHost, S.st));
+    RT_CUDA(ctx, cudaStreamSynchronize(S.st));
+    const unsigned kept = (unsigned)h_counters[3];
+    summary[3] = (int64_t)kept;
+    summary[2] = summary[0] - summary[1] - summary[3];
+    // 5. counts in order within every (gene, codon) and every codon
+    if (kept) {
+        RT_CUDA(ctx, cub::DeviceRadixSort::SortKeys(temp, t2, cnt, val2, kept, 0, gene_bits, S.st));
+        RT_CUDA(ctx, cub::DeviceRadixSort::SortKeys(temp, t3, key, key2, kept, 0, 38, S.st));
+    }
+    RT_CUDA(ctx, cudaEventRecord(S.ev[4], S.st));
+    // 6. codon_stats_kernel over the per-gene cells and the pooled cells
+    auto* gtab = (unsigned long long*)B[kCdGeneTab].p;
+    auto* ptab = (unsigned long long*)B[kCdPooledTab].p;
+    const int64_t gene_cells = 64 * (int64_t)q->n_gene;
+    if (gene_cells) {
+        const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((gene_cells + 7) / 8, big * 4));
+        rt::codon_stats_kernel<<<grid, 256, 0, S.st>>>(val2, (long long)kept, gene_cells, gtab);
+        ctx->launches++;
+        RT_CUDA(ctx, cudaGetLastError());
+    }
+    rt::codon_stats_kernel<<<8, 256, 0, S.st>>>(key2, (long long)kept, 64, ptab);
+    ctx->launches++;
+    RT_CUDA(ctx, cudaGetLastError());
+    RT_CUDA(ctx, cudaEventRecord(S.ev[5], S.st));
+    // 7. copy-back
+    if (gene_cells) RT_CUDA(ctx, cudaMemcpyAsync(gene_tab, gtab, 8 * RT_CODON_CELL * (size_t)gene_cells, cudaMemcpyDeviceToHost, S.st));
+    RT_CUDA(ctx, cudaMemcpyAsync(pooled_tab, ptab, 8 * RT_CODON_CELL * 64, cudaMemcpyDeviceToHost, S.st));
+    RT_CUDA(ctx, cudaEventRecord(S.ev[6], S.st));
+    RT_CUDA(ctx, cudaStreamSynchronize(S.st));
+    if (stage_ms)
+        for (int k = 1; k < RT_CODON_STAGES; ++k) RT_CUDA(ctx, cudaEventElapsedTime(&stage_ms[k], S.ev[k - 1], S.ev[k]));
+    return RT_OK;
 }
 
 }  // extern "C"

@@ -7,12 +7,14 @@
 #include <algorithm>
 #include <atomic>
 #include <charconv>
+#include <cmath>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <memory>
 #include <string>
+#include <string_view>
 #include <unordered_map>
 #include <vector>
 
@@ -349,6 +351,22 @@ int rt_tsv_open(const char* path, int write_header, rt_tsv** out) {
 
 namespace {
 
+// The re-derived ORF id tid_start_end_len of row o (orf.py:101-103) at p; returns the end.  At most the transcript id
+// plus 3 * 21 bytes.
+char* put_oid(char* p, const rt_index* ix, int64_t o) {
+    int tlen = 0;
+    const char* tid = rt_index_field(ix, o, 2, &tlen);
+    const int64_t e0 = ix->exon_ptr[o], e1 = ix->exon_ptr[o + 1];
+    long long L = 0;
+    for (int64_t e = e0; e < e1; ++e) L += (long long)ix->exon_end[e] - ix->exon_start[e] + 1;
+    memcpy(p, tid, (size_t)tlen);
+    p += tlen;
+    *p++ = '_';
+    p = put_int(p, e1 > e0 ? ix->exon_start[e0] : 0); *p++ = '_';
+    p = put_int(p, e1 > e0 ? ix->exon_end[e1 - 1] : 0); *p++ = '_';
+    return put_int(p, L);
+}
+
 // Rows [i0, i1) of the selection, formatted as detect_orfs.py:304-323 prints them.
 bool format_rows(TextBuf& b, const rt_index* ix, int64_t i0, int64_t i1, const int64_t* orf_ids, int64_t orf_lo,
                  const double* score, const int32_t* valid, const int64_t* count, const int32_t* length,
@@ -364,9 +382,6 @@ bool format_rows(TextBuf& b, const rt_index* ix, int64_t i0, int64_t i1, const i
             f[j] = rt_index_field(ix, o, j, &flen[j]);
             text += (size_t)flen[j];
         }
-        const int64_t e0 = ix->exon_ptr[o], e1 = ix->exon_ptr[o + 1];
-        long long L = 0;
-        for (int64_t e = e0; e < e1; ++e) L += (long long)ix->exon_end[e] - ix->exon_start[e] + 1;
         const size_t n_prof = (size_t)(prof_ptr[i + 1] - prof_ptr[i]);
         // everything but the profile: the fields (transcript_id twice), 7 integers of <= 20 characters, 3 doubles of <= 25,
         // the status word, tabs and brackets; a profile value takes <= 11 characters and ", "
@@ -378,11 +393,8 @@ bool format_rows(TextBuf& b, const rt_index* ix, int64_t i0, int64_t i1, const i
             append_repr(num, x);
             put(num.data(), (int)num.size());
         };
-        // oid = tid_start_end_len (orf.py:101-103)
-        put(f[2], flen[2]); *p++ = '_';
-        p = put_int(p, e1 > e0 ? ix->exon_start[e0] : 0); *p++ = '_';
-        p = put_int(p, e1 > e0 ? ix->exon_end[e1 - 1] : 0); *p++ = '_';
-        p = put_int(p, L); *p++ = '\t';
+        p = put_oid(p, ix, o);
+        *p++ = '\t';
         put(f[1], flen[1]); *p++ = '\t';
         if (status[k]) put("translating", 11); else put("nontranslating", 14);
         *p++ = '\t';
@@ -792,6 +804,486 @@ int rt_stream_pack(int64_t n, const int32_t* ref_id, const int32_t* first, const
         return RT_EINVAL;
     }
     if (sweep(true) < 0) return RT_ESTATE;
+    return RT_OK;
+}
+
+}  // extern "C"
+
+// ---- count-orfs-codon, host side (DESIGN.md section 11) ------------------------------------------------------------
+// rt_codon_load_tsv selects the rows of a detected-ORFs TSV and matches them to the index, rt_codon_load_seq checks the
+// orfs-seq nucleotide file against the index, rt_codon_write formats the tables the device computed.
+
+struct rt_codon {
+    HostArr<char> tsv;                   // the detected-ORFs TSV; profiles and gene keys point into it
+    HostArr<char> seq;                   // the orfs-seq file (rt_codon_load_seq)
+    std::vector<int64_t> row, line, prof_off, prof_len;   // per selected TSV row
+    std::vector<int32_t> gene, gseq;
+    std::vector<int64_t> gene_key;       // per gene: offset of "gene_id\tgene_name" in tsv
+    std::vector<int32_t> gene_id_len, gene_key_len;
+    int64_t n_gseq = 0, n_lines = 0;
+    std::vector<int64_t> seq_off;        // per index row: offset of its letters in seq
+};
+
+namespace {
+
+inline bool ws(char c) { return c == ' ' || c == '\t' || c == '\n' || c == '\r' || c == '\v' || c == '\f'; }
+
+// ORF_ID -> index row for the rows whose ORF_type is wanted; a later duplicate replaces an earlier one.  Open addressing
+// over the oid hashes; a probe compares the oid formed again from the index.
+struct OidTable {
+    const rt_index* ix = nullptr;
+    std::vector<uint64_t> hash;          // per index row (0: not a candidate)
+    std::vector<int64_t> slot;           // row + 1, 0 empty
+    uint64_t mask = 0;
+    static uint64_t hash_of(const char* p, size_t n) {
+        uint64_t h = std::hash<std::string_view>()(std::string_view(p, n));
+        return h | 1;                    // 0 marks a row that is not a candidate
+    }
+    bool same(int64_t o, const char* p, size_t n) const {
+        char buf[1 << 12];
+        int tlen = 0;
+        rt_index_field(ix, o, 2, &tlen);
+        if ((size_t)tlen + 70 > sizeof buf) {
+            std::string big((size_t)tlen + 70, '\0');
+            const size_t m = (size_t)(put_oid(&big[0], ix, o) - big.data());
+            return m == n && memcmp(big.data(), p, n) == 0;
+        }
+        const size_t m = (size_t)(put_oid(buf, ix, o) - buf);
+        return m == n && memcmp(buf, p, n) == 0;
+    }
+    void build(const rt_index* index, const std::vector<std::string>& features) {
+        ix = index;
+        const int64_t n = (int64_t)ix->orf_chrom.size();
+        hash.assign((size_t)n, 0);
+        std::atomic<int64_t> n_cand{0};
+        const int64_t block = 1 << 14;
+        claim_parallel(host_threads((size_t)(n / block + 1), 16), (size_t)((n + block - 1) / block), [&](size_t bk) {
+            std::string buf;
+            int64_t cand = 0;
+            for (int64_t o = (int64_t)bk * block; o < std::min(n, (int64_t)(bk + 1) * block); ++o) {
+                int len = 0;
+                const char* type = rt_index_field(ix, o, 1, &len);
+                bool want = false;
+                for (const std::string& f : features) want = want || (f.size() == (size_t)len && memcmp(f.data(), type, (size_t)len) == 0);
+                if (!want) continue;
+                int tlen = 0;
+                rt_index_field(ix, o, 2, &tlen);
+                buf.resize((size_t)tlen + 70);
+                const size_t m = (size_t)(put_oid(&buf[0], ix, o) - buf.data());
+                hash[(size_t)o] = hash_of(buf.data(), m);
+                ++cand;
+            }
+            n_cand += cand;
+        });
+        uint64_t cap = 16;
+        while (cap < 2 * (uint64_t)n_cand.load()) cap <<= 1;
+        slot.assign(cap, 0);
+        mask = cap - 1;
+        std::string buf;
+        for (int64_t o = 0; o < n; ++o) {
+            if (!hash[(size_t)o]) continue;
+            int tlen = 0;
+            rt_index_field(ix, o, 2, &tlen);
+            buf.resize((size_t)tlen + 70);
+            const size_t m = (size_t)(put_oid(&buf[0], ix, o) - buf.data());
+            for (uint64_t s = hash[(size_t)o] & mask;; s = (s + 1) & mask) {
+                const int64_t r = slot[s] - 1;
+                if (r < 0 || (hash[(size_t)r] == hash[(size_t)o] && same(r, buf.data(), m))) { slot[s] = o + 1; break; }
+            }
+        }
+    }
+    int64_t find(const char* p, size_t n) const {
+        const uint64_t h = hash_of(p, n);
+        for (uint64_t s = h & mask;; s = (s + 1) & mask) {
+            const int64_t r = slot[s] - 1;
+            if (r < 0) return -1;
+            if (hash[(size_t)r] == h && same(r, p, n)) return r;
+        }
+    }
+};
+
+// Python's repr of S1 / n, the correctly rounded quotient of two integers (n > 0).
+double exact_ratio(uint64_t s1, uint64_t n) {
+    if (s1 < (1ull << 53) && n < (1ull << 53)) return (double)s1 / (double)n;
+    // a quotient of at least 55 bits, its last bit set when the division is inexact, then one rounding to 53 bits
+    const int bits_s = 64 - __builtin_clzll(s1), bits_n = 64 - __builtin_clzll(n);
+    const int shift = std::max(0, 55 + bits_n - bits_s);
+    const unsigned __int128 num = (unsigned __int128)s1 << shift;
+    const unsigned __int128 q = num / n;
+    const uint64_t sticky = num % n != 0;
+    return std::ldexp((double)(uint64_t)(q | sticky), -shift);
+}
+
+// One row of a table: occurrences, total, mean, median, var (rule 9).  cell = n, S1, S2 low, S2 high, middle sum.
+void put_stats(TextBuf& b, const uint64_t* cell, std::string& num) {
+    const uint64_t n = cell[0], s1 = cell[1];
+    const unsigned __int128 s2 = (unsigned __int128)cell[3] << 64 | cell[2];
+    const unsigned __int128 var_num = (unsigned __int128)n * s2 - (unsigned __int128)s1 * s1;
+    const unsigned __int128 var_den = (unsigned __int128)n * n;
+    num.clear();
+    append_repr(num, exact_ratio(s1, n));
+    num += '\t';
+    append_repr(num, (double)cell[4] / 2.0);
+    num += '\t';
+    append_repr(num, (double)var_num / (double)var_den);
+    char* p = b.need(2 * 21 + num.size() + 4);
+    if (!p) return;
+    p = put_int(p, (long long)n); *p++ = '\t';
+    p = put_int(p, (long long)s1); *p++ = '\t';
+    memcpy(p, num.data(), num.size());
+    p += num.size();
+    *p++ = '\n';
+    b.advance_to(p);
+}
+
+void put_codon(TextBuf& b, int c) {
+    if (char* p = b.need(4)) {
+        p[0] = "ACGT"[c >> 4]; p[1] = "ACGT"[(c >> 2) & 3]; p[2] = "ACGT"[c & 3]; p[3] = '\t';
+        b.advance_to(p + 4);
+    }
+}
+
+}  // namespace
+
+extern "C" {
+
+int rt_codon_load_tsv(const rt_index* ix, const char* path, int n_features, const char* const* features, int report_all,
+                      rt_codon** out) {
+    if (!ix || !path || !out || n_features < 0 || (n_features && !features)) return RT_EINVAL;
+    *out = nullptr;
+    std::unique_ptr<rt_codon> h(new rt_codon());
+    if (const int rc = read_file(path, h->tsv)) return rc;
+    std::vector<std::string> feats;
+    for (int k = 0; k < n_features; ++k) feats.emplace_back(features[k] ? features[k] : "");
+    OidTable oids;
+    oids.build(ix, feats);
+    auto wanted = [&](const char* p, size_t n) {
+        for (const std::string& f : feats)
+            if (f.size() == n && memcmp(f.data(), p, n) == 0) return true;
+        return false;
+    };
+    const char* base = h->tsv.data();
+    const size_t size = h->tsv.size();
+    const char* end = base + size;
+    const char* body = (const char*)memchr(base, '\n', size);   // the first line is skipped, as count_orfs does
+    body = body ? body + 1 : end;
+    const int n_thr = host_threads(size >> 22, 16, "RT_CODON_THREADS");
+
+    // 1. line-aligned chunks: fields, selection, ORF_ID lookup, gene keys interned per chunk
+    struct Chunk {
+        const char *lo, *hi;
+        std::vector<int64_t> row, line, prof_off, prof_len;
+        std::vector<int32_t> gene, gseq;
+        std::vector<std::string_view> genes;            // "gene_id\tgene_name", first appearance within the chunk
+        std::vector<uint64_t> gseqs;                    // local gene << 32 | chrom << 2 | strand
+        int64_t lines = 0;
+        int err = 0;                                    // 1: field count, 2: unknown ORF_ID; at local line err_line
+        int64_t err_line = 0, err_fields = 0;
+        std::string_view err_id;
+    };
+    std::vector<Chunk> chunks((size_t)n_thr);
+    const std::vector<const char*> cut = cut_lines(body, end, n_thr);
+    run_parallel(n_thr, [&](int k) {
+        Chunk& ck = chunks[(size_t)k];
+        std::unordered_map<std::string_view, int32_t> gene_id;
+        std::unordered_map<uint64_t, int32_t> gseq_id;
+        for (const char* p = cut[(size_t)k]; p < cut[(size_t)k + 1]; ++ck.lines) {
+            const char* eol = (const char*)memchr(p, '\n', (size_t)(cut[(size_t)k + 1] - p));
+            const char* lo = p;
+            const char* hi = eol ? eol : cut[(size_t)k + 1];
+            p = hi + 1;
+            while (lo < hi && ws(*lo)) ++lo;                 // line.strip()
+            while (hi > lo && ws(hi[-1])) --hi;
+            const char* f[19];
+            int n_f = 1;
+            f[0] = lo;
+            for (const char* q = lo; (q = (const char*)memchr(q, '\t', (size_t)(hi - q))) != nullptr; ++q) {
+                if (n_f < 18) f[n_f] = q + 1;
+                ++n_f;
+            }
+            if (n_f != 18) { ck.err = 1; ck.err_line = ck.lines; ck.err_fields = n_f; return; }
+            f[18] = hi + 1;
+            auto len = [&](int j) { return (size_t)(f[j + 1] - 1 - f[j]); };
+            if (!wanted(f[1], len(1))) continue;
+            if (!report_all && len(2) == 14 && memcmp(f[2], "nontranslating", 14) == 0) continue;
+            const int64_t o = oids.find(f[0], len(0));
+            if (o < 0) { ck.err = 2; ck.err_line = ck.lines; ck.err_id = std::string_view(f[0], len(0)); return; }
+            const std::string_view key(f[11], (size_t)(f[13] - 1 - f[11]));
+            auto g = gene_id.emplace(key, (int32_t)ck.genes.size());
+            if (g.second) ck.genes.push_back(key);
+            const uint64_t sk = (uint64_t)g.first->second << 32 | (uint64_t)ix->orf_chrom[o] << 2 | ix->orf_strand[o];
+            auto s = gseq_id.emplace(sk, (int32_t)ck.gseqs.size());
+            if (s.second) ck.gseqs.push_back(sk);
+            ck.row.push_back(o);
+            ck.line.push_back(ck.lines);
+            ck.prof_off.push_back(f[17] - base);
+            ck.prof_len.push_back(len(17));
+            ck.gene.push_back(g.first->second);
+            ck.gseq.push_back(s.first->second);
+        }
+    });
+    // 2. the first error in file order; line 1 is the header
+    int64_t lines_before = 2;
+    for (const Chunk& ck : chunks) {
+        if (ck.err == 1) {
+            g_io_error = std::string(path) + " line " + std::to_string(lines_before + ck.err_line) + ": " +
+                         std::to_string(ck.err_fields) + " tab-separated fields, 18 expected";
+            return RT_EINVAL;
+        }
+        if (ck.err == 2) {
+            g_io_error = std::string(path) + " line " + std::to_string(lines_before + ck.err_line) + ": ORF_ID " +
+                         std::string(ck.err_id.substr(0, 200)) + " is not in the index with an ORF_type of the features";
+            return RT_EINVAL;
+        }
+        lines_before += ck.lines;
+    }
+    h->n_lines = lines_before - 2;
+    // 3. merge in file order: gene and (gene, chrom, strand) ids follow first appearance
+    std::unordered_map<std::string_view, int32_t> gene_id;
+    std::unordered_map<uint64_t, int32_t> gseq_id;
+    std::vector<std::vector<int32_t>> gene_map(chunks.size()), gseq_map(chunks.size());
+    size_t n_sel = 0;
+    for (size_t k = 0; k < chunks.size(); ++k) {
+        for (const std::string_view& key : chunks[k].genes) {
+            auto g = gene_id.emplace(key, (int32_t)h->gene_key.size());
+            if (g.second) {
+                h->gene_key.push_back(key.data() - base);
+                h->gene_key_len.push_back((int32_t)key.size());
+                h->gene_id_len.push_back((int32_t)(std::find(key.begin(), key.end(), '\t') - key.begin()));
+            }
+            gene_map[k].push_back(g.first->second);
+        }
+        for (uint64_t sk : chunks[k].gseqs) {
+            const uint64_t gk = (uint64_t)gene_map[k][(size_t)(sk >> 32)] << 32 | (sk & 0xffffffffu);
+            auto s = gseq_id.emplace(gk, (int32_t)gseq_id.size());
+            gseq_map[k].push_back(s.first->second);
+        }
+        n_sel += chunks[k].row.size();
+    }
+    h->n_gseq = (int64_t)gseq_id.size();
+    h->row.resize(n_sel); h->line.resize(n_sel); h->prof_off.resize(n_sel); h->prof_len.resize(n_sel);
+    h->gene.resize(n_sel); h->gseq.resize(n_sel);
+    std::vector<size_t> sel0(chunks.size() + 1, 0);
+    std::vector<int64_t> line0(chunks.size() + 1, 2);
+    for (size_t k = 0; k < chunks.size(); ++k) {
+        sel0[k + 1] = sel0[k] + chunks[k].row.size();
+        line0[k + 1] = line0[k] + chunks[k].lines;
+    }
+    run_parallel(n_thr, [&](int kk) {
+        const size_t k = (size_t)kk, s0 = sel0[k];
+        const Chunk& ck = chunks[k];
+        for (size_t i = 0; i < ck.row.size(); ++i) {
+            h->row[s0 + i] = ck.row[i];
+            h->line[s0 + i] = line0[k] + ck.line[i];
+            h->prof_off[s0 + i] = ck.prof_off[i];
+            h->prof_len[s0 + i] = ck.prof_len[i];
+            h->gene[s0 + i] = gene_map[k][(size_t)ck.gene[i]];
+            h->gseq[s0 + i] = gseq_map[k][(size_t)ck.gseq[i]];
+        }
+    });
+    *out = h.release();
+    return RT_OK;
+}
+
+int rt_codon_load_seq(rt_codon* h, const rt_index* ix, const char* path) {
+    if (!h || !ix || !path) return RT_EINVAL;
+    if (const int rc = read_file(path, h->seq)) return rc;
+    const char* text = h->seq.data();
+    const int64_t size = (int64_t)h->seq.size();
+    const int64_t n = (int64_t)ix->orf_chrom.size();
+    const std::string where = std::string(path) + " line ";
+    const char* hint = "; was it written by orfs-seq from this index, without --protein?";
+    static const char kHeader[] = "ORF_ID\tsequence";
+    const char* nl = (const char*)memchr(text, '\n', (size_t)size);
+    const int64_t head_end = nl ? nl - text : size;
+    if (head_end != (int64_t)sizeof kHeader - 1 || memcmp(text, kHeader, sizeof kHeader - 1) != 0) {
+        g_io_error = where + "1: the header is not ORF_ID<tab>sequence" + hint;
+        return RT_EINVAL;
+    }
+    // every line's place is known from the index: row k is id, tab, length letters, newline at line_off[k]
+    std::vector<int64_t> id_off((size_t)n + 1), L((size_t)n), line_off((size_t)n + 1);
+    rt_index_ids(ix, id_off.data(), nullptr);
+    line_off[0] = head_end + 1;
+    for (int64_t k = 0; k < n; ++k) {
+        int64_t len = 0;
+        for (int64_t e = ix->exon_ptr[k]; e < ix->exon_ptr[k + 1]; ++e) len += (int64_t)ix->exon_end[e] - ix->exon_start[e] + 1;
+        L[(size_t)k] = len;
+        line_off[(size_t)k + 1] = line_off[(size_t)k] + (id_off[(size_t)k + 1] - id_off[(size_t)k]) + 1 + len + 1;
+    }
+    std::vector<char> ids((size_t)std::max<int64_t>(1, id_off[(size_t)n]));
+    rt_index_ids(ix, id_off.data(), ids.data());
+    static const struct Letters {
+        bool ok[256] = {};
+        Letters() { for (char c : std::string("ACGTN")) ok[(unsigned char)c] = true; }
+    } letters;
+    auto row_ok = [&](int64_t k) {
+        const int64_t off = line_off[(size_t)k], id_len = id_off[(size_t)k + 1] - id_off[(size_t)k];
+        const int64_t stop = off + id_len + 1 + L[(size_t)k];
+        if (stop > size || memcmp(text + off, ids.data() + id_off[(size_t)k], (size_t)id_len) != 0 || text[off + id_len] != '\t')
+            return false;
+        if (stop < size && text[stop] != '\n') return false;
+        for (const unsigned char* q = (const unsigned char*)text + off + id_len + 1; q < (const unsigned char*)text + stop; ++q)
+            if (!letters.ok[*q]) return false;
+        return true;
+    };
+    const int64_t block = 1 << 12, n_blocks = (n + block - 1) / block;
+    std::vector<int64_t> first_bad((size_t)std::max<int64_t>(1, n_blocks), INT64_MAX);
+    claim_parallel(host_threads((size_t)(size >> 22) + 1, 16, "RT_CODON_THREADS"), (size_t)n_blocks, [&](size_t b) {
+        for (int64_t k = (int64_t)b * block; k < std::min(n, (int64_t)(b + 1) * block); ++k)
+            if (!row_ok(k)) { first_bad[b] = k; return; }
+    });
+    const int64_t bad = *std::min_element(first_bad.begin(), first_bad.end());
+    if (bad != INT64_MAX) {
+        // rows before `bad` matched exactly, so its line starts at line_off[bad]
+        const int64_t k = bad, off = line_off[(size_t)k], line_no = k + 2;
+        const std::string want(ids.data() + id_off[(size_t)k], (size_t)(id_off[(size_t)k + 1] - id_off[(size_t)k]));
+        if (off >= size) {
+            g_io_error = std::string(path) + ": the file ends after line " + std::to_string(k + 1) + ", the index has " +
+                         std::to_string(n) + " rows" + hint;
+            return RT_EINVAL;
+        }
+        const char* eol = (const char*)memchr(text + off, '\n', (size_t)(size - off));
+        const int64_t stop = eol ? eol - text : size;
+        const char* tab = (const char*)memchr(text + off, '\t', (size_t)(stop - off));
+        if (!tab || std::string(text + off, tab) != want) {
+            const int64_t got = (tab ? tab - text : stop) - off;
+            g_io_error = where + std::to_string(line_no) + ": ORF_ID " + std::string(text + off, (size_t)std::min<int64_t>(got, 200)) +
+                         " is not " + want + ", the ORF_ID of index row " + std::to_string(k + 1) + hint;
+            return RT_EINVAL;
+        }
+        const int64_t got = stop - (tab + 1 - text);
+        if (got != L[(size_t)k]) {
+            g_io_error = where + std::to_string(line_no) + ": the sequence of " + want + " has " + std::to_string(got) +
+                         " letters, the index row has " + std::to_string(L[(size_t)k]) + " nt" + hint;
+            return RT_EINVAL;
+        }
+        int64_t at = 0;
+        while (letters.ok[(unsigned char)tab[1 + at]]) ++at;
+        g_io_error = where + std::to_string(line_no) + ": the sequence of " + want + " holds a letter other than A, C, G, T and N at " +
+                     "position " + std::to_string(at + 1) + hint;
+        return RT_EINVAL;
+    }
+    const int64_t done = std::min(line_off[(size_t)n], size);
+    if (done < size) {
+        g_io_error = where + std::to_string(n + 2) + ": the file has more lines than the index has rows (" + std::to_string(n) + ")" + hint;
+        return RT_EINVAL;
+    }
+    h->seq_off.resize((size_t)n);
+    for (int64_t k = 0; k < n; ++k) h->seq_off[(size_t)k] = line_off[(size_t)k] + (id_off[(size_t)k + 1] - id_off[(size_t)k]) + 1;
+    return RT_OK;
+}
+
+void rt_codon_free(rt_codon* h) { delete h; }
+
+int rt_codon_sizes(const rt_codon* h, int64_t* sizes) {
+    if (!h || !sizes) return RT_EINVAL;
+    sizes[0] = (int64_t)h->row.size();
+    sizes[1] = (int64_t)h->gene_key.size();
+    sizes[2] = h->n_gseq;
+    sizes[3] = h->n_lines;
+    return RT_OK;
+}
+
+int rt_codon_copy(const rt_codon* h, int64_t* row, int32_t* gene, int32_t* gseq, int64_t* line, int64_t* prof_off,
+                  int64_t* prof_len, int64_t* seq_off) {
+    if (!h) return RT_EINVAL;
+    auto copy = [](void* dst, const void* src, size_t bytes) { if (dst && bytes) memcpy(dst, src, bytes); };
+    const size_t n = h->row.size();
+    copy(row, h->row.data(), 8 * n);
+    copy(gene, h->gene.data(), 4 * n);
+    copy(gseq, h->gseq.data(), 4 * n);
+    copy(line, h->line.data(), 8 * n);
+    copy(prof_off, h->prof_off.data(), 8 * n);
+    copy(prof_len, h->prof_len.data(), 8 * n);
+    copy(seq_off, h->seq_off.data(), 8 * h->seq_off.size());
+    return RT_OK;
+}
+
+const char* rt_codon_gene(const rt_codon* h, int64_t g, int* id_len, int* name_len) {
+    if (!h || g < 0 || g >= (int64_t)h->gene_key.size()) return nullptr;
+    const int il = h->gene_id_len[(size_t)g];
+    if (id_len) *id_len = il;
+    if (name_len) *name_len = h->gene_key_len[(size_t)g] - il - 1;
+    return h->tsv.data() + h->gene_key[(size_t)g];
+}
+
+const char* rt_codon_text(const rt_codon* h, int which, int64_t* len) {
+    if (!h || (which != 0 && which != 1)) return nullptr;
+    const HostArr<char>& t = which == 0 ? h->tsv : h->seq;
+    if (len) *len = (int64_t)t.size();
+    return t.data();
+}
+
+int rt_codon_write(const rt_codon* h, const uint64_t* gene_tab, const uint64_t* pooled_tab, const char* gene_path,
+                   const char* pooled_path) {
+    if (!h || !gene_path || !pooled_path || !pooled_tab || (!h->gene_key.empty() && !gene_tab)) return RT_EINVAL;
+    const int64_t n_gene = (int64_t)h->gene_key.size();
+    // genes by (gene_id, gene_name): byte order equals Python's str order
+    auto part = [&](int64_t g, int which) {
+        int il = 0, nl = 0;
+        const char* p = rt_codon_gene(h, g, &il, &nl);
+        return which == 0 ? std::string_view(p, (size_t)il) : std::string_view(p + il + 1, (size_t)nl);
+    };
+    std::vector<int64_t> order((size_t)n_gene);
+    for (int64_t g = 0; g < n_gene; ++g) order[(size_t)g] = g;
+    std::sort(order.begin(), order.end(), [&](int64_t a, int64_t b) {
+        const int c = part(a, 0).compare(part(b, 0));
+        return c != 0 ? c < 0 : part(a, 1) < part(b, 1);
+    });
+    const int n_thr = host_threads((size_t)(n_gene >> 10), 16);
+    std::vector<TextBuf> parts((size_t)n_thr + 1);
+    parts[0].append("gene_id\tcodon\tcodon_occurrences\ttotal_codon_coverage\tmean_codon_coverage\tmedian_codon_coverage\t"
+                    "var_codon_coverage\n", 114);
+    std::vector<char> ok_part((size_t)n_thr, 1);
+    run_parallel(n_thr, [&](int k) {
+        TextBuf& b = parts[(size_t)k + 1];
+        std::string num;
+        for (int64_t i = n_gene * k / n_thr; i < n_gene * (k + 1) / n_thr; ++i) {
+            const int64_t g = order[(size_t)i];
+            const std::string_view id = part(g, 0);
+            for (int c = 0; c < 64; ++c) {
+                const uint64_t* cell = gene_tab + 5 * (64 * g + c);
+                if (!cell[0]) continue;
+                if (!b.need(id.size() + 256)) { ok_part[(size_t)k] = 0; return; }   // room for the whole row
+                b.append(id.data(), id.size());
+                b.append("\t", 1);
+                put_codon(b, c);
+                put_stats(b, cell, num);
+            }
+        }
+    });
+    TextBuf pooled;
+    pooled.append("codon\tcodon_occurrences\ttotal_codon_coverage\tmean_codon_coverage\tmedian_codon_coverage\t"
+                  "var_codon_coverage\n", 106);
+    std::string num;
+    for (int c = 0; c < 64; ++c)
+        if (pooled_tab[5 * c]) { put_codon(pooled, c); put_stats(pooled, pooled_tab + 5 * c, num); }
+    if (!parts[0].base || !pooled.base || std::find(ok_part.begin(), ok_part.end(), 0) != ok_part.end()) {
+        g_io_error = "out of memory";
+        return RT_ENOMEM;
+    }
+    bool ok = true;
+    FILE* fg = fopen(gene_path, "wb");
+    if (!fg) { g_io_error = std::string("cannot open ") + gene_path; return RT_EINVAL; }
+    {
+        WriteBehind w(fg);
+        for (TextBuf& b : parts) ok = ok && w.put(std::move(b));
+        ok = w.finish() && ok;
+    }
+    ok = fclose(fg) == 0 && ok;
+    FILE* fp = ok ? fopen(pooled_path, "wb") : nullptr;
+    if (fp) {
+        ok = fwrite(pooled.base, 1, pooled.len, fp) == pooled.len;
+        ok = fclose(fp) == 0 && ok;
+    } else {
+        ok = false;
+    }
+    if (!ok) {
+        g_io_error = std::string("cannot write ") + gene_path + " or " + pooled_path;
+        remove(gene_path);
+        remove(pooled_path);
+        return RT_EINVAL;
+    }
     return RT_OK;
 }
 

@@ -2685,4 +2685,232 @@ __global__ void __launch_bounds__(kSeqWarps * 32) orf_seq_kernel(SeqArgs A, long
     }
 }
 
+// ---------------------------------------------------------------------------------------------- count-orfs-codon
+// codon_emit_kernel: one warp per selected TSV row, claimed dynamically (profiles run from "[]" to more than 100 knt).
+// The warp reads the profile text in 32-byte windows: every byte is checked against the grammar "[" (D(", "D)*)? "]"
+// with D = 0 | [1-9][0-9]*, a ballot of the digits that follow a non-digit finds the values, and each lane parses the
+// value it starts and adds it to the count of its codon (a zero adds nothing).  Then codon k < min(values, length) / 3
+// is named from the row's letters (6-bit code 16 b0 + 4 b1 + b2, A C G T = 0 1 2 3) and placed on the genome: its first
+// oriented nt, through the row's intervals ('-' rows walk them from the right).  Slot k of the row gets the place key
+// gseq << 32 | first nt and the value (gene * 64 + code) << 32 | count; a codon with N, or past the profile, gets the key
+// ~0 (dropped).
+struct CodonArgs {
+    const char* prof;                 // profile text of the selected rows, back to back
+    const long long* prof_base;       // n_sel + 1
+    const char* seq;                  // their letters, back to back
+    const long long* seq_base;        // n_sel + 1: row lengths
+    const long long* slot_base;       // n_sel + 1: floor(length / 3) slots per row
+    const long long* row;             // index row of each selected row
+    const long long* exon_ptr;
+    const int* ex_start;
+    const int* ex_end;
+    const uint8_t* strand;            // per index row, 1: reverse
+    const int* gene;
+    const int* gseq;
+    unsigned long long* cnt;          // per slot: codon count, zeroed before the launch
+    unsigned long long* pos_key;      // per slot: place key
+    unsigned long long* val;          // per slot: (gene * 64 + codon) << 32 | count
+    unsigned long long* counters;     // [0] codons named, [1] with N, [2] first refused row (atomicMin), zeroed / ~0
+    uint8_t* flag;                    // per selected row: 1 malformed, 2 value above 2^31 - 1, 4 codon count above 2^32 - 1
+    long long n_sel;
+    unsigned* claim;                  // work counter, zeroed before the launch
+};
+
+constexpr int kCodonWarps = 8;
+
+__device__ __forceinline__ bool is_digit(char c) { return c >= '0' && c <= '9'; }
+
+__global__ void __launch_bounds__(kCodonWarps * 32) codon_emit_kernel(const CodonArgs A) {
+    const int lane = threadIdx.x & 31;
+    const unsigned below = (1u << lane) - 1u;
+    for (;;) {
+        unsigned t = 0;
+        if (lane == 0) t = atomicAdd(A.claim, 1u);
+        t = __shfl_sync(kFull, t, 0);
+        if ((long long)t >= A.n_sel) return;
+        const char* s = A.prof + A.prof_base[t];
+        const long long n = A.prof_base[t + 1] - A.prof_base[t];
+        const long long L = A.seq_base[t + 1] - A.seq_base[t];
+        const long long s0 = A.slot_base[t], n_slot = A.slot_base[t + 1] - s0;
+        unsigned bad = 0;
+        long long P = 0;                                   // values parsed
+        if (n < 2 || s[0] != '[' || s[n - 1] != ']') {
+            bad = 1;
+        } else {
+            const char* b = s + 1;
+            const long long nb = n - 2;
+            for (long long w = 0; w < nb; w += 32) {
+                const long long i = w + lane;
+                bool start = false;
+                unsigned long long v = 0;
+                if (i < nb) {
+                    const char c = b[i], p = i > 0 ? b[i - 1] : ' ', q = i + 1 < nb ? b[i + 1] : ',';
+                    if (is_digit(c)) {                     // the defaults of p and q refuse a separator at either end
+                        start = !is_digit(p);
+                    } else if (c == ',') {
+                        if (!is_digit(p) || q != ' ') bad |= 1;
+                    } else if (c == ' ') {
+                        if (p != ',' || !is_digit(q)) bad |= 1;
+                    } else {
+                        bad |= 1;
+                    }
+                    if (start) {
+                        if (c == '0' && i + 1 < nb && is_digit(b[i + 1])) bad |= 1;   // a leading zero
+                        int d = 0;
+                        for (long long j = i; j < nb && is_digit(b[j]) && d < 11; ++j, ++d) v = v * 10 + (b[j] - '0');
+                        if (d > 10 || v > 2147483647ull) bad |= 2;
+                    }
+                }
+                const unsigned starts = __ballot_sync(kFull, start);
+                if (start && v && !bad) {
+                    const long long j = P + __popc(starts & below);
+                    if (j / 3 < n_slot) atomicAdd(A.cnt + s0 + j / 3, v);
+                }
+                P += __popc(starts);
+            }
+        }
+        bad = __reduce_or_sync(kFull, bad);
+        __syncwarp();                                      // the counts of this row are in place (read through L2 below)
+        if (bad) {
+            if (lane == 0) {
+                A.flag[t] = (uint8_t)bad;
+                atomicMin(A.counters + 2, (unsigned long long)t);
+            }
+            continue;
+        }
+        const long long n_cod = min(P, L) / 3;
+        const long long r = A.row[t], e0 = A.exon_ptr[r], e1 = A.exon_ptr[r + 1];
+        const bool rev = A.strand[r] == 1;
+        const char* letters = A.seq + A.seq_base[t];
+        const unsigned long long hi_gene = (unsigned long long)A.gene[t] * 64ull;
+        const unsigned long long hi_place = (unsigned long long)(unsigned)A.gseq[t] << 32;
+        // per lane: interval cursor `e` and the nt of the intervals left of it, `before` (ascending order)
+        long long e = rev ? e1 - 1 : e0, before = 0;
+        if (rev) {
+            long long tail = 0;
+            for (long long x = e0; x < e1 - 1; ++x) tail += A.ex_end[x] - A.ex_start[x] + 1;
+            before = tail;
+        }
+        unsigned named = 0, with_n = 0, over = 0;
+        for (long long k = lane; k < n_slot; k += 32) {
+            unsigned long long key = ~0ull, value = 0;
+            if (k < n_cod) {
+                const unsigned long long c = __ldcg(A.cnt + s0 + k);
+                over |= c > 0xffffffffull;
+                const char* l3 = letters + 3 * k;
+                int code = 0;
+                bool has_n = false;
+#pragma unroll
+                for (int u = 0; u < 3; ++u) {
+                    const char x = l3[u];
+                    has_n |= x == 'N';
+                    code = code * 4 + (x == 'C' ? 1 : x == 'G' ? 2 : x == 'T' ? 3 : 0);
+                }
+                ++named;
+                if (has_n) {
+                    ++with_n;
+                } else {
+                    const long long a = rev ? L - 1 - 3 * k : 3 * k;      // ascending index of the first oriented nt
+                    if (rev) {
+                        while (a < before) { --e; before -= A.ex_end[e] - A.ex_start[e] + 1; }
+                    } else {
+                        while (a >= before + (A.ex_end[e] - A.ex_start[e] + 1)) { before += A.ex_end[e] - A.ex_start[e] + 1; ++e; }
+                    }
+                    const int pos = A.ex_start[e] + (int)(a - before);
+                    key = hi_place | (unsigned)pos;
+                    value = (hi_gene + (unsigned long long)code) << 32 | (c & 0xffffffffull);
+                }
+            }
+            A.pos_key[s0 + k] = key;
+            A.val[s0 + k] = value;
+        }
+        named = __reduce_add_sync(kFull, named);
+        with_n = __reduce_add_sync(kFull, with_n);
+        over = __reduce_or_sync(kFull, over);
+        if (lane == 0) {
+            if (named) atomicAdd(A.counters + 0, (unsigned long long)named);
+            if (with_n) atomicAdd(A.counters + 1, (unsigned long long)with_n);
+            if (over) {
+                A.flag[t] = 4;
+                atomicMin(A.counters + 2, (unsigned long long)t);
+            }
+        }
+    }
+}
+
+// After the stable sort by place key: the first slot of every place is kept.  Appends its value to `kept` and its
+// pooled key (codon << 32 | count) to `pooled`; the order of the appends does not matter (both are sorted next).
+__global__ void __launch_bounds__(256) codon_keep_kernel(const unsigned long long* __restrict__ key,
+                                                         const unsigned long long* __restrict__ val, long long n,
+                                                         unsigned long long* kept, unsigned long long* pooled,
+                                                         unsigned long long* n_kept) {
+    const int lane = threadIdx.x & 31;
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    for (long long w = (long long)blockIdx.x * blockDim.x + (threadIdx.x & ~31); w < n; w += stride) {
+        const long long i = w + lane;
+        bool keep = false;
+        if (i < n) {
+            const unsigned long long k = key[i];
+            keep = k != ~0ull && (i == 0 || key[i - 1] != k);
+        }
+        const unsigned b = __ballot_sync(kFull, keep);
+        unsigned long long at = 0;
+        if (lane == 0 && b) at = atomicAdd(n_kept, (unsigned long long)__popc(b));
+        at = __shfl_sync(kFull, at, 0);
+        if (keep) {
+            const unsigned long long v = val[i], o = at + __popc(b & ((1u << lane) - 1u));
+            kept[o] = v;
+            pooled[o] = ((v >> 32) & 63ull) << 32 | (v & 0xffffffffull);
+        }
+    }
+}
+
+// One warp per cell (the keys whose high 32 bits equal the cell, counts in the low 32 bits, sorted): n, S1, S2 (two
+// 64-bit halves) and the sum of the middle two counts (twice the middle one for odd n).  Exact integers: the result
+// does not depend on the order of the additions.
+__global__ void __launch_bounds__(256) codon_stats_kernel(const unsigned long long* __restrict__ keys, long long n,
+                                                          long long n_cells, unsigned long long* __restrict__ out) {
+    const int lane = threadIdx.x & 31;
+    const long long warps = (long long)gridDim.x * (blockDim.x >> 5);
+    auto lower = [&](unsigned long long x) {              // first key >= x (every lane searches the same addresses)
+        long long a = 0, b = n;
+        while (a < b) {
+            const long long m = (a + b) >> 1;
+            if (keys[m] < x) a = m + 1; else b = m;
+        }
+        return a;
+    };
+    for (long long c = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; c < n_cells; c += warps) {
+        const long long lo = lower((unsigned long long)c << 32), hi = lower((unsigned long long)(c + 1) << 32);
+        unsigned long long s1 = 0, s2_lo = 0, s2_hi = 0;
+        for (long long i = lo + lane; i < hi; i += 32) {
+            const unsigned long long x = keys[i] & 0xffffffffull, sq = x * x;
+            s1 += x;
+            s2_lo += sq;
+            s2_hi += s2_lo < sq;
+        }
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) {
+            s1 += __shfl_xor_sync(kFull, s1, d);
+            const unsigned long long o_lo = __shfl_xor_sync(kFull, s2_lo, d), o_hi = __shfl_xor_sync(kFull, s2_hi, d);
+            s2_lo += o_lo;
+            s2_hi += o_hi + (s2_lo < o_lo);
+        }
+        if (lane == 0) {
+            const long long m = hi - lo;
+            unsigned long long mid = 0;
+            if (m) {
+                const unsigned long long x1 = keys[lo + m / 2] & 0xffffffffull;
+                mid = m & 1 ? 2 * x1 : x1 + (keys[lo + m / 2 - 1] & 0xffffffffull);
+            }
+            unsigned long long* o = out + 5 * c;
+            o[0] = (unsigned long long)m;
+            o[1] = s1;
+            o[2] = s2_lo;
+            o[3] = s2_hi;
+            o[4] = mid;
+        }
+    }
+}
+
 }  // namespace rt

@@ -500,3 +500,31 @@ class Engine:
         self._check(rc)
         if stage_ms is not None:
             stage_ms[:] = ms
+
+    # --------------------------------------------------------------- count-orfs-codon
+    def codon_counts(self, sel: dict, tsv, seq, exon_ptr, exon_start, exon_end, orf_strand, n_gene: int, n_gseq: int,
+                     stage_ms: np.ndarray | None = None):
+        """The codon tables of DESIGN.md section 11 (``rt_codon_counts``).  ``sel`` holds the columns of the selected
+        TSV rows (``row``, ``gene``, ``gseq``, ``prof_off``, ``prof_len``) and ``seq_off`` per index row; ``tsv`` and
+        ``seq`` are the two file texts (uint8).  Returns (gene table [n_gene * 64, 5], pooled table [64, 5], summary[6])
+        as uint64 / int64 arrays: see ``rt_codon_counts`` in the header."""
+        arr = lambda a, dt: np.ascontiguousarray(a, dt)  # noqa: E731
+        row, gene, gseq = arr(sel["row"], np.int64), arr(sel["gene"], np.int32), arr(sel["gseq"], np.int32)
+        prof_off, prof_len, seq_off = arr(sel["prof_off"], np.int64), arr(sel["prof_len"], np.int64), arr(sel["seq_off"], np.int64)
+        exon_ptr, exon_start, exon_end = arr(exon_ptr, np.int64), arr(exon_start, np.int32), arr(exon_end, np.int32)
+        orf_strand = arr(orf_strand, np.uint8)
+        q = _lib.CodonQuery(len(row), _np_ptr(row), _np_ptr(gene), _np_ptr(gseq), _np_ptr(prof_off), _np_ptr(prof_len),
+                            _np_ptr(tsv), _np_ptr(seq_off), _np_ptr(seq), len(exon_ptr) - 1, _np_ptr(exon_ptr),
+                            _np_ptr(exon_start), _np_ptr(exon_end), _np_ptr(orf_strand), int(n_gene), int(n_gseq))
+        gene_tab = np.zeros((64 * int(n_gene), _lib.RT_CODON_CELL), np.uint64)
+        pooled_tab = np.zeros((64, _lib.RT_CODON_CELL), np.uint64)
+        summary = np.zeros(6, np.int64)
+        ms = np.zeros(_lib.RT_CODON_STAGES, np.float32)
+        rc = self.lib.rt_codon_counts(self.ctx, C.byref(q), _np_ptr(gene_tab), _np_ptr(pooled_tab), _np_ptr(summary),
+                                      _np_ptr(ms))
+        if rc == _lib.RT_EINVAL:
+            raise ValueError(self.lib.rt_last_error(self.ctx).decode())
+        self._check(rc)
+        if stage_ms is not None:
+            stage_ms[:] = ms
+        return gene_tab, pooled_tab, summary
