@@ -7,6 +7,7 @@
 #include <cstring>
 #include <atomic>
 #include <chrono>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <unordered_map>
@@ -25,23 +26,80 @@ namespace {
 
 thread_local std::string g_last_error;
 
-struct DevBuf {
-    void* p = nullptr;
-    size_t cap = 0;
-    cudaError_t reserve(size_t bytes) {
-        if (bytes <= cap) return cudaSuccess;
+// Device memory for at least n elements of T, freed with its owner.  reserve() only grows and keeps nothing; it
+// allocates one element and 16 bytes at the least, so an empty table is still a valid kernel argument.
+template <class T>
+struct DevArr {
+    T* p = nullptr;
+    size_t n = 0;
+    DevArr() = default;
+    DevArr(DevArr&& o) noexcept : p(o.p), n(o.n) { o.p = nullptr; o.n = 0; }
+    DevArr& operator=(DevArr&& o) noexcept { std::swap(p, o.p); std::swap(n, o.n); return *this; }
+    ~DevArr() { if (p) cudaFree(p); }
+    cudaError_t reserve(size_t m) {
+        if (m <= n) return cudaSuccess;
         if (p) cudaFree(p);
         p = nullptr;
-        cap = 0;
+        n = 0;
+        const size_t bytes = std::max<size_t>(sizeof(T) * std::max<size_t>(m, 1), 16);
         cudaError_t e = cudaMalloc(&p, bytes);
-        if (e == cudaSuccess) cap = bytes;
+        if (e == cudaSuccess) n = bytes / sizeof(T);
         return e;
     }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
+    // reserve(m), then the first m elements from the host (S: a host type of the same size, e.g. int64_t for long long)
+    template <class S>
+    cudaError_t upload(const S* src, size_t m) {
+        static_assert(sizeof(S) == sizeof(T), "host and device elements differ in size");
+        cudaError_t e = reserve(m);
+        return e != cudaSuccess || m == 0 ? e : cudaMemcpy(p, src, sizeof(T) * m, cudaMemcpyHostToDevice);
     }
+    template <class S>
+    cudaError_t upload(const S* src, size_t m, cudaStream_t st) {
+        static_assert(sizeof(S) == sizeof(T), "host and device elements differ in size");
+        cudaError_t e = reserve(m);
+        return e != cudaSuccess || m == 0 ? e : cudaMemcpyAsync(p, src, sizeof(T) * m, cudaMemcpyHostToDevice, st);
+    }
+};
+
+// Page-locked host memory for n elements of T, freed with its owner.
+template <class T>
+struct PinnedArr {
+    T* p = nullptr;
+    size_t n = 0;
+    PinnedArr() = default;
+    PinnedArr(const PinnedArr&) = delete;
+    PinnedArr& operator=(const PinnedArr&) = delete;
+    ~PinnedArr() { if (p) cudaFreeHost(p); }
+    cudaError_t alloc(size_t m) {
+        if (p) cudaFreeHost(p);
+        p = nullptr;
+        n = 0;
+        cudaError_t e = cudaHostAlloc(&p, sizeof(T) * m, cudaHostAllocDefault);
+        if (e == cudaSuccess) n = m;
+        return e;
+    }
+};
+
+// A non-blocking stream, destroyed with its owner; create() does nothing once the stream exists.
+struct Stream {
+    cudaStream_t s = nullptr;
+    Stream() = default;
+    Stream(const Stream&) = delete;
+    Stream& operator=(const Stream&) = delete;
+    ~Stream() { if (s) cudaStreamDestroy(s); }
+    cudaError_t create() { return s ? cudaSuccess : cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking); }
+    operator cudaStream_t() const { return s; }
+};
+
+// An event, destroyed with its owner; create() does nothing once the event exists.
+struct Event {
+    cudaEvent_t e = nullptr;
+    Event() = default;
+    Event(const Event&) = delete;
+    Event& operator=(const Event&) = delete;
+    ~Event() { if (e) cudaEventDestroy(e); }
+    cudaError_t create(unsigned flags = cudaEventDefault) { return e ? cudaSuccess : cudaEventCreateWithFlags(&e, flags); }
+    operator cudaEvent_t() const { return e; }
 };
 
 }  // namespace
@@ -58,85 +116,102 @@ struct rt_ctx {
     int pad = 0;
     int64_t plane = 0;
     std::vector<int64_t> contig_len, contig_base;
-    int2* d_contig_tab = nullptr;                    // per contig: (length, first slot >> 5)
-    double2* d_uv_table = nullptr;                   // unit vectors of small codons (rt::fill_uv_table), for phase B's seam windows
+    DevArr<int2> contig_tab;                         // per contig: (length, first slot >> 5)
+    DevArr<double2> uv_table;                        // unit vectors of small codons (rt::fill_uv_table), for phase B's seam windows
 
     // read-length table
-    int32_t* d_len_table = nullptr;
+    DevArr<int32_t> len_table;
     bool have_len_table = false;
     int len_base = 20;   // first of the 16 read lengths K1 counts in registers
     int zone_delta_plus = 0, zone_delta_minus = 0;   // smallest P-site displacement from `first` on either strand
 
-    // index
-    int64_t n_orf = 0;
-    uint64_t* d_orf_desc = nullptr;
-    int32_t* d_orf_len = nullptr;
-    cudaEvent_t ev_scored = nullptr;                 // rt_score_host: a part's columns are ready for their copy
-    uint64_t* d_exon_entries = nullptr;
-    std::vector<int64_t> bytes_prefix;  // n_orf + 1: prefix of 4L + 8E + 42
-    std::vector<int64_t> nt_prefix;     // n_orf + 1: prefix of L
-    unsigned long long* d_work_counter = nullptr;   // 4 x u64: work counters of phase A (0) and the fallback (2), fallback count (3)
-
-    // two-phase scoring: atoms (coverage intervals no ORF exon boundary splits) and per-ORF atom refs
-    int64_t n_atoms = 0;
-    uint64_t* d_atoms = nullptr;                     // (slot offset << 24) | len
-    rt::AtomSummary* d_summaries = nullptr;          // per-library scratch, written by phase A
-    uint8_t* d_atom_nonzero = nullptr;               // per-library scratch: atom holds at least one read
-    // compact layout: the coverage buffer holds the exon union only (atoms back to back, genome order)
-    int layout = RT_LAYOUT_DENSE;
-    int64_t compact_elems = 0;                       // int32 elements of a compact coverage buffer (with guard)
-    unsigned* d_cbits = nullptr;                     // one bit per cmap word: the word has members
-    unsigned compact_plus_end = 0, compact_end = 0;  // compact index after the last '+' slot / after the last slot
-    DevBuf zone_buf, spill_buf;                      // rt_bin_stream_fresh: zone boundaries, spill list + its counter
-    uint2* d_cmap = nullptr;                         // per 32 dense slots: member mask | compact index after the last member
-    uint64_t* d_atoms_c = nullptr;                   // the same tables with compact slot offsets
-    uint64_t* d_exon_entries_c = nullptr;
-    std::vector<uint64_t> h_atoms;                   // host copies used to build per-range atom lists
-    std::vector<uint64_t> h_atoms_c;                 // ... with compact slot offsets
-    std::vector<uint64_t> h_orf_refs_desc;           // per ORF: ref begin | n_refs << 40 | reverse << 63
-    std::vector<uint32_t> h_ref_atom;                // atom id of every ref (0xffffffff: reads as zeros)
-    std::vector<uint64_t> h_ref_ent;                 // refs in profile order
+    Event ev_scored;                                 // rt_score_host: a part's columns are ready for their copy
+    DevArr<unsigned long long> work_counter;         // 4 x u64: work counters of phase A (0) and the fallback (2), fallback count (3)
 
     // score plan: the work lists of the three scoring launches for one ORF range
     struct ScorePlan {
         int64_t lo = -1, hi = -1;
-        int32_t* d_fallback = nullptr;  // ORFs redone by score_orfs_kernel; capacity hi - lo
-        int32_t* d_atom_list = nullptr; // atoms the range touches, similar lengths adjacent
+        DevArr<int32_t> fallback;       // ORFs redone by score_orfs_kernel; capacity hi - lo
+        DevArr<int32_t> atom_list;      // atoms the range touches, similar lengths adjacent
         int64_t n_atom_list = 0;
-        rt::PassDesc* d_passes = nullptr;      // compact layout: runs of adjacent atoms for atom_pass_kernel
+        DevArr<rt::PassDesc> passes;    // compact layout: runs of adjacent atoms for atom_pass_kernel
         int64_t n_passes = 0;
-        rt::RefRec* d_refs = nullptr;          // compose_refs_kernel: one slot per atom reference, groups of 32
-        rt::RefWarp* d_ref_warps = nullptr;
-        rt::LongAcc* d_long_acc = nullptr;     // one per ORF with more than 32 references
+        DevArr<rt::RefRec> refs;        // compose_refs_kernel: one slot per atom reference, groups of 32
+        DevArr<rt::RefWarp> ref_warps;
+        DevArr<rt::LongAcc> long_acc;   // one per ORF with more than 32 references
         int64_t n_ref_warps = 0;
     };
-    std::vector<ScorePlan> plans;
+
+    // Everything rt_set_index derives from the index; rt_set_index and rt_set_genome replace it as a whole.
+    struct Index {
+        int64_t n_orf = 0;
+        DevArr<uint64_t> orf_desc;
+        DevArr<int32_t> orf_len;
+        DevArr<uint64_t> exon_entries;
+        std::vector<int64_t> bytes_prefix{0};            // n_orf + 1: prefix of 4L + 8E + 42
+        std::vector<int64_t> nt_prefix{0};               // n_orf + 1: prefix of L
+
+        // two-phase scoring: atoms (coverage intervals no ORF exon boundary splits) and per-ORF atom refs
+        int64_t n_atoms = 0;
+        DevArr<uint64_t> atoms;                          // (slot offset << 24) | len
+        DevArr<rt::AtomSummary> summaries;               // per-library scratch, written by phase A
+        DevArr<uint8_t> atom_nonzero;                    // per-library scratch: atom holds at least one read
+        // compact layout: the coverage buffer holds the exon union only (atoms back to back, genome order)
+        int layout = RT_LAYOUT_DENSE;
+        int64_t compact_elems = 0;                       // int32 elements of a compact coverage buffer (with guard)
+        DevArr<unsigned> cbits;                          // one bit per cmap word: the word has members
+        unsigned compact_plus_end = 0, compact_end = 0;  // compact index after the last '+' slot / after the last slot
+        DevArr<uint2> cmap;                              // per 32 dense slots: member mask | compact index after the last member
+        DevArr<uint64_t> atoms_c;                        // the same tables with compact slot offsets
+        DevArr<uint64_t> exon_entries_c;
+        std::vector<uint64_t> h_atoms;                   // host copies used to build per-range atom lists
+        std::vector<uint64_t> h_atoms_c;                 // ... with compact slot offsets
+        std::vector<uint64_t> h_orf_refs_desc;           // per ORF: ref begin | n_refs << 40 | reverse << 63
+        std::vector<uint32_t> h_ref_atom;                // atom id of every ref (0xffffffff: reads as zeros)
+        std::vector<uint64_t> h_ref_ent;                 // refs in profile order
+
+        std::vector<ScorePlan> plans;
+    } ix;
+    DevArr<unsigned> zone_buf, spill_buf;            // rt_bin_stream_fresh: zone boundaries; spill counter (16 B), spill list
 
     // scratch for the host-buffer entry points
     struct HostStage {                               // page-locked staging of one chunk's record stream
-        uint32_t* rec = nullptr;
-        int32_t* hdr = nullptr;
-        cudaEvent_t copied = nullptr;
+        PinnedArr<uint32_t> rec;
+        PinnedArr<int32_t> hdr;
+        Event copied;
         bool busy = false;
     } host_stage[16];
     std::mutex launch_mutex;                         // the packing threads of rt_bin_reads_host launch K1 one at a time
-    DevBuf read_slot[16];
-    cudaStream_t slot_stream[16] = {};
-    DevBuf stats_buf, score_buf;
+    DevArr<char> read_slot[16];
+    Stream slot_stream[16];
+    DevArr<int64_t> stats_buf;                       // stats, then length counts
+    DevArr<char> score_buf;
 
     // sparse clear: slots touched by K1 since the last rt_clear_touched
     bool track_touched = false;
-    DevBuf touched_buf;
-    unsigned long long* d_n_touched = nullptr;
+    DevArr<unsigned long long> touched_buf;
+    DevArr<unsigned long long> n_touched;
     int64_t touched_reserved = 0;    // reads binned (weight +1) since the last clear
 
     // prepare-orfs (rt_orf_search / rt_orf_fetch): the last search's tables and rows stay on the device until fetched
-    DevBuf orf_buf[32];
+    struct OrfBufs {
+        DevArr<uint8_t> codes, ex_rev, tx_rev, seq, row_type, row_codon;
+        DevArr<long long> ex_src, ex_dst, tx_seq, tx_exon, tx_rows, row_off, iv_count, iv_off;
+        DevArr<int> ex_len, ex_start, ex_end, ex_before, row_tx, row_start, row_stop, iv_start, iv_end;
+        DevArr<int2> tx_cds;
+        DevArr<unsigned> claim;
+    } orf;
     std::vector<int64_t> orf_iv_ptr;                 // n_rows + 1: interval offsets of the last search
     int64_t orf_rows = 0;
 
     // orfs-seq (rt_orf_seq_write): the uploaded tables and the two chunk buffers, kept for the next call
-    DevBuf seq_buf[16];
+    struct SeqBufs {
+        DevArr<uint8_t> codes, strand;
+        DevArr<long long> exon_ptr, base, id_off, line_off;
+        DevArr<int> ex_start, ex_end, contig;
+        DevArr<char> ids, out[2];
+        DevArr<unsigned> claim;
+    } seq;
 };
 
 namespace {
@@ -174,17 +249,15 @@ struct DeviceGuard {
 
 // The touched-slot list holds one entry per read binned since the last clear; grow it keeping its content.
 int ensure_touched_capacity(rt_ctx* ctx, int64_t reads) {
-    const size_t need = sizeof(unsigned long long) * (size_t)reads;
-    if (need <= ctx->touched_buf.cap) return RT_OK;
-    DevBuf bigger;
-    RT_CUDA(ctx, bigger.reserve(std::max(need, ctx->touched_buf.cap * 2)));
+    if ((size_t)reads <= ctx->touched_buf.n) return RT_OK;
+    DevArr<unsigned long long> bigger;
+    RT_CUDA(ctx, bigger.reserve(std::max((size_t)reads, ctx->touched_buf.n * 2)));
     if (ctx->touched_buf.p) {
         RT_CUDA(ctx, cudaDeviceSynchronize());
         RT_CUDA(ctx, cudaMemcpy(bigger.p, ctx->touched_buf.p, sizeof(unsigned long long) * (size_t)ctx->touched_reserved,
                                 cudaMemcpyDeviceToDevice));
-        ctx->touched_buf.release();
     }
-    ctx->touched_buf = bigger;
+    ctx->touched_buf = std::move(bigger);
     return RT_OK;
 }
 
@@ -192,6 +265,7 @@ int ensure_touched_capacity(rt_ctx* ctx, int64_t reads) {
 // (no ORF exon boundary falls inside an atom; atoms longer than kAtomMaxNt are chopped) and express
 // every ORF as its sequence of atoms in profile order.
 int build_atoms(rt_ctx* ctx, const std::vector<uint64_t>& desc, const std::vector<uint64_t>& entries) {
+    rt_ctx::Index& ix = ctx->ix;
     const uint64_t kZero = rt::kZeroOff;
     std::vector<uint64_t> pts;
     pts.reserve(entries.size() * 2);
@@ -235,98 +309,87 @@ int build_atoms(rt_ctx* ctx, const std::vector<uint64_t>& desc, const std::vecto
     }
     // atoms of interval i are [atom_begin[i], atom_begin[i+1])
     std::vector<uint32_t> atom_begin(pts.size() + 1, 0);
-    ctx->h_atoms.clear();
+    ix.h_atoms.clear();
     int64_t cover = 0;
     for (size_t i = 0; i + 1 < pts.size(); ++i) {
         cover += diff[i];
-        atom_begin[i] = (uint32_t)ctx->h_atoms.size();
+        atom_begin[i] = (uint32_t)ix.h_atoms.size();
         if (cover > 0) {
             uint64_t at = pts[i];
             while (at < pts[i + 1]) {
                 const uint64_t piece = std::min<uint64_t>(pts[i + 1] - at, (uint64_t)rt::kAtomMaxNt);
-                ctx->h_atoms.push_back((at << rt::kLenBits) | piece);
+                ix.h_atoms.push_back((at << rt::kLenBits) | piece);
                 at += piece;
             }
         }
     }
-    if (!pts.empty()) atom_begin[pts.size() - 1] = atom_begin[pts.size()] = (uint32_t)ctx->h_atoms.size();
-    if (ctx->h_atoms.size() >= 0xffffffffull) return fail(ctx, RT_EINVAL, "rt_set_index: too many atoms");
+    if (!pts.empty()) atom_begin[pts.size() - 1] = atom_begin[pts.size()] = (uint32_t)ix.h_atoms.size();
+    if (ix.h_atoms.size() >= 0xffffffffull) return fail(ctx, RT_EINVAL, "rt_set_index: too many atoms");
     // per-ORF refs in profile order
     const size_t n_orf = desc.size();
-    ctx->h_orf_refs_desc.assign(n_orf, 0);
-    ctx->h_ref_ent.clear();
-    ctx->h_ref_atom.clear();
-    ctx->h_ref_ent.reserve(entries.size() * 3 / 2);
-    ctx->h_ref_atom.reserve(entries.size() * 3 / 2);
+    ix.h_orf_refs_desc.assign(n_orf, 0);
+    ix.h_ref_ent.clear();
+    ix.h_ref_atom.clear();
+    ix.h_ref_ent.reserve(entries.size() * 3 / 2);
+    ix.h_ref_atom.reserve(entries.size() * 3 / 2);
     for (size_t o = 0; o < n_orf; ++o) {
         const uint64_t begin = desc[o] & rt::kBeginMask;
         const int n_ent = (int)((desc[o] >> 40) & rt::kMaxEntriesPerOrf);
         const bool rev = (desc[o] >> 63) != 0;
-        const size_t ref_begin = ctx->h_ref_ent.size();
+        const size_t ref_begin = ix.h_ref_ent.size();
         for (int k = 0; k < n_ent; ++k) {
             const size_t e = begin + (size_t)(rev ? n_ent - 1 - k : k);
             const uint64_t ent = entries[e];
             const uint64_t off = ent >> rt::kLenBits;
             if (off == kZero) {
-                ctx->h_ref_ent.push_back(ent);
-                ctx->h_ref_atom.push_back(0xffffffffu);   // reads-as-zero stretch: no atom
+                ix.h_ref_ent.push_back(ent);
+                ix.h_ref_atom.push_back(0xffffffffu);   // reads-as-zero stretch: no atom
                 continue;
             }
             const uint32_t a0 = atom_begin[ilo[e]], a1 = atom_begin[ihi[e]];
             for (uint32_t a = 0; a < a1 - a0; ++a) {
                 const uint32_t atom = rev ? a1 - 1 - a : a0 + a;
-                ctx->h_ref_ent.push_back(ctx->h_atoms[atom]);
-                ctx->h_ref_atom.push_back(atom);
+                ix.h_ref_ent.push_back(ix.h_atoms[atom]);
+                ix.h_ref_atom.push_back(atom);
             }
         }
-        const size_t cnt = ctx->h_ref_ent.size() - ref_begin;
+        const size_t cnt = ix.h_ref_ent.size() - ref_begin;
         if (cnt > (size_t)rt::kMaxEntriesPerOrf) return fail(ctx, RT_EINVAL, "rt_set_index: ORF %zu has too many atoms", o);
-        ctx->h_orf_refs_desc[o] = (uint64_t)ref_begin | ((uint64_t)cnt << 40) | ((uint64_t)rev << 63);
+        ix.h_orf_refs_desc[o] = (uint64_t)ref_begin | ((uint64_t)cnt << 40) | ((uint64_t)rev << 63);
     }
-    ctx->n_atoms = (int64_t)ctx->h_atoms.size();
+    ix.n_atoms = (int64_t)ix.h_atoms.size();
     // compact layout: atom i starts at the sum of the lengths of the atoms before it
-    std::vector<uint64_t>& atoms_c = ctx->h_atoms_c;
-    atoms_c.assign(ctx->h_atoms.size(), 0);
+    std::vector<uint64_t>& atoms_c = ix.h_atoms_c;
+    atoms_c.assign(ix.h_atoms.size(), 0);
     std::vector<uint64_t> entries_c(entries.size());
     uint64_t cat = 0;
     for (size_t i = 0; i < atoms_c.size(); ++i) {
-        const uint64_t len = ctx->h_atoms[i] & rt::kLenMask;
+        const uint64_t len = ix.h_atoms[i] & rt::kLenMask;
         atoms_c[i] = (cat << rt::kLenBits) | len;
         cat += len;
     }
-    ctx->compact_elems = (int64_t)((cat + 31) / 32 * 32 + 32);
-    ctx->compact_end = (unsigned)std::min<uint64_t>(cat, 0xffffffffull);
-    ctx->compact_plus_end = ctx->compact_end;        // atoms are in slot order: the first one of the '-' plane ends the '+' part
+    ix.compact_elems = (int64_t)((cat + 31) / 32 * 32 + 32);
+    ix.compact_end = (unsigned)std::min<uint64_t>(cat, 0xffffffffull);
+    ix.compact_plus_end = ix.compact_end;        // atoms are in slot order: the first one of the '-' plane ends the '+' part
     for (size_t i = 0; i < atoms_c.size(); ++i)
-        if ((ctx->h_atoms[i] >> rt::kLenBits) >= (uint64_t)ctx->plane) {
-            ctx->compact_plus_end = (unsigned)(atoms_c[i] >> rt::kLenBits);
+        if ((ix.h_atoms[i] >> rt::kLenBits) >= (uint64_t)ctx->plane) {
+            ix.compact_plus_end = (unsigned)(atoms_c[i] >> rt::kLenBits);
             break;
         }
     for (size_t k = 0; k < entries.size(); ++k) {
         const uint64_t off = entries[k] >> rt::kLenBits, len = entries[k] & rt::kLenMask;
         entries_c[k] = off == kZero ? entries[k] : ((atoms_c[atom_begin[ilo[k]]] >> rt::kLenBits) << rt::kLenBits) | len;
     }
-    auto upload = [&](auto** dptr, const auto& vec) -> cudaError_t {
-        using T = typename std::remove_reference<decltype(vec)>::type::value_type;
-        cudaError_t e = cudaMalloc(dptr, sizeof(T) * (vec.size() + 4));   // slack: atom_pass_kernel copies descriptor pairs
-        if (e == cudaSuccess && !vec.empty()) e = cudaMemcpy(*dptr, vec.data(), sizeof(T) * vec.size(), cudaMemcpyHostToDevice);
-        return e;
+    auto upload = [&](DevArr<uint64_t>& d, const std::vector<uint64_t>& vec) {
+        cudaError_t e = d.reserve(vec.size() + 4);   // slack: atom_pass_kernel copies descriptor pairs
+        return e == cudaSuccess ? d.upload(vec.data(), vec.size()) : e;
     };
-    RT_CUDA(ctx, upload(&ctx->d_atoms, ctx->h_atoms));
-    RT_CUDA(ctx, upload(&ctx->d_atoms_c, atoms_c));
-    RT_CUDA(ctx, upload(&ctx->d_exon_entries_c, entries_c));
-    RT_CUDA(ctx, cudaMalloc(&ctx->d_summaries, sizeof(rt::AtomSummary) * std::max<size_t>(1, ctx->h_atoms.size())));
-    RT_CUDA(ctx, cudaMalloc(&ctx->d_atom_nonzero, std::max<size_t>(1, ctx->h_atoms.size())));
+    RT_CUDA(ctx, upload(ix.atoms, ix.h_atoms));
+    RT_CUDA(ctx, upload(ix.atoms_c, atoms_c));
+    RT_CUDA(ctx, upload(ix.exon_entries_c, entries_c));
+    RT_CUDA(ctx, ix.summaries.reserve(ix.h_atoms.size()));
+    RT_CUDA(ctx, ix.atom_nonzero.reserve(ix.h_atoms.size()));
     return RT_OK;   // the host copies stay: build_plan_host makes the atom lists and the families from them
-}
-
-void free_plan(rt_ctx::ScorePlan& p) {
-    cudaFree(p.d_fallback);
-    cudaFree(p.d_atom_list);
-    cudaFree(p.d_passes);
-    cudaFree(p.d_refs);
-    cudaFree(p.d_ref_warps);
-    cudaFree(p.d_long_acc);
 }
 
 constexpr size_t kReadBytes = 4 + 4 + 4 + 2 + 2 + 1 + 1;
@@ -368,59 +431,23 @@ int rt_create(int device, rt_ctx** out) {
     if (prop.major < 10)
         return fail(nullptr, RT_ECUDA, "rt_create: device %d is sm_%d%d; this library is built for sm_100a only",
                     device, prop.major, prop.minor);
-    rt_ctx* ctx = new rt_ctx();
+    std::unique_ptr<rt_ctx> ctx(new rt_ctx());
     ctx->device = device;
     ctx->n_sm = prop.multiProcessorCount;
-    if (cudaMalloc(&ctx->d_work_counter, 4 * sizeof(unsigned long long)) != cudaSuccess ||
-        cudaMalloc(&ctx->d_len_table, sizeof(int32_t) * RT_LEN_TABLE) != cudaSuccess) {
-        delete ctx;
+    if (ctx->work_counter.reserve(4) != cudaSuccess || ctx->len_table.reserve(RT_LEN_TABLE) != cudaSuccess ||
+        ctx->uv_table.reserve(rt::kUvEntries) != cudaSuccess)
         return fail(nullptr, RT_ENOMEM, "rt_create: cudaMalloc failed");
-    }
-    if (cudaMalloc(&ctx->d_uv_table, sizeof(double2) * rt::kUvEntries) != cudaSuccess) {
-        delete ctx;
-        return fail(nullptr, RT_ENOMEM, "rt_create: cudaMalloc failed");
-    }
-    rt::fill_uv_table_kernel<<<1, 256>>>(ctx->d_uv_table);
-    if (cudaDeviceSynchronize() != cudaSuccess) {
-        delete ctx;
+    rt::fill_uv_table_kernel<<<1, 256>>>(ctx->uv_table.p);
+    if (cudaDeviceSynchronize() != cudaSuccess)
         return fail(nullptr, RT_ECUDA, "rt_create: %s", cudaGetErrorString(cudaGetLastError()));
-    }
-    *out = ctx;
+    *out = ctx.release();
     return RT_OK;
 }
 
 void rt_destroy(rt_ctx* ctx) {
     if (!ctx) return;
     DeviceGuard guard(ctx->device);
-    for (auto& b : ctx->orf_buf) b.release();
-    for (auto& b : ctx->seq_buf) b.release();
-    cudaFree(ctx->d_contig_tab);
-    cudaFree(ctx->d_uv_table);
-    cudaFree(ctx->d_len_table);
-    cudaFree(ctx->d_orf_desc);
-    cudaFree(ctx->d_orf_len);
-    cudaFree(ctx->d_exon_entries);
-    cudaFree(ctx->d_atoms);
-    cudaFree(ctx->d_summaries);
-    cudaFree(ctx->d_atom_nonzero);
-    cudaFree(ctx->d_cmap);
-    cudaFree(ctx->d_cbits);
-    cudaFree(ctx->d_atoms_c);
-    cudaFree(ctx->d_exon_entries_c);
-    cudaFree(ctx->d_work_counter);
-    if (ctx->ev_scored) cudaEventDestroy(ctx->ev_scored);
-    for (auto& p : ctx->plans) free_plan(p);
-    for (int s = 0; s < 16; ++s) {
-        if (ctx->host_stage[s].rec) cudaFreeHost(ctx->host_stage[s].rec);
-        if (ctx->host_stage[s].hdr) cudaFreeHost(ctx->host_stage[s].hdr);
-        if (ctx->host_stage[s].copied) cudaEventDestroy(ctx->host_stage[s].copied);
-        ctx->read_slot[s].release();
-        if (ctx->slot_stream[s]) cudaStreamDestroy(ctx->slot_stream[s]);
-    }
-    ctx->stats_buf.release();
-    ctx->score_buf.release();
-    ctx->touched_buf.release();
-    cudaFree(ctx->d_n_touched);
+    cudaDeviceSynchronize();   // no stream or page-locked buffer of the ctx goes while work of the ctx may still use it
     delete ctx;
 }
 
@@ -447,15 +474,11 @@ int rt_set_genome(rt_ctx* ctx, int n_contig, const int64_t* h_contig_len, int pa
     ctx->plane = n_contig ? at : 32;
     if (2 * ctx->plane >= (int64_t)rt::kZeroOff || 2 * ctx->plane / 32 >= 0xffffffffll)
         return fail(ctx, RT_EINVAL, "rt_set_genome: genome too large (2 x plane must stay below 2^37 slots)");
-    cudaFree(ctx->d_contig_tab);
-    ctx->d_contig_tab = nullptr;
     std::vector<int2> tab((size_t)std::max(1, n_contig));
     for (int c = 0; c < n_contig; ++c) tab[c] = make_int2((int)h_contig_len[c], (int)(ctx->contig_base[c] >> 5));
-    RT_CUDA(ctx, cudaMalloc(&ctx->d_contig_tab, sizeof(int2) * tab.size()));
-    RT_CUDA(ctx, cudaMemcpy(ctx->d_contig_tab, tab.data(), sizeof(int2) * tab.size(), cudaMemcpyHostToDevice));
+    RT_CUDA(ctx, ctx->contig_tab.upload(tab.data(), tab.size()));
     // a new genome invalidates the index encoding
-    ctx->n_orf = 0;
-    ctx->layout = RT_LAYOUT_DENSE;
+    ctx->ix = rt_ctx::Index();
     return RT_OK;
 }
 
@@ -474,7 +497,7 @@ int rt_set_length_table(rt_ctx* ctx, const int32_t* h_len_table) {
         if (h_len_table[i] > RT_LEN_FILTERED && (h_len_table[i] < -RT_MAX_OFFSET || h_len_table[i] > RT_MAX_OFFSET))
             return fail(ctx, RT_EINVAL, "rt_set_length_table: entry %d = %d is neither a sentinel nor an offset in [-%d, %d]", i,
                         h_len_table[i], RT_MAX_OFFSET, RT_MAX_OFFSET);
-    RT_CUDA(ctx, cudaMemcpy(ctx->d_len_table, h_len_table, sizeof(int32_t) * RT_LEN_TABLE, cudaMemcpyHostToDevice));
+    RT_CUDA(ctx, cudaMemcpy(ctx->len_table.p, h_len_table, sizeof(int32_t) * RT_LEN_TABLE, cudaMemcpyHostToDevice));
     ctx->have_len_table = true;
     ctx->len_base = 20;
     for (int i = 0; i < RT_LEN_TABLE; ++i)
@@ -499,7 +522,7 @@ int rt_clear_coverage(rt_ctx* ctx, int32_t* d_cov, void* stream) {
     if (!ctx || !d_cov) return fail(ctx, RT_EINVAL, "rt_clear_coverage: NULL argument");
     if (ctx->plane == 0) return fail(ctx, RT_ESTATE, "rt_clear_coverage: call rt_set_genome first");
     DeviceGuard guard(ctx->device);
-    const size_t elems = ctx->layout == RT_LAYOUT_COMPACT ? (size_t)ctx->compact_elems : 2 * (size_t)ctx->plane;
+    const size_t elems = ctx->ix.layout == RT_LAYOUT_COMPACT ? (size_t)ctx->ix.compact_elems : 2 * (size_t)ctx->plane;
     RT_CUDA(ctx, cudaMemsetAsync(d_cov, 0, sizeof(int32_t) * elems, (cudaStream_t)stream));
     return RT_OK;
 }
@@ -508,25 +531,25 @@ int rt_set_layout(rt_ctx* ctx, int layout) {
     if (!ctx) return fail(nullptr, RT_EINVAL, "rt_set_layout: ctx is NULL");
     if (layout != RT_LAYOUT_DENSE && layout != RT_LAYOUT_COMPACT) return fail(ctx, RT_EINVAL, "rt_set_layout: unknown layout %d", layout);
     if (layout == RT_LAYOUT_COMPACT) {
-        if (ctx->n_orf == 0) return fail(ctx, RT_ESTATE, "rt_set_layout: the compact layout is derived from the index; call rt_set_index first");
-        if (ctx->compact_elems >= 0xffffffffll) return fail(ctx, RT_EINVAL, "rt_set_layout: exon union too large for 32-bit compact slots");
+        if (ctx->ix.n_orf == 0) return fail(ctx, RT_ESTATE, "rt_set_layout: the compact layout is derived from the index; call rt_set_index first");
+        if (ctx->ix.compact_elems >= 0xffffffffll) return fail(ctx, RT_EINVAL, "rt_set_layout: exon union too large for 32-bit compact slots");
         DeviceGuard guard(ctx->device);
-        if (!ctx->d_cmap) {
+        if (!ctx->ix.cmap.p) {
             const size_t words = (size_t)(2 * ctx->plane / 32);
-            RT_CUDA(ctx, cudaMalloc(&ctx->d_cmap, sizeof(uint2) * words));
-            RT_CUDA(ctx, cudaMemset(ctx->d_cmap, 0, sizeof(uint2) * words));
-            if (ctx->n_atoms > 0) {
-                const unsigned grid = (unsigned)std::min<int64_t>((ctx->n_atoms + 7) / 8, (int64_t)ctx->n_sm * 16);
-                rt::build_cmap_kernel<<<grid, 256>>>(ctx->d_atoms, ctx->d_atoms_c, ctx->n_atoms, ctx->d_cmap);
+            RT_CUDA(ctx, ctx->ix.cmap.reserve(words));
+            RT_CUDA(ctx, cudaMemset(ctx->ix.cmap.p, 0, sizeof(uint2) * words));
+            if (ctx->ix.n_atoms > 0) {
+                const unsigned grid = (unsigned)std::min<int64_t>((ctx->ix.n_atoms + 7) / 8, (int64_t)ctx->n_sm * 16);
+                rt::build_cmap_kernel<<<grid, 256>>>(ctx->ix.atoms.p, ctx->ix.atoms_c.p, ctx->ix.n_atoms, ctx->ix.cmap.p);
                 ctx->launches++;
                 RT_CUDA(ctx, cudaGetLastError());
             }
             {   // empty words carry the compact index of the next member (cmap_rank: zone boundaries of rt_bin_stream_fresh)
                 const size_t tiles = (words + rt::kGapTile - 1) / rt::kGapTile;
-                DevBuf tile_buf;
-                RT_CUDA(ctx, tile_buf.reserve(sizeof(unsigned) * tiles));
-                unsigned* d_tile = static_cast<unsigned*>(tile_buf.p);
-                rt::cmap_tile_last_kernel<<<(unsigned)tiles, 256>>>(ctx->d_cmap, (long long)words, d_tile);
+                DevArr<unsigned> tile_buf;
+                RT_CUDA(ctx, tile_buf.reserve(tiles));
+                unsigned* d_tile = tile_buf.p;
+                rt::cmap_tile_last_kernel<<<(unsigned)tiles, 256>>>(ctx->ix.cmap.p, (long long)words, d_tile);
                 std::vector<unsigned> h_tile(tiles);
                 RT_CUDA(ctx, cudaMemcpy(h_tile.data(), d_tile, sizeof(unsigned) * tiles, cudaMemcpyDeviceToHost));
                 unsigned carry = 0;
@@ -536,34 +559,33 @@ int rt_set_layout(rt_ctx* ctx, int layout) {
                     carry = std::max(carry, last);
                 }
                 RT_CUDA(ctx, cudaMemcpy(d_tile, h_tile.data(), sizeof(unsigned) * tiles, cudaMemcpyHostToDevice));
-                rt::cmap_fill_gaps_kernel<<<(unsigned)tiles, 256>>>(ctx->d_cmap, (long long)words, d_tile);
+                rt::cmap_fill_gaps_kernel<<<(unsigned)tiles, 256>>>(ctx->ix.cmap.p, (long long)words, d_tile);
                 ctx->launches += 2;
                 RT_CUDA(ctx, cudaGetLastError());
                 RT_CUDA(ctx, cudaDeviceSynchronize());
-                tile_buf.release();
             }
-            RT_CUDA(ctx, cudaMalloc(&ctx->d_cbits, sizeof(unsigned) * ((words + 31) / 32)));
-            rt::build_cbits_kernel<<<(unsigned)((words + 255) / 256), 256>>>(ctx->d_cmap, (long long)words, ctx->d_cbits);
+            RT_CUDA(ctx, ctx->ix.cbits.reserve((words + 31) / 32));
+            rt::build_cbits_kernel<<<(unsigned)((words + 255) / 256), 256>>>(ctx->ix.cmap.p, (long long)words, ctx->ix.cbits.p);
             ctx->launches++;
             RT_CUDA(ctx, cudaGetLastError());
             RT_CUDA(ctx, cudaDeviceSynchronize());
         }
     }
-    ctx->layout = layout;
+    ctx->ix.layout = layout;
     return RT_OK;
 }
 
 int64_t rt_coverage_elems(const rt_ctx* ctx) {
     if (!ctx) return 0;
-    return ctx->layout == RT_LAYOUT_COMPACT ? ctx->compact_elems : 2 * ctx->plane;
+    return ctx->ix.layout == RT_LAYOUT_COMPACT ? ctx->ix.compact_elems : 2 * ctx->plane;
 }
 
 int rt_track_touched(rt_ctx* ctx, int enable) {
     if (!ctx) return fail(nullptr, RT_EINVAL, "rt_track_touched: ctx is NULL");
     DeviceGuard guard(ctx->device);
-    if (enable && !ctx->d_n_touched) {
-        RT_CUDA(ctx, cudaMalloc(&ctx->d_n_touched, sizeof(unsigned long long)));
-        RT_CUDA(ctx, cudaMemset(ctx->d_n_touched, 0, sizeof(unsigned long long)));
+    if (enable && !ctx->n_touched.p) {
+        RT_CUDA(ctx, ctx->n_touched.reserve(1));
+        RT_CUDA(ctx, cudaMemset(ctx->n_touched.p, 0, sizeof(unsigned long long)));
     }
     ctx->track_touched = enable != 0;
     return RT_OK;
@@ -571,21 +593,21 @@ int rt_track_touched(rt_ctx* ctx, int enable) {
 
 int rt_clear_touched(rt_ctx* ctx, int32_t* d_cov, void* stream) {
     if (!ctx || !d_cov) return fail(ctx, RT_EINVAL, "rt_clear_touched: NULL argument");
-    if (!ctx->d_n_touched && ctx->layout != RT_LAYOUT_COMPACT)
+    if (!ctx->n_touched.p && ctx->ix.layout != RT_LAYOUT_COMPACT)
         return fail(ctx, RT_ESTATE, "rt_clear_touched: call rt_track_touched(ctx, 1) first");
     DeviceGuard guard(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
-    if (ctx->layout == RT_LAYOUT_COMPACT) {   // the whole buffer is the exon union: a plain memset is the sparse clear
-        RT_CUDA(ctx, cudaMemsetAsync(d_cov, 0, sizeof(int32_t) * (size_t)ctx->compact_elems, st));
+    if (ctx->ix.layout == RT_LAYOUT_COMPACT) {   // the whole buffer is the exon union: a plain memset is the sparse clear
+        RT_CUDA(ctx, cudaMemsetAsync(d_cov, 0, sizeof(int32_t) * (size_t)ctx->ix.compact_elems, st));
         return RT_OK;
     }
     if (ctx->touched_buf.p) {
         rt::clear_touched_kernel<<<(unsigned)ctx->n_sm * 8, 256, 0, st>>>(
-            d_cov, static_cast<const unsigned long long*>(ctx->touched_buf.p), ctx->d_n_touched);
+            d_cov, ctx->touched_buf.p, ctx->n_touched.p);
         ctx->launches++;
         RT_CUDA(ctx, cudaGetLastError());
     }
-    RT_CUDA(ctx, cudaMemsetAsync(ctx->d_n_touched, 0, sizeof(unsigned long long), st));
+    RT_CUDA(ctx, cudaMemsetAsync(ctx->n_touched.p, 0, sizeof(unsigned long long), st));
     ctx->touched_reserved = 0;
     return RT_OK;
 }
@@ -609,8 +631,8 @@ int launch_bin(rt_ctx* ctx, const char* who, rt::BinArgs& a, int32_t* d_cov, int
     a.protocol = protocol;
     a.weight = weight;
     a.len_base = ctx->len_base;
-    a.len_table = ctx->d_len_table;
-    a.contig_tab = ctx->d_contig_tab;
+    a.len_table = ctx->len_table.p;
+    a.contig_tab = ctx->contig_tab.p;
     a.n_contig = ctx->n_contig;
     a.pad = ctx->pad;
     a.plane_words = (unsigned)(ctx->plane >> 5);
@@ -618,14 +640,14 @@ int launch_bin(rt_ctx* ctx, const char* who, rt::BinArgs& a, int32_t* d_cov, int
     a.len_counts = reinterpret_cast<unsigned long long*>(d_len_counts);
     a.touched = nullptr;
     a.n_touched = nullptr;
-    a.cmap = ctx->layout == RT_LAYOUT_COMPACT ? ctx->d_cmap : nullptr;
-    a.cbits = ctx->d_cbits;
+    a.cmap = ctx->ix.layout == RT_LAYOUT_COMPACT ? ctx->ix.cmap.p : nullptr;
+    a.cbits = ctx->ix.cbits.p;
     if (ctx->track_touched && weight == 1 && !a.cmap) {
         int rc = ensure_touched_capacity(ctx, ctx->touched_reserved + n);
         if (rc != RT_OK) return rc;
         ctx->touched_reserved += n;
-        a.touched = static_cast<unsigned long long*>(ctx->touched_buf.p);
-        a.n_touched = ctx->d_n_touched;
+        a.touched = ctx->touched_buf.p;
+        a.n_touched = ctx->n_touched.p;
     }
     const int64_t per_block = (int64_t)rt::kBinThreads * rt::kBinReadsPerThread;
     const int64_t blocks = (n + per_block - 1) / per_block;
@@ -666,14 +688,14 @@ static int launch_stream(rt_ctx* ctx, const char* who, bool fresh, int32_t* d_co
         return fail(ctx, RT_EINVAL, "%s: NULL argument or bad n_blocks", who);
     if ((reinterpret_cast<uintptr_t>(d_records) | reinterpret_cast<uintptr_t>(d_hdr)) & 15)
         return fail(ctx, RT_EINVAL, "%s: d_records and d_hdr must be 16-byte aligned", who);
-    if (ctx->track_touched && ctx->layout != RT_LAYOUT_COMPACT)
+    if (ctx->track_touched && ctx->ix.layout != RT_LAYOUT_COMPACT)
         return fail(ctx, RT_ESTATE, "%s: the touched-slot list of the dense layout is kept by rt_bin_reads only", who);
-    if (fresh && ctx->layout != RT_LAYOUT_COMPACT) return fail(ctx, RT_ESTATE, "%s: needs the compact layout (rt_set_layout)", who);
+    if (fresh && ctx->ix.layout != RT_LAYOUT_COMPACT) return fail(ctx, RT_ESTATE, "%s: needs the compact layout (rt_set_layout)", who);
     if (fresh && (reinterpret_cast<uintptr_t>(d_cov) & 15)) return fail(ctx, RT_EINVAL, "%s: d_cov must be 16-byte aligned", who);
     DeviceGuard guard(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
     if (n_blocks == 0) {
-        if (fresh) RT_CUDA(ctx, cudaMemsetAsync(d_cov, 0, sizeof(int32_t) * (size_t)ctx->compact_elems, st));
+        if (fresh) RT_CUDA(ctx, cudaMemsetAsync(d_cov, 0, sizeof(int32_t) * (size_t)ctx->ix.compact_elems, st));
         return RT_OK;
     }
     rt::StreamArgs a{};
@@ -684,10 +706,10 @@ static int launch_stream(rt_ctx* ctx, const char* who, bool fresh, int32_t* d_co
     a.protocol = protocol;
     a.weight = weight;
     a.len_base = ctx->len_base;
-    a.cmap = ctx->layout == RT_LAYOUT_COMPACT ? ctx->d_cmap : nullptr;
-    a.cbits = ctx->d_cbits;
-    a.len_table = ctx->d_len_table;
-    a.contig_tab = ctx->d_contig_tab;
+    a.cmap = ctx->ix.layout == RT_LAYOUT_COMPACT ? ctx->ix.cmap.p : nullptr;
+    a.cbits = ctx->ix.cbits.p;
+    a.len_table = ctx->len_table.p;
+    a.contig_tab = ctx->contig_tab.p;
     a.n_contig = ctx->n_contig;
     a.pad = ctx->pad;
     a.plane_words = (unsigned)(ctx->plane >> 5);
@@ -698,22 +720,22 @@ static int launch_stream(rt_ctx* ctx, const char* who, bool fresh, int32_t* d_co
     if (fresh) {
         // zone boundaries of the blocks (rank of the first position a read of the block can reach), made monotone
         const int64_t tiles = (n_blocks + 1 + rt::kZoneTile - 1) / rt::kZoneTile;
-        RT_CUDA(ctx, ctx->zone_buf.reserve(sizeof(unsigned) * (2 * (size_t)(n_blocks + 1) + 4 * (size_t)tiles)));
-        RT_CUDA(ctx, ctx->spill_buf.reserve(sizeof(unsigned) * (size_t)n_blocks * RT_STREAM_BLOCK + 16));
+        RT_CUDA(ctx, ctx->zone_buf.reserve(2 * (size_t)(n_blocks + 1) + 4 * (size_t)tiles));
+        RT_CUDA(ctx, ctx->spill_buf.reserve((size_t)n_blocks * RT_STREAM_BLOCK + 4));
         rt::ZoneArgs z{};
         z.hdr = a.hdr;
         z.n_blocks = n_blocks;
-        z.bounds = static_cast<unsigned*>(ctx->zone_buf.p);
-        z.cmap = ctx->d_cmap;
-        z.contig_tab = ctx->d_contig_tab;
+        z.bounds = ctx->zone_buf.p;
+        z.cmap = ctx->ix.cmap.p;
+        z.contig_tab = ctx->contig_tab.p;
         z.n_contig = ctx->n_contig;
         z.pad = ctx->pad;
         z.plane_words = a.plane_words;
         z.delta_plus = ctx->zone_delta_plus;
         z.delta_minus = ctx->zone_delta_minus;
-        z.plus_end = ctx->compact_plus_end;
-        z.minus_end = ctx->compact_end;
-        unsigned long long* d_n_spill = reinterpret_cast<unsigned long long*>(static_cast<char*>(ctx->spill_buf.p));
+        z.plus_end = ctx->ix.compact_plus_end;
+        z.minus_end = ctx->ix.compact_end;
+        unsigned long long* d_n_spill = reinterpret_cast<unsigned long long*>(ctx->spill_buf.p);
         unsigned* d_tile_max = z.bounds + 2 * (size_t)(n_blocks + 1);
         unsigned* d_tile_carry = d_tile_max + 2 * (size_t)tiles;
         a.zone_bounds = z.bounds;
@@ -723,7 +745,7 @@ static int launch_stream(rt_ctx* ctx, const char* who, bool fresh, int32_t* d_co
         a.n_spill = d_n_spill;
         RT_CUDA(ctx, cudaMemsetAsync(d_n_spill, 0, sizeof(unsigned long long), st));
         // the few guard slots behind the last zone belong to no block
-        RT_CUDA(ctx, cudaMemsetAsync(d_cov + ctx->compact_end, 0, sizeof(int32_t) * (size_t)(ctx->compact_elems - ctx->compact_end), st));
+        RT_CUDA(ctx, cudaMemsetAsync(d_cov + ctx->ix.compact_end, 0, sizeof(int32_t) * (size_t)(ctx->ix.compact_elems - ctx->ix.compact_end), st));
         rt::zone_bounds_kernel<<<dim3((unsigned)tiles, 2), rt::kZoneTile, 0, st>>>(z, d_tile_max);
         rt::zone_carry_kernel<<<2, 1024, 0, st>>>(d_tile_max, d_tile_carry, tiles, z.plus_end);
         rt::bin_stream_kernel<true, true><<<grid, rt::kStreamThreads, 0, st>>>(a);
@@ -755,11 +777,11 @@ int rt_bin_stream_host(rt_ctx* ctx, int32_t* d_cov, int64_t n_blocks, const uint
     if (n_blocks < 0 || (n_blocks > 0 && (!h_records || !h_hdr))) return fail(ctx, RT_EINVAL, "rt_bin_stream_host: NULL stream");
     DeviceGuard guard(ctx->device);
     const size_t acc_bytes = sizeof(int64_t) * (RT_N_STATS + RT_LEN_TABLE);
-    RT_CUDA(ctx, ctx->stats_buf.reserve(acc_bytes));
-    int64_t* d_stats = static_cast<int64_t*>(ctx->stats_buf.p);
+    RT_CUDA(ctx, ctx->stats_buf.reserve(RT_N_STATS + RT_LEN_TABLE));
+    int64_t* d_stats = ctx->stats_buf.p;
     int64_t* d_len_counts = d_stats + RT_N_STATS;
     for (int s = 0; s < 2; ++s)
-        if (!ctx->slot_stream[s]) RT_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->slot_stream[s], cudaStreamNonBlocking));
+        RT_CUDA(ctx, ctx->slot_stream[s].create());
     RT_CUDA(ctx, cudaMemsetAsync(d_stats, 0, acc_bytes, ctx->slot_stream[0]));
     RT_CUDA(ctx, cudaStreamSynchronize(ctx->slot_stream[0]));
     // chunks of 16 MB of records alternate between two device slots: copy of one || K1 of the other
@@ -769,8 +791,8 @@ int rt_bin_stream_host(rt_ctx* ctx, int32_t* d_cov, int64_t n_blocks, const uint
     for (int64_t at = 0; at < n_blocks; at += chunk, slot ^= 1) {
         const int64_t m = std::min(chunk, n_blocks - at);
         RT_CUDA(ctx, ctx->read_slot[slot].reserve(rec_bytes + sizeof(int32_t) * 4 * (size_t)chunk));
-        uint32_t* d_rec = static_cast<uint32_t*>(ctx->read_slot[slot].p);
-        int32_t* d_hdr = reinterpret_cast<int32_t*>(static_cast<char*>(ctx->read_slot[slot].p) + rec_bytes);
+        uint32_t* d_rec = reinterpret_cast<uint32_t*>(ctx->read_slot[slot].p);
+        int32_t* d_hdr = reinterpret_cast<int32_t*>(ctx->read_slot[slot].p + rec_bytes);
         cudaStream_t st = ctx->slot_stream[slot];   // stream order protects the slot's previous use
         RT_CUDA(ctx, cudaMemcpyAsync(d_rec, h_records + at * RT_STREAM_BLOCK, sizeof(uint32_t) * RT_STREAM_BLOCK * (size_t)m, cudaMemcpyHostToDevice, st));
         RT_CUDA(ctx, cudaMemcpyAsync(d_hdr, h_hdr + 4 * at, sizeof(int32_t) * 4 * (size_t)m, cudaMemcpyHostToDevice, st));
@@ -795,16 +817,16 @@ int rt_bin_reads_host(rt_ctx* ctx, int32_t* d_cov, int64_t n, const int32_t* h_r
         return fail(ctx, RT_EINVAL, "rt_bin_reads_host: NULL column");
     DeviceGuard guard(ctx->device);
     // the sparse-clear list of the dense layout is kept by the column kernel only
-    const bool use_stream = sorted_hint && !(ctx->track_touched && ctx->layout != RT_LAYOUT_COMPACT);
+    const bool use_stream = sorted_hint && !(ctx->track_touched && ctx->ix.layout != RT_LAYOUT_COMPACT);
     const size_t acc_bytes = sizeof(int64_t) * (RT_N_STATS + RT_LEN_TABLE);
-    RT_CUDA(ctx, ctx->stats_buf.reserve(acc_bytes));
-    int64_t* d_stats = static_cast<int64_t*>(ctx->stats_buf.p);
+    RT_CUDA(ctx, ctx->stats_buf.reserve(RT_N_STATS + RT_LEN_TABLE));
+    int64_t* d_stats = ctx->stats_buf.p;
     int64_t* d_len_counts = d_stats + RT_N_STATS;
     for (int s = 0; s < 2; ++s)
-        if (!ctx->slot_stream[s]) RT_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->slot_stream[s], cudaStreamNonBlocking));
+        RT_CUDA(ctx, ctx->slot_stream[s].create());
     RT_CUDA(ctx, cudaMemsetAsync(d_stats, 0, acc_bytes, ctx->slot_stream[0]));
     RT_CUDA(ctx, cudaStreamSynchronize(ctx->slot_stream[0]));
-    if (ctx->track_touched && ctx->layout != RT_LAYOUT_COMPACT) {   // one growth up front instead of one per chunk
+    if (ctx->track_touched && ctx->ix.layout != RT_LAYOUT_COMPACT) {   // one growth up front instead of one per chunk
         int rc = ensure_touched_capacity(ctx, ctx->touched_reserved + n);
         if (rc != RT_OK) return rc;
     }
@@ -826,13 +848,13 @@ int rt_bin_reads_host(rt_ctx* ctx, int32_t* d_cov, int64_t n, const int32_t* h_r
     // per-slot layout: a chunk's record stream (records, then block headers) or its plain columns, widest column first
     const size_t slot_bytes = std::max((size_t)chunk, (size_t)(use_stream ? kPackChunkReads : 0)) * kReadBytes + 64;
     for (int s = 0; s < n_pipes; ++s) {
-        if (!ctx->slot_stream[s]) RT_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->slot_stream[s], cudaStreamNonBlocking));
+        RT_CUDA(ctx, ctx->slot_stream[s].create());
         RT_CUDA(ctx, ctx->read_slot[s].reserve(slot_bytes));
         rt_ctx::HostStage& hs = ctx->host_stage[s];
-        if (use_stream && !hs.rec) {
-            RT_CUDA(ctx, cudaHostAlloc(&hs.rec, sizeof(uint32_t) * RT_STREAM_BLOCK * (size_t)kChunkBlockCap, cudaHostAllocDefault));
-            RT_CUDA(ctx, cudaHostAlloc(&hs.hdr, sizeof(int32_t) * 4 * (size_t)kChunkBlockCap, cudaHostAllocDefault));
-            RT_CUDA(ctx, cudaEventCreateWithFlags(&hs.copied, cudaEventDisableTiming));
+        if (use_stream && !hs.rec.p) {
+            RT_CUDA(ctx, hs.rec.alloc(RT_STREAM_BLOCK * (size_t)kChunkBlockCap));
+            RT_CUDA(ctx, hs.hdr.alloc(4 * (size_t)kChunkBlockCap));
+            RT_CUDA(ctx, hs.copied.create(cudaEventDisableTiming));
         }
         hs.busy = false;
     }
@@ -841,7 +863,7 @@ int rt_bin_reads_host(rt_ctx* ctx, int32_t* d_cov, int64_t n, const int32_t* h_r
     std::string first_error;
     auto pipeline = [&](int s) {
         cudaSetDevice(ctx->device);
-        char* base = static_cast<char*>(ctx->read_slot[s].p);
+        char* base = ctx->read_slot[s].p;
         // a chunk is either a record stream (records, then block headers) or plain columns
         uint32_t* d_rec = reinterpret_cast<uint32_t*>(base);
         int32_t* d_hdr = reinterpret_cast<int32_t*>(d_rec + RT_STREAM_BLOCK * (size_t)kChunkBlockCap);
@@ -871,7 +893,7 @@ int rt_bin_reads_host(rt_ctx* ctx, int32_t* d_cov, int64_t n, const int32_t* h_r
                 hs.busy = false;
                 const auto t1 = std::chrono::steady_clock::now();
                 blocks = rt_stream_pack_range(h_ref_id + at, h_first + at, h_last + at, h_mlen + at, h_flag + at, h_mapq + at, h_nh + at, m,
-                                              hs.rec, hs.hdr, kChunkBlockCap);
+                                              hs.rec.p, hs.hdr.p, kChunkBlockCap);
                 if (timing) {
                     wait_ns += std::chrono::duration_cast<std::chrono::nanoseconds>(t1 - t0).count();
                     pack_ns += std::chrono::duration_cast<std::chrono::nanoseconds>(std::chrono::steady_clock::now() - t1).count();
@@ -880,8 +902,8 @@ int rt_bin_reads_host(rt_ctx* ctx, int32_t* d_cov, int64_t n, const int32_t* h_r
             const auto t2 = std::chrono::steady_clock::now();
             int rc;
             if (blocks >= 0) {
-                if (!check(cudaMemcpyAsync(d_rec, hs.rec, sizeof(uint32_t) * RT_STREAM_BLOCK * (size_t)blocks, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync") ||
-                    !check(cudaMemcpyAsync(d_hdr, hs.hdr, sizeof(int32_t) * 4 * (size_t)blocks, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync") ||
+                if (!check(cudaMemcpyAsync(d_rec, hs.rec.p, sizeof(uint32_t) * RT_STREAM_BLOCK * (size_t)blocks, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync") ||
+                    !check(cudaMemcpyAsync(d_hdr, hs.hdr.p, sizeof(int32_t) * 4 * (size_t)blocks, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync") ||
                     !check(cudaEventRecord(hs.copied, st), "cudaEventRecord"))
                     break;
                 hs.busy = true;
@@ -940,8 +962,7 @@ int rt_set_index(rt_ctx* ctx, int64_t n_orf, const int64_t* h_exon_ptr, const in
     std::vector<uint64_t> desc((size_t)n_orf);
     std::vector<uint64_t> entries;
     entries.reserve((size_t)(h_exon_ptr[n_orf] - h_exon_ptr[0]) + 16);
-    ctx->bytes_prefix.assign((size_t)n_orf + 1, 0);
-    ctx->nt_prefix.assign((size_t)n_orf + 1, 0);
+    std::vector<int64_t> bytes_prefix((size_t)n_orf + 1, 0), nt_prefix((size_t)n_orf + 1, 0);
     auto push = [&](int64_t off, int64_t len) {   // off < 0: zeros
         while (len > 0) {
             const int64_t piece = std::min(len, max_piece);
@@ -984,83 +1005,58 @@ int rt_set_index(rt_ctx* ctx, int64_t n_orf, const int64_t* h_exon_ptr, const in
             return fail(ctx, RT_EINVAL, "rt_set_index: ORF %lld has too many intervals", (long long)o);
         if (begin >= rt::kBeginMask) return fail(ctx, RT_EINVAL, "rt_set_index: index too large");
         desc[o] = (uint64_t)begin | ((uint64_t)cnt << 40) | ((uint64_t)(s == 1) << 63);
-        ctx->nt_prefix[o + 1] = ctx->nt_prefix[o] + L;
-        ctx->bytes_prefix[o + 1] = ctx->bytes_prefix[o] + 4 * L + 8 * (e1 - e0) + 42;
+        nt_prefix[o + 1] = nt_prefix[o] + L;
+        bytes_prefix[o + 1] = bytes_prefix[o] + 4 * L + 8 * (e1 - e0) + 42;
     }
-    cudaFree(ctx->d_orf_desc);
-    cudaFree(ctx->d_orf_len);
-    cudaFree(ctx->d_exon_entries);
-    ctx->d_orf_desc = ctx->d_exon_entries = nullptr;
-    ctx->d_orf_len = nullptr;
-    ctx->n_orf = 0;
-    for (auto& p : ctx->plans) free_plan(p);
-    ctx->plans.clear();
-    cudaFree(ctx->d_atoms);
-    cudaFree(ctx->d_summaries);
-    cudaFree(ctx->d_atom_nonzero);
-    ctx->d_atom_nonzero = nullptr;
-    cudaFree(ctx->d_cmap);
-    cudaFree(ctx->d_cbits);
-    cudaFree(ctx->d_atoms_c);
-    cudaFree(ctx->d_exon_entries_c);
-    ctx->d_cmap = nullptr;
-    ctx->d_cbits = nullptr;
-    ctx->d_atoms_c = ctx->d_exon_entries_c = nullptr;
-    ctx->layout = RT_LAYOUT_DENSE;
-    ctx->compact_elems = 0;
-    ctx->d_atoms = nullptr;
-    ctx->d_summaries = nullptr;
-    ctx->n_atoms = 0;
+    // the old index goes only now, so that an index refused above leaves it intact; a failure from here on (a CUDA
+    // error, too many atoms) leaves an empty index
+    rt_ctx::Index& ix = ctx->ix;
+    ix = rt_ctx::Index();
+    ix.bytes_prefix = std::move(bytes_prefix);
+    ix.nt_prefix = std::move(nt_prefix);
     {
         std::vector<int32_t> lens((size_t)n_orf);
-        for (int64_t o = 0; o < n_orf; ++o) lens[o] = (int32_t)(ctx->nt_prefix[o + 1] - ctx->nt_prefix[o]);
-        RT_CUDA(ctx, cudaMalloc(&ctx->d_orf_len, sizeof(int32_t) * std::max<size_t>(1, lens.size())));
-        if (!lens.empty())
-            RT_CUDA(ctx, cudaMemcpy(ctx->d_orf_len, lens.data(), sizeof(int32_t) * lens.size(), cudaMemcpyHostToDevice));
+        for (int64_t o = 0; o < n_orf; ++o) lens[o] = (int32_t)(ix.nt_prefix[o + 1] - ix.nt_prefix[o]);
+        RT_CUDA(ctx, ix.orf_len.upload(lens.data(), lens.size()));
     }
-    RT_CUDA(ctx, cudaMalloc(&ctx->d_orf_desc, sizeof(uint64_t) * std::max<size_t>(1, desc.size())));
-    RT_CUDA(ctx, cudaMalloc(&ctx->d_exon_entries, sizeof(uint64_t) * std::max<size_t>(1, entries.size())));
-    if (!desc.empty())
-        RT_CUDA(ctx, cudaMemcpy(ctx->d_orf_desc, desc.data(), sizeof(uint64_t) * desc.size(), cudaMemcpyHostToDevice));
-    if (!entries.empty())
-        RT_CUDA(ctx, cudaMemcpy(ctx->d_exon_entries, entries.data(), sizeof(uint64_t) * entries.size(),
-                                cudaMemcpyHostToDevice));
+    RT_CUDA(ctx, ix.orf_desc.upload(desc.data(), desc.size()));
+    RT_CUDA(ctx, ix.exon_entries.upload(entries.data(), entries.size()));
     {
         const auto t_atoms = std::chrono::steady_clock::now();
         int rc = build_atoms(ctx, desc, entries);
         if (getenv("RT_HOST_TIMING"))
             fprintf(stderr, "rt_set_index: build_atoms %.1f ms (%zu ORFs, %zu exon entries, %zu atoms)\n",
                     std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_atoms).count(), desc.size(), entries.size(),
-                    ctx->h_atoms.size());
+                    ix.h_atoms.size());
         if (rc != RT_OK) return rc;
     }
-    ctx->n_orf = n_orf;
+    ix.n_orf = n_orf;
     return RT_OK;
 }
 
-int64_t rt_index_orfs(const rt_ctx* ctx) { return ctx ? ctx->n_orf : 0; }
+int64_t rt_index_orfs(const rt_ctx* ctx) { return ctx ? ctx->ix.n_orf : 0; }
 
 int64_t rt_index_score_bytes(const rt_ctx* ctx, int64_t lo, int64_t hi) {
-    if (!ctx || lo < 0 || hi > ctx->n_orf || lo > hi) return -1;
-    return ctx->bytes_prefix[hi] - ctx->bytes_prefix[lo];
+    if (!ctx || lo < 0 || hi > ctx->ix.n_orf || lo > hi) return -1;
+    return ctx->ix.bytes_prefix[hi] - ctx->ix.bytes_prefix[lo];
 }
 
 int64_t rt_index_total_nt(const rt_ctx* ctx, int64_t lo, int64_t hi) {
-    if (!ctx || lo < 0 || hi > ctx->n_orf || lo > hi) return -1;
-    return ctx->nt_prefix[hi] - ctx->nt_prefix[lo];
+    if (!ctx || lo < 0 || hi > ctx->ix.n_orf || lo > hi) return -1;
+    return ctx->ix.nt_prefix[hi] - ctx->ix.nt_prefix[lo];
 }
 
 int rt_shard_bounds(const rt_ctx* ctx, int n_shards, int64_t* h_bounds) {
     if (!ctx || n_shards < 1 || !h_bounds) return RT_EINVAL;
-    const int64_t total = ctx->bytes_prefix.empty() ? 0 : ctx->bytes_prefix.back();
+    const int64_t total = ctx->ix.bytes_prefix.back();
     h_bounds[0] = 0;
     for (int s = 1; s < n_shards; ++s) {
         const int64_t target = (int64_t)((__int128)total * s / n_shards);
-        auto it = std::lower_bound(ctx->bytes_prefix.begin(), ctx->bytes_prefix.end(), target);
-        h_bounds[s] = std::max<int64_t>(h_bounds[s - 1], it - ctx->bytes_prefix.begin());
-        if (h_bounds[s] > ctx->n_orf) h_bounds[s] = ctx->n_orf;
+        auto it = std::lower_bound(ctx->ix.bytes_prefix.begin(), ctx->ix.bytes_prefix.end(), target);
+        h_bounds[s] = std::max<int64_t>(h_bounds[s - 1], it - ctx->ix.bytes_prefix.begin());
+        if (h_bounds[s] > ctx->ix.n_orf) h_bounds[s] = ctx->ix.n_orf;
     }
-    h_bounds[n_shards] = ctx->n_orf;
+    h_bounds[n_shards] = ctx->ix.n_orf;
     return RT_OK;
 }
 
@@ -1095,19 +1091,19 @@ void build_plan_host(const rt_ctx* ctx, int64_t lo, int64_t hi, PlanHost& ph) {
     };
     {   // atoms the ORFs of the range refer to; sorted by length inside windows so that the four atoms of
         // a warp are balanced while genomic neighbours stay close in time
-        std::vector<uint8_t> used((size_t)ctx->n_atoms, 0);
+        std::vector<uint8_t> used((size_t)ctx->ix.n_atoms, 0);
         for (int64_t o = lo; o < hi; ++o) {
-            const uint64_t d = ctx->h_orf_refs_desc[o];
+            const uint64_t d = ctx->ix.h_orf_refs_desc[o];
             const uint64_t b = d & rt::kBeginMask, c = (d >> 40) & rt::kMaxEntriesPerOrf;
             for (uint64_t k = b; k < b + c; ++k)
-                if (ctx->h_ref_atom[k] != 0xffffffffu) used[ctx->h_ref_atom[k]] = 1;
+                if (ctx->ix.h_ref_atom[k] != 0xffffffffu) used[ctx->ix.h_ref_atom[k]] = 1;
         }
         std::vector<int32_t>& alist = ph.alist;
-        for (int64_t a = 0; a < ctx->n_atoms; ++a)
+        for (int64_t a = 0; a < ctx->ix.n_atoms; ++a)
             if (used[a]) alist.push_back((int32_t)a);
         {   // passes of the streamed phase A: consecutive atom ids are adjacent in the compact buffer
             std::vector<rt::PassDesc>& passes = ph.passes;
-            const uint64_t* ac = ctx->h_atoms_c.data();
+            const uint64_t* ac = ctx->ix.h_atoms_c.data();
             size_t i = 0;
             while (i < alist.size()) {
                 const uint32_t a0 = (uint32_t)alist[i];
@@ -1129,7 +1125,7 @@ void build_plan_host(const rt_ctx* ctx, int64_t lo, int64_t hi, PlanHost& ph) {
         for (size_t w0 = 0; w0 < alist.size(); w0 += kAtomWindow) {
             auto b = alist.begin() + w0, e = alist.begin() + std::min(alist.size(), w0 + kAtomWindow);
             std::stable_sort(b, e, [&](int32_t x, int32_t y) {
-                return (ctx->h_atoms[x] & rt::kLenMask) > (ctx->h_atoms[y] & rt::kLenMask);
+                return (ctx->ix.h_atoms[x] & rt::kLenMask) > (ctx->ix.h_atoms[y] & rt::kLenMask);
             });
         }
     }
@@ -1143,7 +1139,7 @@ void build_plan_host(const rt_ctx* ctx, int64_t lo, int64_t hi, PlanHost& ph) {
         // Families never straddle a group of 32 slots; ORFs with more than 32 references stay alone and fill whole groups.
         std::vector<rt::RefRec>& refs = ph.refs;
         std::vector<rt::RefWarp>& warps = ph.warps;
-        refs.reserve((size_t)(ctx->h_ref_ent.size() / std::max<int64_t>(1, ctx->n_orf) * n * 3 / 4 + 64));
+        refs.reserve((size_t)(ctx->ix.h_ref_ent.size() / std::max<int64_t>(1, ctx->ix.n_orf) * n * 3 / 4 + 64));
         const rt::RefRec pad_rec{0xffffffffu, 0u, 0u, -1};
         int& n_long = ph.n_long_b;
         auto pad_group = [&]() {
@@ -1151,7 +1147,7 @@ void build_plan_host(const rt_ctx* ctx, int64_t lo, int64_t hi, PlanHost& ph) {
             warps.resize(refs.size() / 32, rt::RefWarp{-1, 0, -1, 0});
         };
         auto desc_of = [&](int64_t o, uint64_t& rb, uint64_t& cnt, uint32_t& rev) {
-            const uint64_t d = ctx->h_orf_refs_desc[o];
+            const uint64_t d = ctx->ix.h_orf_refs_desc[o];
             rb = d & rt::kBeginMask;
             cnt = (d >> 40) & (uint64_t)rt::kMaxEntriesPerOrf;
             rev = (uint32_t)(d >> 63);
@@ -1160,7 +1156,7 @@ void build_plan_host(const rt_ctx* ctx, int64_t lo, int64_t hi, PlanHost& ph) {
         // hash of the child that is that suffix
         const uint64_t kB = 0x9E3779B97F4A7C15ull;
         auto elem = [&](uint64_t k) {
-            uint64_t x = ((uint64_t)ctx->h_ref_atom[k] << 25) ^ (ctx->h_ref_ent[k] & rt::kLenMask);
+            uint64_t x = ((uint64_t)ctx->ix.h_ref_atom[k] << 25) ^ (ctx->ix.h_ref_ent[k] & rt::kLenMask);
             x ^= x >> 31; x *= 0xD6E8FEB86659FD93ull; x ^= x >> 29;
             return x | 1ull;
         };
@@ -1179,7 +1175,7 @@ void build_plan_host(const rt_ctx* ctx, int64_t lo, int64_t hi, PlanHost& ph) {
         std::vector<int32_t> parent_of((size_t)n, -1);                   // -1: not a child
         std::vector<int64_t> order((size_t)n);
         for (int64_t i = 0; i < n; ++i) order[i] = lo + i;
-        auto refs_of = [&](int64_t o) { return (ctx->h_orf_refs_desc[o] >> 40) & (uint64_t)rt::kMaxEntriesPerOrf; };
+        auto refs_of = [&](int64_t o) { return (ctx->ix.h_orf_refs_desc[o] >> 40) & (uint64_t)rt::kMaxEntriesPerOrf; };
         std::stable_sort(order.begin(), order.end(), [&](int64_t x, int64_t y) { return refs_of(x) > refs_of(y); });
         // children[o - lo]: (position in the parent's list, child ORF)
         std::vector<std::vector<std::pair<int, int64_t>>> children((size_t)n);
@@ -1201,11 +1197,11 @@ void build_plan_host(const rt_ctx* ctx, int64_t lo, int64_t hi, PlanHost& ph) {
                     if (crev != rev || ccnt != cnt - k) continue;
                     // a child's first reference must hold two values: then every seam window of the references after it
                     // starts inside the child (with one value, the window two before the next reference would not)
-                    if ((ctx->h_ref_ent[crb] & rt::kLenMask) < 2) continue;
+                    if ((ctx->ix.h_ref_ent[crb] & rt::kLenMask) < 2) continue;
                     bool same = true;
                     for (uint64_t j = 0; j < ccnt && same; ++j)
-                        same = ctx->h_ref_atom[crb + j] == ctx->h_ref_atom[rb + k + j] &&
-                               (ctx->h_ref_ent[crb + j] & rt::kLenMask) == (ctx->h_ref_ent[rb + k + j] & rt::kLenMask);
+                        same = ctx->ix.h_ref_atom[crb + j] == ctx->ix.h_ref_atom[rb + k + j] &&
+                               (ctx->ix.h_ref_ent[crb + j] & rt::kLenMask) == (ctx->ix.h_ref_ent[rb + k + j] & rt::kLenMask);
                     if (!same) continue;
                     parent_of[c - lo] = (int32_t)(o - lo);
                     children[o - lo].push_back({(int)k, c});
@@ -1221,24 +1217,24 @@ void build_plan_host(const rt_ctx* ctx, int64_t lo, int64_t hi, PlanHost& ph) {
             if (cnt > 32 || refs.size() % 32 + std::max<uint64_t>(cnt, 1) > 32) pad_group();
             const size_t w0 = refs.size() / 32, first_slot = refs.size();
             uint64_t P = 0;
-            const uint64_t L = (uint64_t)(ctx->nt_prefix[o + 1] - ctx->nt_prefix[o]);
+            const uint64_t L = (uint64_t)(ctx->ix.nt_prefix[o + 1] - ctx->ix.nt_prefix[o]);
             auto flags_of = [&](uint64_t len, uint64_t l_mod3) -> uint32_t {
                 return ((uint32_t)(P % 3) << rt::kRefPmod3Shift) | (P >= 1 ? rt::kRefPge1 : 0u) | (P >= 2 ? rt::kRefPge2 : 0u) |
                        (P + len == L ? rt::kRefLast : 0u) | ((uint32_t)l_mod3 << rt::kRefLmod3Shift) | (rev ? rt::kRefRev : 0u);
             };
             for (uint64_t k = 0; k < cnt; ++k) {
-                const uint32_t len = (uint32_t)(ctx->h_ref_ent[rb + k] & rt::kLenMask);
+                const uint32_t len = (uint32_t)(ctx->ix.h_ref_ent[rb + k] & rt::kLenMask);
                 // L mod 3 of the ORF that starts on this slot; a long ORF carries its own on every slot (its last
                 // group applies the trailing partial codon itself)
                 const uint64_t lm3 = (k == 0 || cnt > 32) ? L % 3 : 0;
-                refs.push_back({ctx->h_ref_atom[rb + k], len | flags_of(len, lm3), (uint32_t)((len + P) % 3) | (k == 0 ? rt::kRefFamilyHead : 0u),
+                refs.push_back({ctx->ix.h_ref_atom[rb + k], len | flags_of(len, lm3), (uint32_t)((len + P) % 3) | (k == 0 ? rt::kRefFamilyHead : 0u),
                                 k == 0 ? (int32_t)o : -2});
                 P += len;
             }
             if (cnt == 0) refs.push_back({0xffffffffu, flags_of(0, L % 3), rt::kRefFamilyHead, (int32_t)o});   // an ORF without intervals still gets its row
             for (const auto& ch : children[o - lo]) {
                 rt::RefRec& r = refs[first_slot + (size_t)ch.first];
-                const uint64_t Lc = (uint64_t)(ctx->nt_prefix[ch.second + 1] - ctx->nt_prefix[ch.second]);
+                const uint64_t Lc = (uint64_t)(ctx->ix.nt_prefix[ch.second + 1] - ctx->ix.nt_prefix[ch.second]);
                 r.orf = (int32_t)ch.second;
                 r.len_flags = (r.len_flags & ~(3u << rt::kRefLmod3Shift)) | ((uint32_t)(Lc % 3) << rt::kRefLmod3Shift);
             }
@@ -1260,43 +1256,30 @@ void build_plan_host(const rt_ctx* ctx, int64_t lo, int64_t hi, PlanHost& ph) {
 // The device side of a plan: the host arrays of `ph` uploaded, the plan entered into the (bounded) cache of the ctx.
 int upload_plan(rt_ctx* ctx, PlanHost& ph, rt_ctx::ScorePlan** out) {
     const int64_t lo = ph.lo, hi = ph.hi, n = hi - lo;
-    if (ctx->plans.size() >= 24) {   // bounded cache (rt_score_host keeps four part plans per range it is asked for)
-        free_plan(ctx->plans.front());
-        ctx->plans.erase(ctx->plans.begin());
-    }
+    if (ctx->ix.plans.size() >= 24)   // bounded cache (rt_score_host keeps four part plans per range it is asked for)
+        ctx->ix.plans.erase(ctx->ix.plans.begin());
     rt_ctx::ScorePlan p;
     p.lo = lo;
     p.hi = hi;
-    RT_CUDA(ctx, cudaMalloc(&p.d_fallback, sizeof(int32_t) * std::max<int64_t>(1, n)));
+    RT_CUDA(ctx, p.fallback.reserve((size_t)n));
     p.n_passes = (int64_t)ph.passes.size();
-    RT_CUDA(ctx, cudaMalloc(&p.d_passes, sizeof(rt::PassDesc) * std::max<size_t>(1, ph.passes.size())));
-    if (!ph.passes.empty())
-        RT_CUDA(ctx, cudaMemcpy(p.d_passes, ph.passes.data(), sizeof(rt::PassDesc) * ph.passes.size(), cudaMemcpyHostToDevice));
+    RT_CUDA(ctx, p.passes.upload(ph.passes.data(), ph.passes.size()));
     p.n_atom_list = (int64_t)ph.alist.size();
-    RT_CUDA(ctx, cudaMalloc(&p.d_atom_list, sizeof(int32_t) * std::max<size_t>(1, ph.alist.size())));
-    if (!ph.alist.empty())
-        RT_CUDA(ctx, cudaMemcpy(p.d_atom_list, ph.alist.data(), sizeof(int32_t) * ph.alist.size(), cudaMemcpyHostToDevice));
-    const std::vector<rt::RefRec>& refs = ph.refs;
-    const std::vector<rt::RefWarp>& warps = ph.warps;
-    p.n_ref_warps = (int64_t)warps.size();
-    RT_CUDA(ctx, cudaMalloc(&p.d_refs, sizeof(rt::RefRec) * std::max<size_t>(1, refs.size())));
-    RT_CUDA(ctx, cudaMalloc(&p.d_ref_warps, sizeof(rt::RefWarp) * std::max<size_t>(1, warps.size())));
-    if (!refs.empty()) {
-        RT_CUDA(ctx, cudaMemcpy(p.d_refs, refs.data(), sizeof(rt::RefRec) * refs.size(), cudaMemcpyHostToDevice));
-        RT_CUDA(ctx, cudaMemcpy(p.d_ref_warps, warps.data(), sizeof(rt::RefWarp) * warps.size(), cudaMemcpyHostToDevice));
-    }
+    RT_CUDA(ctx, p.atom_list.upload(ph.alist.data(), ph.alist.size()));
+    p.n_ref_warps = (int64_t)ph.warps.size();
+    RT_CUDA(ctx, p.refs.upload(ph.refs.data(), ph.refs.size()));
+    RT_CUDA(ctx, p.ref_warps.upload(ph.warps.data(), ph.warps.size()));
     std::vector<rt::LongAcc> acc((size_t)std::max(1, ph.n_long_b));
     memset(acc.data(), 0, sizeof(rt::LongAcc) * acc.size());
     for (auto& a : acc) a.mn = 0xffffffffu;
-    RT_CUDA(ctx, cudaMalloc(&p.d_long_acc, sizeof(rt::LongAcc) * acc.size()));
-    RT_CUDA(ctx, cudaMemcpy(p.d_long_acc, acc.data(), sizeof(rt::LongAcc) * acc.size(), cudaMemcpyHostToDevice));
-    ctx->plans.push_back(p);
-    *out = &ctx->plans.back();
+    RT_CUDA(ctx, p.long_acc.upload(acc.data(), acc.size()));
+    ctx->ix.plans.push_back(std::move(p));
+    *out = &ctx->ix.plans.back();
     return RT_OK;
 }
 
 int get_plan(rt_ctx* ctx, int64_t lo, int64_t hi, rt_ctx::ScorePlan** out) {
-    for (auto& p : ctx->plans)
+    for (auto& p : ctx->ix.plans)
         if (p.lo == lo && p.hi == hi) {
             *out = &p;
             return RT_OK;
@@ -1313,7 +1296,7 @@ int prebuild_plans(rt_ctx* ctx, const std::vector<int64_t>& cut) {
     for (size_t i = 0; i + 1 < cut.size(); ++i) {
         const int64_t a = cut[i], b = cut[i + 1];
         bool cached = a == b;
-        for (auto& p : ctx->plans) cached = cached || (p.lo == a && p.hi == b);
+        for (auto& p : ctx->ix.plans) cached = cached || (p.lo == a && p.hi == b);
         if (!cached) {
             todo.emplace_back();
             todo.back().lo = a;
@@ -1347,9 +1330,9 @@ int rt_score(rt_ctx* ctx, const int32_t* d_cov, int64_t orf_lo, int64_t orf_hi, 
              const rt_score_out* d_out, void* stream) {
     if (!ctx) return fail(nullptr, RT_EINVAL, "rt_score: ctx is NULL");
     if (!d_cov || !params || !d_out) return fail(ctx, RT_EINVAL, "rt_score: NULL argument");
-    if (orf_lo < 0 || orf_hi > ctx->n_orf || orf_lo > orf_hi)
+    if (orf_lo < 0 || orf_hi > ctx->ix.n_orf || orf_lo > orf_hi)
         return fail(ctx, RT_EINVAL, "rt_score: ORF range [%lld,%lld) outside the index [0,%lld)", (long long)orf_lo,
-                    (long long)orf_hi, (long long)ctx->n_orf);
+                    (long long)orf_hi, (long long)ctx->ix.n_orf);
     if (orf_lo == orf_hi) return RT_OK;
     if (!d_out->score || !d_out->valid || !d_out->count || !d_out->length)
         return fail(ctx, RT_EINVAL, "rt_score: score/valid/count/length columns are required");
@@ -1358,15 +1341,15 @@ int rt_score(rt_ctx* ctx, const int32_t* d_cov, int64_t orf_lo, int64_t orf_hi, 
     rt_ctx::ScorePlan* plan = nullptr;
     int rc = get_plan(ctx, orf_lo, orf_hi, &plan);
     if (rc != RT_OK) return rc;
-    RT_CUDA(ctx, cudaMemsetAsync(ctx->d_work_counter, 0, 4 * sizeof(unsigned long long), st));
+    RT_CUDA(ctx, cudaMemsetAsync(ctx->work_counter.p, 0, 4 * sizeof(unsigned long long), st));
     rt::ScoreArgs a;
     a.cov = d_cov;
-    a.orf_desc = ctx->d_orf_desc;
-    const bool compact = ctx->layout == RT_LAYOUT_COMPACT;
-    a.exon_entries = compact ? ctx->d_exon_entries_c : ctx->d_exon_entries;
-    a.orf_len = ctx->d_orf_len;
+    a.orf_desc = ctx->ix.orf_desc.p;
+    const bool compact = ctx->ix.layout == RT_LAYOUT_COMPACT;
+    a.exon_entries = compact ? ctx->ix.exon_entries_c.p : ctx->ix.exon_entries.p;
+    a.orf_len = ctx->ix.orf_len.p;
     a.orf_lo = orf_lo;
-    a.n_fallback = reinterpret_cast<unsigned*>(ctx->d_work_counter + 3);
+    a.n_fallback = reinterpret_cast<unsigned*>(ctx->work_counter.p + 3);
     a.prm = *params;
     a.out = *d_out;
     const int threads = rt::kScoreWarps * 32;
@@ -1378,11 +1361,11 @@ int rt_score(rt_ctx* ctx, const int32_t* d_cov, int64_t orf_lo, int64_t orf_hi, 
             // streamed phase A: the compact buffer is read once, front to back, through TMA into shared memory
             rt::PassArgs pa;
             pa.cov = d_cov;
-            pa.atoms = ctx->d_atoms_c;
-            pa.passes = plan->d_passes;
+            pa.atoms = ctx->ix.atoms_c.p;
+            pa.passes = plan->passes.p;
             pa.n_passes = (unsigned)plan->n_passes;
-            pa.out = ctx->d_summaries;
-            pa.nonzero = ctx->d_atom_nonzero;
+            pa.out = ctx->ix.summaries.p;
+            pa.nonzero = ctx->ix.atom_nonzero.p;
             const size_t smem = rt::kUvEntries * sizeof(double2) + (size_t)rt::kPassWarps * rt::kPassStages * rt::kPassStageBytes;
             const auto kern = want_min ? rt::atom_pass_kernel<true> : rt::atom_pass_kernel<false>;
             RT_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1392,12 +1375,12 @@ int rt_score(rt_ctx* ctx, const int32_t* d_cov, int64_t orf_lo, int64_t orf_hi, 
         } else {
             rt::AtomArgs aa;
             aa.cov = d_cov;
-            aa.atoms = ctx->d_atoms;
-            aa.list = plan->d_atom_list;
+            aa.atoms = ctx->ix.atoms.p;
+            aa.list = plan->atom_list.p;
             aa.n_list = plan->n_atom_list;
-            aa.work_counter = ctx->d_work_counter + 0;
-            aa.out = ctx->d_summaries;
-            aa.nonzero = ctx->d_atom_nonzero;
+            aa.work_counter = ctx->work_counter.p + 0;
+            aa.out = ctx->ix.summaries.p;
+            aa.nonzero = ctx->ix.atom_nonzero.p;
             const auto kern = want_min ? rt::atom_summary_kernel<true> : rt::atom_summary_kernel<false>;
             const int g = 32 / rt::kAtomLPO;
             kern<<<persistent_grid(ctx, kern, (plan->n_atom_list + g - 1) / g), threads, 0, st>>>(aa);
@@ -1406,18 +1389,18 @@ int rt_score(rt_ctx* ctx, const int32_t* d_cov, int64_t orf_lo, int64_t orf_hi, 
     }
     // phase B: the ORFs of every family from the summaries of their atoms
     rt::RefComposeArgs ra;
-    ra.refs = plan->d_refs;
-    ra.warps = plan->d_ref_warps;
+    ra.refs = plan->refs.p;
+    ra.warps = plan->ref_warps.p;
     ra.n_warps = plan->n_ref_warps;
-    ra.summaries = ctx->d_summaries;
-    ra.atom_nonzero = ctx->d_atom_nonzero;
-    ra.uv_table = ctx->d_uv_table;
+    ra.summaries = ctx->ix.summaries.p;
+    ra.atom_nonzero = ctx->ix.atom_nonzero.p;
+    ra.uv_table = ctx->uv_table.p;
     ra.want_min = want_min ? 1 : 0;
-    ra.orf_len = ctx->d_orf_len;
+    ra.orf_len = ctx->ix.orf_len.p;
     ra.orf_lo = orf_lo;
-    ra.fallback = plan->d_fallback;
+    ra.fallback = plan->fallback.p;
     ra.n_fallback = a.n_fallback;
-    ra.long_acc = plan->d_long_acc;
+    ra.long_acc = plan->long_acc.p;
     ra.prm = *params;
     ra.out = *d_out;
     if (ra.n_warps > 0) {
@@ -1426,10 +1409,10 @@ int rt_score(rt_ctx* ctx, const int32_t* d_cov, int64_t orf_lo, int64_t orf_hi, 
     }
     ctx->launches++;
     // ORFs holding counts >= 2^20: redone by the generic kernel (normally none)
-    a.list = plan->d_fallback;
+    a.list = plan->fallback.p;
     a.n_list = 0;
     a.n_list_dev = a.n_fallback;
-    a.work_counter = ctx->d_work_counter + 2;
+    a.work_counter = ctx->work_counter.p + 2;
     rt::score_orfs_kernel<<<(unsigned)ctx->n_sm, threads, 0, st>>>(a);
     ctx->launches++;
     RT_CUDA(ctx, cudaGetLastError());
@@ -1440,14 +1423,14 @@ int rt_score_host(rt_ctx* ctx, const int32_t* d_cov, int64_t orf_lo, int64_t orf
                   const rt_score_out* h_out) {
     if (!ctx) return fail(nullptr, RT_EINVAL, "rt_score_host: ctx is NULL");
     if (!h_out || !params) return fail(ctx, RT_EINVAL, "rt_score_host: NULL argument");
-    if (orf_lo < 0 || orf_hi > ctx->n_orf || orf_lo > orf_hi) return fail(ctx, RT_EINVAL, "rt_score_host: bad ORF range");
+    if (orf_lo < 0 || orf_hi > ctx->ix.n_orf || orf_lo > orf_hi) return fail(ctx, RT_EINVAL, "rt_score_host: bad ORF range");
     const int64_t n = orf_hi - orf_lo;
     if (n == 0) return RT_OK;
     DeviceGuard guard(ctx->device);
     // one scratch allocation, 8-byte columns first
     const size_t bytes = (size_t)n * (8 + 8 + 24 + 4 + 4 + 4 + 12 + 1) + 256;
     RT_CUDA(ctx, ctx->score_buf.reserve(bytes));
-    char* p = static_cast<char*>(ctx->score_buf.p);
+    char* p = ctx->score_buf.p;
     rt_score_out d{};
     d.score = reinterpret_cast<double*>(p); p += 8 * n;
     d.count = reinterpret_cast<int64_t*>(p); p += 8 * n;
@@ -1464,7 +1447,7 @@ int rt_score_host(rt_ctx* ctx, const int32_t* d_cov, int64_t orf_lo, int64_t orf
     n_parts = (int)std::min<int64_t>(n_parts, n);
     std::vector<int64_t> cut((size_t)n_parts + 1, orf_lo);
     cut[(size_t)n_parts] = orf_hi;
-    const int64_t* bp = ctx->bytes_prefix.data();
+    const int64_t* bp = ctx->ix.bytes_prefix.data();
     for (int i = 1; i < n_parts; ++i) {
         const int64_t target = bp[orf_lo] + (bp[orf_hi] - bp[orf_lo]) * i / n_parts;
         cut[(size_t)i] = std::max<int64_t>(cut[(size_t)i - 1], std::lower_bound(bp + orf_lo, bp + orf_hi, target) - bp);
@@ -1473,9 +1456,9 @@ int rt_score_host(rt_ctx* ctx, const int32_t* d_cov, int64_t orf_lo, int64_t orf
         const int rc = prebuild_plans(ctx, cut);
         if (rc != RT_OK) return rc;
     }
-    if (!ctx->slot_stream[0]) RT_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->slot_stream[0], cudaStreamNonBlocking));
-    cudaStream_t copy = n_parts > 1 ? ctx->slot_stream[0] : nullptr;
-    if (n_parts > 1 && !ctx->ev_scored) RT_CUDA(ctx, cudaEventCreateWithFlags(&ctx->ev_scored, cudaEventDisableTiming));
+    RT_CUDA(ctx, ctx->slot_stream[0].create());
+    cudaStream_t copy = n_parts > 1 ? ctx->slot_stream[0].s : nullptr;
+    if (n_parts > 1) RT_CUDA(ctx, ctx->ev_scored.create(cudaEventDisableTiming));
     for (int i = 0; i < n_parts; ++i) {
         const int64_t a = cut[(size_t)i], b = cut[(size_t)i + 1], m = b - a, k = a - orf_lo;
         if (m == 0) continue;
@@ -1515,7 +1498,7 @@ int rt_phasescore_values(rt_ctx* ctx, const double* h_values, int64_t n, double*
     DeviceGuard guard(ctx->device);
     const size_t bytes = sizeof(double) * (size_t)std::max<int64_t>(n, 1) + 64;
     RT_CUDA(ctx, ctx->score_buf.reserve(bytes));
-    double* d_vals = static_cast<double*>(ctx->score_buf.p);
+    double* d_vals = reinterpret_cast<double*>(ctx->score_buf.p);
     double* d_score = d_vals + std::max<int64_t>(n, 1);
     int* d_valid = reinterpret_cast<int*>(d_score + 1);
     if (n) RT_CUDA(ctx, cudaMemcpyAsync(d_vals, h_values, sizeof(double) * n, cudaMemcpyHostToDevice, nullptr));
@@ -1533,13 +1516,13 @@ int rt_gather_profiles(rt_ctx* ctx, const int32_t* d_cov, int64_t n_sel, const i
     if (!ctx) return fail(nullptr, RT_EINVAL, "rt_gather_profiles: ctx is NULL");
     if (n_sel < 0 || !d_cov || (n_sel > 0 && (!d_orf_ids || !d_out_ptr || !d_out)))
         return fail(ctx, RT_EINVAL, "rt_gather_profiles: NULL argument");
-    if (ctx->n_orf == 0 && n_sel > 0) return fail(ctx, RT_ESTATE, "rt_gather_profiles: no index");
+    if (ctx->ix.n_orf == 0 && n_sel > 0) return fail(ctx, RT_ESTATE, "rt_gather_profiles: no index");
     if (n_sel == 0) return RT_OK;
     DeviceGuard guard(ctx->device);
     rt::GatherArgs a;
     a.cov = d_cov;
-    a.orf_desc = ctx->d_orf_desc;
-    a.exon_entries = ctx->layout == RT_LAYOUT_COMPACT ? ctx->d_exon_entries_c : ctx->d_exon_entries;
+    a.orf_desc = ctx->ix.orf_desc.p;
+    a.exon_entries = ctx->ix.layout == RT_LAYOUT_COMPACT ? ctx->ix.exon_entries_c.p : ctx->ix.exon_entries.p;
     a.orf_ids = d_orf_ids;
     a.out_ptr = d_out_ptr;
     a.out = d_out;
@@ -1556,11 +1539,11 @@ int rt_gather_profiles(rt_ctx* ctx, const int32_t* d_cov, int64_t n_sel, const i
 int rt_compact_from_dense(rt_ctx* ctx, const int32_t* d_dense, int32_t* d_compact, void* stream) {
     if (!ctx) return fail(nullptr, RT_EINVAL, "rt_compact_from_dense: ctx is NULL");
     if (!d_dense || !d_compact) return fail(ctx, RT_EINVAL, "rt_compact_from_dense: NULL argument");
-    if (ctx->n_orf == 0 || !ctx->d_atoms_c) return fail(ctx, RT_ESTATE, "rt_compact_from_dense: call rt_set_index first");
-    if (ctx->n_atoms == 0) return RT_OK;
+    if (ctx->ix.n_orf == 0 || !ctx->ix.atoms_c.p) return fail(ctx, RT_ESTATE, "rt_compact_from_dense: call rt_set_index first");
+    if (ctx->ix.n_atoms == 0) return RT_OK;
     DeviceGuard guard(ctx->device);
-    const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((ctx->n_atoms + 7) / 8, (int64_t)ctx->n_sm * 16));
-    rt::compact_from_dense_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(ctx->d_atoms, ctx->d_atoms_c, ctx->n_atoms, d_dense, d_compact);
+    const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((ctx->ix.n_atoms + 7) / 8, (int64_t)ctx->n_sm * 16));
+    rt::compact_from_dense_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(ctx->ix.atoms.p, ctx->ix.atoms_c.p, ctx->ix.n_atoms, d_dense, d_compact);
     ctx->launches++;
     RT_CUDA(ctx, cudaGetLastError());
     return RT_OK;
@@ -1600,7 +1583,7 @@ int rt_interval_sums(rt_ctx* ctx, const int32_t* d_cov, int64_t n_iv, const int6
     if (!ctx) return fail(nullptr, RT_EINVAL, "rt_interval_sums: ctx is NULL");
     if (n_iv < 0 || !d_cov || !d_sums || (n_iv > 0 && (!d_iv_off || !d_iv_len || !d_iv_group)))
         return fail(ctx, RT_EINVAL, "rt_interval_sums: NULL argument");
-    if (ctx->layout != RT_LAYOUT_DENSE)
+    if (ctx->ix.layout != RT_LAYOUT_DENSE)
         return fail(ctx, RT_ESTATE, "rt_interval_sums: interval offsets address the dense planes; switch the layout back first");
     if (n_iv == 0) return RT_OK;
     DeviceGuard guard(ctx->device);
@@ -1625,37 +1608,23 @@ int rt_bootstrap_medians(rt_ctx* ctx, const double* h_values, int64_t n, const i
     DeviceGuard guard(ctx->device);
     const size_t key_bytes = sizeof(unsigned long long) * (size_t)n_sel;
     const bool in_smem = key_bytes <= 160 * 1024;
-    DevBuf vals, idx, outb, scratch;
-    auto cleanup = [&]() { vals.release(); idx.release(); outb.release(); scratch.release(); };
-    cudaError_t e = vals.reserve(sizeof(double) * (size_t)n);
-    if (e == cudaSuccess) e = idx.reserve(sizeof(int64_t) * (size_t)(n_sel * reps));
-    if (e == cudaSuccess) e = outb.reserve(sizeof(double) * (size_t)reps);
-    if (e == cudaSuccess && !in_smem) e = scratch.reserve(key_bytes * (size_t)reps);
-    if (e == cudaSuccess) e = cudaMemcpy(vals.p, h_values, sizeof(double) * (size_t)n, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMemcpy(idx.p, h_idx, sizeof(int64_t) * (size_t)(n_sel * reps), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && in_smem)
-        e = cudaFuncSetAttribute(rt::bootstrap_median_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)key_bytes);
-    if (e == cudaSuccess) {
-        rt::bootstrap_median_kernel<<<(unsigned)reps, 256, in_smem ? key_bytes : 0>>>(
-            static_cast<const double*>(vals.p), static_cast<const long long*>(idx.p), n_sel, reps,
-            static_cast<unsigned long long*>(scratch.p), in_smem ? 1 : 0, static_cast<double*>(outb.p));
-        ctx->launches++;
-        e = cudaGetLastError();
-    }
-    if (e == cudaSuccess) e = cudaMemcpy(h_out, outb.p, sizeof(double) * (size_t)reps, cudaMemcpyDeviceToHost);
-    cleanup();
-    if (e != cudaSuccess) return fail(ctx, e == cudaErrorMemoryAllocation ? RT_ENOMEM : RT_ECUDA, "rt_bootstrap_medians: %s", cudaGetErrorString(e));
+    DevArr<double> vals, outb;
+    DevArr<long long> idx;
+    DevArr<unsigned long long> scratch;
+    RT_CUDA(ctx, vals.upload(h_values, (size_t)n));
+    RT_CUDA(ctx, idx.upload(h_idx, (size_t)(n_sel * reps)));
+    RT_CUDA(ctx, outb.reserve((size_t)reps));
+    if (!in_smem) RT_CUDA(ctx, scratch.reserve((size_t)n_sel * (size_t)reps));
+    if (in_smem) RT_CUDA(ctx, cudaFuncSetAttribute(rt::bootstrap_median_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)key_bytes));
+    rt::bootstrap_median_kernel<<<(unsigned)reps, 256, in_smem ? key_bytes : 0>>>(vals.p, idx.p, n_sel, reps, scratch.p,
+                                                                                 in_smem ? 1 : 0, outb.p);
+    ctx->launches++;
+    RT_CUDA(ctx, cudaGetLastError());
+    RT_CUDA(ctx, cudaMemcpy(h_out, outb.p, sizeof(double) * (size_t)reps, cudaMemcpyDeviceToHost));
     return RT_OK;
 }
 
 // ------------------------------------------------------------------------------------------------ prepare-orfs
-namespace {
-enum OrfBuf { kCodes, kExSrc, kExDst, kExLen, kExRev, kTxSeq, kTxCds, kTxExon, kTxRev, kExStart, kExEnd, kExBefore, kSeq,
-              kTxRows, kRowOff, kRowTx, kRowStart, kRowStop, kRowType, kRowCodon, kIvCount, kIvOff, kIvStart, kIvEnd,
-              kClaim, kOrfBufs };
-static_assert(kOrfBufs <= 32, "rt_ctx::orf_buf is too small");
-}  // namespace
-
 int rt_orf_search(rt_ctx* ctx, const rt_orf_query* q, int64_t* n_rows, int64_t* n_iv, float* stage_ms) {
     if (!ctx) return fail(nullptr, RT_EINVAL, "rt_orf_search: ctx is NULL");
     if (!q || !n_rows || !n_iv || q->n_tx < 0 || q->n_codes < 0 || q->min_orf_length < 0 ||
@@ -1693,87 +1662,83 @@ int rt_orf_search(rt_ctx* ctx, const rt_orf_query* q, int64_t* n_rows, int64_t* 
     }
     const int64_t n_seq = tx_seq[(size_t)n_tx];
     DeviceGuard guard(ctx->device);
-    DevBuf* B = ctx->orf_buf;
-    auto reserve = [&](int k, size_t bytes) { return B[k].reserve(std::max<size_t>(bytes, 16)); };
-    RT_CUDA(ctx, reserve(kCodes, (size_t)q->n_codes));
-    RT_CUDA(ctx, reserve(kExSrc, 8 * (size_t)n_ex));
-    RT_CUDA(ctx, reserve(kExDst, 8 * (size_t)n_ex));
-    RT_CUDA(ctx, reserve(kExLen, 4 * (size_t)n_ex));
-    RT_CUDA(ctx, reserve(kExRev, (size_t)n_ex));
-    RT_CUDA(ctx, reserve(kTxSeq, 8 * (size_t)(n_tx + 1)));
-    RT_CUDA(ctx, reserve(kTxCds, 8 * (size_t)n_tx));
-    RT_CUDA(ctx, reserve(kTxExon, 8 * (size_t)(n_tx + 1)));
-    RT_CUDA(ctx, reserve(kTxRev, (size_t)n_tx));
-    RT_CUDA(ctx, reserve(kExStart, 4 * (size_t)n_ex));
-    RT_CUDA(ctx, reserve(kExEnd, 4 * (size_t)n_ex));
-    RT_CUDA(ctx, reserve(kExBefore, 4 * (size_t)n_ex));
-    RT_CUDA(ctx, reserve(kSeq, (size_t)n_seq + 4));
-    RT_CUDA(ctx, reserve(kTxRows, 8 * (size_t)n_tx));
-    RT_CUDA(ctx, reserve(kRowOff, 8 * (size_t)n_tx));
-    RT_CUDA(ctx, reserve(kClaim, 4));
+    rt_ctx::OrfBufs& B = ctx->orf;
+    const size_t nt = (size_t)n_tx, ne = (size_t)n_ex;
+    RT_CUDA(ctx, B.codes.reserve((size_t)q->n_codes));
+    RT_CUDA(ctx, B.ex_src.reserve(ne));
+    RT_CUDA(ctx, B.ex_dst.reserve(ne));
+    RT_CUDA(ctx, B.ex_len.reserve(ne));
+    RT_CUDA(ctx, B.ex_rev.reserve(ne));
+    RT_CUDA(ctx, B.tx_seq.reserve(nt + 1));
+    RT_CUDA(ctx, B.tx_cds.reserve(nt));
+    RT_CUDA(ctx, B.tx_exon.reserve(nt + 1));
+    RT_CUDA(ctx, B.tx_rev.reserve(nt));
+    RT_CUDA(ctx, B.ex_start.reserve(ne));
+    RT_CUDA(ctx, B.ex_end.reserve(ne));
+    RT_CUDA(ctx, B.ex_before.reserve(ne));
+    RT_CUDA(ctx, B.seq.reserve((size_t)n_seq + 4));
+    RT_CUDA(ctx, B.tx_rows.reserve(nt));
+    RT_CUDA(ctx, B.row_off.reserve(nt));
+    RT_CUDA(ctx, B.claim.reserve(1));
     cudaStream_t st = 0;
-    cudaEvent_t ev[RT_ORF_STAGES + 1];
-    for (auto& e : ev) RT_CUDA(ctx, cudaEventCreate(&e));
-    struct EvGuard { cudaEvent_t* ev; ~EvGuard() { for (int i = 0; i <= RT_ORF_STAGES; ++i) cudaEventDestroy(ev[i]); } } evg{ev};
-    auto up = [&](int k, const void* src, size_t bytes) { return bytes ? cudaMemcpyAsync(B[k].p, src, bytes, cudaMemcpyHostToDevice, st) : cudaSuccess; };
+    Event ev[RT_ORF_STAGES + 1];
+    for (auto& e : ev) RT_CUDA(ctx, e.create());
     RT_CUDA(ctx, cudaEventRecord(ev[0], st));
     // 1. upload: contig codes, the transcript and exon tables
-    RT_CUDA(ctx, up(kCodes, q->codes, (size_t)q->n_codes));
-    RT_CUDA(ctx, up(kExSrc, ex_src.data(), 8 * (size_t)n_ex));
-    RT_CUDA(ctx, up(kExDst, ex_dst.data(), 8 * (size_t)n_ex));
-    RT_CUDA(ctx, up(kExLen, ex_len.data(), 4 * (size_t)n_ex));
-    RT_CUDA(ctx, up(kExRev, ex_rev.data(), (size_t)n_ex));
-    RT_CUDA(ctx, up(kTxSeq, tx_seq.data(), 8 * (size_t)(n_tx + 1)));
-    RT_CUDA(ctx, up(kTxCds, q->tx_cds, 8 * (size_t)n_tx));
-    RT_CUDA(ctx, up(kTxExon, q->exon_ptr, 8 * (size_t)(n_tx + 1)));
-    RT_CUDA(ctx, up(kTxRev, q->tx_strand, (size_t)n_tx));
-    RT_CUDA(ctx, up(kExStart, q->exon_start, 4 * (size_t)n_ex));
-    RT_CUDA(ctx, up(kExEnd, q->exon_end, 4 * (size_t)n_ex));
-    RT_CUDA(ctx, up(kExBefore, ex_before.data(), 4 * (size_t)n_ex));
+    RT_CUDA(ctx, B.codes.upload(q->codes, (size_t)q->n_codes, st));
+    RT_CUDA(ctx, B.ex_src.upload(ex_src.data(), ne, st));
+    RT_CUDA(ctx, B.ex_dst.upload(ex_dst.data(), ne, st));
+    RT_CUDA(ctx, B.ex_len.upload(ex_len.data(), ne, st));
+    RT_CUDA(ctx, B.ex_rev.upload(ex_rev.data(), ne, st));
+    RT_CUDA(ctx, B.tx_seq.upload(tx_seq.data(), nt + 1, st));
+    RT_CUDA(ctx, B.tx_cds.upload(reinterpret_cast<const int2*>(q->tx_cds), nt, st));
+    RT_CUDA(ctx, B.tx_exon.upload(q->exon_ptr, nt + 1, st));
+    RT_CUDA(ctx, B.tx_rev.upload(q->tx_strand, nt, st));
+    RT_CUDA(ctx, B.ex_start.upload(q->exon_start, ne, st));
+    RT_CUDA(ctx, B.ex_end.upload(q->exon_end, ne, st));
+    RT_CUDA(ctx, B.ex_before.upload(ex_before.data(), ne, st));
     RT_CUDA(ctx, cudaEventRecord(ev[1], st));
     const unsigned big = (unsigned)std::max(1, ctx->n_sm * 8);
     // 2. spliced, oriented sequences
     if (n_ex) {
         rt::orf_splice_kernel<<<(unsigned)std::min<int64_t>((n_ex + 7) / 8, big), 256, 0, st>>>(
-            (const uint8_t*)B[kCodes].p, (const long long*)B[kExSrc].p, (const long long*)B[kExDst].p, (const int*)B[kExLen].p,
-            (const uint8_t*)B[kExRev].p, n_ex, (uint8_t*)B[kSeq].p);
+            B.codes.p, B.ex_src.p, B.ex_dst.p, B.ex_len.p, B.ex_rev.p, n_ex, B.seq.p);
         ctx->launches++;
         RT_CUDA(ctx, cudaGetLastError());
     }
     RT_CUDA(ctx, cudaEventRecord(ev[2], st));
     // 3. rows per transcript
-    rt::OrfArgs A{(const long long*)B[kTxSeq].p, (const int2*)B[kTxCds].p, (uint8_t*)B[kSeq].p, q->start_mask, q->stop_mask,
-                  (int)n_tx, q->min_orf_length, q->longest ? 1 : 0, (unsigned*)B[kClaim].p};
+    rt::OrfArgs A{B.tx_seq.p, B.tx_cds.p, B.seq.p, q->start_mask, q->stop_mask, (int)n_tx, q->min_orf_length, q->longest ? 1 : 0,
+                  B.claim.p};
     const unsigned walk_grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((n_tx + 7) / 8, big));
     if (n_tx) {
-        RT_CUDA(ctx, cudaMemsetAsync(B[kClaim].p, 0, 4, st));
-        rt::orf_walk_kernel<false><<<walk_grid, 256, 0, st>>>(A, (long long*)B[kTxRows].p, nullptr, nullptr, nullptr, nullptr,
-                                                                nullptr, nullptr);
+        RT_CUDA(ctx, cudaMemsetAsync(B.claim.p, 0, sizeof(unsigned), st));
+        rt::orf_walk_kernel<false><<<walk_grid, 256, 0, st>>>(A, B.tx_rows.p, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);
         ctx->launches++;
         RT_CUDA(ctx, cudaGetLastError());
     }
     RT_CUDA(ctx, cudaEventRecord(ev[3], st));
     // 4. exclusive scan of the row counts (host: one int64 per transcript)
     std::vector<int64_t> cnt((size_t)n_tx), off((size_t)n_tx + 1, 0);
-    if (n_tx) RT_CUDA(ctx, cudaMemcpyAsync(cnt.data(), B[kTxRows].p, 8 * (size_t)n_tx, cudaMemcpyDeviceToHost, st));
+    if (n_tx) RT_CUDA(ctx, cudaMemcpyAsync(cnt.data(), B.tx_rows.p, sizeof(long long) * nt, cudaMemcpyDeviceToHost, st));
     RT_CUDA(ctx, cudaStreamSynchronize(st));
     for (int64_t t = 0; t < n_tx; ++t) off[(size_t)t + 1] = off[(size_t)t] + cnt[(size_t)t];
     const int64_t rows = off[(size_t)n_tx];
-    RT_CUDA(ctx, reserve(kRowTx, 4 * (size_t)rows));
-    RT_CUDA(ctx, reserve(kRowStart, 4 * (size_t)rows));
-    RT_CUDA(ctx, reserve(kRowStop, 4 * (size_t)rows));
-    RT_CUDA(ctx, reserve(kRowType, (size_t)rows));
-    RT_CUDA(ctx, reserve(kRowCodon, (size_t)rows));
-    RT_CUDA(ctx, reserve(kIvCount, 8 * (size_t)rows));
-    RT_CUDA(ctx, reserve(kIvOff, 8 * (size_t)rows));
-    RT_CUDA(ctx, up(kRowOff, off.data(), 8 * (size_t)n_tx));
+    const size_t nr = (size_t)rows;
+    RT_CUDA(ctx, B.row_tx.reserve(nr));
+    RT_CUDA(ctx, B.row_start.reserve(nr));
+    RT_CUDA(ctx, B.row_stop.reserve(nr));
+    RT_CUDA(ctx, B.row_type.reserve(nr));
+    RT_CUDA(ctx, B.row_codon.reserve(nr));
+    RT_CUDA(ctx, B.iv_count.reserve(nr));
+    RT_CUDA(ctx, B.iv_off.reserve(nr));
+    RT_CUDA(ctx, B.row_off.upload(off.data(), nt, st));
     RT_CUDA(ctx, cudaEventRecord(ev[4], st));
     // 5. the rows
     if (rows) {
-        RT_CUDA(ctx, cudaMemsetAsync(B[kClaim].p, 0, 4, st));
-        rt::orf_walk_kernel<true><<<walk_grid, 256, 0, st>>>(A, (long long*)B[kTxRows].p, (const long long*)B[kRowOff].p,
-                                                               (int*)B[kRowTx].p, (int*)B[kRowStart].p, (int*)B[kRowStop].p,
-                                                               (uint8_t*)B[kRowType].p, (uint8_t*)B[kRowCodon].p);
+        RT_CUDA(ctx, cudaMemsetAsync(B.claim.p, 0, sizeof(unsigned), st));
+        rt::orf_walk_kernel<true><<<walk_grid, 256, 0, st>>>(A, B.tx_rows.p, B.row_off.p, B.row_tx.p, B.row_start.p, B.row_stop.p,
+                                                               B.row_type.p, B.row_codon.p);
         ctx->launches++;
         RT_CUDA(ctx, cudaGetLastError());
     }
@@ -1782,15 +1747,13 @@ int rt_orf_search(rt_ctx* ctx, const rt_orf_query* q, int64_t* n_rows, int64_t* 
     const unsigned row_grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((rows + 255) / 256, (int64_t)big * 4));
     auto intervals = [&](bool count) {
         if (count)
-            rt::orf_interval_kernel<true><<<row_grid, 256, 0, st>>>(
-                rows, (const int*)B[kRowTx].p, (const int*)B[kRowStart].p, (const int*)B[kRowStop].p, (const long long*)B[kTxExon].p,
-                (const long long*)B[kTxSeq].p, (const uint8_t*)B[kTxRev].p, (const int*)B[kExStart].p, (const int*)B[kExEnd].p,
-                (const int*)B[kExBefore].p, (long long*)B[kIvCount].p, nullptr, nullptr, nullptr);
+            rt::orf_interval_kernel<true><<<row_grid, 256, 0, st>>>(rows, B.row_tx.p, B.row_start.p, B.row_stop.p, B.tx_exon.p,
+                                                                      B.tx_seq.p, B.tx_rev.p, B.ex_start.p, B.ex_end.p, B.ex_before.p,
+                                                                      B.iv_count.p, nullptr, nullptr, nullptr);
         else
-            rt::orf_interval_kernel<false><<<row_grid, 256, 0, st>>>(
-                rows, (const int*)B[kRowTx].p, (const int*)B[kRowStart].p, (const int*)B[kRowStop].p, (const long long*)B[kTxExon].p,
-                (const long long*)B[kTxSeq].p, (const uint8_t*)B[kTxRev].p, (const int*)B[kExStart].p, (const int*)B[kExEnd].p,
-                (const int*)B[kExBefore].p, nullptr, (const long long*)B[kIvOff].p, (int*)B[kIvStart].p, (int*)B[kIvEnd].p);
+            rt::orf_interval_kernel<false><<<row_grid, 256, 0, st>>>(rows, B.row_tx.p, B.row_start.p, B.row_stop.p, B.tx_exon.p,
+                                                                       B.tx_seq.p, B.tx_rev.p, B.ex_start.p, B.ex_end.p, B.ex_before.p,
+                                                                       nullptr, B.iv_off.p, B.iv_start.p, B.iv_end.p);
         ctx->launches++;
         return cudaGetLastError();
     };
@@ -1799,14 +1762,14 @@ int rt_orf_search(rt_ctx* ctx, const rt_orf_query* q, int64_t* n_rows, int64_t* 
     if (rows) {
         RT_CUDA(ctx, intervals(true));
         std::vector<int64_t> ivc((size_t)rows);
-        RT_CUDA(ctx, cudaMemcpyAsync(ivc.data(), B[kIvCount].p, 8 * (size_t)rows, cudaMemcpyDeviceToHost, st));
+        RT_CUDA(ctx, cudaMemcpyAsync(ivc.data(), B.iv_count.p, sizeof(long long) * nr, cudaMemcpyDeviceToHost, st));
         RT_CUDA(ctx, cudaStreamSynchronize(st));
         for (int64_t r = 0; r < rows; ++r) ivp[(size_t)r + 1] = ivp[(size_t)r] + ivc[(size_t)r];
     }
     const int64_t ivs = ivp.back();
-    RT_CUDA(ctx, reserve(kIvStart, 4 * (size_t)ivs));
-    RT_CUDA(ctx, reserve(kIvEnd, 4 * (size_t)ivs));
-    RT_CUDA(ctx, up(kIvOff, ivp.data(), 8 * (size_t)rows));
+    RT_CUDA(ctx, B.iv_start.reserve((size_t)ivs));
+    RT_CUDA(ctx, B.iv_end.reserve((size_t)ivs));
+    RT_CUDA(ctx, B.iv_off.upload(ivp.data(), nr, st));
     RT_CUDA(ctx, cudaEventRecord(ev[6], st));
     // 7. the intervals
     if (rows) RT_CUDA(ctx, intervals(false));
@@ -1827,16 +1790,18 @@ int rt_orf_fetch(rt_ctx* ctx, int32_t* row_tx, int32_t* row_start, int32_t* row_
     if ((int64_t)ctx->orf_iv_ptr.size() != rows + 1) return fail(ctx, RT_ESTATE, "rt_orf_fetch: call rt_orf_search first");
     const int64_t ivs = ctx->orf_iv_ptr.back();
     DeviceGuard guard(ctx->device);
-    DevBuf* B = ctx->orf_buf;
+    const rt_ctx::OrfBufs& B = ctx->orf;
     cudaStream_t st = 0;
-    auto down = [&](void* dst, int k, size_t bytes) { return dst && bytes ? cudaMemcpyAsync(dst, B[k].p, bytes, cudaMemcpyDeviceToHost, st) : cudaSuccess; };
-    RT_CUDA(ctx, down(row_tx, kRowTx, 4 * (size_t)rows));
-    RT_CUDA(ctx, down(row_start, kRowStart, 4 * (size_t)rows));
-    RT_CUDA(ctx, down(row_stop, kRowStop, 4 * (size_t)rows));
-    RT_CUDA(ctx, down(row_type, kRowType, (size_t)rows));
-    RT_CUDA(ctx, down(row_codon, kRowCodon, (size_t)rows));
-    RT_CUDA(ctx, down(iv_start, kIvStart, 4 * (size_t)ivs));
-    RT_CUDA(ctx, down(iv_end, kIvEnd, 4 * (size_t)ivs));
+    auto down = [&](void* dst, const auto& src, int64_t m) {
+        return dst && m ? cudaMemcpyAsync(dst, src.p, sizeof(*src.p) * (size_t)m, cudaMemcpyDeviceToHost, st) : cudaSuccess;
+    };
+    RT_CUDA(ctx, down(row_tx, B.row_tx, rows));
+    RT_CUDA(ctx, down(row_start, B.row_start, rows));
+    RT_CUDA(ctx, down(row_stop, B.row_stop, rows));
+    RT_CUDA(ctx, down(row_type, B.row_type, rows));
+    RT_CUDA(ctx, down(row_codon, B.row_codon, rows));
+    RT_CUDA(ctx, down(iv_start, B.iv_start, ivs));
+    RT_CUDA(ctx, down(iv_end, B.iv_end, ivs));
     if (iv_ptr) memcpy(iv_ptr, ctx->orf_iv_ptr.data(), 8 * (size_t)(rows + 1));
     RT_CUDA(ctx, cudaStreamSynchronize(st));
     return RT_OK;
@@ -1844,29 +1809,20 @@ int rt_orf_fetch(rt_ctx* ctx, int32_t* row_tx, int32_t* row_start, int32_t* row_
 
 // ---------------------------------------------------------------------------------------------------- orfs-seq
 namespace {
-enum SeqBuf { kSqCodes, kSqExPtr, kSqExStart, kSqExEnd, kSqContig, kSqStrand, kSqBase, kSqIdOff, kSqIds, kSqLineOff,
-              kSqOut0, kSqOut1, kSqClaim, kSeqBufs };
-static_assert(kSeqBufs <= 16, "rt_ctx::seq_buf is too small");
 constexpr int64_t kSeqChunkDefault = int64_t(64) << 20;
 
 // Streams, events, page-locked buffers and the writer of one rt_orf_seq_write call; the destructor joins the writer and
-// waits for both streams before anything is freed, so every early return leaves nothing behind.
+// waits for both streams before the members are freed, so every early return leaves nothing behind.
 struct SeqPipeline {
-    cudaStream_t ks = nullptr, cs = nullptr;   // kernels + uploads, copy-back
-    cudaEvent_t ev[10] = {};                   // upload begin / end, then per buffer b: kernel begin/end, copy begin/end
-    char* pinned[2] = {};
+    Stream ks, cs;                             // kernels + uploads, copy-back
+    Event ev[10];                              // upload begin / end, then per buffer b: kernel begin/end, copy begin/end
+    PinnedArr<char> pinned[2];
     WriteBehind writer;
     explicit SeqPipeline(FILE* fh) : writer(fh) {}
     ~SeqPipeline() {
         writer.finish();                       // before the page-locked buffers it writes from are freed
         if (ks) cudaStreamSynchronize(ks);
         if (cs) cudaStreamSynchronize(cs);
-        for (char* p : pinned)
-            if (p) cudaFreeHost(p);
-        for (cudaEvent_t e : ev)
-            if (e) cudaEventDestroy(e);
-        if (ks) cudaStreamDestroy(ks);
-        if (cs) cudaStreamDestroy(cs);
     }
 };
 
@@ -1874,39 +1830,36 @@ int seq_emit(rt_ctx* ctx, const rt_seq_query* q, const std::vector<int64_t>& lin
              int64_t buf_bytes, FILE* fh, float* stage_ms) {
     const int64_t n = q->n_orf, n_ex = n ? q->exon_ptr[n] : 0, n_ids = n ? q->id_off[n] : 0;
     const int64_t n_chunks = (int64_t)cut.size() - 1;
-    DevBuf* B = ctx->seq_buf;
-    auto reserve = [&](int k, size_t bytes) { return B[k].reserve(std::max<size_t>(bytes, 16)); };
-    RT_CUDA(ctx, reserve(kSqCodes, (size_t)q->n_codes));
-    RT_CUDA(ctx, reserve(kSqExPtr, 8 * (size_t)(n + 1)));
-    RT_CUDA(ctx, reserve(kSqExStart, 4 * (size_t)n_ex));
-    RT_CUDA(ctx, reserve(kSqExEnd, 4 * (size_t)n_ex));
-    RT_CUDA(ctx, reserve(kSqContig, 4 * (size_t)n));
-    RT_CUDA(ctx, reserve(kSqStrand, (size_t)n));
-    RT_CUDA(ctx, reserve(kSqBase, 8 * (size_t)q->n_contig));
-    RT_CUDA(ctx, reserve(kSqIdOff, 8 * (size_t)(n + 1)));
-    RT_CUDA(ctx, reserve(kSqIds, (size_t)n_ids));
-    RT_CUDA(ctx, reserve(kSqLineOff, 8 * (size_t)(n + 1)));
-    RT_CUDA(ctx, reserve(kSqClaim, 4));
+    rt_ctx::SeqBufs& B = ctx->seq;
+    const size_t nr = (size_t)n, ne = (size_t)n_ex;
+    RT_CUDA(ctx, B.codes.reserve((size_t)q->n_codes));
+    RT_CUDA(ctx, B.exon_ptr.reserve(nr + 1));
+    RT_CUDA(ctx, B.ex_start.reserve(ne));
+    RT_CUDA(ctx, B.ex_end.reserve(ne));
+    RT_CUDA(ctx, B.contig.reserve(nr));
+    RT_CUDA(ctx, B.strand.reserve(nr));
+    RT_CUDA(ctx, B.base.reserve((size_t)q->n_contig));
+    RT_CUDA(ctx, B.id_off.reserve(nr + 1));
+    RT_CUDA(ctx, B.ids.reserve((size_t)n_ids));
+    RT_CUDA(ctx, B.line_off.reserve(nr + 1));
+    RT_CUDA(ctx, B.claim.reserve(1));
     SeqPipeline P(fh);
-    RT_CUDA(ctx, cudaStreamCreateWithFlags(&P.ks, cudaStreamNonBlocking));
-    RT_CUDA(ctx, cudaStreamCreateWithFlags(&P.cs, cudaStreamNonBlocking));
-    for (auto& e : P.ev) RT_CUDA(ctx, cudaEventCreate(&e));
-    cudaEvent_t *k_begin = P.ev + 2, *k_end = P.ev + 4, *c_begin = P.ev + 6, *c_end = P.ev + 8;
+    RT_CUDA(ctx, P.ks.create());
+    RT_CUDA(ctx, P.cs.create());
+    for (auto& e : P.ev) RT_CUDA(ctx, e.create());
+    const Event *k_begin = P.ev + 2, *k_end = P.ev + 4, *c_begin = P.ev + 6, *c_end = P.ev + 8;
     // 1. upload: the contig codes and the tables, once
-    auto up = [&](int k, const void* src, size_t bytes) {
-        return bytes ? cudaMemcpyAsync(B[k].p, src, bytes, cudaMemcpyHostToDevice, P.ks) : cudaSuccess;
-    };
     RT_CUDA(ctx, cudaEventRecord(P.ev[0], P.ks));
-    RT_CUDA(ctx, up(kSqCodes, q->codes, (size_t)q->n_codes));
-    RT_CUDA(ctx, up(kSqExPtr, q->exon_ptr, 8 * (size_t)(n + 1)));
-    RT_CUDA(ctx, up(kSqExStart, q->exon_start, 4 * (size_t)n_ex));
-    RT_CUDA(ctx, up(kSqExEnd, q->exon_end, 4 * (size_t)n_ex));
-    RT_CUDA(ctx, up(kSqContig, q->orf_contig, 4 * (size_t)n));
-    RT_CUDA(ctx, up(kSqStrand, q->orf_strand, (size_t)n));
-    RT_CUDA(ctx, up(kSqBase, q->contig_base, 8 * (size_t)q->n_contig));
-    RT_CUDA(ctx, up(kSqIdOff, q->id_off, 8 * (size_t)(n + 1)));
-    RT_CUDA(ctx, up(kSqIds, q->ids, (size_t)n_ids));
-    RT_CUDA(ctx, up(kSqLineOff, line_off.data(), 8 * (size_t)(n + 1)));
+    RT_CUDA(ctx, B.codes.upload(q->codes, (size_t)q->n_codes, P.ks));
+    RT_CUDA(ctx, B.exon_ptr.upload(q->exon_ptr, nr + 1, P.ks));
+    RT_CUDA(ctx, B.ex_start.upload(q->exon_start, ne, P.ks));
+    RT_CUDA(ctx, B.ex_end.upload(q->exon_end, ne, P.ks));
+    RT_CUDA(ctx, B.contig.upload(q->orf_contig, nr, P.ks));
+    RT_CUDA(ctx, B.strand.upload(q->orf_strand, nr, P.ks));
+    RT_CUDA(ctx, B.base.upload(q->contig_base, (size_t)q->n_contig, P.ks));
+    RT_CUDA(ctx, B.id_off.upload(q->id_off, nr + 1, P.ks));
+    RT_CUDA(ctx, B.ids.upload(q->ids, (size_t)n_ids, P.ks));
+    RT_CUDA(ctx, B.line_off.upload(line_off.data(), nr + 1, P.ks));
     RT_CUDA(ctx, cudaEventRecord(P.ev[1], P.ks));
     if (stage_ms) stage_ms[1] = stage_ms[2] = 0.f;
     if (n_chunks == 0) {
@@ -1916,13 +1869,11 @@ int seq_emit(rt_ctx* ctx, const rt_seq_query* q, const std::vector<int64_t>& lin
     }
     // 2. the chunks: kernel k+1 runs while chunk k is copied back and chunk k-1 is written
     for (int b = 0; b < 2 && b < n_chunks; ++b) {
-        RT_CUDA(ctx, reserve(kSqOut0 + b, (size_t)buf_bytes));
-        RT_CUDA(ctx, cudaHostAlloc((void**)&P.pinned[b], (size_t)buf_bytes, cudaHostAllocDefault));
+        RT_CUDA(ctx, B.out[b].reserve((size_t)buf_bytes));
+        RT_CUDA(ctx, P.pinned[b].alloc((size_t)buf_bytes));
     }
-    const rt::SeqArgs A{(const uint8_t*)B[kSqCodes].p, (const long long*)B[kSqExPtr].p, (const int*)B[kSqExStart].p,
-                        (const int*)B[kSqExEnd].p, (const int*)B[kSqContig].p, (const uint8_t*)B[kSqStrand].p,
-                        (const long long*)B[kSqBase].p, (const long long*)B[kSqIdOff].p, (const char*)B[kSqIds].p,
-                        (const long long*)B[kSqLineOff].p, (unsigned*)B[kSqClaim].p};
+    const rt::SeqArgs A{B.codes.p, B.exon_ptr.p, B.ex_start.p, B.ex_end.p, B.contig.p, B.strand.p, B.base.p, B.id_off.p, B.ids.p,
+                        B.line_off.p, B.claim.p};
     const int64_t big = std::max(1, ctx->n_sm * 8);
     auto bytes_of = [&](int64_t k) { return (size_t)(line_off[(size_t)cut[(size_t)k + 1]] - line_off[(size_t)cut[(size_t)k]]); };
     // chunk k is on the host: add its times, hand it to the writer
@@ -1936,20 +1887,20 @@ int seq_emit(rt_ctx* ctx, const rt_seq_query* q, const std::vector<int64_t>& lin
             stage_ms[1] += kms;
             stage_ms[2] += cms;
         }
-        if (!P.writer.put_view(P.pinned[b], bytes_of(k))) return fail(ctx, RT_EINVAL, "rt_orf_seq_write: write error");
+        if (!P.writer.put_view(P.pinned[b].p, bytes_of(k))) return fail(ctx, RT_EINVAL, "rt_orf_seq_write: write error");
         return RT_OK;
     };
     for (int64_t k = 0; k < n_chunks; ++k) {
         const int b = (int)(k & 1);
         const int64_t r0 = cut[(size_t)k], rows = cut[(size_t)k + 1] - r0;
         // device buffer b is free: chunk k-2's copy finished before collect(k-2) returned
-        RT_CUDA(ctx, cudaMemsetAsync(B[kSqClaim].p, 0, 4, P.ks));
+        RT_CUDA(ctx, cudaMemsetAsync(B.claim.p, 0, sizeof(unsigned), P.ks));
         RT_CUDA(ctx, cudaEventRecord(k_begin[b], P.ks));
         const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((rows + rt::kSeqWarps - 1) / rt::kSeqWarps, big));
         if (q->protein)
-            rt::orf_seq_kernel<true><<<grid, rt::kSeqWarps * 32, 0, P.ks>>>(A, r0, rows, (char*)B[kSqOut0 + b].p);
+            rt::orf_seq_kernel<true><<<grid, rt::kSeqWarps * 32, 0, P.ks>>>(A, r0, rows, B.out[b].p);
         else
-            rt::orf_seq_kernel<false><<<grid, rt::kSeqWarps * 32, 0, P.ks>>>(A, r0, rows, (char*)B[kSqOut0 + b].p);
+            rt::orf_seq_kernel<false><<<grid, rt::kSeqWarps * 32, 0, P.ks>>>(A, r0, rows, B.out[b].p);
         ctx->launches++;
         RT_CUDA(ctx, cudaGetLastError());
         RT_CUDA(ctx, cudaEventRecord(k_end[b], P.ks));
@@ -1961,7 +1912,7 @@ int seq_emit(rt_ctx* ctx, const rt_seq_query* q, const std::vector<int64_t>& lin
         if (k >= 2 && !P.writer.wait_written(k - 1)) return fail(ctx, RT_EINVAL, "rt_orf_seq_write: write error");
         RT_CUDA(ctx, cudaStreamWaitEvent(P.cs, k_end[b], 0));
         RT_CUDA(ctx, cudaEventRecord(c_begin[b], P.cs));
-        RT_CUDA(ctx, cudaMemcpyAsync(P.pinned[b], B[kSqOut0 + b].p, bytes_of(k), cudaMemcpyDeviceToHost, P.cs));
+        RT_CUDA(ctx, cudaMemcpyAsync(P.pinned[b].p, B.out[b].p, bytes_of(k), cudaMemcpyDeviceToHost, P.cs));
         RT_CUDA(ctx, cudaEventRecord(c_end[b], P.cs));
     }
     const int rc = collect(n_chunks - 1);
@@ -2039,22 +1990,17 @@ int rt_orf_seq_write(rt_ctx* ctx, const rt_seq_query* q, const char* path, float
 }  // extern "C"
 
 namespace {
-enum CodonBuf { kCdProf, kCdSeq, kCdProfBase, kCdSeqBase, kCdSlotBase, kCdRow, kCdGene, kCdGseq, kCdExPtr, kCdExStart,
-                kCdExEnd, kCdStrand, kCdCnt, kCdKey, kCdVal, kCdKey2, kCdVal2, kCdCounters, kCdFlag, kCdClaim, kCdTemp,
-                kCdGeneTab, kCdPooledTab, kCodonBufs };
-
-// The device buffers and events of one rt_codon_counts call; everything is freed on every return.
+// The stream, events and device buffers of one rt_codon_counts call; everything is freed on every return.
 struct CodonScratch {
-    DevBuf b[kCodonBufs];
-    cudaStream_t st = nullptr;
-    cudaEvent_t ev[7] = {};
-    ~CodonScratch() {
-        if (st) cudaStreamSynchronize(st);
-        for (DevBuf& x : b) x.release();
-        for (cudaEvent_t e : ev)
-            if (e) cudaEventDestroy(e);
-        if (st) cudaStreamDestroy(st);
-    }
+    Stream st;
+    Event ev[7];
+    DevArr<char> prof, seq, temp;
+    DevArr<long long> prof_base, seq_base, slot_base, row, ex_ptr;
+    DevArr<int> gene, gseq, ex_start, ex_end;
+    DevArr<uint8_t> strand, flag;
+    DevArr<unsigned long long> cnt, key, val, key2, val2, counters, gene_tab, pooled_tab;
+    DevArr<unsigned> claim;
+    ~CodonScratch() { if (st) cudaStreamSynchronize(st); }
 };
 
 int bit_length(unsigned long long x) { return x ? 64 - __builtin_clzll(x) : 0; }
@@ -2109,68 +2055,55 @@ int rt_codon_counts(rt_ctx* ctx, const rt_codon_query* q, uint64_t* gene_tab, ui
     // 2. uploads
     DeviceGuard guard(ctx->device);
     CodonScratch S;
-    DevBuf* B = S.b;
-    RT_CUDA(ctx, cudaStreamCreateWithFlags(&S.st, cudaStreamNonBlocking));
-    for (auto& e : S.ev) RT_CUDA(ctx, cudaEventCreate(&e));
-    auto reserve = [&](int k, size_t bytes) { return B[k].reserve(std::max<size_t>(bytes, 16)); };
-    auto up = [&](int k, const void* src, size_t bytes) {
-        return bytes ? cudaMemcpyAsync(B[k].p, src, bytes, cudaMemcpyHostToDevice, S.st) : cudaSuccess;
-    };
-    const size_t ns = (size_t)n_slot;
-    RT_CUDA(ctx, reserve(kCdProf, prof.size()));
-    RT_CUDA(ctx, reserve(kCdSeq, letters.size()));
-    RT_CUDA(ctx, reserve(kCdProfBase, 8 * ((size_t)n + 1)));
-    RT_CUDA(ctx, reserve(kCdSeqBase, 8 * ((size_t)n + 1)));
-    RT_CUDA(ctx, reserve(kCdSlotBase, 8 * ((size_t)n + 1)));
-    RT_CUDA(ctx, reserve(kCdRow, 8 * (size_t)n));
-    RT_CUDA(ctx, reserve(kCdGene, 4 * (size_t)n));
-    RT_CUDA(ctx, reserve(kCdGseq, 4 * (size_t)n));
-    RT_CUDA(ctx, reserve(kCdExPtr, 8 * ((size_t)q->n_orf + 1)));
-    RT_CUDA(ctx, reserve(kCdExStart, 4 * (size_t)n_ex));
-    RT_CUDA(ctx, reserve(kCdExEnd, 4 * (size_t)n_ex));
-    RT_CUDA(ctx, reserve(kCdStrand, (size_t)q->n_orf));
-    RT_CUDA(ctx, reserve(kCdCnt, 8 * ns));
-    RT_CUDA(ctx, reserve(kCdKey, 8 * ns));
-    RT_CUDA(ctx, reserve(kCdVal, 8 * ns));
-    RT_CUDA(ctx, reserve(kCdKey2, 8 * ns));
-    RT_CUDA(ctx, reserve(kCdVal2, 8 * ns));
-    RT_CUDA(ctx, reserve(kCdCounters, 8 * 4));
-    RT_CUDA(ctx, reserve(kCdFlag, (size_t)n));
-    RT_CUDA(ctx, reserve(kCdClaim, 4));
-    RT_CUDA(ctx, reserve(kCdGeneTab, 8 * RT_CODON_CELL * 64 * (size_t)q->n_gene));
-    RT_CUDA(ctx, reserve(kCdPooledTab, 8 * RT_CODON_CELL * 64));
+    RT_CUDA(ctx, S.st.create());
+    for (auto& e : S.ev) RT_CUDA(ctx, e.create());
+    const size_t ns = (size_t)n_slot, nn = (size_t)n, no = (size_t)q->n_orf, ne = (size_t)n_ex;
+    RT_CUDA(ctx, S.prof.reserve(prof.size()));
+    RT_CUDA(ctx, S.seq.reserve(letters.size()));
+    RT_CUDA(ctx, S.prof_base.reserve(nn + 1));
+    RT_CUDA(ctx, S.seq_base.reserve(nn + 1));
+    RT_CUDA(ctx, S.slot_base.reserve(nn + 1));
+    RT_CUDA(ctx, S.row.reserve(nn));
+    RT_CUDA(ctx, S.gene.reserve(nn));
+    RT_CUDA(ctx, S.gseq.reserve(nn));
+    RT_CUDA(ctx, S.ex_ptr.reserve(no + 1));
+    RT_CUDA(ctx, S.ex_start.reserve(ne));
+    RT_CUDA(ctx, S.ex_end.reserve(ne));
+    RT_CUDA(ctx, S.strand.reserve(no));
+    RT_CUDA(ctx, S.cnt.reserve(ns));
+    RT_CUDA(ctx, S.key.reserve(ns));
+    RT_CUDA(ctx, S.val.reserve(ns));
+    RT_CUDA(ctx, S.key2.reserve(ns));
+    RT_CUDA(ctx, S.val2.reserve(ns));
+    RT_CUDA(ctx, S.counters.reserve(4));
+    RT_CUDA(ctx, S.flag.reserve(nn));
+    RT_CUDA(ctx, S.claim.reserve(1));
+    RT_CUDA(ctx, S.gene_tab.reserve(RT_CODON_CELL * 64 * (size_t)q->n_gene));
+    RT_CUDA(ctx, S.pooled_tab.reserve(RT_CODON_CELL * 64));
     RT_CUDA(ctx, cudaEventRecord(S.ev[0], S.st));
-    RT_CUDA(ctx, up(kCdProf, prof.p, prof.size()));
-    RT_CUDA(ctx, up(kCdSeq, letters.p, letters.size()));
-    RT_CUDA(ctx, up(kCdProfBase, prof_base.data(), 8 * ((size_t)n + 1)));
-    RT_CUDA(ctx, up(kCdSeqBase, seq_base.data(), 8 * ((size_t)n + 1)));
-    RT_CUDA(ctx, up(kCdSlotBase, slot_base.data(), 8 * ((size_t)n + 1)));
-    RT_CUDA(ctx, up(kCdRow, q->row, 8 * (size_t)n));
-    RT_CUDA(ctx, up(kCdGene, q->gene, 4 * (size_t)n));
-    RT_CUDA(ctx, up(kCdGseq, q->gseq, 4 * (size_t)n));
+    RT_CUDA(ctx, S.prof.upload(prof.p, prof.size(), S.st));
+    RT_CUDA(ctx, S.seq.upload(letters.p, letters.size(), S.st));
+    RT_CUDA(ctx, S.prof_base.upload(prof_base.data(), nn + 1, S.st));
+    RT_CUDA(ctx, S.seq_base.upload(seq_base.data(), nn + 1, S.st));
+    RT_CUDA(ctx, S.slot_base.upload(slot_base.data(), nn + 1, S.st));
+    RT_CUDA(ctx, S.row.upload(q->row, nn, S.st));
+    RT_CUDA(ctx, S.gene.upload(q->gene, nn, S.st));
+    RT_CUDA(ctx, S.gseq.upload(q->gseq, nn, S.st));
     if (n) {
-        RT_CUDA(ctx, up(kCdExPtr, q->exon_ptr, 8 * ((size_t)q->n_orf + 1)));
-        RT_CUDA(ctx, up(kCdExStart, q->exon_start, 4 * (size_t)n_ex));
-        RT_CUDA(ctx, up(kCdExEnd, q->exon_end, 4 * (size_t)n_ex));
-        RT_CUDA(ctx, up(kCdStrand, q->orf_strand, (size_t)q->n_orf));
+        RT_CUDA(ctx, S.ex_ptr.upload(q->exon_ptr, no + 1, S.st));
+        RT_CUDA(ctx, S.ex_start.upload(q->exon_start, ne, S.st));
+        RT_CUDA(ctx, S.ex_end.upload(q->exon_end, ne, S.st));
+        RT_CUDA(ctx, S.strand.upload(q->orf_strand, no, S.st));
     }
     const unsigned long long counters0[4] = {0, 0, ~0ull, 0};
-    RT_CUDA(ctx, up(kCdCounters, counters0, sizeof counters0));
-    RT_CUDA(ctx, cudaMemsetAsync(B[kCdCnt].p, 0, 8 * ns, S.st));
-    RT_CUDA(ctx, cudaMemsetAsync(B[kCdClaim].p, 0, 4, S.st));
+    RT_CUDA(ctx, S.counters.upload(counters0, 4, S.st));
+    RT_CUDA(ctx, cudaMemsetAsync(S.cnt.p, 0, sizeof(unsigned long long) * ns, S.st));
+    RT_CUDA(ctx, cudaMemsetAsync(S.claim.p, 0, sizeof(unsigned), S.st));
     RT_CUDA(ctx, cudaEventRecord(S.ev[1], S.st));
     // 3. codon_emit_kernel
-    auto* cnt = (unsigned long long*)B[kCdCnt].p;
-    auto* key = (unsigned long long*)B[kCdKey].p;
-    auto* val = (unsigned long long*)B[kCdVal].p;
-    auto* key2 = (unsigned long long*)B[kCdKey2].p;
-    auto* val2 = (unsigned long long*)B[kCdVal2].p;
-    auto* counters = (unsigned long long*)B[kCdCounters].p;
-    const rt::CodonArgs A{(const char*)B[kCdProf].p, (const long long*)B[kCdProfBase].p, (const char*)B[kCdSeq].p,
-                          (const long long*)B[kCdSeqBase].p, (const long long*)B[kCdSlotBase].p, (const long long*)B[kCdRow].p,
-                          (const long long*)B[kCdExPtr].p, (const int*)B[kCdExStart].p, (const int*)B[kCdExEnd].p,
-                          (const uint8_t*)B[kCdStrand].p, (const int*)B[kCdGene].p, (const int*)B[kCdGseq].p, cnt, key, val,
-                          counters, (uint8_t*)B[kCdFlag].p, (long long)n, (unsigned*)B[kCdClaim].p};
+    unsigned long long *cnt = S.cnt.p, *key = S.key.p, *val = S.val.p, *key2 = S.key2.p, *val2 = S.val2.p, *counters = S.counters.p;
+    const rt::CodonArgs A{S.prof.p, S.prof_base.p, S.seq.p, S.seq_base.p, S.slot_base.p, S.row.p, S.ex_ptr.p, S.ex_start.p,
+                          S.ex_end.p, S.strand.p, S.gene.p, S.gseq.p, cnt, key, val, counters, S.flag.p, (long long)n, S.claim.p};
     const int64_t big = std::max(1, ctx->n_sm * 8);
     if (n) {
         const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((n + rt::kCodonWarps - 1) / rt::kCodonWarps, big));
@@ -2186,7 +2119,7 @@ int rt_codon_counts(rt_ctx* ctx, const rt_codon_query* q, uint64_t* gene_tab, ui
     summary[1] = (int64_t)h_counters[1];
     if (h_counters[2] != ~0ull) {                      // a refused profile: no tables
         uint8_t f = 0;
-        RT_CUDA(ctx, cudaMemcpyAsync(&f, (uint8_t*)B[kCdFlag].p + h_counters[2], 1, cudaMemcpyDeviceToHost, S.st));
+        RT_CUDA(ctx, cudaMemcpyAsync(&f, S.flag.p + h_counters[2], 1, cudaMemcpyDeviceToHost, S.st));
         RT_CUDA(ctx, cudaStreamSynchronize(S.st));
         summary[4] = (int64_t)h_counters[2];
         summary[5] = f;
@@ -2201,8 +2134,8 @@ int rt_codon_counts(rt_ctx* ctx, const rt_codon_query* q, uint64_t* gene_tab, ui
     RT_CUDA(ctx, cub::DeviceRadixSort::SortPairs(nullptr, t1, key, key2, val, val2, items, 0, place_bits, S.st));
     RT_CUDA(ctx, cub::DeviceRadixSort::SortKeys(nullptr, t2, val, val2, items, 0, gene_bits, S.st));
     RT_CUDA(ctx, cub::DeviceRadixSort::SortKeys(nullptr, t3, val, val2, items, 0, 38, S.st));
-    RT_CUDA(ctx, reserve(kCdTemp, std::max({t1, t2, t3})));
-    void* temp = B[kCdTemp].p;
+    RT_CUDA(ctx, S.temp.reserve(std::max({t1, t2, t3})));
+    void* temp = S.temp.p;
     if (items) RT_CUDA(ctx, cub::DeviceRadixSort::SortPairs(temp, t1, key, key2, val, val2, items, 0, place_bits, S.st));
     // kept values -> cnt (free now), pooled keys -> key (free now)
     const unsigned keep_grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((int64_t)(ns + 255) / 256, big));
@@ -2224,8 +2157,7 @@ int rt_codon_counts(rt_ctx* ctx, const rt_codon_query* q, uint64_t* gene_tab, ui
     }
     RT_CUDA(ctx, cudaEventRecord(S.ev[4], S.st));
     // 6. codon_stats_kernel over the per-gene cells and the pooled cells
-    auto* gtab = (unsigned long long*)B[kCdGeneTab].p;
-    auto* ptab = (unsigned long long*)B[kCdPooledTab].p;
+    unsigned long long *gtab = S.gene_tab.p, *ptab = S.pooled_tab.p;
     const int64_t gene_cells = 64 * (int64_t)q->n_gene;
     if (gene_cells) {
         const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((gene_cells + 7) / 8, big * 4));
