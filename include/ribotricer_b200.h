@@ -308,8 +308,11 @@ int rt_phasescore_values(rt_ctx* ctx, const double* h_values, int64_t n, double*
  */
 typedef struct rt_index rt_index;
 typedef struct rt_tsv rt_tsv;
+typedef struct rt_text rt_text;
 const char* rt_io_last_error(void);
 int rt_index_load(const char* path, rt_index** out);
+/* the same from a text in memory (rt_text below), which the call takes over in every case; `path` names it */
+int rt_index_load_text(rt_text* text, const char* path, rt_index** out);
 void rt_index_free(rt_index* ix);
 int64_t rt_index_n_orf(const rt_index* ix);
 int64_t rt_index_n_exon(const rt_index* ix);
@@ -391,6 +394,7 @@ uint32_t rt_crc32(const uint8_t* p, int64_t n);
  */
 typedef struct rt_gtf rt_gtf;
 int rt_gtf_load(const char* path, rt_gtf** out);
+int rt_gtf_load_text(rt_text* text, const char* path, rt_gtf** out);   /* takes `text` over, like rt_index_load_text */
 void rt_gtf_free(rt_gtf* g);
 int64_t rt_gtf_n_lines(const rt_gtf* g);
 int64_t rt_gtf_n_strings(const rt_gtf* g);
@@ -402,6 +406,7 @@ int rt_gtf_copy(const rt_gtf* g, int64_t* line_no, uint8_t* feature, int32_t* ch
  * codes (A C G T in either case -> 0-3, anything else -> 4).  Nothing is written next to the input. */
 typedef struct rt_fasta rt_fasta;
 int rt_fasta_load(const char* path, rt_fasta** out);
+int rt_fasta_load_text(rt_text* text, const char* path, rt_fasta** out);   /* takes `text` over */
 void rt_fasta_free(rt_fasta* fa);
 int rt_fasta_n_contig(const rt_fasta* fa);
 const char* rt_fasta_contig_name(const rt_fasta* fa, int i);
@@ -491,6 +496,10 @@ typedef struct rt_codon rt_codon;
 int rt_codon_load_tsv(const rt_index* ix, const char* path, int n_features, const char* const* features, int report_all,
                       rt_codon** out);
 int rt_codon_load_seq(rt_codon* h, const rt_index* ix, const char* path);
+/* the same from texts in memory, taken over in every case; `path` names the file in messages */
+int rt_codon_load_tsv_text(const rt_index* ix, rt_text* text, const char* path, int n_features, const char* const* features,
+                           int report_all, rt_codon** out);
+int rt_codon_load_seq_text(rt_codon* h, const rt_index* ix, rt_text* text, const char* path);
 void rt_codon_free(rt_codon* h);
 /* sizes[4]: selected lines, genes, (gene, chrom, strand) groups, data lines of the TSV */
 int rt_codon_sizes(const rt_codon* h, int64_t* sizes);
@@ -537,6 +546,35 @@ typedef struct rt_codon_query {
 } rt_codon_query;
 int rt_codon_counts(rt_ctx* ctx, const rt_codon_query* q, uint64_t* gene_tab, uint64_t* pooled_tab, int64_t* summary,
                     float* stage_ms);
+
+/*
+ * ---- text inputs in memory, and BGZF-compressed text inflated on the GPU (DESIGN.md section 12) -------------------
+ * An rt_text is an owned host buffer of rt_text_len bytes followed by a NUL.  rt_text_alloc makes one of n bytes (content
+ * undefined) for the caller to fill through rt_text_data; every *_load_text loader takes its rt_text over, whatever it
+ * returns, so the caller frees only a text it has not handed to a loader.  Host side; errors in rt_io_last_error.
+ */
+int rt_text_alloc(int64_t n, rt_text** out);
+char* rt_text_data(rt_text* t);
+int64_t rt_text_len(const rt_text* t);
+void rt_text_free(rt_text* t);
+/* rt_bgzf_inflate reads a BGZF file (SAM spec 4.1: a chain of gzip members with a 'BC' extra subfield, each a raw
+ * DEFLATE stream of at most 64 KiB of output; the 28-byte EOF member is optional) and returns its inflated text.  The
+ * host walks the member headers into a block table (payload offset and length, output offset, ISIZE, CRC-32); launches
+ * of bgzf_inflate_kernel, each as many members as the GPU has resident warps and each after the upload of its members,
+ * decode one member per warp (claimed dynamically): stored, fixed
+ * and dynamic Huffman blocks, decode tables built by the warp in shared memory, every read and write bounds-checked
+ * against the member's own ranges, the result checked against ISIZE and the CRC-32 on the device.  The text comes back
+ * in 64 MiB pieces through two page-locked buffers that host threads drain into the rt_text, overlapped with the next
+ * piece's copy and the later launches.  Members the device
+ * refuses are decoded again on the host (rt_inflate.cpp, then zlib).  RT_EINVAL naming the file, the member number and
+ * its byte offset when a member does not parse, is truncated, is followed by bytes that are not a member, or does not
+ * inflate to its ISIZE and CRC-32 on either side.  summary[4] (optional): members, compressed bytes, inflated bytes,
+ * members decoded on the host (also filled when a member fails on both sides).  stage_ms (optional) receives
+ * RT_BGZF_STAGES times: file read, header walk (host clocks); upload (summed), bgzf_inflate_kernel (first launch's start
+ * to last launch's end), copy-back into the page-locked buffers (summed; device events); drain into the rt_text (summed)
+ * and host decode of refused members (host clocks).  Errors in rt_last_error(ctx). */
+#define RT_BGZF_STAGES 7
+int rt_bgzf_inflate(rt_ctx* ctx, const char* path, rt_text** out, int64_t* summary, float* stage_ms);
 
 /* number of kernel launches issued through this ctx so far (bench.py's gpu_launches) */
 int64_t rt_launch_count(const rt_ctx* ctx);

@@ -36,12 +36,15 @@ EXPORTS = (
     "rt_orf_write", "rt_orf_search", "rt_orf_fetch", "rt_index_ids", "rt_orf_seq_write",
     "rt_codon_load_tsv", "rt_codon_load_seq", "rt_codon_free", "rt_codon_sizes", "rt_codon_copy", "rt_codon_gene",
     "rt_codon_text", "rt_codon_write", "rt_codon_counts",
+    "rt_text_alloc", "rt_text_data", "rt_text_len", "rt_text_free", "rt_bgzf_inflate", "rt_index_load_text",
+    "rt_gtf_load_text", "rt_fasta_load_text", "rt_codon_load_tsv_text", "rt_codon_load_seq_text",
 )
 RT_EINVAL = -1
 RT_ORF_STAGES = 7
 RT_SEQ_STAGES = 3
 RT_CODON_STAGES = 7
 RT_CODON_CELL = 5
+RT_BGZF_STAGES = 7
 
 
 class ScoreParams(C.Structure):
@@ -213,6 +216,19 @@ def load():
     lib.rt_codon_text.restype = vp
     lib.rt_codon_write.argtypes = [vp, vp, vp, C.c_char_p, C.c_char_p]
     lib.rt_codon_counts.argtypes = [vp, C.POINTER(CodonQuery), vp, vp, vp, vp]
+    lib.rt_text_alloc.argtypes = [i64, C.POINTER(vp)]
+    lib.rt_text_data.argtypes = [vp]
+    lib.rt_text_data.restype = vp
+    lib.rt_text_len.argtypes = [vp]
+    lib.rt_text_len.restype = i64
+    lib.rt_text_free.argtypes = [vp]
+    lib.rt_text_free.restype = None
+    lib.rt_bgzf_inflate.argtypes = [vp, C.c_char_p, C.POINTER(vp), vp, vp]
+    lib.rt_index_load_text.argtypes = [vp, C.c_char_p, C.POINTER(vp)]
+    lib.rt_gtf_load_text.argtypes = [vp, C.c_char_p, C.POINTER(vp)]
+    lib.rt_fasta_load_text.argtypes = [vp, C.c_char_p, C.POINTER(vp)]
+    lib.rt_codon_load_tsv_text.argtypes = [vp, vp, C.c_char_p, i32, C.POINTER(C.c_char_p), i32, C.POINTER(vp)]
+    lib.rt_codon_load_seq_text.argtypes = [vp, vp, vp, C.c_char_p]
     if lib.rt_abi_version() != 4:
         raise RtError(f"ABI mismatch: library reports {lib.rt_abi_version()}, binding expects 4")
     _lib = lib

@@ -4,8 +4,8 @@
 The flag names, defaults, flag -> argument renames (``--min_read_density`` -> ``min_density_over_orf``,
 ``--stranded yes`` -> ``forward``, ``--meta-min-reads``) and every validation message are those of the
 reference command line (ribotricer/cli.py:127-289, 292-339, 435-560), so existing invocations keep working.
-``prepare-orfs``, ``orfs-seq`` and ``count-orfs-codon`` take the reference's flags (ribotricer/cli.py) and read
-plain-text files only.
+``prepare-orfs``, ``orfs-seq`` and ``count-orfs-codon`` take the reference's flags (ribotricer/cli.py) and read plain-text
+or BGZF files (inflated on the GPU); other gzip files are refused.
 The commands are assembled from option tables below.  ``--bam`` also accepts a ``.npz`` of decoded columns.
 """
 from __future__ import annotations
@@ -21,6 +21,7 @@ from . import const as K
 CONTEXT_SETTINGS = {"help_option_names": ["-h", "--help"]}
 _INDEX_HELP = "Path to the index file of ribotricer\nThis file should be generated using ribotricer prepare-orfs"
 _REPORT_ALL_HELP = "Whether output all ORFs including those non-translating ones"
+_TEXT_INDEX_HELP = _INDEX_HELP + " (plain text or BGZF)"
 
 try:   # colours are cosmetic; the package is absent in some environments
     from click_help_colors import HelpColorsGroup
@@ -84,8 +85,10 @@ def _prepare(gtf, fasta, prefix, min_orf_length, start_codons, stop_codons, long
 
     _need_file(gtf, "GTF file")
     _need_file(fasta, "FASTA file")
+    from .bgzf import sniff
+
     for path, what in ((gtf, "GTF"), (fasta, "FASTA")):
-        if path.endswith((".gz", ".bgz")):
+        if path.endswith((".gz", ".bgz")) and sniff(path) != "bgzf":
             _fail(f"{what} file {path} is compressed; prepare-orfs reads plain text only (decompress it first)")
     if min_orf_length < 0:
         _fail("min_orf_length must be >= 0")
@@ -97,8 +100,8 @@ def _prepare(gtf, fasta, prefix, min_orf_length, start_codons, stop_codons, long
 
 
 _register("prepare-orfs", "Extract candidate ORFs based on GTF and FASTA files", [
-    ("--gtf", dict(help="Path to GTF file", required=True)),
-    ("--fasta", dict(help="Path to FASTA file", required=True)),
+    ("--gtf", dict(help="Path to GTF file (plain text or BGZF)", required=True)),
+    ("--fasta", dict(help="Path to FASTA file (plain text or BGZF)", required=True)),
     ("--prefix", dict(help="Prefix to output file", required=True)),
     ("--min_orf_length", dict(type=int, default=60, show_default=True, help="The minimum length (nts) of ORF to include")),
     ("--start_codons", dict(default="ATG", show_default=True, help="Comma separated list of start codons")),
@@ -248,8 +251,8 @@ def _seq(ribotricer_index, fasta, saveto, protein) -> None:
 
 
 _register("orfs-seq", "Generate sequence for ORFs in ribotricer's index", [
-    ("--ribotricer_index", dict(help=_INDEX_HELP, required=True)),
-    ("--fasta", dict(help="Path to FASTA file", required=True)),
+    ("--ribotricer_index", dict(help=_TEXT_INDEX_HELP, required=True)),
+    ("--fasta", dict(help="Path to FASTA file (plain text or BGZF)", required=True)),
     ("--saveto", dict(help="Path to output file", required=True)),
     ("--protein", dict(is_flag=True, help="Output protein sequence instead of nucleotide sequence")),
 ], _seq)
@@ -270,12 +273,13 @@ def _count_codon(ribotricer_index, detected_orfs, features, ribotricer_index_fas
 
 
 _register("count-orfs-codon", "Count reads for detected ORFs at codon level", [
-    ("--ribotricer_index", dict(help=_INDEX_HELP, required=True)),
+    ("--ribotricer_index", dict(help=_TEXT_INDEX_HELP, required=True)),
     ("--detected_orfs", dict(required=True, help="Path to the detected orfs file\nThis file should be generated "
-                                                 "using ribotricer detect-orfs")),
+                                                 "using ribotricer detect-orfs (plain text or BGZF)")),
     ("--features", dict(help="ORF types separated with comma", required=True)),
     ("--ribotricer_index_fasta", dict(required=True, help="Path to the nucleotide sequence file of the index\nThis "
-                                                          "file should be generated using ribotricer orfs-seq")),
+                                                          "file should be generated using ribotricer orfs-seq (plain "
+                                                          "text or BGZF)")),
     ("--prefix", dict(help="Prefix to output file", required=True)),
     ("--report_all", dict(is_flag=True, help=_REPORT_ALL_HELP)),
 ], _count_codon)

@@ -197,14 +197,22 @@ class CodonInput:
     """The selected rows of a detected-ORFs TSV matched to the index (``rt_codon_load_tsv``) and, after
     ``load_seq``, the checked orfs-seq nucleotide file (``rt_codon_load_seq``).  Rule violations raise ValueError."""
 
-    def __init__(self, idx, detected_orfs: str, features, report_all: bool = False):
+    def __init__(self, idx, detected_orfs, features, report_all: bool = False):
+        from .bgzf import NativeText
+
         self._lib = lib = _lib.load()
         self.idx = idx
         feats = [f.encode() for f in features]
         arr = (C.c_char_p * max(1, len(feats)))(*feats)
         handle = C.c_void_p()
-        if lib.rt_codon_load_tsv(idx.handle, str(detected_orfs).encode(), len(feats), arr, int(bool(report_all)),
-                                 C.byref(handle)) != 0:
+        if isinstance(detected_orfs, NativeText):
+            path = detected_orfs.path.encode()
+            rc = lib.rt_codon_load_tsv_text(idx.handle, detected_orfs.take(), path, len(feats), arr, int(bool(report_all)),
+                                            C.byref(handle))
+        else:
+            rc = lib.rt_codon_load_tsv(idx.handle, str(detected_orfs).encode(), len(feats), arr, int(bool(report_all)),
+                                       C.byref(handle))
+        if rc != 0:
             raise ValueError(lib.rt_io_last_error().decode())
         self.handle = handle
         sizes = np.zeros(4, np.int64)
@@ -222,8 +230,15 @@ class CodonInput:
         self._lib.rt_codon_copy(self.handle, p(s["row"]), p(s["gene"]), p(s["gseq"]), p(s["line"]), p(s["prof_off"]),
                                 p(s["prof_len"]), p(s["seq_off"]))
 
-    def load_seq(self, path: str) -> None:
-        if self._lib.rt_codon_load_seq(self.handle, self.idx.handle, str(path).encode()) != 0:
+    def load_seq(self, src) -> None:
+        """The orfs-seq nucleotide file: a path or a ``bgzf.NativeText``."""
+        from .bgzf import NativeText
+
+        if isinstance(src, NativeText):
+            rc = self._lib.rt_codon_load_seq_text(self.handle, self.idx.handle, src.take(), src.path.encode())
+        else:
+            rc = self._lib.rt_codon_load_seq(self.handle, self.idx.handle, str(src).encode())
+        if rc != 0:
             raise ValueError(self._lib.rt_io_last_error().decode())
         self._copy()
 
@@ -269,8 +284,8 @@ def count_orfs_codon(ribotricer_index, detected_orfs, features, ribotricer_index
     index, a detected-ORFs TSV and the orfs-seq nucleotide file of the same index.  ``features`` is a set of ORF types.
     Every check runs before either file is opened.  ``stage_ms``, when given, receives the time of every stage in
     milliseconds.  Returns a summary dict."""
+    from .bgzf import open_texts
     from .detect_orfs import get_engine
-    from .prepare_orfs import _refuse_gzip
 
     times = {} if stage_ms is None else stage_ms
     clock = time.perf_counter()
@@ -281,13 +296,13 @@ def count_orfs_codon(ribotricer_index, detected_orfs, features, ribotricer_index
         times[name] = (now - clock) * 1e3
         clock = now
 
-    for path in (ribotricer_index, detected_orfs, ribotricer_index_fasta):
-        _refuse_gzip(path, "count-orfs-codon")
-    idx = load_native_index(ribotricer_index)
+    index_src, tsv_src, seq_src = open_texts([ribotricer_index, detected_orfs, ribotricer_index_fasta], "count-orfs-codon")
+    lap("inflate")
+    idx = load_native_index(index_src)
     lap("index_load")
-    inp = CodonInput(idx, detected_orfs, features, report_all)
+    inp = CodonInput(idx, tsv_src, features, report_all)
     lap("tsv_load")
-    inp.load_seq(ribotricer_index_fasta)
+    inp.load_seq(seq_src)
     lap("seq_check")
     dev_ms = np.zeros(_lib.RT_CODON_STAGES, np.float32)
     gene_tab, pooled_tab, summary = get_engine().codon_counts(

@@ -15,6 +15,7 @@
 
 #include <cub/device/device_radix_sort.cuh>
 
+#include "rt_bgzf.h"
 #include "rt_host.h"
 #include "rt_kernels.cuh"
 
@@ -2176,6 +2177,206 @@ int rt_codon_counts(rt_ctx* ctx, const rt_codon_query* q, uint64_t* gene_tab, ui
     RT_CUDA(ctx, cudaStreamSynchronize(S.st));
     if (stage_ms)
         for (int k = 1; k < RT_CODON_STAGES; ++k) RT_CUDA(ctx, cudaEventElapsedTime(&stage_ms[k], S.ev[k - 1], S.ev[k]));
+    return RT_OK;
+}
+
+}  // extern "C"
+
+// -------------------------------------------------------------------------------------------------- BGZF text inputs
+namespace {
+constexpr size_t kInflatePiece = size_t(64) << 20;   // text bytes per page-locked copy-back buffer
+
+// Streams, events and buffers of one rt_bgzf_inflate call; the destructor waits for the streams before the members are
+// freed, so every early return leaves nothing behind.
+struct InflatePipeline {
+    Stream ks, us, cs;                                     // kernels, uploads, copy-back
+    std::unique_ptr<Event[]> up_begin, up_end, k_begin, k_end;   // per kernel launch
+    Event c_begin[2], c_end[2];                            // per page-locked buffer
+    PinnedArr<char> pinned[2];
+    DevArr<uint8_t> comp, text, status;
+    DevArr<rt::BgzfBlock> tab;
+    DevArr<unsigned> claim;                                // one work counter per launch
+    explicit InflatePipeline(size_t n)
+        : up_begin(new Event[n]), up_end(new Event[n]), k_begin(new Event[n]), k_end(new Event[n]) {}
+    ~InflatePipeline() {
+        for (cudaStream_t s : {ks.s, us.s, cs.s})
+            if (s) cudaStreamSynchronize(s);
+    }
+};
+
+float ms_since(std::chrono::steady_clock::time_point t) {
+    return std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t).count();
+}
+
+// The members inflated on the device and the text copied into `out`.  Launches of one member per resident warp (so each
+// fills the GPU) run in order on one stream, each after the upload of its members' payload on another.  The text comes
+// back in pieces of kInflatePiece bytes through two page-locked buffers, each piece as soon as the launches that write
+// it have finished, and host threads drain a piece into `out` while the next piece is copied and later launches run: a
+// single copy into pageable memory runs at the rate one thread faults in the destination's pages.
+// ms[2..5]: upload (summed), kernels (first start to last end), copy-back into the page-locked buffers (summed), drain.
+int inflate_on_device(rt_ctx* ctx, const uint8_t* base, size_t size, const std::vector<rt::BgzfBlock>& tab, size_t total,
+                      char* out, std::vector<uint8_t>& status, float* ms) {
+    const size_t nb = tab.size();
+    DeviceGuard guard(ctx->device);
+    int per_sm = 0;
+    RT_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, rt::bgzf_inflate_kernel, rt::kInflateWarps * 32, 0));
+    const size_t ctas = (size_t)std::max(1, per_sm) * (size_t)std::max(1, ctx->n_sm);
+    const size_t per_launch = ctas * rt::kInflateWarps;
+    const size_t n_launch = (nb + per_launch - 1) / per_launch;
+    InflatePipeline P(n_launch);
+    RT_CUDA(ctx, P.ks.create());
+    RT_CUDA(ctx, P.us.create());
+    RT_CUDA(ctx, P.cs.create());
+    for (size_t c = 0; c < n_launch; ++c)
+        for (Event* e : {&P.up_begin[c], &P.up_end[c], &P.k_begin[c], &P.k_end[c]}) RT_CUDA(ctx, e->create());
+    for (int b = 0; b < 2; ++b) {
+        RT_CUDA(ctx, P.c_begin[b].create());
+        RT_CUDA(ctx, P.c_end[b].create());
+    }
+    RT_CUDA(ctx, P.comp.reserve(size));
+    RT_CUDA(ctx, P.text.reserve(total));
+    RT_CUDA(ctx, P.status.reserve(nb));
+    RT_CUDA(ctx, P.tab.reserve(nb));
+    RT_CUDA(ctx, P.claim.reserve(n_launch));
+    RT_CUDA(ctx, P.tab.upload(tab.data(), nb, P.ks));
+    RT_CUDA(ctx, cudaMemsetAsync(P.claim.p, 0, sizeof(unsigned) * n_launch, P.ks));
+    // 1. uploads and launches, in order
+    std::vector<size_t> launch_out(n_launch);             // first text byte each launch writes
+    for (size_t c = 0; c < n_launch; ++c) {
+        const size_t m0 = c * per_launch, m1 = std::min(nb, m0 + per_launch);
+        const size_t lo = tab[m0].in_off, hi = tab[m1 - 1].in_off + tab[m1 - 1].in_len;
+        launch_out[c] = tab[m0].out_off;
+        RT_CUDA(ctx, cudaEventRecord(P.up_begin[c], P.us));
+        if (hi > lo) RT_CUDA(ctx, cudaMemcpyAsync(P.comp.p + lo, base + lo, hi - lo, cudaMemcpyHostToDevice, P.us));
+        RT_CUDA(ctx, cudaEventRecord(P.up_end[c], P.us));
+        RT_CUDA(ctx, cudaStreamWaitEvent(P.ks, P.up_end[c], 0));
+        RT_CUDA(ctx, cudaEventRecord(P.k_begin[c], P.ks));
+        const unsigned grid = (unsigned)std::min(ctas, (m1 - m0 + rt::kInflateWarps - 1) / rt::kInflateWarps);
+        rt::bgzf_inflate_kernel<<<grid, rt::kInflateWarps * 32, 0, P.ks>>>(P.comp.p, P.tab.p + m0, (long long)(m1 - m0), P.text.p,
+                                                                          P.status.p + m0, P.claim.p + c);
+        ctx->launches++;
+        RT_CUDA(ctx, cudaGetLastError());
+        RT_CUDA(ctx, cudaEventRecord(P.k_end[c], P.ks));
+    }
+    RT_CUDA(ctx, cudaMemcpyAsync(status.data(), P.status.p, nb, cudaMemcpyDeviceToHost, P.ks));
+    // 2. the text, piece by piece: copy-back of piece p overlaps the drain of piece p - 1
+    const size_t n_pieces = (total + kInflatePiece - 1) / kInflatePiece;
+    for (size_t b = 0; b < 2 && b < n_pieces; ++b) RT_CUDA(ctx, P.pinned[b].alloc(std::min(kInflatePiece, total)));
+    auto piece_bytes = [&](size_t p) { return std::min(kInflatePiece, total - p * kInflatePiece); };
+    auto drain = [&](size_t p) -> int {
+        const int b = (int)(p & 1);
+        RT_CUDA(ctx, cudaEventSynchronize(P.c_end[b]));
+        float c_ms = 0.f;
+        RT_CUDA(ctx, cudaEventElapsedTime(&c_ms, P.c_begin[b], P.c_end[b]));
+        ms[4] += c_ms;
+        const auto t = std::chrono::steady_clock::now();
+        const size_t n = piece_bytes(p), slice = size_t(1) << 20, n_slices = (n + slice - 1) / slice;
+        char* dst = out + p * kInflatePiece;
+        const char* src = P.pinned[b].p;
+        claim_parallel(host_threads(n_slices, 64), n_slices, [&](size_t k) {
+            memcpy(dst + k * slice, src + k * slice, std::min(slice, n - k * slice));
+        });
+        ms[5] += ms_since(t);
+        return RT_OK;
+    };
+    for (size_t p = 0; p < n_pieces; ++p) {
+        const int b = (int)(p & 1);                        // buffer b was drained with piece p - 2
+        const size_t hi = p * kInflatePiece + piece_bytes(p);
+        const size_t last = (size_t)(std::upper_bound(launch_out.begin(), launch_out.end(), hi - 1) - launch_out.begin()) - 1;
+        RT_CUDA(ctx, cudaStreamWaitEvent(P.cs, P.k_end[last], 0));
+        RT_CUDA(ctx, cudaEventRecord(P.c_begin[b], P.cs));
+        RT_CUDA(ctx, cudaMemcpyAsync(P.pinned[b].p, P.text.p + p * kInflatePiece, piece_bytes(p), cudaMemcpyDeviceToHost, P.cs));
+        RT_CUDA(ctx, cudaEventRecord(P.c_end[b], P.cs));
+        if (p >= 1)
+            if (const int rc = drain(p - 1)) return rc;
+    }
+    if (n_pieces)
+        if (const int rc = drain(n_pieces - 1)) return rc;
+    RT_CUDA(ctx, cudaStreamSynchronize(P.ks));
+    RT_CUDA(ctx, cudaStreamSynchronize(P.us));
+    for (size_t c = 0; c < n_launch; ++c) {
+        float u = 0.f;
+        RT_CUDA(ctx, cudaEventElapsedTime(&u, P.up_begin[c], P.up_end[c]));
+        ms[2] += u;
+    }
+    RT_CUDA(ctx, cudaEventElapsedTime(&ms[3], P.k_begin[0], P.k_end[n_launch - 1]));
+    return RT_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int rt_bgzf_inflate(rt_ctx* ctx, const char* path, rt_text** out, int64_t* summary, float* stage_ms) {
+    if (!ctx) return fail(nullptr, RT_EINVAL, "rt_bgzf_inflate: ctx is NULL");
+    if (!path || !out) return fail(ctx, RT_EINVAL, "rt_bgzf_inflate: NULL argument");
+    *out = nullptr;
+    float ms[RT_BGZF_STAGES] = {};
+    // 1. the file, read in slices by all threads
+    auto t0 = std::chrono::steady_clock::now();
+    HostArr<char> file;
+    if (const int rc = read_file(path, file)) return fail(ctx, rc, "%s", rt_io_last_error());
+    ms[0] = ms_since(t0);
+    // 2. the member chain: block table and output offsets
+    t0 = std::chrono::steady_clock::now();
+    const uint8_t* base = reinterpret_cast<const uint8_t*>(file.data());
+    const size_t size = file.size();
+    std::vector<rt::BgzfBlock> tab;
+    std::vector<size_t> at;                           // byte offset of every member, for messages
+    unsigned long long total = 0;
+    for (size_t off = 0; off < size;) {
+        Block b;
+        size_t next;
+        const long long k = (long long)tab.size();
+        if (!parse_block(base, size, off, b, next)) {
+            const int why = block_refusal(base, size, off);
+            if (why == 2 && k > 0)
+                return fail(ctx, RT_EINVAL, "%s: BGZF block %lld at byte %zu: %zu bytes after the last member are not a BGZF member",
+                            path, k, off, size - off);
+            if (why == 1) return fail(ctx, RT_EINVAL, "%s: BGZF block %lld at byte %zu: truncated, the file ends inside it", path, k, off);
+            return fail(ctx, RT_EINVAL, "%s: BGZF block %lld at byte %zu: not a BGZF member header", path, k, off);
+        }
+        tab.push_back({(unsigned long long)b.in_off, total, (unsigned)b.in_len, b.out_len, b.crc, 0u});
+        at.push_back(off);
+        total += b.out_len;
+        off = next;
+    }
+    rt_text* raw = nullptr;
+    if (rt_text_alloc((int64_t)total, &raw) != RT_OK)
+        return fail(ctx, RT_ENOMEM, "rt_bgzf_inflate: no host memory for the %llu inflated bytes of %s", total, path);
+    std::unique_ptr<rt_text, void (*)(rt_text*)> text(raw, rt_text_free);
+    ms[1] = ms_since(t0);
+    // 3. device: inflate, copy back
+    const size_t nb = tab.size();
+    std::vector<uint8_t> status(nb, 0);
+    if (nb)
+        if (const int rc = inflate_on_device(ctx, base, size, tab, (size_t)total, text->p, status, ms)) return rc;
+    // 4. members the device refused, decoded again on the host (rt_inflate.cpp, then zlib)
+    t0 = std::chrono::steady_clock::now();
+    std::vector<size_t> redo;
+    for (size_t k = 0; k < nb; ++k)
+        if (status[k] != rt::kInfOk) redo.push_back(k);
+    std::vector<char> ok(redo.size(), 0);
+    claim_parallel(host_threads(redo.size(), SIZE_MAX), redo.size(), [&](size_t j) {
+        const rt::BgzfBlock& b = tab[redo[j]];
+        ok[j] = inflate_block(base + b.in_off, b.in_len, reinterpret_cast<uint8_t*>(text->p) + b.out_off, b.out_len, b.crc, false) &&
+                (b.out_len != 0 || b.crc == 0);
+    });
+    if (summary) {
+        summary[0] = (int64_t)nb;
+        summary[1] = (int64_t)size;
+        summary[2] = (int64_t)total;
+        summary[3] = (int64_t)redo.size();
+    }
+    for (size_t j = 0; j < redo.size(); ++j)
+        if (!ok[j]) {
+            const rt::BgzfBlock& b = tab[redo[j]];
+            return fail(ctx, RT_EINVAL, "%s: BGZF block %zu at byte %zu: does not inflate to its ISIZE of %u bytes and CRC-32 %08x", path,
+                        redo[j], at[redo[j]], b.out_len, b.crc);
+        }
+    ms[6] = ms_since(t0);
+    if (stage_ms)
+        for (int k = 0; k < RT_BGZF_STAGES; ++k) stage_ms[k] = ms[k];
+    *out = text.release();
     return RT_OK;
 }
 

@@ -24,6 +24,12 @@
 
 void rt_io_set_error(const std::string& msg);   // rt_host_io.cpp: the slot rt_io_last_error reads
 
+// The buffer behind an rt_text handle: malloc storage of n bytes and a NUL at p[n] (rt_text_alloc, rt_bgzf_inflate).
+struct rt_text {
+    char* p = nullptr;
+    size_t n = 0;
+};
+
 namespace {
 
 // Plain uninitialised malloc storage: the threads that fill a large array are the first to touch its pages (a
@@ -131,6 +137,14 @@ inline int read_file(const char* path, HostArr<char>& buf) {
     buf.n = size;
     if (!ok) { rt_io_set_error(std::string("short read of ") + path); return RT_EINVAL; }
     return RT_OK;
+}
+
+// The text of `t` moved into `buf` without a copy; `t` itself is freed.  The *_text loaders take their input so.
+inline void adopt_text(rt_text* t, HostArr<char>& buf) {
+    free(buf.p);
+    buf.p = t->p;
+    buf.n = t->n;
+    delete t;
 }
 
 // Boundaries of n chunks of [lo, hi): n + 1 pointers; every chunk but the last ends after a '\n'.

@@ -13,6 +13,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <memory>
+#include <new>
 #include <string>
 #include <string_view>
 #include <unordered_map>
@@ -106,18 +107,34 @@ extern "C" {
 
 const char* rt_io_last_error(void) { return g_io_error.c_str(); }
 
+int rt_text_alloc(int64_t n, rt_text** out) {
+    if (!out || n < 0) return RT_EINVAL;
+    *out = nullptr;
+    std::unique_ptr<rt_text> t(new (std::nothrow) rt_text());
+    if (!t || !(t->p = static_cast<char*>(malloc((size_t)n + 1)))) { g_io_error = "out of memory"; return RT_ENOMEM; }
+    t->n = (size_t)n;
+    t->p[n] = '\0';
+    *out = t.release();
+    return RT_OK;
+}
+
+char* rt_text_data(rt_text* t) { return t ? t->p : nullptr; }
+int64_t rt_text_len(const rt_text* t) { return t ? (int64_t)t->n : 0; }
+
+void rt_text_free(rt_text* t) {
+    if (!t) return;
+    free(t->p);
+    delete t;
+}
+
 }  // extern "C"
 
 void rt_io_set_error(const std::string& msg) { g_io_error = msg; }   // rt_prepare.cpp reports through the same slot
 
 extern "C" {
 
-int rt_index_load(const char* path, rt_index** out) {
-    if (!path || !out) return RT_EINVAL;
-    *out = nullptr;
-    std::unique_ptr<rt_index> ix(new rt_index());
-    // 1. the file, read in slices by all threads
-    if (const int rc = read_file(path, ix->text)) return rc;
+// rt_index_load and rt_index_load_text once ix->text holds the file
+static int index_parse(std::unique_ptr<rt_index> ix, rt_index** out) {
     const size_t size = ix->text.size();
     const char* base = ix->text.data();
     const char* end = base + size;
@@ -276,6 +293,23 @@ int rt_index_load(const char* path, rt_index** out) {
     });
     *out = ix.release();
     return RT_OK;
+}
+
+int rt_index_load(const char* path, rt_index** out) {
+    if (!path || !out) return RT_EINVAL;
+    *out = nullptr;
+    std::unique_ptr<rt_index> ix(new rt_index());
+    // the file, read in slices by all threads
+    if (const int rc = read_file(path, ix->text)) return rc;
+    return index_parse(std::move(ix), out);
+}
+
+int rt_index_load_text(rt_text* text, const char* path, rt_index** out) {
+    if (!text || !path || !out) { rt_text_free(text); return RT_EINVAL; }
+    *out = nullptr;
+    std::unique_ptr<rt_index> ix(new rt_index());
+    adopt_text(text, ix->text);
+    return index_parse(std::move(ix), out);
 }
 
 void rt_index_free(rt_index* ix) { delete ix; }
@@ -947,12 +981,9 @@ void put_codon(TextBuf& b, int c) {
 
 extern "C" {
 
-int rt_codon_load_tsv(const rt_index* ix, const char* path, int n_features, const char* const* features, int report_all,
-                      rt_codon** out) {
-    if (!ix || !path || !out || n_features < 0 || (n_features && !features)) return RT_EINVAL;
-    *out = nullptr;
-    std::unique_ptr<rt_codon> h(new rt_codon());
-    if (const int rc = read_file(path, h->tsv)) return rc;
+// rt_codon_load_tsv and rt_codon_load_tsv_text once h->tsv holds the file; `path` names it in messages
+static int codon_parse_tsv(std::unique_ptr<rt_codon> h, const rt_index* ix, const char* path, int n_features,
+                           const char* const* features, int report_all, rt_codon** out) {
     std::vector<std::string> feats;
     for (int k = 0; k < n_features; ++k) feats.emplace_back(features[k] ? features[k] : "");
     OidTable oids;
@@ -1085,9 +1116,26 @@ int rt_codon_load_tsv(const rt_index* ix, const char* path, int n_features, cons
     return RT_OK;
 }
 
-int rt_codon_load_seq(rt_codon* h, const rt_index* ix, const char* path) {
-    if (!h || !ix || !path) return RT_EINVAL;
-    if (const int rc = read_file(path, h->seq)) return rc;
+int rt_codon_load_tsv(const rt_index* ix, const char* path, int n_features, const char* const* features, int report_all,
+                      rt_codon** out) {
+    if (!ix || !path || !out || n_features < 0 || (n_features && !features)) return RT_EINVAL;
+    *out = nullptr;
+    std::unique_ptr<rt_codon> h(new rt_codon());
+    if (const int rc = read_file(path, h->tsv)) return rc;
+    return codon_parse_tsv(std::move(h), ix, path, n_features, features, report_all, out);
+}
+
+int rt_codon_load_tsv_text(const rt_index* ix, rt_text* text, const char* path, int n_features, const char* const* features,
+                           int report_all, rt_codon** out) {
+    if (!ix || !text || !path || !out || n_features < 0 || (n_features && !features)) { rt_text_free(text); return RT_EINVAL; }
+    *out = nullptr;
+    std::unique_ptr<rt_codon> h(new rt_codon());
+    adopt_text(text, h->tsv);
+    return codon_parse_tsv(std::move(h), ix, path, n_features, features, report_all, out);
+}
+
+// rt_codon_load_seq and rt_codon_load_seq_text once h->seq holds the file; `path` names it in messages
+static int codon_parse_seq(rt_codon* h, const rt_index* ix, const char* path) {
     const char* text = h->seq.data();
     const int64_t size = (int64_t)h->seq.size();
     const int64_t n = (int64_t)ix->orf_chrom.size();
@@ -1171,6 +1219,18 @@ int rt_codon_load_seq(rt_codon* h, const rt_index* ix, const char* path) {
     h->seq_off.resize((size_t)n);
     for (int64_t k = 0; k < n; ++k) h->seq_off[(size_t)k] = line_off[(size_t)k] + (id_off[(size_t)k + 1] - id_off[(size_t)k]) + 1;
     return RT_OK;
+}
+
+int rt_codon_load_seq(rt_codon* h, const rt_index* ix, const char* path) {
+    if (!h || !ix || !path) return RT_EINVAL;
+    if (const int rc = read_file(path, h->seq)) return rc;
+    return codon_parse_seq(h, ix, path);
+}
+
+int rt_codon_load_seq_text(rt_codon* h, const rt_index* ix, rt_text* text, const char* path) {
+    if (!h || !ix || !text || !path) { rt_text_free(text); return RT_EINVAL; }
+    adopt_text(text, h->seq);
+    return codon_parse_seq(h, ix, path);
 }
 
 void rt_codon_free(rt_codon* h) { delete h; }

@@ -2913,4 +2913,371 @@ __global__ void __launch_bounds__(256) codon_stats_kernel(const unsigned long lo
     }
 }
 
+
+// ---------------------------------------------------------------------------------------------------- BGZF inflate
+// bgzf_inflate_kernel (DESIGN.md section 12): one warp per BGZF member, claimed dynamically.  Lane 0 walks the DEFLATE
+// bit stream (RFC 1951) and writes the literals; the back-references it meets go to a queue of kInfQueue entries in
+// shared memory, which the whole warp then copies in order, one byte per lane (a copy that overlaps its own output reads
+// source byte k mod distance).  The Huffman decode tables of every DEFLATE block are built by the warp in shared memory:
+// code lengths counted and ranked with __match_any_sync, then a kInfLitFast-bit (literal/length) or kInfDistFast-bit
+// (distance) lookup table of (symbol << 4 | code length); longer codes take the canonical walk over the per-length counts.
+// Every read stays inside the member's payload and every write inside [out_off, out_off + ISIZE).  Then each lane takes
+// the CRC-32 of a 32nd of the output and the lanes combine theirs by multiplication with x^(8n) mod P (zlib's
+// crc32_combine).  status[b] = kInfOk when member b inflated to exactly ISIZE bytes with the CRC-32 of its footer.
+struct BgzfBlock {
+    unsigned long long in_off, out_off;   // DEFLATE payload in the compressed file; first byte in the text
+    unsigned in_len, out_len, crc, pad;
+};
+
+constexpr int kInflateWarps = 8;
+constexpr int kInfLitFast = 10, kInfDistFast = 8, kInfQueue = 32;
+enum : int { kInfOk = 0, kInfBadBlock = 1, kInfBadCode = 2, kInfBadSymbol = 3, kInfOverrun = 4, kInfSize = 5, kInfCrc = 6 };
+
+__constant__ uint16_t kInfLenBase[29] = {3, 4, 5, 6, 7, 8, 9, 10, 11, 13, 15, 17, 19, 23, 27, 31, 35, 43, 51, 59, 67, 83, 99,
+                                         115, 131, 163, 195, 227, 258};
+__constant__ uint8_t kInfLenExtra[29] = {0, 0, 0, 0, 0, 0, 0, 0, 1, 1, 1, 1, 2, 2, 2, 2, 3, 3, 3, 3, 4, 4, 4, 4, 5, 5, 5, 5, 0};
+__constant__ uint16_t kInfDistBase[30] = {1, 2, 3, 4, 5, 7, 9, 13, 17, 25, 33, 49, 65, 97, 129, 193, 257, 385, 513, 769, 1025,
+                                          1537, 2049, 3073, 4097, 6145, 8193, 12289, 16385, 24577};
+__constant__ uint8_t kInfDistExtra[30] = {0, 0, 0, 0, 1, 1, 2, 2, 3, 3, 4, 4, 5, 5, 6, 6, 7, 7, 8, 8, 9, 9, 10, 10, 11, 11, 12,
+                                          12, 13, 13};
+__constant__ uint8_t kInfClOrder[19] = {16, 17, 18, 0, 8, 7, 9, 6, 10, 5, 11, 4, 12, 3, 13, 2, 14, 1, 15};
+
+struct InflateWarp {                              // the shared memory of one warp
+    uint16_t lit_fast[1 << kInfLitFast];          // (symbol << 4) | code length; 0: a longer code, or none
+    uint16_t dist_fast[1 << kInfDistFast];
+    uint16_t lit_sorted[288], dist_sorted[32];    // symbols in canonical order (code length, then symbol)
+    uint16_t lit_count[16], dist_count[16];       // codes of each length
+    uint16_t run[16], code0[16];                  // table build: next rank of each length; first code minus first rank
+    uint8_t lens[320];                            // code lengths: literal/length 0..287, distance 288..319
+    uint8_t cl_lens[20];                          // the code length code of a dynamic block
+    unsigned q_pos[kInfQueue];                    // back-references waiting for the warp: output offset, length, distance
+    uint16_t q_len[kInfQueue], q_dist[kInfQueue];
+};
+
+// Lane 0's view of the member's bits, least significant first; bytes past the payload read as 0 and are caught by the
+// callers (pos > n + 8 means bits past the end have been consumed).
+struct InflateBits {
+    const uint8_t* in;
+    unsigned n, pos;
+    unsigned long long bb;
+    int bc;
+    __device__ __forceinline__ void refill() {
+        while (bc <= 56) {
+            const unsigned long long b = pos < n ? in[pos] : 0u;
+            ++pos;
+            bb |= b << bc;
+            bc += 8;
+        }
+    }
+    __device__ __forceinline__ unsigned take(int k) {
+        const unsigned v = (unsigned)(bb & ((1ull << k) - 1));
+        bb >>= k;
+        bc -= k;
+        return v;
+    }
+};
+
+// The decode table of one canonical code, built by the whole warp.  false when the lengths over-subscribe the code, or
+// leave it incomplete with a longest code above 1 bit (zlib accepts a lone 1-bit code), or, for the code length code,
+// leave it incomplete at all.
+__device__ bool inflate_build(const uint8_t* lens, int n, int fast_bits, uint16_t* fast, uint16_t* sorted, uint16_t* count,
+                              InflateWarp& w, bool cl_code, int lane) {
+    if (lane < 16) count[lane] = 0;
+    for (int i = lane; i < (1 << fast_bits); i += 32) fast[i] = 0;
+    __syncwarp();
+    for (int c = 0; c < n; c += 32) {
+        const int L = c + lane < n ? lens[c + lane] : 0;
+        const unsigned m = __match_any_sync(kFull, L);
+        if (L && lane == __ffs(m) - 1) count[L] += (uint16_t)__popc(m);
+        __syncwarp();
+    }
+    int left = 1, longest = 0, offs = 0, code = 0;
+    for (int L = 1; L < 16; ++L) {
+        const int k = count[L];
+        left = (left << 1) - k;
+        if (left < 0) return false;
+        if (k) longest = L;
+        if (lane == 0) {
+            w.run[L] = (uint16_t)offs;
+            w.code0[L] = (uint16_t)(code - offs);
+        }
+        offs += k;
+        code = (code + k) << 1;
+    }
+    if (left > 0 && (longest > 1 || cl_code)) return false;
+    __syncwarp();
+    for (int c = 0; c < n; c += 32) {
+        const int s = c + lane;
+        const int L = s < n ? lens[s] : 0;
+        const unsigned m = __match_any_sync(kFull, L);
+        const int idx = w.run[L] + __popc(m & ((1u << lane) - 1u));
+        __syncwarp();
+        if (L) {
+            if (lane == __ffs(m) - 1) w.run[L] += (uint16_t)__popc(m);
+            sorted[idx] = (uint16_t)s;
+            if (L <= fast_bits) {
+                const unsigned rev = __brev((unsigned)(w.code0[L] + idx)) >> (32 - L);
+                for (unsigned k = rev; k < (1u << fast_bits); k += 1u << L) fast[k] = (uint16_t)(s << 4 | L);
+            }
+        }
+        __syncwarp();
+    }
+    return true;
+}
+
+// One symbol (lane 0; at least 15 bits in the buffer): the table entry, else the canonical walk bit by bit.  -1: no code.
+__device__ __forceinline__ int inflate_symbol(InflateBits& br, const uint16_t* fast, int fast_bits, const uint16_t* count,
+                                              const uint16_t* sorted) {
+    const unsigned e = fast[br.bb & ((1u << fast_bits) - 1)];
+    if (e & 15) {
+        br.bb >>= e & 15;
+        br.bc -= (int)(e & 15);
+        return (int)(e >> 4);
+    }
+    int code = 0, first = 0, index = 0;
+    for (int len = 1; len < 16; ++len) {
+        code |= (int)((br.bb >> (len - 1)) & 1);
+        const int k = count[len];
+        if (code - k < first) {
+            br.bb >>= len;
+            br.bc -= len;
+            return sorted[index + (code - first)];
+        }
+        index += k;
+        first = (first + k) << 1;
+        code <<= 1;
+    }
+    return -1;
+}
+
+// The DEFLATE stream of one member into out[0, out_len), by the whole warp; returns the same status in every lane.
+__device__ int inflate_member(InflateWarp& w, const uint8_t* __restrict__ in, unsigned in_len, uint8_t* out,
+                              unsigned out_len, int lane) {
+    InflateBits br{in, in_len, 0u, 0ull, 0};
+    unsigned op = 0;                                  // bytes written; lane 0's count is the one that matters
+    int err = kInfOk, last = 0;
+    while (!last) {
+        int type = 0;
+        if (lane == 0) {
+            br.refill();
+            if (br.pos > in_len + 8) err = kInfOverrun;
+            last = (int)br.take(1);
+            type = (int)br.take(2);
+        }
+        err = __shfl_sync(kFull, err, 0);
+        if (err) return err;
+        type = __shfl_sync(kFull, type, 0);
+        last = __shfl_sync(kFull, last, 0);
+        if (type == 0) {                              // stored: LEN, NLEN, then LEN bytes from the next byte boundary
+            unsigned src = 0, n = 0;
+            if (lane == 0) {
+                br.take(br.bc & 7);
+                src = br.pos - (unsigned)(br.bc >> 3);
+                br.bb = 0;
+                br.bc = 0;
+                if (src + 4 > in_len) {
+                    err = kInfOverrun;
+                } else {
+                    n = in[src] | (unsigned)in[src + 1] << 8;
+                    const unsigned nn = in[src + 2] | (unsigned)in[src + 3] << 8;
+                    if (n != (~nn & 0xffffu)) err = kInfBadBlock;
+                    else if (src + 4 + n > in_len) err = kInfOverrun;
+                    else if (n > out_len - op) err = kInfSize;
+                }
+                br.pos = src + 4 + n;
+            }
+            err = __shfl_sync(kFull, err, 0);
+            if (err) return err;
+            src = __shfl_sync(kFull, src, 0) + 4;
+            n = __shfl_sync(kFull, n, 0);
+            op = __shfl_sync(kFull, op, 0);
+            for (unsigned k = lane; k < n; k += 32) out[op + k] = in[src + k];
+            op += n;
+            continue;
+        }
+        if (type == 3) return kInfBadBlock;
+        if (type == 1) {                              // fixed codes (RFC 1951 3.2.6); symbols 286, 287, 30, 31 are refused
+            for (int i = lane; i < 320; i += 32) w.lens[i] = i < 144 ? 8 : i < 256 ? 9 : i < 280 ? 7 : i < 288 ? 8 : 5;
+            __syncwarp();
+        } else {                                      // dynamic: HLIT, HDIST, HCLEN, the code length code, the lengths
+            int nlit = 0, ndist = 0;
+            for (int i = lane; i < 320; i += 32) w.lens[i] = 0;
+            if (lane == 0) {
+                br.refill();
+                nlit = (int)br.take(5) + 257;
+                ndist = (int)br.take(5) + 1;
+                const int ncl = (int)br.take(4) + 4;
+                for (int i = 0; i < 19; ++i) {
+                    if (br.bc < 3) br.refill();
+                    w.cl_lens[kInfClOrder[i]] = (uint8_t)(i < ncl ? br.take(3) : 0);
+                }
+                if (nlit > 286 || ndist > 30) err = kInfBadBlock;
+            }
+            err = __shfl_sync(kFull, err, 0);
+            if (err) return err;
+            __syncwarp();
+            if (!inflate_build(w.cl_lens, 19, 7, w.lit_fast, w.dist_sorted, w.dist_count, w, true, lane)) return kInfBadCode;
+            if (lane == 0) {
+                const int total = nlit + ndist;
+                int prev = -1;
+                for (int i = 0; i < total;) {
+                    if (br.bc < 16) {
+                        br.refill();
+                        if (br.pos > in_len + 8) { err = kInfOverrun; break; }
+                    }
+                    const int sym = inflate_symbol(br, w.lit_fast, 7, w.dist_count, w.dist_sorted);
+                    int len = 0, rep = 1;
+                    if (sym < 0) { err = kInfBadSymbol; break; }
+                    if (sym < 16) {
+                        len = sym;
+                    } else if (sym == 16) {
+                        if (prev < 0) { err = kInfBadBlock; break; }
+                        len = prev;
+                        rep = 3 + (int)br.take(2);
+                    } else {
+                        rep = sym == 17 ? 3 + (int)br.take(3) : 11 + (int)br.take(7);
+                    }
+                    if (rep > total - i) { err = kInfBadBlock; break; }
+                    prev = len;
+                    for (; rep > 0; --rep, ++i) w.lens[i < nlit ? i : 288 + i - nlit] = (uint8_t)len;
+                }
+                if (!err && w.lens[256] == 0) err = kInfBadCode;   // no end-of-block code
+            }
+            err = __shfl_sync(kFull, err, 0);
+            if (err) return err;
+            __syncwarp();
+        }
+        if (!inflate_build(w.lens, 288, kInfLitFast, w.lit_fast, w.lit_sorted, w.lit_count, w, false, lane)) return kInfBadCode;
+        if (!inflate_build(w.lens + 288, 32, kInfDistFast, w.dist_fast, w.dist_sorted, w.dist_count, w, false, lane))
+            return kInfBadCode;
+        for (;;) {                                    // batches: lane 0 decodes up to kInfQueue back-references, the warp copies
+            int nq = 0, eob = 0;
+            if (lane == 0) {
+                while (nq < kInfQueue) {
+                    if (br.bc < 48) {                 // a length and a distance with their extra bits take at most 48
+                        br.refill();
+                        if (br.pos > in_len + 8) { err = kInfOverrun; break; }
+                    }
+                    int sym = inflate_symbol(br, w.lit_fast, kInfLitFast, w.lit_count, w.lit_sorted);
+                    if (sym < 256) {
+                        if (sym < 0) { err = kInfBadSymbol; break; }
+                        if (op >= out_len) { err = kInfSize; break; }
+                        out[op++] = (uint8_t)sym;
+                        continue;
+                    }
+                    if (sym == 256) { eob = 1; break; }
+                    sym -= 257;
+                    if (sym >= 29) { err = kInfBadSymbol; break; }
+                    const unsigned len = kInfLenBase[sym] + br.take(kInfLenExtra[sym]);
+                    const int ds = inflate_symbol(br, w.dist_fast, kInfDistFast, w.dist_count, w.dist_sorted);
+                    if (ds < 0 || ds >= 30) { err = kInfBadSymbol; break; }
+                    const unsigned dist = kInfDistBase[ds] + br.take(kInfDistExtra[ds]);
+                    if (dist > op) { err = kInfBadSymbol; break; }
+                    if (len > out_len - op) { err = kInfSize; break; }
+                    w.q_pos[nq] = op;
+                    w.q_len[nq] = (uint16_t)len;
+                    w.q_dist[nq] = (uint16_t)dist;
+                    ++nq;
+                    op += len;
+                }
+            }
+            err = __shfl_sync(kFull, err, 0);
+            if (err) return err;
+            nq = __shfl_sync(kFull, nq, 0);
+            eob = __shfl_sync(kFull, eob, 0);
+            __syncwarp();
+            for (int q = 0; q < nq; ++q) {
+                const unsigned len = w.q_len[q], dist = w.q_dist[q];
+                uint8_t* dst = out + w.q_pos[q];
+                const uint8_t* src = dst - dist;
+                if (dist >= len) {
+                    for (unsigned k = lane; k < len; k += 32) dst[k] = src[k];
+                } else {
+                    unsigned s = (unsigned)lane % dist;
+                    const unsigned step = 32u % dist;
+                    for (unsigned k = lane; k < len; k += 32) {
+                        dst[k] = src[s];
+                        s += step;
+                        if (s >= dist) s -= dist;
+                    }
+                }
+                __syncwarp();
+            }
+            if (eob) break;
+        }
+    }
+    if (lane == 0) {
+        if ((unsigned long long)br.pos * 8 - (unsigned long long)br.bc > (unsigned long long)in_len * 8) err = kInfOverrun;
+        else if (op != out_len) err = kInfSize;
+    }
+    return __shfl_sync(kFull, err, 0);
+}
+
+// a * b mod P over GF(2), bit-reflected (zlib's multmodp)
+__device__ __forceinline__ unsigned crc_multmodp(unsigned a, unsigned b) {
+    unsigned p = 0;
+    for (unsigned m = 1u << 31; m; m >>= 1) {
+        if (a & m) p ^= b;
+        b = b & 1 ? (b >> 1) ^ 0xedb88320u : b >> 1;
+    }
+    return p;
+}
+
+// x^(8n) mod P from x2n[k] = x^(2^k) mod P
+__device__ __forceinline__ unsigned crc_x8n(unsigned n, const unsigned* x2n) {
+    unsigned p = 1u << 31;
+    for (int k = 3; n; n >>= 1, ++k)
+        if (n & 1) p = crc_multmodp(x2n[k & 31], p);
+    return p;
+}
+
+__global__ void __launch_bounds__(kInflateWarps * 32) bgzf_inflate_kernel(const uint8_t* __restrict__ comp,
+                                                                          const BgzfBlock* __restrict__ blocks,
+                                                                          long long n_blocks, uint8_t* text,
+                                                                          uint8_t* __restrict__ status, unsigned* claim) {
+    __shared__ InflateWarp warps[kInflateWarps];
+    __shared__ unsigned crc_tab[256], x2n[32];
+    for (int i = threadIdx.x; i < 256; i += blockDim.x) {
+        unsigned c = (unsigned)i;
+        for (int k = 0; k < 8; ++k) c = c & 1 ? (c >> 1) ^ 0xedb88320u : c >> 1;
+        crc_tab[i] = c;
+    }
+    if (threadIdx.x == 0) {
+        unsigned p = 1u << 30;                        // x^1
+        for (int k = 0; k < 32; ++k) {
+            x2n[k] = p;
+            p = crc_multmodp(p, p);
+        }
+    }
+    __syncthreads();
+    InflateWarp& w = warps[threadIdx.x >> 5];
+    const int lane = threadIdx.x & 31;
+    for (;;) {
+        unsigned t = 0;
+        if (lane == 0) t = atomicAdd(claim, 1u);
+        t = __shfl_sync(kFull, t, 0);
+        if ((long long)t >= n_blocks) return;
+        const BgzfBlock B = blocks[t];
+        uint8_t* out = text + B.out_off;
+        int err = inflate_member(w, comp + B.in_off, B.in_len, out, B.out_len, lane);
+        if (err == kInfOk) {
+            __syncwarp();
+            const unsigned L = B.out_len, S = (L + 31) >> 5;
+            const unsigned lo = min(lane * S, L), hi = min(lo + S, L);
+            unsigned c = ~0u;
+            for (unsigned k = lo; k < hi; ++k) c = crc_tab[(c ^ out[k]) & 255u] ^ (c >> 8);
+            c = ~c;
+            for (int d = 1; d < 32; d <<= 1) {
+                const unsigned other = __shfl_down_sync(kFull, c, d);
+                if ((lane & (2 * d - 1)) == 0) {
+                    const unsigned b0 = min((lane + d) * S, L), b1 = min((lane + 2 * d) * S, L);
+                    c = crc_multmodp(crc_x8n(b1 - b0, x2n), c) ^ other;
+                }
+            }
+            if (__shfl_sync(kFull, c, 0) != B.crc) err = kInfCrc;
+        }
+        if (lane == 0) status[t] = (uint8_t)err;
+    }
+}
+
 }  // namespace rt

@@ -134,11 +134,8 @@ void parse_gtf_chunk(GtfChunk& ck) {
 
 extern "C" {
 
-int rt_gtf_load(const char* path, rt_gtf** out) {
-    if (!path || !out) return RT_EINVAL;
-    *out = nullptr;
-    HostArr<char> text;
-    if (const int rc = read_file(path, text)) return rc;
+// rt_gtf_load and rt_gtf_load_text once `text` holds the file
+static int gtf_parse(const HostArr<char>& text, rt_gtf** out) {
     const int n_thr = host_threads(text.size() >> 20, 32, "RT_GTF_THREADS");
     const char* base = text.data();
     std::vector<const char*> cut = cut_lines(base, base + text.size(), n_thr);
@@ -203,6 +200,22 @@ int rt_gtf_load(const char* path, rt_gtf** out) {
     return RT_OK;
 }
 
+int rt_gtf_load(const char* path, rt_gtf** out) {
+    if (!path || !out) return RT_EINVAL;
+    *out = nullptr;
+    HostArr<char> text;
+    if (const int rc = read_file(path, text)) return rc;
+    return gtf_parse(text, out);
+}
+
+int rt_gtf_load_text(rt_text* text, const char* path, rt_gtf** out) {
+    if (!text || !path || !out) { rt_text_free(text); return RT_EINVAL; }
+    *out = nullptr;
+    HostArr<char> buf;
+    adopt_text(text, buf);
+    return gtf_parse(buf, out);
+}
+
 void rt_gtf_free(rt_gtf* g) { delete g; }
 int64_t rt_gtf_n_lines(const rt_gtf* g) { return g ? (int64_t)g->line_no.size() : 0; }
 int64_t rt_gtf_n_strings(const rt_gtf* g) { return g ? g->n_strings : 0; }
@@ -238,11 +251,8 @@ struct rt_fasta {
 
 extern "C" {
 
-int rt_fasta_load(const char* path, rt_fasta** out) {
-    if (!path || !out) return RT_EINVAL;
-    *out = nullptr;
-    std::unique_ptr<rt_fasta> fa(new rt_fasta());
-    if (const int rc = read_file(path, fa->text)) return rc;
+// rt_fasta_load and rt_fasta_load_text once fa->text holds the file
+static int fasta_parse(std::unique_ptr<rt_fasta> fa, rt_fasta** out) {
     const char* base = fa->text.data();
     const size_t size = fa->text.size();
     fa->n_thr = host_threads(size >> 20, 32, "RT_FASTA_THREADS");
@@ -298,6 +308,22 @@ int rt_fasta_load(const char* path, rt_fasta** out) {
     }
     *out = fa.release();
     return RT_OK;
+}
+
+int rt_fasta_load(const char* path, rt_fasta** out) {
+    if (!path || !out) return RT_EINVAL;
+    *out = nullptr;
+    std::unique_ptr<rt_fasta> fa(new rt_fasta());
+    if (const int rc = read_file(path, fa->text)) return rc;
+    return fasta_parse(std::move(fa), out);
+}
+
+int rt_fasta_load_text(rt_text* text, const char* path, rt_fasta** out) {
+    if (!text || !path || !out) { rt_text_free(text); return RT_EINVAL; }
+    *out = nullptr;
+    std::unique_ptr<rt_fasta> fa(new rt_fasta());
+    adopt_text(text, fa->text);
+    return fasta_parse(std::move(fa), out);
 }
 
 void rt_fasta_free(rt_fasta* fa) { delete fa; }

@@ -528,3 +528,26 @@ class Engine:
         if stage_ms is not None:
             stage_ms[:] = ms
         return gene_tab, pooled_tab, summary
+
+    # --------------------------------------------------------------- BGZF text inputs
+    def inflate_bgzf(self, path: str, summary: np.ndarray | None = None, stage_ms: np.ndarray | None = None):
+        """The inflated text of a BGZF file (``rt_bgzf_inflate``: bgzf_inflate_kernel, members the device refuses
+        decoded again on the host) as a ``bgzf.NativeText``.  A file that is not a clean chain of BGZF members, or a
+        member that does not inflate to its ISIZE and CRC-32, raises ValueError naming the member and its byte offset.
+        ``summary`` (4) receives members, compressed bytes, inflated bytes, members decoded on the host (also when
+        the call raises); ``stage_ms``
+        (``RT_BGZF_STAGES``) the stage times of the header."""
+        from .bgzf import NativeText
+
+        h = C.c_void_p()
+        sm = np.zeros(4, np.int64)
+        ms = np.zeros(_lib.RT_BGZF_STAGES, np.float32)
+        rc = self.lib.rt_bgzf_inflate(self.ctx, str(path).encode(), C.byref(h), _np_ptr(sm), _np_ptr(ms))
+        if summary is not None:
+            summary[:] = sm
+        if rc == _lib.RT_EINVAL:
+            raise ValueError(self.lib.rt_last_error(self.ctx).decode())
+        self._check(rc)
+        if stage_ms is not None:
+            stage_ms[:] = ms
+        return NativeText(h, str(path))

@@ -149,16 +149,23 @@ class _RowView:
 
 
 class NativeIndex:
-    """The whole index in columns, parsed by ``rt_index_load``.  Duck-types ``PackedIndex``."""
+    """The whole index in columns, parsed by ``rt_index_load``.  Duck-types ``PackedIndex``.  ``src`` is a path or a
+    ``bgzf.NativeText`` (``rt_index_load_text``)."""
 
-    def __init__(self, path: str):
+    def __init__(self, src):
         import ctypes as C
 
         from . import _lib
+        from .bgzf import NativeText
 
         self._lib = lib = _lib.load()
         handle = C.c_void_p()
-        rc = lib.rt_index_load(path.encode(), C.byref(handle))
+        if isinstance(src, NativeText):
+            path = src.path
+            rc = lib.rt_index_load_text(src.take(), path.encode(), C.byref(handle))
+        else:
+            path = src
+            rc = lib.rt_index_load(path.encode(), C.byref(handle))
         if rc != 0:
             msg = lib.rt_io_last_error().decode()
             if msg.startswith("Error: unexpected number of columns"):
@@ -236,5 +243,5 @@ class NativeIndex:
                     orf_contig=np.ascontiguousarray(contig, np.int32), orf_strand=self.orf_strand_code)
 
 
-def load_native_index(path: str) -> NativeIndex:
-    return NativeIndex(path)
+def load_native_index(src) -> NativeIndex:
+    return NativeIndex(src)

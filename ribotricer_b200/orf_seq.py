@@ -6,7 +6,8 @@
                    overlapped with the next chunk's kernel, a writer thread
 
 The rules are those of DESIGN.md section 10.  Same name and argument order as the reference's ``orf_seq``
-(orf_seq.py:128-179).  Inputs are plain text; gzipped files are refused.
+(orf_seq.py:128-179).  Inputs are plain text or BGZF (inflated on the GPU, ``bgzf.open_texts``); other gzip files are
+refused.
 """
 from __future__ import annotations
 
@@ -17,8 +18,9 @@ import time
 import numpy as np
 
 from . import _lib
+from .bgzf import open_texts
 from .index import load_native_index
-from .prepare_orfs import Genome, _refuse_gzip
+from .prepare_orfs import Genome
 
 
 def orf_seq(ribotricer_index, genome_fasta, saveto, translate=False, chunk_bytes: int = 0,
@@ -36,12 +38,12 @@ def orf_seq(ribotricer_index, genome_fasta, saveto, translate=False, chunk_bytes
         times[name] = (now - clock) * 1e3
         clock = now
 
-    _refuse_gzip(ribotricer_index, "orfs-seq")
-    _refuse_gzip(genome_fasta, "orfs-seq")
-    idx = load_native_index(ribotricer_index)
+    index_src, fasta_src = open_texts([ribotricer_index, genome_fasta], "orfs-seq")
+    lap("inflate")
+    idx = load_native_index(index_src)
     id_off, ids = idx.ids()
     lap("index_load")
-    genome = Genome(genome_fasta)
+    genome = Genome(fasta_src)
     lap("fasta_load")
     lut = {name: i for i, name in enumerate(genome.names)}
     table = np.array([lut.get(c, -1) for c in idx.chrom_names], np.int64)

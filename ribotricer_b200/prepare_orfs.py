@@ -7,7 +7,8 @@
     index file          rt_orf_write (all cores, write-behind)
 
 The rules are those of DESIGN.md section 9.  Same name and argument order as the reference's ``prepare_orfs``
-(prepare_orfs.py:278).  Inputs are plain text; gzipped files are refused.
+(prepare_orfs.py:278).  Inputs are plain text or BGZF (inflated on the GPU, ``bgzf.open_texts``); other gzip files are
+refused.
 """
 from __future__ import annotations
 
@@ -18,6 +19,7 @@ import pathlib
 import numpy as np
 
 from . import _lib
+from .bgzf import NativeText, open_text, open_texts
 
 TYPES = ("annotated", "uORF", "overlap_uORF", "super_uORF", "overlap_dORF", "dORF", "novel", "internal")
 BASES = "ACGT"
@@ -38,12 +40,6 @@ def codon_mask(codons) -> int:
     return mask
 
 
-def _refuse_gzip(path: str, command: str = "prepare-orfs") -> None:
-    with open(path, "rb") as fh:
-        if fh.read(2) == b"\x1f\x8b":
-            raise ValueError(f"{path} is gzip-compressed; {command} reads plain text only")
-
-
 def _np_ptr(a: np.ndarray):
     return a.ctypes.data_as(C.c_void_p)
 
@@ -53,13 +49,21 @@ def _io_error(what: str):
 
 
 class Genome:
-    """A FASTA indexed by ``rt_fasta_load``; ``codes`` translates contigs to 1-byte codes on demand."""
+    """A FASTA indexed by ``rt_fasta_load``; ``codes`` translates contigs to 1-byte codes on demand.  ``src`` is a path
+    (plain text or BGZF) or a ``NativeText``."""
 
-    def __init__(self, path: str):
-        _refuse_gzip(path)
+    def __init__(self, src):
+        self.handle = None
+        src = open_text(src, "prepare-orfs") if isinstance(src, str) else src
         self._lib = lib = _lib.load()
         h = C.c_void_p()
-        if lib.rt_fasta_load(path.encode(), C.byref(h)) != 0:
+        if isinstance(src, NativeText):
+            path = src.path
+            rc = lib.rt_fasta_load_text(src.take(), path.encode(), C.byref(h))
+        else:
+            path = src
+            rc = lib.rt_fasta_load(path.encode(), C.byref(h))
+        if rc != 0:
             raise _io_error(f"cannot load FASTA {path}")
         self.handle = h
         n = lib.rt_fasta_n_contig(h)
@@ -82,13 +86,20 @@ class Genome:
     __del__ = close
 
 
-def load_gtf(path: str) -> dict:
+def load_gtf(src) -> dict:
     """The exon and CDS lines of a GTF (``rt_gtf_load``) as columns; ``attr`` holds 5 string ids per line (gene_id,
-    transcript_id, gene_name, gene_type, transcript_type with their fallbacks; -1 absent) into ``strings``."""
-    _refuse_gzip(path)
+    transcript_id, gene_name, gene_type, transcript_type with their fallbacks; -1 absent) into ``strings``.  ``src`` is
+    a path (plain text or BGZF) or a ``NativeText``."""
+    src = open_text(src, "prepare-orfs") if isinstance(src, str) else src
     lib = _lib.load()
     h = C.c_void_p()
-    if lib.rt_gtf_load(path.encode(), C.byref(h)) != 0:
+    if isinstance(src, NativeText):
+        path = src.path
+        rc = lib.rt_gtf_load_text(src.take(), path.encode(), C.byref(h))
+    else:
+        path = src
+        rc = lib.rt_gtf_load(path.encode(), C.byref(h))
+    if rc != 0:
         raise _io_error(f"cannot load GTF {path}")
     try:
         n = int(lib.rt_gtf_n_lines(h))
@@ -283,9 +294,11 @@ def prepare_orfs(gtf, fasta, prefix, min_orf_length=60, start_codons={"ATG"}, st
         times[name] = (now - clock) * 1e3
         clock = now
 
-    genome = Genome(fasta)
+    fasta_src, gtf_src = open_texts([fasta, gtf], "prepare-orfs")
+    lap("inflate")
+    genome = Genome(fasta_src)
     lap("fasta_load")
-    g = load_gtf(gtf)
+    g = load_gtf(gtf_src)
     lap("gtf_load")
     tx = build_transcripts(g, genome)
     used = np.unique(tx["contig"]).astype(np.int32)
