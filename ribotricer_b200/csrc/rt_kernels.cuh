@@ -470,7 +470,8 @@ constexpr int kUvCenter = (kUvMax - 1) * kUvStride + (kUvMax - 1);
 // ulp is 2^-42).  Sums of up to 1,024 such values are EXACT in fp64 (every partial sum is a multiple of 2^-42 below
 // 2^10), so the per-atom sums do not depend on the order of summation: any lane / tile / layout decomposition of
 // phase A gives bit-identical summaries, and phase B adds them as 64-bit integers (units of 2^-42).  The rounding
-// moves a score by less than 2^-43 (the sums are divided by the number of codons).
+// moves a unit vector by at most 2^-42 (2^-43 in A / n, sqrt(3) * 2^-43 in the sqrt(3) B / n it stands for), so a score
+// |sum u| / sqrt(K * M) (M non-uniform codons) moves by at most M * 2^-42 / sqrt(K * M) <= 2^-42.
 constexpr double kUvGridMagic = 1536.0;
 constexpr double kUvGridScale = 4398046511104.0;      // 2^42
 __device__ __forceinline__ double2 uv_grid(double A, double B) {     // (A, B) != (0, 0); |A|, |B| < 2^22: D is exact
