@@ -548,6 +548,36 @@ int rt_codon_counts(rt_ctx* ctx, const rt_codon_query* q, uint64_t* gene_tab, ui
                     float* stage_ms);
 
 /*
+ * ---- count-orfs: per-gene read counts of detected ORFs from the TSV text (DESIGN.md section 13) --------------------
+ * The selected lines come from rt_codon_load_tsv (rt_codon_copy: row, gene, prof_off, prof_len; rt_codon_text: tsv).
+ * rt_count_orfs gathers their profile text on all cores and uploads it with the index intervals.  count_emit_kernel
+ * (one warp per line, claimed dynamically) checks every profile and gives oriented nt k < m = min(values, row length)
+ * of the line the key gene << 32 | genomic coordinate and the value; a stable radix sort on the key and
+ * count_keep_kernel keep the first slot of every key, in (line, oriented nt) order, and sum per gene.
+ * total[n_gene] and length[n_gene]: per gene, the sum of the kept values and the number of distinct coordinates.
+ * summary[4]: positions named (sum of m), positions kept, the first selected line whose profile is refused (-1: none)
+ * and its reasons (1 malformed, 2 a value above 2^31 - 1); when a line is refused the counts are not computed.  At most
+ * 2^32 - 1 nt in the selected rows.  stage_ms (optional) receives RT_COUNT_STAGES times: host gather (host clock),
+ * upload, count_emit_kernel, sort, count_keep_kernel, copy-back. */
+#define RT_COUNT_STAGES 6
+typedef struct rt_count_query {
+    int64_t n_sel;
+    const int64_t* row;             /* index row of each selected TSV line */
+    const int32_t* gene;            /* gene id, < n_gene */
+    const int64_t* prof_off;        /* profile field of each in `tsv` */
+    const int64_t* prof_len;
+    const char* tsv;
+    int64_t n_orf;
+    const int64_t* exon_ptr;        /* n_orf + 1 */
+    const int32_t* exon_start;      /* 1-based closed, ascending within a row */
+    const int32_t* exon_end;
+    const uint8_t* orf_strand;      /* 1 reverse, anything else forward */
+    int32_t n_gene;
+} rt_count_query;
+int rt_count_orfs(rt_ctx* ctx, const rt_count_query* q, uint64_t* total, uint64_t* length, int64_t* summary,
+                  float* stage_ms);
+
+/*
  * ---- text inputs in memory, and BGZF-compressed text inflated on the GPU (DESIGN.md section 12) -------------------
  * An rt_text is an owned host buffer of rt_text_len bytes followed by a NUL.  rt_text_alloc makes one of n bytes (content
  * undefined) for the caller to fill through rt_text_data; every *_load_text loader takes its rt_text over, whatever it

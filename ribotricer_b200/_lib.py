@@ -37,7 +37,7 @@ EXPORTS = (
     "rt_codon_load_tsv", "rt_codon_load_seq", "rt_codon_free", "rt_codon_sizes", "rt_codon_copy", "rt_codon_gene",
     "rt_codon_text", "rt_codon_write", "rt_codon_counts",
     "rt_text_alloc", "rt_text_data", "rt_text_len", "rt_text_free", "rt_bgzf_inflate", "rt_index_load_text",
-    "rt_gtf_load_text", "rt_fasta_load_text", "rt_codon_load_tsv_text", "rt_codon_load_seq_text",
+    "rt_gtf_load_text", "rt_fasta_load_text", "rt_codon_load_tsv_text", "rt_codon_load_seq_text", "rt_count_orfs",
 )
 RT_EINVAL = -1
 RT_ORF_STAGES = 7
@@ -45,6 +45,7 @@ RT_SEQ_STAGES = 3
 RT_CODON_STAGES = 7
 RT_CODON_CELL = 5
 RT_BGZF_STAGES = 7
+RT_COUNT_STAGES = 6
 
 
 class ScoreParams(C.Structure):
@@ -78,6 +79,12 @@ class CodonQuery(C.Structure):
                 ("prof_off", C.c_void_p), ("prof_len", C.c_void_p), ("tsv", C.c_void_p), ("seq_off", C.c_void_p),
                 ("seq", C.c_void_p), ("n_orf", C.c_int64), ("exon_ptr", C.c_void_p), ("exon_start", C.c_void_p),
                 ("exon_end", C.c_void_p), ("orf_strand", C.c_void_p), ("n_gene", C.c_int32), ("n_gseq", C.c_int32)]
+
+
+class CountQuery(C.Structure):
+    _fields_ = [("n_sel", C.c_int64), ("row", C.c_void_p), ("gene", C.c_void_p), ("prof_off", C.c_void_p),
+                ("prof_len", C.c_void_p), ("tsv", C.c_void_p), ("n_orf", C.c_int64), ("exon_ptr", C.c_void_p),
+                ("exon_start", C.c_void_p), ("exon_end", C.c_void_p), ("orf_strand", C.c_void_p), ("n_gene", C.c_int32)]
 
 
 class RtError(RuntimeError):
@@ -229,6 +236,7 @@ def load():
     lib.rt_fasta_load_text.argtypes = [vp, C.c_char_p, C.POINTER(vp)]
     lib.rt_codon_load_tsv_text.argtypes = [vp, vp, C.c_char_p, i32, C.POINTER(C.c_char_p), i32, C.POINTER(vp)]
     lib.rt_codon_load_seq_text.argtypes = [vp, vp, vp, C.c_char_p]
+    lib.rt_count_orfs.argtypes = [vp, C.POINTER(CountQuery), vp, vp, vp, vp]
     if lib.rt_abi_version() != 4:
         raise RtError(f"ABI mismatch: library reports {lib.rt_abi_version()}, binding expects 4")
     _lib = lib

@@ -1,4 +1,5 @@
-"""Text inputs of ``prepare-orfs``, ``orfs-seq`` and ``count-orfs-codon``: plain text, or BGZF inflated on the GPU.
+"""Text inputs of ``prepare-orfs``, ``orfs-seq``, ``count-orfs`` and ``count-orfs-codon``: plain text, or BGZF
+inflated on the GPU.
 
 ``open_texts(paths, command)`` looks at the first bytes of every input (DESIGN.md section 12):
 

@@ -4,8 +4,8 @@
 The flag names, defaults, flag -> argument renames (``--min_read_density`` -> ``min_density_over_orf``,
 ``--stranded yes`` -> ``forward``, ``--meta-min-reads``) and every validation message are those of the
 reference command line (ribotricer/cli.py:127-289, 292-339, 435-560), so existing invocations keep working.
-``prepare-orfs``, ``orfs-seq`` and ``count-orfs-codon`` take the reference's flags (ribotricer/cli.py) and read plain-text
-or BGZF files (inflated on the GPU); other gzip files are refused.
+``prepare-orfs``, ``orfs-seq``, ``count-orfs`` and ``count-orfs-codon`` take the reference's flags (ribotricer/cli.py)
+and read plain-text or BGZF files (inflated on the GPU); other gzip files are refused.
 The commands are assembled from option tables below.  ``--bam`` also accepts a ``.npz`` of decoded columns.
 """
 from __future__ import annotations
@@ -34,7 +34,7 @@ except ImportError:
 @click.version_option(version=__version__)
 def cli() -> None:
     """ribotricer: Tool for detecting translating ORF from Ribo-seq data (B200-native prepare-orfs, detect-orfs,
-    orfs-seq and count-orfs-codon)"""
+    count-orfs, orfs-seq and count-orfs-codon)"""
 
 
 def _register(name: str, summary: str, options, handler) -> None:
@@ -172,17 +172,21 @@ _register("detect-orfs", "Detect translating ORFs from BAM file", [
 
 # ------------------------------------------------------------------------------------ count-orfs
 def _count(ribotricer_index, detected_orfs, features, out, report_all) -> None:
-    from .count_orfs import count_orfs
+    from .count_orfs import count_orfs_gpu
 
     _need_file(ribotricer_index, "ribotricer index file")
     _need_file(detected_orfs, "detected orfs file")
-    count_orfs(ribotricer_index, detected_orfs, {item.strip() for item in features.strip().split(",")}, out, report_all)
+    try:
+        count_orfs_gpu(ribotricer_index, detected_orfs, {item.strip() for item in features.strip().split(",")}, out,
+                       report_all)
+    except ValueError as exc:
+        _fail(str(exc))
 
 
 _register("count-orfs", "Count reads for detected ORFs at gene level", [
-    ("--ribotricer_index", dict(help=_INDEX_HELP, required=True)),
+    ("--ribotricer_index", dict(help=_TEXT_INDEX_HELP, required=True)),
     ("--detected_orfs", dict(required=True, help="Path to the detected orfs file\nThis file should be generated "
-                                                 "using ribotricer detect-orfs")),
+                                                 "using ribotricer detect-orfs (plain text or BGZF)")),
     ("--features", dict(help="ORF types separated with comma", required=True)),
     ("--out", dict(help="Path to output file", required=True)),
     ("--report_all", dict(is_flag=True, help=_REPORT_ALL_HELP)),

@@ -8,7 +8,15 @@ points give the same table:
 * ``count_orfs_device``  works on what ``detect_orfs`` already holds in HBM -- the dense P-site planes, the
   packed index and the status column -- so no profile is ever turned into text: the union intervals of every
   gene are merged on the host (a sort over exon intervals) and summed by ``rt_interval_sums``;
-* ``count_orfs``         keeps the reference's signature (index path, TSV path) for existing pipelines.
+* ``count_orfs_gpu``     keeps the reference's signature (index path, TSV path) and reads the TSV text on the GPU
+  (DESIGN.md section 13); the index and the TSV may be plain text or BGZF.  The ``count-orfs`` command runs it:
+
+    TSV            rt_codon_load_tsv (all cores): fields, selection, ORF_ID -> index row, gene keys
+    counts         Engine.orf_counts: count_emit_kernel, a stable radix sort on (gene, coordinate), count_keep_kernel
+    table          write_counts
+
+* ``count_orfs``         the same table in plain Python, from plain-text files: the statement the GPU path is
+  checked against.
 
 ``count_orfs_codon`` gives the same selection at codon level (DESIGN.md section 11): per gene and pooled over all
 genes, the occurrences, total, mean, median and variance of the read count of every codon.
@@ -191,6 +199,47 @@ def count_orfs(ribotricer_index, detected_orfs, features, outfile, report_all=Fa
         _, first = np.unique(pos, return_index=True)              # first coverage seen at a position wins (:80-82)
         total[g], length[g] = cov[first].sum(), len(first)
     write_counts(outfile, keys, total, length)
+
+
+def count_orfs_gpu(ribotricer_index, detected_orfs, features, outfile, report_all=False, stage_ms: dict | None = None):
+    """``count_orfs`` on the GPU (DESIGN.md section 13): the same table, byte for byte, on every input ``count_orfs``
+    accepts.  Every check runs before ``outfile`` is opened, so a refused input leaves no file; the refusals (a plain
+    gzip input, a line without 18 fields, an unknown ORF_ID, a malformed profile) raise ValueError naming the file and
+    the line.  ``stage_ms``, when given, receives the time of every stage in milliseconds.  Returns a summary dict."""
+    from .bgzf import open_texts
+    from .detect_orfs import get_engine
+
+    times = {} if stage_ms is None else stage_ms
+    clock = time.perf_counter()
+
+    def lap(name):
+        nonlocal clock
+        now = time.perf_counter()
+        times[name] = (now - clock) * 1e3
+        clock = now
+
+    index_src, tsv_src = open_texts([ribotricer_index, detected_orfs], "count-orfs")
+    lap("inflate")
+    idx = load_native_index(index_src)
+    lap("index_load")
+    inp = CodonInput(idx, tsv_src, features, report_all)
+    lap("tsv_load")
+    dev_ms = np.zeros(_lib.RT_COUNT_STAGES, np.float32)
+    total, length, summary = get_engine().orf_counts(inp.sel, inp.text(0), idx.exon_ptr, idx.exon_start, idx.exon_end,
+                                                     idx.orf_strand_code, inp.n_gene, stage_ms=dev_ms)
+    lap("orf_counts")
+    for name, ms in zip(("host_gather", "upload", "count_emit_kernel", "sort", "count_keep_kernel", "copy_back"),
+                        dev_ms.tolist()):
+        times["device:" + name] = ms
+    bad = int(summary[2])
+    if bad >= 0:
+        reason = next(text for bit, text in _PROFILE_REFUSALS if int(summary[3]) & bit)
+        raise ValueError(f"{detected_orfs} line {int(inp.sel['line'][bad])}: {reason}")
+    genes = np.flatnonzero(length)
+    keys = [tuple(part.decode("utf-8") for part in inp.gene(int(g))) for g in genes]
+    write_counts(outfile, keys, total[genes], length[genes])
+    lap("write")
+    return dict(rows=inp.n_sel, genes=len(keys), positions=int(summary[1]), duplicates=int(summary[0] - summary[1]))
 
 
 class CodonInput:

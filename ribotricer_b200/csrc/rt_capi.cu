@@ -2182,6 +2182,166 @@ int rt_codon_counts(rt_ctx* ctx, const rt_codon_query* q, uint64_t* gene_tab, ui
 
 }  // extern "C"
 
+// ---------------------------------------------------------------------------------------------------- count-orfs
+namespace {
+// The stream, events and device buffers of one rt_count_orfs call; everything is freed on every return.
+struct CountScratch {
+    Stream st;
+    Event ev[6];
+    DevArr<char> prof, temp;
+    DevArr<long long> prof_base, slot_base, row, ex_ptr;
+    DevArr<int> gene, ex_start, ex_end;
+    DevArr<uint8_t> strand, flag;
+    DevArr<unsigned long long> key, key2, counters, total, length;
+    DevArr<unsigned> val, val2, claim;
+    ~CountScratch() { if (st) cudaStreamSynchronize(st); }
+};
+}  // namespace
+
+extern "C" {
+
+int rt_count_orfs(rt_ctx* ctx, const rt_count_query* q, uint64_t* total, uint64_t* length, int64_t* summary,
+                  float* stage_ms) {
+    if (!ctx) return fail(nullptr, RT_EINVAL, "rt_count_orfs: ctx is NULL");
+    if (!q || !summary || q->n_sel < 0 || q->n_orf < 0 || q->n_gene < 0 ||
+        (q->n_sel && (!q->row || !q->gene || !q->prof_off || !q->prof_len || !q->tsv || !q->exon_ptr || !q->orf_strand)) ||
+        (q->n_gene && (!total || !length)))
+        return fail(ctx, RT_EINVAL, "rt_count_orfs: NULL or negative argument");
+    const auto t_host = std::chrono::steady_clock::now();
+    const int64_t n = q->n_sel, n_ex = q->n_orf ? q->exon_ptr[q->n_orf] : 0;
+    // 1. host: per selected line its row length and the offset of its profile text
+    std::vector<int64_t> prof_base((size_t)n + 1, 0), slot_base((size_t)n + 1, 0);
+    for (int64_t i = 0; i < n; ++i) {
+        const int64_t r = q->row[i];
+        if (r < 0 || r >= q->n_orf || q->gene[i] < 0 || q->gene[i] >= q->n_gene)
+            return fail(ctx, RT_EINVAL, "rt_count_orfs: selected line %lld lies outside the index or the gene table", (long long)i);
+        int64_t L = 0;
+        for (int64_t e = q->exon_ptr[r]; e < q->exon_ptr[r + 1]; ++e) L += (int64_t)q->exon_end[e] - q->exon_start[e] + 1;
+        prof_base[(size_t)i + 1] = prof_base[(size_t)i] + q->prof_len[i];
+        slot_base[(size_t)i + 1] = slot_base[(size_t)i] + L;
+    }
+    const int64_t n_slot = slot_base[(size_t)n];
+    if (n_slot > (int64_t)0xffffffffll)
+        return fail(ctx, RT_EINVAL, "count-orfs handles at most 2^32 - 1 nt in the selected rows; the selection has %lld",
+                    (long long)n_slot);
+    HostArr<char> prof;
+    if (!prof.alloc((size_t)prof_base[(size_t)n])) return fail(ctx, RT_ENOMEM, "rt_count_orfs: out of host memory");
+    const int64_t block = 1 << 10;
+    claim_parallel(host_threads((size_t)(prof_base[(size_t)n] >> 22) + 1, 32), (size_t)((n + block - 1) / block), [&](size_t bk) {
+        for (int64_t i = (int64_t)bk * block; i < std::min(n, (int64_t)(bk + 1) * block); ++i)
+            memcpy(prof.p + prof_base[(size_t)i], q->tsv + q->prof_off[i], (size_t)q->prof_len[i]);
+    });
+    if (stage_ms) {
+        for (int k = 0; k < RT_COUNT_STAGES; ++k) stage_ms[k] = 0.f;
+        stage_ms[0] = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_host).count();
+    }
+    for (int k = 0; k < 4; ++k) summary[k] = 0;
+    summary[2] = -1;
+    // 2. uploads
+    DeviceGuard guard(ctx->device);
+    CountScratch S;
+    RT_CUDA(ctx, S.st.create());
+    for (auto& e : S.ev) RT_CUDA(ctx, e.create());
+    const size_t ns = (size_t)n_slot, nn = (size_t)n, no = (size_t)q->n_orf, ne = (size_t)n_ex, ng = (size_t)q->n_gene;
+    RT_CUDA(ctx, S.prof.reserve(prof.size()));
+    RT_CUDA(ctx, S.prof_base.reserve(nn + 1));
+    RT_CUDA(ctx, S.slot_base.reserve(nn + 1));
+    RT_CUDA(ctx, S.row.reserve(nn));
+    RT_CUDA(ctx, S.gene.reserve(nn));
+    RT_CUDA(ctx, S.ex_ptr.reserve(no + 1));
+    RT_CUDA(ctx, S.ex_start.reserve(ne));
+    RT_CUDA(ctx, S.ex_end.reserve(ne));
+    RT_CUDA(ctx, S.strand.reserve(no));
+    RT_CUDA(ctx, S.key.reserve(ns));
+    RT_CUDA(ctx, S.key2.reserve(ns));
+    RT_CUDA(ctx, S.val.reserve(ns));
+    RT_CUDA(ctx, S.val2.reserve(ns));
+    RT_CUDA(ctx, S.counters.reserve(2));
+    RT_CUDA(ctx, S.flag.reserve(nn));
+    RT_CUDA(ctx, S.claim.reserve(1));
+    RT_CUDA(ctx, S.total.reserve(ng));
+    RT_CUDA(ctx, S.length.reserve(ng));
+    // the sort looks at the key bits in use: 32 of coordinate and those of the largest gene id, n_gene - 1.  A dropped
+    // slot's key ~0 has all of them set, and a real key's gene field is at most n_gene - 1 < 2^bit_length(n_gene) - 1,
+    // so a dropped slot sorts after every real key and never equals one.
+    const unsigned items = (unsigned)ns;
+    const int key_bits = 32 + bit_length((unsigned long long)q->n_gene);
+    size_t temp_bytes = 0;
+    RT_CUDA(ctx, cub::DeviceRadixSort::SortPairs(nullptr, temp_bytes, S.key.p, S.key2.p, S.val.p, S.val2.p, items, 0,
+                                                 key_bits, S.st.s));
+    RT_CUDA(ctx, S.temp.reserve(temp_bytes));
+    RT_CUDA(ctx, cudaEventRecord(S.ev[0], S.st));
+    RT_CUDA(ctx, S.prof.upload(prof.p, prof.size(), S.st));
+    RT_CUDA(ctx, S.prof_base.upload(prof_base.data(), nn + 1, S.st));
+    RT_CUDA(ctx, S.slot_base.upload(slot_base.data(), nn + 1, S.st));
+    RT_CUDA(ctx, S.row.upload(q->row, nn, S.st));
+    RT_CUDA(ctx, S.gene.upload(q->gene, nn, S.st));
+    if (n) {
+        RT_CUDA(ctx, S.ex_ptr.upload(q->exon_ptr, no + 1, S.st));
+        RT_CUDA(ctx, S.ex_start.upload(q->exon_start, ne, S.st));
+        RT_CUDA(ctx, S.ex_end.upload(q->exon_end, ne, S.st));
+        RT_CUDA(ctx, S.strand.upload(q->orf_strand, no, S.st));
+    }
+    const unsigned long long counters0[2] = {0, ~0ull};
+    RT_CUDA(ctx, S.counters.upload(counters0, 2, S.st));
+    RT_CUDA(ctx, cudaMemsetAsync(S.claim.p, 0, sizeof(unsigned), S.st));
+    RT_CUDA(ctx, cudaMemsetAsync(S.total.p, 0, sizeof(unsigned long long) * ng, S.st));
+    RT_CUDA(ctx, cudaMemsetAsync(S.length.p, 0, sizeof(unsigned long long) * ng, S.st));
+    RT_CUDA(ctx, cudaEventRecord(S.ev[1], S.st));
+    // 3. count_emit_kernel
+    const rt::CountArgs A{S.prof.p, S.prof_base.p, S.slot_base.p, S.row.p, S.ex_ptr.p, S.ex_start.p, S.ex_end.p,
+                          S.strand.p, S.gene.p, S.key.p, S.val.p, S.counters.p, S.flag.p, (long long)n, S.claim.p};
+    const int64_t big = std::max(1, ctx->n_sm * 8);
+    if (n) {
+        const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((n + rt::kCodonWarps - 1) / rt::kCodonWarps, big));
+        rt::count_emit_kernel<<<grid, rt::kCodonWarps * 32, 0, S.st>>>(A);
+        ctx->launches++;
+        RT_CUDA(ctx, cudaGetLastError());
+    }
+    RT_CUDA(ctx, cudaEventRecord(S.ev[2], S.st));
+    unsigned long long h_counters[2];
+    RT_CUDA(ctx, cudaMemcpyAsync(h_counters, S.counters.p, sizeof h_counters, cudaMemcpyDeviceToHost, S.st));
+    RT_CUDA(ctx, cudaStreamSynchronize(S.st));
+    summary[0] = (int64_t)h_counters[0];
+    if (h_counters[1] != ~0ull) {                      // a refused profile: no counts
+        uint8_t f = 0;
+        RT_CUDA(ctx, cudaMemcpyAsync(&f, S.flag.p + h_counters[1], 1, cudaMemcpyDeviceToHost, S.st));
+        RT_CUDA(ctx, cudaStreamSynchronize(S.st));
+        summary[2] = (int64_t)h_counters[1];
+        summary[3] = f;
+        if (stage_ms) RT_CUDA(ctx, cudaEventElapsedTime(&stage_ms[1], S.ev[0], S.ev[1]));
+        return RT_OK;
+    }
+    // 4. stable sort by key: slots are in (line, oriented nt) order, so the first slot of every key is the first pair
+    if (items)
+        RT_CUDA(ctx, cub::DeviceRadixSort::SortPairs(S.temp.p, temp_bytes, S.key.p, S.key2.p, S.val.p, S.val2.p, items, 0,
+                                                     key_bits, S.st.s));
+    RT_CUDA(ctx, cudaEventRecord(S.ev[3], S.st));
+    // 5. count_keep_kernel
+    if (items) {
+        const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((int64_t)(ns + 255) / 256, big));
+        rt::count_keep_kernel<<<grid, 256, 0, S.st>>>(S.key2.p, S.val2.p, (long long)ns, S.total.p, S.length.p);
+        ctx->launches++;
+        RT_CUDA(ctx, cudaGetLastError());
+    }
+    RT_CUDA(ctx, cudaEventRecord(S.ev[4], S.st));
+    // 6. copy-back
+    if (ng) {
+        RT_CUDA(ctx, cudaMemcpyAsync(total, S.total.p, 8 * ng, cudaMemcpyDeviceToHost, S.st));
+        RT_CUDA(ctx, cudaMemcpyAsync(length, S.length.p, 8 * ng, cudaMemcpyDeviceToHost, S.st));
+    }
+    RT_CUDA(ctx, cudaEventRecord(S.ev[5], S.st));
+    RT_CUDA(ctx, cudaStreamSynchronize(S.st));
+    uint64_t kept = 0;
+    for (size_t g = 0; g < ng; ++g) kept += length[g];
+    summary[1] = (int64_t)kept;
+    if (stage_ms)
+        for (int k = 1; k < RT_COUNT_STAGES; ++k) RT_CUDA(ctx, cudaEventElapsedTime(&stage_ms[k], S.ev[k - 1], S.ev[k]));
+    return RT_OK;
+}
+
+}  // extern "C"
+
 // -------------------------------------------------------------------------------------------------- BGZF text inputs
 namespace {
 constexpr size_t kInflatePiece = size_t(64) << 20;   // text bytes per page-locked copy-back buffer

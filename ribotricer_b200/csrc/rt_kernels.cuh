@@ -2721,9 +2721,50 @@ constexpr int kCodonWarps = 8;
 
 __device__ __forceinline__ bool is_digit(char c) { return c >= '0' && c <= '9'; }
 
+// The profile grammar walk shared by codon_emit_kernel and count_emit_kernel, called by the whole warp on the profile
+// text s[0, n) of one row.  Every byte is checked against "[" (D(", "D)*)? "]" with D = 0 | [1-9][0-9]*, 32 bytes a
+// window; a ballot of the digits that follow a non-digit finds the values, and the lane that starts value j calls
+// on_value(j, v) while it has seen nothing wrong.  Returns this lane's refusal bits (1 malformed, 2 a value above
+// 2^31 - 1; the caller reduces them over the warp) and sets P to the number of values.
+template <class OnValue>
+__device__ __forceinline__ unsigned profile_walk(const char* s, long long n, int lane, long long& P, OnValue&& on_value) {
+    const unsigned below = (1u << lane) - 1u;
+    unsigned bad = 0;
+    P = 0;
+    if (n < 2 || s[0] != '[' || s[n - 1] != ']') return 1;
+    const char* b = s + 1;
+    const long long nb = n - 2;
+    for (long long w = 0; w < nb; w += 32) {
+        const long long i = w + lane;
+        bool start = false;
+        unsigned long long v = 0;
+        if (i < nb) {
+            const char c = b[i], p = i > 0 ? b[i - 1] : ' ', q = i + 1 < nb ? b[i + 1] : ',';
+            if (is_digit(c)) {                             // the defaults of p and q refuse a separator at either end
+                start = !is_digit(p);
+            } else if (c == ',') {
+                if (!is_digit(p) || q != ' ') bad |= 1;
+            } else if (c == ' ') {
+                if (p != ',' || !is_digit(q)) bad |= 1;
+            } else {
+                bad |= 1;
+            }
+            if (start) {
+                if (c == '0' && i + 1 < nb && is_digit(b[i + 1])) bad |= 1;   // a leading zero
+                int d = 0;
+                for (long long j = i; j < nb && is_digit(b[j]) && d < 11; ++j, ++d) v = v * 10 + (b[j] - '0');
+                if (d > 10 || v > 2147483647ull) bad |= 2;
+            }
+        }
+        const unsigned starts = __ballot_sync(kFull, start);
+        if (start && !bad) on_value(P + __popc(starts & below), v);
+        P += __popc(starts);
+    }
+    return bad;
+}
+
 __global__ void __launch_bounds__(kCodonWarps * 32) codon_emit_kernel(const CodonArgs A) {
     const int lane = threadIdx.x & 31;
-    const unsigned below = (1u << lane) - 1u;
     for (;;) {
         unsigned t = 0;
         if (lane == 0) t = atomicAdd(A.claim, 1u);
@@ -2733,43 +2774,10 @@ __global__ void __launch_bounds__(kCodonWarps * 32) codon_emit_kernel(const Codo
         const long long n = A.prof_base[t + 1] - A.prof_base[t];
         const long long L = A.seq_base[t + 1] - A.seq_base[t];
         const long long s0 = A.slot_base[t], n_slot = A.slot_base[t + 1] - s0;
-        unsigned bad = 0;
-        long long P = 0;                                   // values parsed
-        if (n < 2 || s[0] != '[' || s[n - 1] != ']') {
-            bad = 1;
-        } else {
-            const char* b = s + 1;
-            const long long nb = n - 2;
-            for (long long w = 0; w < nb; w += 32) {
-                const long long i = w + lane;
-                bool start = false;
-                unsigned long long v = 0;
-                if (i < nb) {
-                    const char c = b[i], p = i > 0 ? b[i - 1] : ' ', q = i + 1 < nb ? b[i + 1] : ',';
-                    if (is_digit(c)) {                     // the defaults of p and q refuse a separator at either end
-                        start = !is_digit(p);
-                    } else if (c == ',') {
-                        if (!is_digit(p) || q != ' ') bad |= 1;
-                    } else if (c == ' ') {
-                        if (p != ',' || !is_digit(q)) bad |= 1;
-                    } else {
-                        bad |= 1;
-                    }
-                    if (start) {
-                        if (c == '0' && i + 1 < nb && is_digit(b[i + 1])) bad |= 1;   // a leading zero
-                        int d = 0;
-                        for (long long j = i; j < nb && is_digit(b[j]) && d < 11; ++j, ++d) v = v * 10 + (b[j] - '0');
-                        if (d > 10 || v > 2147483647ull) bad |= 2;
-                    }
-                }
-                const unsigned starts = __ballot_sync(kFull, start);
-                if (start && v && !bad) {
-                    const long long j = P + __popc(starts & below);
-                    if (j / 3 < n_slot) atomicAdd(A.cnt + s0 + j / 3, v);
-                }
-                P += __popc(starts);
-            }
-        }
+        long long P;                                       // values parsed
+        unsigned bad = profile_walk(s, n, lane, P, [&](long long j, unsigned long long v) {
+            if (v && j / 3 < n_slot) atomicAdd(A.cnt + s0 + j / 3, v);
+        });
         bad = __reduce_or_sync(kFull, bad);
         __syncwarp();                                      // the counts of this row are in place (read through L2 below)
         if (bad) {
@@ -2910,6 +2918,114 @@ __global__ void __launch_bounds__(256) codon_stats_kernel(const unsigned long lo
             o[2] = s2_lo;
             o[3] = s2_hi;
             o[4] = mid;
+        }
+    }
+}
+
+// ---------------------------------------------------------------------------------------------------- count-orfs
+// count_emit_kernel (DESIGN.md section 13): one warp per selected TSV line, claimed dynamically.  The warp checks the
+// profile grammar (profile_walk) and stores value j < L of the row's L nt as val[s0 + j].  Then oriented nt k < m =
+// min(values, L) gets the key gene << 32 | (uint32) its genomic coordinate, found through the row's intervals with a
+// per-lane cursor ('-' rows walk them from the right); slots k in [m, L) get the key ~0 (dropped).  A refused line sets
+// its flag and takes part in an atomicMin of the first refused line.
+struct CountArgs {
+    const char* prof;                 // profile text of the selected lines, back to back
+    const long long* prof_base;       // n_sel + 1
+    const long long* slot_base;       // n_sel + 1: row lengths, scanned
+    const long long* row;             // index row of each selected line
+    const long long* exon_ptr;
+    const int* ex_start;
+    const int* ex_end;
+    const uint8_t* strand;            // per index row, 1: reverse
+    const int* gene;
+    unsigned long long* key;          // per slot
+    unsigned* val;                    // per slot
+    unsigned long long* counters;     // [0] positions named (sum of m), [1] first refused line (atomicMin), zeroed / ~0
+    uint8_t* flag;                    // per selected line: 1 malformed, 2 value above 2^31 - 1
+    long long n_sel;
+    unsigned* claim;                  // work counter, zeroed before the launch
+};
+
+__global__ void __launch_bounds__(kCodonWarps * 32) count_emit_kernel(const CountArgs A) {
+    const int lane = threadIdx.x & 31;
+    for (;;) {
+        unsigned t = 0;
+        if (lane == 0) t = atomicAdd(A.claim, 1u);
+        t = __shfl_sync(kFull, t, 0);
+        if ((long long)t >= A.n_sel) return;
+        const long long s0 = A.slot_base[t], L = A.slot_base[t + 1] - s0;
+        long long P;
+        unsigned bad = profile_walk(A.prof + A.prof_base[t], A.prof_base[t + 1] - A.prof_base[t], lane, P,
+                                    [&](long long j, unsigned long long v) {
+            if (j < L) A.val[s0 + j] = (unsigned)v;
+        });
+        bad = __reduce_or_sync(kFull, bad);
+        if (bad) {
+            if (lane == 0) {
+                A.flag[t] = (uint8_t)bad;
+                atomicMin(A.counters + 1, (unsigned long long)t);
+            }
+            continue;
+        }
+        const long long m = min(P, L);
+        const long long r = A.row[t], e0 = A.exon_ptr[r], e1 = A.exon_ptr[r + 1];
+        const bool rev = A.strand[r] == 1;
+        const unsigned long long hi = (unsigned long long)(unsigned)A.gene[t] << 32;
+        // per lane: interval cursor `e` and the nt of the intervals left of it, `before` (ascending order)
+        long long e = rev ? e1 - 1 : e0, before = 0;
+        if (rev)
+            for (long long x = e0; x < e1 - 1; ++x) before += A.ex_end[x] - A.ex_start[x] + 1;
+        for (long long k = lane; k < L; k += 32) {
+            unsigned long long key = ~0ull;
+            if (k < m) {
+                const long long a = rev ? L - 1 - k : k;   // ascending index of oriented nt k
+                if (rev) {
+                    while (a < before) { --e; before -= A.ex_end[e] - A.ex_start[e] + 1; }
+                } else {
+                    while (a >= before + (A.ex_end[e] - A.ex_start[e] + 1)) { before += A.ex_end[e] - A.ex_start[e] + 1; ++e; }
+                }
+                key = hi | (unsigned)(A.ex_start[e] + (int)(a - before));
+            }
+            A.key[s0 + k] = key;
+        }
+        if (lane == 0 && m) atomicAdd(A.counters + 0, (unsigned long long)m);
+    }
+}
+
+// After the stable sort by key: the first slot of every key is kept (TSV order survives a stable sort, so it is the
+// first line's value), and adds its value to total[gene] and 1 to length[gene].  Keys are sorted, so the gene of the
+// slots, key >> 32 (0xffffffff for dropped slots and past the end), never decreases across a warp: a segmented scan over
+// runs of equal gene leaves each run's sums with its last lane, which alone issues the two atomics.
+__global__ void __launch_bounds__(256) count_keep_kernel(const unsigned long long* __restrict__ key,
+                                                         const unsigned* __restrict__ val, long long n,
+                                                         unsigned long long* total, unsigned long long* length) {
+    const int lane = threadIdx.x & 31;
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    for (long long w = (long long)blockIdx.x * blockDim.x + (threadIdx.x & ~31); w < n; w += stride) {
+        const long long i = w + lane;
+        unsigned gene = 0xffffffffu;
+        unsigned long long sum = 0, cnt = 0;
+        if (i < n) {
+            const unsigned long long k = key[i];
+            gene = (unsigned)(k >> 32);
+            if (k != ~0ull && (i == 0 || key[i - 1] != k)) {
+                sum = val[i];
+                cnt = 1;
+            }
+        }
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const unsigned g_up = __shfl_up_sync(kFull, gene, d);
+            const unsigned long long s_up = __shfl_up_sync(kFull, sum, d), c_up = __shfl_up_sync(kFull, cnt, d);
+            if (lane >= d && g_up == gene) {
+                sum += s_up;
+                cnt += c_up;
+            }
+        }
+        const unsigned g_next = __shfl_down_sync(kFull, gene, 1);
+        if ((lane == 31 || g_next != gene) && cnt) {
+            atomicAdd(total + gene, sum);
+            atomicAdd(length + gene, cnt);
         }
     }
 }

@@ -529,6 +529,31 @@ class Engine:
             stage_ms[:] = ms
         return gene_tab, pooled_tab, summary
 
+    # --------------------------------------------------------------- count-orfs
+    def orf_counts(self, sel: dict, tsv, exon_ptr, exon_start, exon_end, orf_strand, n_gene: int,
+                   stage_ms: np.ndarray | None = None):
+        """Per-gene read counts of DESIGN.md section 13 (``rt_count_orfs``).  ``sel`` holds the columns of the selected
+        TSV lines (``row``, ``gene``, ``prof_off``, ``prof_len``); ``tsv`` is the file text (uint8).  Returns (total
+        [n_gene], length [n_gene], summary[4]) as uint64 / int64 arrays: see ``rt_count_orfs`` in the header."""
+        arr = lambda a, dt: np.ascontiguousarray(a, dt)  # noqa: E731
+        row, gene = arr(sel["row"], np.int64), arr(sel["gene"], np.int32)
+        prof_off, prof_len = arr(sel["prof_off"], np.int64), arr(sel["prof_len"], np.int64)
+        exon_ptr, exon_start, exon_end = arr(exon_ptr, np.int64), arr(exon_start, np.int32), arr(exon_end, np.int32)
+        orf_strand = arr(orf_strand, np.uint8)
+        q = _lib.CountQuery(len(row), _np_ptr(row), _np_ptr(gene), _np_ptr(prof_off), _np_ptr(prof_len), _np_ptr(tsv),
+                            len(exon_ptr) - 1, _np_ptr(exon_ptr), _np_ptr(exon_start), _np_ptr(exon_end),
+                            _np_ptr(orf_strand), int(n_gene))
+        total, length = np.zeros(int(n_gene), np.uint64), np.zeros(int(n_gene), np.uint64)
+        summary = np.zeros(4, np.int64)
+        ms = np.zeros(_lib.RT_COUNT_STAGES, np.float32)
+        rc = self.lib.rt_count_orfs(self.ctx, C.byref(q), _np_ptr(total), _np_ptr(length), _np_ptr(summary), _np_ptr(ms))
+        if rc == _lib.RT_EINVAL:
+            raise ValueError(self.lib.rt_last_error(self.ctx).decode())
+        self._check(rc)
+        if stage_ms is not None:
+            stage_ms[:] = ms
+        return total, length, summary
+
     # --------------------------------------------------------------- BGZF text inputs
     def inflate_bgzf(self, path: str, summary: np.ndarray | None = None, stage_ms: np.ndarray | None = None):
         """The inflated text of a BGZF file (``rt_bgzf_inflate``: bgzf_inflate_kernel, members the device refuses
