@@ -92,6 +92,37 @@ def compare_scores(got, ref, tie, params=DEFAULT_PARAMS, what=""):
     return int(tie.sum()), int(near.sum())
 
 
+def compare_tsv(got_text, want_text, phase_score_cutoff, what=""):
+    """Two translating-ORFs TSV texts under the parity bar: same header and row order, phase score within SCORE_TOL,
+    every other column equal except valid codons / ratio / status on frame ties (H1) and status near the cutoff.  A row
+    only one side reports must be a tie or near the cutoff; at most max(2, 5 %) rows differ so.  Returns the number of
+    rows of ``want_text``."""
+    from oracle import oracle_py as O
+
+    split = lambda text: {r.split("\t")[0]: r.split("\t") for r in text.split("\n")[1:] if r}     # noqa: E731
+    assert got_text.split("\n")[0] == want_text.split("\n")[0], f"{what}header differs"
+    got, ref = split(got_text), split(want_text)
+    assert [k for k in got if k in ref] == [k for k in ref if k in got], f"{what}ORF ordering differs"
+    n_exc = 0
+    for oid, r in ref.items():
+        tie = O.is_frame_tie(O.frame_spectra(eval(r[17])))
+        near = abs(float(r[3]) - phase_score_cutoff) <= SCORE_TOL
+        if oid not in got:
+            assert tie or near, (what, oid)
+            n_exc += 1
+            continue
+        g = got[oid]
+        assert abs(float(g[3]) - float(r[3])) <= SCORE_TOL, (what, oid)
+        cols = [0, 1, 4, 5, 8, 9, 10, 11, 12, 13, 14, 15, 16, 17]
+        if not tie:
+            cols += [6, 7] + ([2] if not near else [])
+        for c in cols:
+            assert g[c] == r[c], (what, oid, c, g[c], r[c])
+    n_exc += sum(1 for oid in got if oid not in ref)
+    assert n_exc <= max(2, len(ref) // 20), f"{what}{n_exc} rows differ"
+    return len(ref)
+
+
 def decode_stream(records, hdr, n_blocks, block=256):
     """Checker-side decoder of the record stream of include/ribotricer_b200.h (rt_stream_pack): returns one tuple
     (ref_id, first, last, mlen, meta7) per read record, in order.  Plain Python: small cases only."""

@@ -5,7 +5,7 @@ import os
 import numpy as np
 import pytest
 
-from helpers import SCORE_TOL, alignments_to_reads, load_golden
+from helpers import SCORE_TOL, alignments_to_reads, compare_tsv, load_golden
 
 pytestmark = pytest.mark.gpu
 
@@ -18,11 +18,6 @@ def _read_columns(case, by_length=False):
     if by_length:   # reads grouped by ascending length: read_length_counts insertion order (bam.py:136)
         case = dict(case, alignments=sorted(case["alignments"], key=lambda a: a[0]))
     return ReadColumns(names, lens, alignments_to_reads(case, names))
-
-
-def _rows(text):
-    lines = text.split("\n")
-    return lines[0], {r.split("\t")[0]: r.split("\t") for r in lines[1:] if r}
 
 
 def test_phasescore_function(engine):
@@ -54,7 +49,6 @@ def test_phasescore_function(engine):
 def test_detect_orfs_end_to_end(engine, tmp_path):
     """detect_orfs() with explicit read lengths and offsets: TSV, WIG and bam summary against the
     files written by the reference's export_orf_coverages / export_wig (golden)."""
-    from oracle import oracle_py as O
     from ribotricer_b200 import detect_orfs as D
 
     D._ENGINE = engine
@@ -69,31 +63,8 @@ def test_detect_orfs_end_to_end(engine, tmp_path):
             D.detect_orfs(reads, str(idx_path), prefix, "forward", None, dict(offsets), prm["phase_score_cutoff"],
                           prm["min_valid_codons"], prm["min_reads_per_codon"], prm["min_valid_codons_ratio"],
                           prm["min_density_over_orf"], prm["report_all"], meta_min_reads=10 ** 9)
-            got_hdr, got = _rows(open(f"{prefix}_translating_ORFs.tsv").read())
-            ref_hdr, ref = _rows(run["text"])
-            assert got_hdr == ref_hdr
-            order_got = [k for k in got if k in ref]
-            order_ref = [k for k in ref if k in got]
-            assert order_got == order_ref                      # ORF ordering
-            n_exc = 0
-            for oid, r in ref.items():
-                tie = O.is_frame_tie(O.frame_spectra(eval(r[17])))
-                near = abs(float(r[3]) - prm["phase_score_cutoff"]) <= SCORE_TOL
-                if oid not in got:
-                    assert tie or near, oid
-                    n_exc += 1
-                    continue
-                g = got[oid]
-                assert abs(float(g[3]) - float(r[3])) <= SCORE_TOL
-                cols = [0, 1, 4, 5, 8, 9, 10, 11, 12, 13, 14, 15, 16, 17]
-                if not tie:
-                    cols += [6, 7] + ([2] if not near else [])
-                for c in cols:
-                    assert g[c] == r[c], (case["name"], oid, c, g[c], r[c])
-            for oid in got:
-                if oid not in ref:
-                    n_exc += 1
-            assert n_exc <= max(2, len(ref) // 20)
+            compare_tsv(open(f"{prefix}_translating_ORFs.tsv").read(), run["text"], prm["phase_score_cutoff"],
+                        what=case["name"] + ": ")
         # WIG: every P-site the reference wrote, except those shifted beyond the contig pad
         for tag, text in case["wig"].items():
             assert open(f"{prefix}_{tag}.wig").read() == text
@@ -363,11 +334,12 @@ def test_two_rank_job_is_byte_identical(tmp_path):
 def test_batch_of_libraries_matches_single_runs(engine, tmp_path):
     """BASELINE configs[3] in small: eight libraries against one resident index through detect_orfs_batch (index and
     compact slot map set once, copy / kernels / text pipelined over two coverage buffers).  Every library's TSV and
-    BAM summary must be the bytes detect_orfs() writes for that library alone."""
+    BAM summary must be the bytes detect_orfs() writes for that library alone.  Then the same on the genome of 1,900
+    contigs of test_many_contigs.py (edge-length contigs, contigs with ORFs but no reads at either end and in the
+    middle): a streamed library, one the packer refuses and an unsorted one."""
     from ribotricer_b200 import detect_orfs as D
     from ribotricer_b200 import synth
     from ribotricer_b200.bam import ReadColumns, save_read_columns
-    from ribotricer_b200.batch import detect_orfs_batch
 
     D._ENGINE = engine
     cfg = synth.config("tiny")
@@ -376,22 +348,44 @@ def test_batch_of_libraries_matches_single_runs(engine, tmp_path):
     idx.write_tsv(index_path)
     offsets = {27: 12, 28: 12, 29: 12, 30: 13, 31: 13}
     lengths = [27, 28, 29, 30, 31]
-    libs, singles, batched = [], [], []
+    libs = []
     for k in range(8):
         cols = synth.reads_to_numpy(synth.make_reads(cfg, idx, n_reads=40_000 + 15_000 * k, seed_offset=100 + k, sort=k != 5))
         path = str(tmp_path / f"lib{k}.npz")
         save_read_columns(path, ReadColumns(idx.contig_names, idx.contig_len, cols, k != 5))
         libs.append(path)
-        singles.append(str(tmp_path / f"single{k}"))
-        batched.append(str(tmp_path / "batch" / f"lib{k}"))
     params = (0.3, 3, 0, 0.1, 0.25)
+    _batch_matches_single_runs(engine, tmp_path / "tiny", libs, index_path, lengths, offsets, params)
+
+    import test_many_contigs as M
+
+    names, lens = M.genome()
+    index_path = str(tmp_path / "many_index.tsv")
+    M.write_index(index_path)
+    libs = []
+    for k, kind in enumerate(("dense", "sparse", "dense")):
+        cols = M.library(kind)
+        if k == 2:                      # not coordinate-sorted: the column kernel after a clear
+            cols = {c: v[np.random.default_rng(k).permutation(len(v))] for c, v in cols.items()}
+        path = str(tmp_path / f"many{k}.npz")
+        save_read_columns(path, ReadColumns(names, lens, cols, k != 2))
+        libs.append(path)
+    _batch_matches_single_runs(engine, tmp_path / "many", libs, index_path, None, M.OFFSETS, params)
+
+
+def _batch_matches_single_runs(engine, out_dir, libs, index_path, lengths, offsets, params):
+    from ribotricer_b200 import detect_orfs as D
+    from ribotricer_b200.batch import detect_orfs_batch
+
+    singles = [str(out_dir / f"single{k}") for k in range(len(libs))]
+    batched = [str(out_dir / "batch" / f"lib{k}") for k in range(len(libs))]
     for report_all in (False, True):
-        for k in range(8):
+        for k in range(len(libs)):
             D.detect_orfs(libs[k], index_path, singles[k], "forward", lengths, dict(offsets), *params, report_all)
         done = detect_orfs_batch(libs, index_path, batched, "forward", lengths, offsets, *params, report_all=report_all,
                                  engine=engine)
-        assert [k for k, _ in done] == list(range(8))
-        for k in range(8):
+        assert [k for k, _ in done] == list(range(len(libs)))
+        for k in range(len(libs)):
             for suffix in ("_translating_ORFs.tsv", "_bam_summary.txt"):
                 assert open(batched[k] + suffix, "rb").read() == open(singles[k] + suffix, "rb").read(), (k, suffix)
     assert engine.layout == "dense"

@@ -831,8 +831,7 @@ def test_detect_orfs_host_flow_against_reference_golden(built, tmp_path, monkeyp
     step, the dense -> compact hand-over, row selection and chunking of write_tsv, the native TSV / WIG writers -- against
     the files the unmodified reference wrote for the same inputs (four parameter sets per case).  GPU twin:
     test_gpu_api.py::test_detect_orfs_end_to_end."""
-    from helpers import SCORE_TOL, alignments_to_reads, load_golden
-    from oracle import oracle_py as O
+    from helpers import alignments_to_reads, compare_tsv, load_golden
     from oracle_engine import install
     from ribotricer_b200 import detect_orfs as D
     from ribotricer_b200.bam import ReadColumns
@@ -852,28 +851,8 @@ def test_detect_orfs_host_flow_against_reference_golden(built, tmp_path, monkeyp
                           prm["min_valid_codons"], prm["min_reads_per_codon"], prm["min_valid_codons_ratio"],
                           prm["min_density_over_orf"], prm["report_all"], meta_min_reads=10 ** 9)
             assert "compact_from_dense" in eng.calls and "score_host" in eng.calls      # scored in the compact layout
-            split = lambda text: {r.split("\t")[0]: r.split("\t") for r in text.split("\n")[1:] if r}     # noqa: E731
             got_text = open(f"{prefix}_translating_ORFs.tsv").read()
-            assert got_text.split("\n")[0] == run["text"].split("\n")[0]
-            got, ref = split(got_text), split(run["text"])
-            assert [k for k in got if k in ref] == [k for k in ref if k in got]          # ORF ordering
-            n_exc = 0
-            for oid, r in ref.items():
-                tie = O.is_frame_tie(O.frame_spectra(eval(r[17])))
-                near = abs(float(r[3]) - prm["phase_score_cutoff"]) <= SCORE_TOL
-                if oid not in got:
-                    assert tie or near, oid
-                    n_exc += 1
-                    continue
-                g = got[oid]
-                assert abs(float(g[3]) - float(r[3])) <= SCORE_TOL
-                cols = [0, 1, 4, 5, 8, 9, 10, 11, 12, 13, 14, 15, 16, 17]
-                if not tie:
-                    cols += [6, 7] + ([2] if not near else [])
-                for c in cols:
-                    assert g[c] == r[c], (case["name"], oid, c, g[c], r[c])
-            n_exc += sum(1 for oid in got if oid not in ref)
-            assert n_exc <= max(2, len(ref) // 20)
+            compare_tsv(got_text, run["text"], prm["phase_score_cutoff"], what=case["name"] + ": ")
         for tag, text in case["wig"].items():
             assert open(f"{prefix}_{tag}.wig").read() == text
         summary = open(f"{prefix}_bam_summary.txt").read()
