@@ -16,6 +16,7 @@ GPU name and power limit are read in the same run.
 from __future__ import annotations
 
 import argparse
+import hashlib
 import os
 import subprocess
 import sys
@@ -134,6 +135,8 @@ def main():
         say("")
         say(f"selection {mode}: {info['rows']} rows, {info['genes']} genes, {info['codons']} codons kept, "
             f"{info['duplicates']} duplicates skipped, {info['codons_with_n']} codons with N")
+        say("tables sha256: " + ", ".join(f"{suffix} {hashlib.sha256(open(out + suffix, 'rb').read()).hexdigest()}"
+                                          for suffix in ("_codon_counts_by_gene.tsv", "_codon_counts.tsv")))
         say("stage (ms)                " + "".join(f"run {k + 1:>2}    " for k in range(len(runs))))
         for name in runs[0]:
             say(f"{name:<26}" + "".join(f"{r[name]:>9.1f} " for r in runs))

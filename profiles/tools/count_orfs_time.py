@@ -16,6 +16,7 @@ the CPU arm.  The GPU name and power limit are read in the same run.
 from __future__ import annotations
 
 import argparse
+import hashlib
 import os
 import subprocess
 import sys
@@ -102,6 +103,7 @@ def main():
         say("")
         say(f"selection {mode}: {info['rows']} rows, {info['genes']} genes, {info['positions']} positions kept, "
             f"{info['duplicates']} duplicates skipped")
+        say(f"table sha256: {hashlib.sha256(open(out, 'rb').read()).hexdigest()}")
         say("stage (ms)                " + "".join(f"run {k + 1:>2}    " for k in range(len(runs))))
         for name in STAGES:
             say(f"{name:<26}" + "".join(f"{r[name]:>9.1f} " for r in runs))

@@ -23,6 +23,21 @@ unsigned __cudaPushCallConfiguration(dim3, dim3, size_t, cudaStream_t) { return 
 cudaError_t __cudaPopCallConfiguration(dim3*, dim3*, size_t*, void*) { return cudaSuccess; }
 cudaError_t cudaLaunchKernel(const void*, dim3, dim3, void**, size_t, cudaStream_t) { return cudaSuccess; }
 cudaError_t cudaDeviceSynchronize() { return cudaSuccess; }
+cudaError_t cudaDeviceGetAttribute(int* v, cudaDeviceAttr a, int) {
+    switch (a) {
+        case cudaDevAttrComputeCapabilityMajor: *v = 10; break;
+        case cudaDevAttrComputeCapabilityMinor: *v = 0; break;
+        case cudaDevAttrMultiProcessorCount: *v = 148; break;
+        case cudaDevAttrMaxSharedMemoryPerBlock: *v = 49152; break;
+        case cudaDevAttrMaxSharedMemoryPerBlockOptin: *v = 232448; break;
+        case cudaDevAttrMaxSharedMemoryPerMultiprocessor: *v = 233472; break;
+        default: *v = 1;
+    }
+    return cudaSuccess;
+}
+cudaError_t cudaFuncGetAttributes(cudaFuncAttributes* a, const void*) { memset(a, 0, sizeof *a); a->ptxVersion = a->binaryVersion = 100; a->maxThreadsPerBlock = 1024; return cudaSuccess; }
+cudaError_t cudaPeekAtLastError() { return cudaSuccess; }
+void __cudaRegisterVar(void**, char*, char*, const char*, int, size_t, int, int) {}
 cudaError_t cudaEventCreate(cudaEvent_t* e) { *e = (cudaEvent_t)malloc(8); return cudaSuccess; }
 cudaError_t cudaEventCreateWithFlags(cudaEvent_t* e, unsigned) { *e = (cudaEvent_t)malloc(8); return cudaSuccess; }
 cudaError_t cudaEventElapsedTime(float* ms, cudaEvent_t, cudaEvent_t) { *ms = 0.f; return cudaSuccess; }

@@ -14,6 +14,7 @@ from __future__ import annotations
 
 import ctypes as C
 import struct
+import time
 
 import numpy as np
 
@@ -114,3 +115,21 @@ def open_text(path: str, command: str):
     """``open_texts`` of one input."""
     return open_texts([path], command)[0]
 
+
+class StageClock:
+    """Stage times of one command in milliseconds, written into ``times`` (a new dict when None): ``lap(name)`` records
+    the host time since the previous lap, ``device(names, ms)`` the device stage times a native call reported, each as
+    ``"device:" + name``."""
+
+    def __init__(self, times: dict | None = None):
+        self.times = {} if times is None else times
+        self._clock = time.perf_counter()
+
+    def lap(self, name: str) -> None:
+        now = time.perf_counter()
+        self.times[name] = (now - self._clock) * 1e3
+        self._clock = now
+
+    def device(self, names, ms) -> None:
+        for name, v in zip(names, ms.tolist()):
+            self.times["device:" + name] = v

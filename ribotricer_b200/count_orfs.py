@@ -32,12 +32,12 @@ from __future__ import annotations
 import ctypes as C
 import os
 import pathlib
-import time
 from collections import defaultdict
 
 import numpy as np
 
 from . import _lib
+from .bgzf import NativeText, StageClock, open_texts
 from .index import load_native_index
 
 _POS_BITS = 33          # positions are int32: gene * 2^33 + (pos + 2^31) orders intervals by (gene, pos)
@@ -206,39 +206,20 @@ def count_orfs_gpu(ribotricer_index, detected_orfs, features, outfile, report_al
     accepts.  Every check runs before ``outfile`` is opened, so a refused input leaves no file; the refusals (a plain
     gzip input, a line without 18 fields, an unknown ORF_ID, a malformed profile) raise ValueError naming the file and
     the line.  ``stage_ms``, when given, receives the time of every stage in milliseconds.  Returns a summary dict."""
-    from .bgzf import open_texts
     from .detect_orfs import get_engine
 
-    times = {} if stage_ms is None else stage_ms
-    clock = time.perf_counter()
-
-    def lap(name):
-        nonlocal clock
-        now = time.perf_counter()
-        times[name] = (now - clock) * 1e3
-        clock = now
-
-    index_src, tsv_src = open_texts([ribotricer_index, detected_orfs], "count-orfs")
-    lap("inflate")
-    idx = load_native_index(index_src)
-    lap("index_load")
-    inp = CodonInput(idx, tsv_src, features, report_all)
-    lap("tsv_load")
+    clock = StageClock(stage_ms)
+    idx, inp, _ = _open_selection(clock, "count-orfs", ribotricer_index, detected_orfs, features, report_all)
     dev_ms = np.zeros(_lib.RT_COUNT_STAGES, np.float32)
     total, length, summary = get_engine().orf_counts(inp.sel, inp.text(0), idx.exon_ptr, idx.exon_start, idx.exon_end,
                                                      idx.orf_strand_code, inp.n_gene, stage_ms=dev_ms)
-    lap("orf_counts")
-    for name, ms in zip(("host_gather", "upload", "count_emit_kernel", "sort", "count_keep_kernel", "copy_back"),
-                        dev_ms.tolist()):
-        times["device:" + name] = ms
-    bad = int(summary[2])
-    if bad >= 0:
-        reason = next(text for bit, text in _PROFILE_REFUSALS if int(summary[3]) & bit)
-        raise ValueError(f"{detected_orfs} line {int(inp.sel['line'][bad])}: {reason}")
+    clock.lap("orf_counts")
+    clock.device(("host_gather", "upload", "count_emit_kernel", "sort", "count_keep_kernel", "copy_back"), dev_ms)
+    _raise_refused(detected_orfs, inp, summary[2:4])
     genes = np.flatnonzero(length)
     keys = [tuple(part.decode("utf-8") for part in inp.gene(int(g))) for g in genes]
     write_counts(outfile, keys, total[genes], length[genes])
-    lap("write")
+    clock.lap("write")
     return dict(rows=inp.n_sel, genes=len(keys), positions=int(summary[1]), duplicates=int(summary[0] - summary[1]))
 
 
@@ -247,8 +228,6 @@ class CodonInput:
     ``load_seq``, the checked orfs-seq nucleotide file (``rt_codon_load_seq``).  Rule violations raise ValueError."""
 
     def __init__(self, idx, detected_orfs, features, report_all: bool = False):
-        from .bgzf import NativeText
-
         self._lib = lib = _lib.load()
         self.idx = idx
         feats = [f.encode() for f in features]
@@ -281,8 +260,6 @@ class CodonInput:
 
     def load_seq(self, src) -> None:
         """The orfs-seq nucleotide file: a path or a ``bgzf.NativeText``."""
-        from .bgzf import NativeText
-
         if isinstance(src, NativeText):
             rc = self._lib.rt_codon_load_seq_text(self.handle, self.idx.handle, src.take(), src.path.encode())
         else:
@@ -327,48 +304,52 @@ _PROFILE_REFUSALS = ((1, "the profile is not a list of integers written as str(l
                      (4, "a codon count exceeds 4294967295"))
 
 
+def _open_selection(clock, command, ribotricer_index, detected_orfs, features, report_all, *more):
+    """The input stage of count-orfs and count-orfs-codon: every input opened (``bgzf.open_texts``), the index loaded
+    and the selected TSV rows matched to it.  Returns (index, ``CodonInput``, the opened ``more`` inputs)."""
+    index_src, tsv_src, *more_src = open_texts([ribotricer_index, detected_orfs, *more], command)
+    clock.lap("inflate")
+    idx = load_native_index(index_src)
+    clock.lap("index_load")
+    inp = CodonInput(idx, tsv_src, features, report_all)
+    clock.lap("tsv_load")
+    return idx, inp, more_src
+
+
+def _raise_refused(detected_orfs, inp, refusal):
+    """A ValueError naming the TSV line of the first refused profile, when ``refusal`` (the first refused selected row,
+    -1 for none, and its reasons: the two summary fields of the emit kernel) names one."""
+    bad, bits = int(refusal[0]), int(refusal[1])
+    if bad >= 0:
+        reason = next(text for bit, text in _PROFILE_REFUSALS if bits & bit)
+        raise ValueError(f"{detected_orfs} line {int(inp.sel['line'][bad])}: {reason}")
+
+
 def count_orfs_codon(ribotricer_index, detected_orfs, features, ribotricer_index_fasta, prefix, report_all=False,
                      stage_ms: dict | None = None):
     """Write ``{prefix}_codon_counts_by_gene.tsv`` and ``{prefix}_codon_counts.tsv`` (DESIGN.md section 11) from the
     index, a detected-ORFs TSV and the orfs-seq nucleotide file of the same index.  ``features`` is a set of ORF types.
     Every check runs before either file is opened.  ``stage_ms``, when given, receives the time of every stage in
     milliseconds.  Returns a summary dict."""
-    from .bgzf import open_texts
     from .detect_orfs import get_engine
 
-    times = {} if stage_ms is None else stage_ms
-    clock = time.perf_counter()
-
-    def lap(name):
-        nonlocal clock
-        now = time.perf_counter()
-        times[name] = (now - clock) * 1e3
-        clock = now
-
-    index_src, tsv_src, seq_src = open_texts([ribotricer_index, detected_orfs, ribotricer_index_fasta], "count-orfs-codon")
-    lap("inflate")
-    idx = load_native_index(index_src)
-    lap("index_load")
-    inp = CodonInput(idx, tsv_src, features, report_all)
-    lap("tsv_load")
+    clock = StageClock(stage_ms)
+    idx, inp, (seq_src,) = _open_selection(clock, "count-orfs-codon", ribotricer_index, detected_orfs, features,
+                                           report_all, ribotricer_index_fasta)
     inp.load_seq(seq_src)
-    lap("seq_check")
+    clock.lap("seq_check")
     dev_ms = np.zeros(_lib.RT_CODON_STAGES, np.float32)
     gene_tab, pooled_tab, summary = get_engine().codon_counts(
         inp.sel, inp.text(0), inp.text(1), idx.exon_ptr, idx.exon_start, idx.exon_end, idx.orf_strand_code,
         inp.n_gene, inp.n_gseq, stage_ms=dev_ms)
-    lap("codon_counts")
-    for name, ms in zip(("host_gather", "upload", "codon_emit_kernel", "dedup", "count_sorts", "codon_stats_kernel",
-                         "copy_back"), dev_ms.tolist()):
-        times["device:" + name] = ms
-    bad = int(summary[4])
-    if bad >= 0:
-        reason = next(text for bit, text in _PROFILE_REFUSALS if int(summary[5]) & bit)
-        raise ValueError(f"{detected_orfs} line {int(inp.sel['line'][bad])}: {reason}")
+    clock.lap("codon_counts")
+    clock.device(("host_gather", "upload", "codon_emit_kernel", "dedup", "count_sorts", "codon_stats_kernel",
+                  "copy_back"), dev_ms)
+    _raise_refused(detected_orfs, inp, summary[4:6])
     gene_path, pooled_path = f"{prefix}_codon_counts_by_gene.tsv", f"{prefix}_codon_counts.tsv"
     pathlib.Path(os.path.dirname(os.path.abspath(gene_path))).mkdir(parents=True, exist_ok=True)
     inp.write(gene_tab, pooled_tab, gene_path, pooled_path)
-    lap("write")
+    clock.lap("write")
     genes = int(np.count_nonzero(gene_tab[:, 0].reshape(-1, 64).any(axis=1))) if inp.n_gene else 0
     result = dict(rows=inp.n_sel, genes=genes, codons=int(summary[3]), duplicates=int(summary[2]),
                   codons_with_n=int(summary[1]), gene_table=gene_path, codon_table=pooled_path)

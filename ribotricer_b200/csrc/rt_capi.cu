@@ -103,6 +103,13 @@ struct Event {
     operator cudaEvent_t() const { return e; }
 };
 
+// stage_ms[k] = the time from ev[k] to ev[k + 1] for k < n: consecutive events bound consecutive stages.
+cudaError_t stage_times(const Event* ev, int n, float* stage_ms) {
+    for (int k = 0; k < n; ++k)
+        if (cudaError_t e = cudaEventElapsedTime(&stage_ms[k], ev[k], ev[k + 1])) return e;
+    return cudaSuccess;
+}
+
 }  // namespace
 
 struct rt_ctx {
@@ -1776,8 +1783,7 @@ int rt_orf_search(rt_ctx* ctx, const rt_orf_query* q, int64_t* n_rows, int64_t* 
     if (rows) RT_CUDA(ctx, intervals(false));
     RT_CUDA(ctx, cudaEventRecord(ev[7], st));
     RT_CUDA(ctx, cudaStreamSynchronize(st));
-    if (stage_ms)
-        for (int i = 0; i < RT_ORF_STAGES; ++i) RT_CUDA(ctx, cudaEventElapsedTime(&stage_ms[i], ev[i], ev[i + 1]));
+    if (stage_ms) RT_CUDA(ctx, stage_times(ev, RT_ORF_STAGES, stage_ms));
     ctx->orf_rows = rows;
     *n_rows = rows;
     *n_iv = ivs;
@@ -1987,20 +1993,128 @@ int rt_orf_seq_write(rt_ctx* ctx, const rt_seq_query* q, const char* path, float
     return rc;
 }
 
-// ---------------------------------------------------------------------------------------------- count-orfs-codon
+// ---------------------------------------------------------------------- selected detected-ORF rows, count-orfs-codon
 }  // extern "C"
 
 namespace {
-// The stream, events and device buffers of one rt_codon_counts call; everything is freed on every return.
+// The selected rows of a detected-ORFs TSV (rt_codon_load_tsv), the half rt_codon_counts and rt_count_orfs share.
+// scan<slot_nt>() checks the query fields both take and scans per row its profile text, its length in nt and its slots
+// of slot_nt nt; gather() copies the profile text together on all cores; reserve() and upload() put it on the device with
+// the rows' index intervals for the emit kernels (rt::RowArgs); read_refusal() reads back the first refused row.
+struct SelectedRows {
+    rt_count_query q{};
+    int64_t n = 0, n_ex = 0;
+    HostArr<int64_t> prof_base, len_base, slot_base;         // n + 1 each
+    HostArr<char> prof;
+    DevArr<char> d_prof;
+    DevArr<long long> d_prof_base, d_len_base, d_row, d_ex_ptr;
+    DevArr<int> d_gene, d_ex_start, d_ex_end;
+    DevArr<uint8_t> d_strand, d_flag;
+    DevArr<unsigned> d_claim;
+
+    template <int slot_nt>
+    int scan(rt_ctx* ctx, const char* who, const rt_count_query& query) {
+        q = query;
+        if (q.n_sel < 0 || q.n_orf < 0 || q.n_gene < 0 ||
+            (q.n_sel && (!q.row || !q.gene || !q.prof_off || !q.prof_len || !q.tsv || !q.exon_ptr || !q.orf_strand)))
+            return fail(ctx, RT_EINVAL, "%s: NULL or negative argument", who);
+        n = q.n_sel;
+        n_ex = n ? q.exon_ptr[q.n_orf] : 0;
+        if (!prof_base.alloc((size_t)n + 1) || !len_base.alloc((size_t)n + 1) || !slot_base.alloc((size_t)n + 1))
+            return fail(ctx, RT_ENOMEM, "%s: out of host memory", who);
+        prof_base[0] = len_base[0] = slot_base[0] = 0;
+        for (int64_t i = 0; i < n; ++i) {
+            const int64_t r = q.row[i];
+            if (r < 0 || r >= q.n_orf || q.gene[i] < 0 || q.gene[i] >= q.n_gene)
+                return fail(ctx, RT_EINVAL, "%s: selected row %lld lies outside the index or the gene table", who, (long long)i);
+            int64_t L = 0;
+            for (int64_t e = q.exon_ptr[r]; e < q.exon_ptr[r + 1]; ++e) L += (int64_t)q.exon_end[e] - q.exon_start[e] + 1;
+            prof_base[(size_t)i + 1] = prof_base[(size_t)i] + q.prof_len[i];
+            len_base[(size_t)i + 1] = len_base[(size_t)i] + L;
+            slot_base[(size_t)i + 1] = slot_base[(size_t)i] + L / slot_nt;
+        }
+        return RT_OK;
+    }
+    int64_t slots() const { return slot_base[(size_t)n]; }
+
+    // also(i) runs for every row i in the same pass; also_bytes is what it copies in all.
+    template <class F>
+    int gather(rt_ctx* ctx, const char* who, int64_t also_bytes, F&& also) {
+        if (!prof.alloc((size_t)prof_base[(size_t)n])) return fail(ctx, RT_ENOMEM, "%s: out of host memory", who);
+        const int64_t block = 1 << 10;
+        claim_parallel(host_threads((size_t)((prof_base[(size_t)n] + also_bytes) >> 22) + 1, 32),
+                       (size_t)((n + block - 1) / block), [&](size_t bk) {
+            for (int64_t i = (int64_t)bk * block; i < std::min(n, (int64_t)(bk + 1) * block); ++i) {
+                memcpy(prof.p + prof_base[(size_t)i], q.tsv + q.prof_off[i], (size_t)q.prof_len[i]);
+                also(i);
+            }
+        });
+        return RT_OK;
+    }
+
+    int reserve(rt_ctx* ctx) {
+        const size_t nn = (size_t)n, no = (size_t)q.n_orf, ne = (size_t)n_ex;
+        RT_CUDA(ctx, d_prof.reserve(prof.size()));
+        RT_CUDA(ctx, d_prof_base.reserve(nn + 1));
+        RT_CUDA(ctx, d_len_base.reserve(nn + 1));
+        RT_CUDA(ctx, d_row.reserve(nn));
+        RT_CUDA(ctx, d_gene.reserve(nn));
+        RT_CUDA(ctx, d_ex_ptr.reserve(no + 1));
+        RT_CUDA(ctx, d_ex_start.reserve(ne));
+        RT_CUDA(ctx, d_ex_end.reserve(ne));
+        RT_CUDA(ctx, d_strand.reserve(no));
+        RT_CUDA(ctx, d_flag.reserve(nn));
+        RT_CUDA(ctx, d_claim.reserve(1));
+        return RT_OK;
+    }
+
+    int upload(rt_ctx* ctx, cudaStream_t st) {
+        const size_t nn = (size_t)n, no = (size_t)q.n_orf, ne = (size_t)n_ex;
+        RT_CUDA(ctx, d_prof.upload(prof.p, prof.size(), st));
+        RT_CUDA(ctx, d_prof_base.upload(prof_base.data(), nn + 1, st));
+        RT_CUDA(ctx, d_len_base.upload(len_base.data(), nn + 1, st));
+        RT_CUDA(ctx, d_row.upload(q.row, nn, st));
+        RT_CUDA(ctx, d_gene.upload(q.gene, nn, st));
+        if (n) {
+            RT_CUDA(ctx, d_ex_ptr.upload(q.exon_ptr, no + 1, st));
+            RT_CUDA(ctx, d_ex_start.upload(q.exon_start, ne, st));
+            RT_CUDA(ctx, d_ex_end.upload(q.exon_end, ne, st));
+            RT_CUDA(ctx, d_strand.upload(q.orf_strand, no, st));
+        }
+        RT_CUDA(ctx, cudaMemsetAsync(d_claim.p, 0, sizeof(unsigned), st));
+        return RT_OK;
+    }
+
+    rt::RowArgs args() const {
+        return {d_prof.p, d_prof_base.p, d_len_base.p, d_row.p, d_ex_ptr.p, d_ex_start.p, d_ex_end.p, d_strand.p, d_gene.p,
+                d_flag.p, (long long)n, d_claim.p};
+    }
+    // blocks of kCodonWarps warps, one warp a row, at most `cap` blocks
+    unsigned emit_grid(int64_t cap) const {
+        return (unsigned)std::max<int64_t>(1, std::min<int64_t>((n + rt::kCodonWarps - 1) / rt::kCodonWarps, cap));
+    }
+
+    // out[0] = first, the first refused row, and out[1] = its refusal bits
+    int read_refusal(rt_ctx* ctx, cudaStream_t st, unsigned long long first, int64_t* out) {
+        uint8_t f = 0;
+        RT_CUDA(ctx, cudaMemcpyAsync(&f, d_flag.p + first, 1, cudaMemcpyDeviceToHost, st));
+        RT_CUDA(ctx, cudaStreamSynchronize(st));
+        out[0] = (int64_t)first;
+        out[1] = f;
+        return RT_OK;
+    }
+};
+
+// The stream, events and buffers of one rt_codon_counts call; everything is freed on every return.
 struct CodonScratch {
     Stream st;
     Event ev[7];
-    DevArr<char> prof, seq, temp;
-    DevArr<long long> prof_base, seq_base, slot_base, row, ex_ptr;
-    DevArr<int> gene, gseq, ex_start, ex_end;
-    DevArr<uint8_t> strand, flag;
+    SelectedRows rows;                 // len_base: where the rows' letters start in `letters`
+    HostArr<char> letters;
+    DevArr<char> seq, temp;
+    DevArr<long long> slot_base;
+    DevArr<int> gseq;
     DevArr<unsigned long long> cnt, key, val, key2, val2, counters, gene_tab, pooled_tab;
-    DevArr<unsigned> claim;
     ~CodonScratch() { if (st) cudaStreamSynchronize(st); }
 };
 
@@ -2012,41 +2126,32 @@ extern "C" {
 int rt_codon_counts(rt_ctx* ctx, const rt_codon_query* q, uint64_t* gene_tab, uint64_t* pooled_tab, int64_t* summary,
                     float* stage_ms) {
     if (!ctx) return fail(nullptr, RT_EINVAL, "rt_codon_counts: ctx is NULL");
-    if (!q || !pooled_tab || !summary || q->n_sel < 0 || q->n_orf < 0 || q->n_gene < 0 || q->n_gseq < 0 ||
-        (q->n_sel && (!q->row || !q->gene || !q->gseq || !q->prof_off || !q->prof_len || !q->tsv || !q->seq_off || !q->seq ||
-                      !q->exon_ptr || !q->orf_strand)) || (q->n_gene && !gene_tab))
+    if (!q || !pooled_tab || !summary || q->n_gseq < 0 || (q->n_sel && (!q->gseq || !q->seq_off || !q->seq)) ||
+        (q->n_gene && !gene_tab))
         return fail(ctx, RT_EINVAL, "rt_codon_counts: NULL or negative argument");
     if (q->n_gene > (1 << 26))
         return fail(ctx, RT_EINVAL, "count-orfs-codon handles at most 2^26 genes; the selection has %d", q->n_gene);
+    DeviceGuard guard(ctx->device);
+    CodonScratch S;
+    SelectedRows& R = S.rows;
     const auto t_host = std::chrono::steady_clock::now();
-    const int64_t n = q->n_sel, n_ex = q->n_orf ? q->exon_ptr[q->n_orf] : 0;
-    // 1. host: per selected row its length, slots and the offsets of its profile text and letters
-    std::vector<int64_t> prof_base((size_t)n + 1, 0), seq_base((size_t)n + 1, 0), slot_base((size_t)n + 1, 0);
-    for (int64_t i = 0; i < n; ++i) {
-        const int64_t r = q->row[i];
-        if (r < 0 || r >= q->n_orf || q->gene[i] < 0 || q->gene[i] >= q->n_gene || q->gseq[i] < 0 || q->gseq[i] >= q->n_gseq)
-            return fail(ctx, RT_EINVAL, "rt_codon_counts: selected row %lld lies outside the index or the gene tables", (long long)i);
-        int64_t L = 0;
-        for (int64_t e = q->exon_ptr[r]; e < q->exon_ptr[r + 1]; ++e) L += (int64_t)q->exon_end[e] - q->exon_start[e] + 1;
-        prof_base[(size_t)i + 1] = prof_base[(size_t)i] + q->prof_len[i];
-        seq_base[(size_t)i + 1] = seq_base[(size_t)i] + L;
-        slot_base[(size_t)i + 1] = slot_base[(size_t)i] + L / 3;
-    }
-    const int64_t n_slot = slot_base[(size_t)n];
+    // 1. host: per selected row its profile text, length and codons, and its letters
+    if (int rc = R.scan<3>(ctx, "rt_codon_counts", {q->n_sel, q->row, q->gene, q->prof_off, q->prof_len, q->tsv, q->n_orf,
+                                                    q->exon_ptr, q->exon_start, q->exon_end, q->orf_strand, q->n_gene}))
+        return rc;
+    const int64_t n = R.n, n_slot = R.slots();
+    for (int64_t i = 0; i < n; ++i)
+        if (q->gseq[i] < 0 || q->gseq[i] >= q->n_gseq)
+            return fail(ctx, RT_EINVAL, "rt_codon_counts: selected row %lld lies outside the gene tables", (long long)i);
     if (n_slot > (int64_t)0xffffffffll)
         return fail(ctx, RT_EINVAL, "count-orfs-codon handles at most 2^32 - 1 codons; the selection has %lld", (long long)n_slot);
-    // the profile text and the letters of the selected rows, gathered by all cores
-    HostArr<char> prof, letters;
-    if (!prof.alloc((size_t)prof_base[(size_t)n]) || !letters.alloc((size_t)seq_base[(size_t)n]))
-        return fail(ctx, RT_ENOMEM, "rt_codon_counts: out of host memory");
-    const int64_t block = 1 << 10;
-    claim_parallel(host_threads((size_t)((prof_base[(size_t)n] + seq_base[(size_t)n]) >> 22) + 1, 32),
-                   (size_t)((n + block - 1) / block), [&](size_t bk) {
-        for (int64_t i = (int64_t)bk * block; i < std::min(n, (int64_t)(bk + 1) * block); ++i) {
-            memcpy(prof.p + prof_base[(size_t)i], q->tsv + q->prof_off[i], (size_t)q->prof_len[i]);
-            memcpy(letters.p + seq_base[(size_t)i], q->seq + q->seq_off[q->row[i]], (size_t)(seq_base[(size_t)i + 1] - seq_base[(size_t)i]));
-        }
-    });
+    const int64_t* seq_base = R.len_base.data();
+    if (!S.letters.alloc((size_t)seq_base[(size_t)n])) return fail(ctx, RT_ENOMEM, "rt_codon_counts: out of host memory");
+    if (int rc = R.gather(ctx, "rt_codon_counts", seq_base[(size_t)n], [&](int64_t i) {
+            memcpy(S.letters.p + seq_base[(size_t)i], q->seq + q->seq_off[q->row[i]],
+                   (size_t)(seq_base[(size_t)i + 1] - seq_base[(size_t)i]));
+        }))
+        return rc;
     if (stage_ms) {
         for (int k = 0; k < RT_CODON_STAGES; ++k) stage_ms[k] = 0.f;
         stage_ms[0] = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_host).count();
@@ -2054,61 +2159,36 @@ int rt_codon_counts(rt_ctx* ctx, const rt_codon_query* q, uint64_t* gene_tab, ui
     for (int k = 0; k < 6; ++k) summary[k] = 0;
     summary[4] = -1;
     // 2. uploads
-    DeviceGuard guard(ctx->device);
-    CodonScratch S;
     RT_CUDA(ctx, S.st.create());
     for (auto& e : S.ev) RT_CUDA(ctx, e.create());
-    const size_t ns = (size_t)n_slot, nn = (size_t)n, no = (size_t)q->n_orf, ne = (size_t)n_ex;
-    RT_CUDA(ctx, S.prof.reserve(prof.size()));
-    RT_CUDA(ctx, S.seq.reserve(letters.size()));
-    RT_CUDA(ctx, S.prof_base.reserve(nn + 1));
-    RT_CUDA(ctx, S.seq_base.reserve(nn + 1));
+    const size_t ns = (size_t)n_slot, nn = (size_t)n;
+    if (int rc = R.reserve(ctx)) return rc;
+    RT_CUDA(ctx, S.seq.reserve(S.letters.size()));
     RT_CUDA(ctx, S.slot_base.reserve(nn + 1));
-    RT_CUDA(ctx, S.row.reserve(nn));
-    RT_CUDA(ctx, S.gene.reserve(nn));
     RT_CUDA(ctx, S.gseq.reserve(nn));
-    RT_CUDA(ctx, S.ex_ptr.reserve(no + 1));
-    RT_CUDA(ctx, S.ex_start.reserve(ne));
-    RT_CUDA(ctx, S.ex_end.reserve(ne));
-    RT_CUDA(ctx, S.strand.reserve(no));
     RT_CUDA(ctx, S.cnt.reserve(ns));
     RT_CUDA(ctx, S.key.reserve(ns));
     RT_CUDA(ctx, S.val.reserve(ns));
     RT_CUDA(ctx, S.key2.reserve(ns));
     RT_CUDA(ctx, S.val2.reserve(ns));
     RT_CUDA(ctx, S.counters.reserve(4));
-    RT_CUDA(ctx, S.flag.reserve(nn));
-    RT_CUDA(ctx, S.claim.reserve(1));
     RT_CUDA(ctx, S.gene_tab.reserve(RT_CODON_CELL * 64 * (size_t)q->n_gene));
     RT_CUDA(ctx, S.pooled_tab.reserve(RT_CODON_CELL * 64));
     RT_CUDA(ctx, cudaEventRecord(S.ev[0], S.st));
-    RT_CUDA(ctx, S.prof.upload(prof.p, prof.size(), S.st));
-    RT_CUDA(ctx, S.seq.upload(letters.p, letters.size(), S.st));
-    RT_CUDA(ctx, S.prof_base.upload(prof_base.data(), nn + 1, S.st));
-    RT_CUDA(ctx, S.seq_base.upload(seq_base.data(), nn + 1, S.st));
-    RT_CUDA(ctx, S.slot_base.upload(slot_base.data(), nn + 1, S.st));
-    RT_CUDA(ctx, S.row.upload(q->row, nn, S.st));
-    RT_CUDA(ctx, S.gene.upload(q->gene, nn, S.st));
+    if (int rc = R.upload(ctx, S.st)) return rc;
+    RT_CUDA(ctx, S.seq.upload(S.letters.p, S.letters.size(), S.st));
+    RT_CUDA(ctx, S.slot_base.upload(R.slot_base.data(), nn + 1, S.st));
     RT_CUDA(ctx, S.gseq.upload(q->gseq, nn, S.st));
-    if (n) {
-        RT_CUDA(ctx, S.ex_ptr.upload(q->exon_ptr, no + 1, S.st));
-        RT_CUDA(ctx, S.ex_start.upload(q->exon_start, ne, S.st));
-        RT_CUDA(ctx, S.ex_end.upload(q->exon_end, ne, S.st));
-        RT_CUDA(ctx, S.strand.upload(q->orf_strand, no, S.st));
-    }
     const unsigned long long counters0[4] = {0, 0, ~0ull, 0};
     RT_CUDA(ctx, S.counters.upload(counters0, 4, S.st));
     RT_CUDA(ctx, cudaMemsetAsync(S.cnt.p, 0, sizeof(unsigned long long) * ns, S.st));
-    RT_CUDA(ctx, cudaMemsetAsync(S.claim.p, 0, sizeof(unsigned), S.st));
     RT_CUDA(ctx, cudaEventRecord(S.ev[1], S.st));
     // 3. codon_emit_kernel
     unsigned long long *cnt = S.cnt.p, *key = S.key.p, *val = S.val.p, *key2 = S.key2.p, *val2 = S.val2.p, *counters = S.counters.p;
-    const rt::CodonArgs A{S.prof.p, S.prof_base.p, S.seq.p, S.seq_base.p, S.slot_base.p, S.row.p, S.ex_ptr.p, S.ex_start.p,
-                          S.ex_end.p, S.strand.p, S.gene.p, S.gseq.p, cnt, key, val, counters, S.flag.p, (long long)n, S.claim.p};
+    const rt::CodonArgs A{R.args(), S.seq.p, S.slot_base.p, S.gseq.p, cnt, key, val, counters};
     const int64_t big = std::max(1, ctx->n_sm * 8);
     if (n) {
-        const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((n + rt::kCodonWarps - 1) / rt::kCodonWarps, big));
-        rt::codon_emit_kernel<<<grid, rt::kCodonWarps * 32, 0, S.st>>>(A);
+        rt::codon_emit_kernel<<<R.emit_grid(big), rt::kCodonWarps * 32, 0, S.st>>>(A);
         ctx->launches++;
         RT_CUDA(ctx, cudaGetLastError());
     }
@@ -2119,12 +2199,8 @@ int rt_codon_counts(rt_ctx* ctx, const rt_codon_query* q, uint64_t* gene_tab, ui
     summary[0] = (int64_t)h_counters[0];
     summary[1] = (int64_t)h_counters[1];
     if (h_counters[2] != ~0ull) {                      // a refused profile: no tables
-        uint8_t f = 0;
-        RT_CUDA(ctx, cudaMemcpyAsync(&f, S.flag.p + h_counters[2], 1, cudaMemcpyDeviceToHost, S.st));
-        RT_CUDA(ctx, cudaStreamSynchronize(S.st));
-        summary[4] = (int64_t)h_counters[2];
-        summary[5] = f;
-        if (stage_ms) RT_CUDA(ctx, cudaEventElapsedTime(&stage_ms[1], S.ev[0], S.ev[1]));
+        if (int rc = R.read_refusal(ctx, S.st, h_counters[2], summary + 4)) return rc;
+        if (stage_ms) RT_CUDA(ctx, stage_times(S.ev, 1, stage_ms + 1));
         return RT_OK;
     }
     // 4. dedup: stable sort by place, keep the first slot of every place
@@ -2175,8 +2251,7 @@ int rt_codon_counts(rt_ctx* ctx, const rt_codon_query* q, uint64_t* gene_tab, ui
     RT_CUDA(ctx, cudaMemcpyAsync(pooled_tab, ptab, 8 * RT_CODON_CELL * 64, cudaMemcpyDeviceToHost, S.st));
     RT_CUDA(ctx, cudaEventRecord(S.ev[6], S.st));
     RT_CUDA(ctx, cudaStreamSynchronize(S.st));
-    if (stage_ms)
-        for (int k = 1; k < RT_CODON_STAGES; ++k) RT_CUDA(ctx, cudaEventElapsedTime(&stage_ms[k], S.ev[k - 1], S.ev[k]));
+    if (stage_ms) RT_CUDA(ctx, stage_times(S.ev, RT_CODON_STAGES - 1, stage_ms + 1));
     return RT_OK;
 }
 
@@ -2184,16 +2259,14 @@ int rt_codon_counts(rt_ctx* ctx, const rt_codon_query* q, uint64_t* gene_tab, ui
 
 // ---------------------------------------------------------------------------------------------------- count-orfs
 namespace {
-// The stream, events and device buffers of one rt_count_orfs call; everything is freed on every return.
+// The stream, events and buffers of one rt_count_orfs call; everything is freed on every return.
 struct CountScratch {
     Stream st;
     Event ev[6];
-    DevArr<char> prof, temp;
-    DevArr<long long> prof_base, slot_base, row, ex_ptr;
-    DevArr<int> gene, ex_start, ex_end;
-    DevArr<uint8_t> strand, flag;
+    SelectedRows rows;                 // len_base: the slots of every row, one a nt
+    DevArr<char> temp;
     DevArr<unsigned long long> key, key2, counters, total, length;
-    DevArr<unsigned> val, val2, claim;
+    DevArr<unsigned> val, val2;
     ~CountScratch() { if (st) cudaStreamSynchronize(st); }
 };
 }  // namespace
@@ -2203,34 +2276,19 @@ extern "C" {
 int rt_count_orfs(rt_ctx* ctx, const rt_count_query* q, uint64_t* total, uint64_t* length, int64_t* summary,
                   float* stage_ms) {
     if (!ctx) return fail(nullptr, RT_EINVAL, "rt_count_orfs: ctx is NULL");
-    if (!q || !summary || q->n_sel < 0 || q->n_orf < 0 || q->n_gene < 0 ||
-        (q->n_sel && (!q->row || !q->gene || !q->prof_off || !q->prof_len || !q->tsv || !q->exon_ptr || !q->orf_strand)) ||
-        (q->n_gene && (!total || !length)))
+    if (!q || !summary || (q->n_gene && (!total || !length)))
         return fail(ctx, RT_EINVAL, "rt_count_orfs: NULL or negative argument");
+    DeviceGuard guard(ctx->device);
+    CountScratch S;
+    SelectedRows& R = S.rows;
     const auto t_host = std::chrono::steady_clock::now();
-    const int64_t n = q->n_sel, n_ex = q->n_orf ? q->exon_ptr[q->n_orf] : 0;
-    // 1. host: per selected line its row length and the offset of its profile text
-    std::vector<int64_t> prof_base((size_t)n + 1, 0), slot_base((size_t)n + 1, 0);
-    for (int64_t i = 0; i < n; ++i) {
-        const int64_t r = q->row[i];
-        if (r < 0 || r >= q->n_orf || q->gene[i] < 0 || q->gene[i] >= q->n_gene)
-            return fail(ctx, RT_EINVAL, "rt_count_orfs: selected line %lld lies outside the index or the gene table", (long long)i);
-        int64_t L = 0;
-        for (int64_t e = q->exon_ptr[r]; e < q->exon_ptr[r + 1]; ++e) L += (int64_t)q->exon_end[e] - q->exon_start[e] + 1;
-        prof_base[(size_t)i + 1] = prof_base[(size_t)i] + q->prof_len[i];
-        slot_base[(size_t)i + 1] = slot_base[(size_t)i] + L;
-    }
-    const int64_t n_slot = slot_base[(size_t)n];
+    // 1. host: per selected line its profile text and row length
+    if (int rc = R.scan<1>(ctx, "rt_count_orfs", *q)) return rc;
+    const int64_t n = R.n, n_slot = R.slots();
     if (n_slot > (int64_t)0xffffffffll)
         return fail(ctx, RT_EINVAL, "count-orfs handles at most 2^32 - 1 nt in the selected rows; the selection has %lld",
                     (long long)n_slot);
-    HostArr<char> prof;
-    if (!prof.alloc((size_t)prof_base[(size_t)n])) return fail(ctx, RT_ENOMEM, "rt_count_orfs: out of host memory");
-    const int64_t block = 1 << 10;
-    claim_parallel(host_threads((size_t)(prof_base[(size_t)n] >> 22) + 1, 32), (size_t)((n + block - 1) / block), [&](size_t bk) {
-        for (int64_t i = (int64_t)bk * block; i < std::min(n, (int64_t)(bk + 1) * block); ++i)
-            memcpy(prof.p + prof_base[(size_t)i], q->tsv + q->prof_off[i], (size_t)q->prof_len[i]);
-    });
+    if (int rc = R.gather(ctx, "rt_count_orfs", 0, [](int64_t) {})) return rc;
     if (stage_ms) {
         for (int k = 0; k < RT_COUNT_STAGES; ++k) stage_ms[k] = 0.f;
         stage_ms[0] = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_host).count();
@@ -2238,27 +2296,15 @@ int rt_count_orfs(rt_ctx* ctx, const rt_count_query* q, uint64_t* total, uint64_
     for (int k = 0; k < 4; ++k) summary[k] = 0;
     summary[2] = -1;
     // 2. uploads
-    DeviceGuard guard(ctx->device);
-    CountScratch S;
     RT_CUDA(ctx, S.st.create());
     for (auto& e : S.ev) RT_CUDA(ctx, e.create());
-    const size_t ns = (size_t)n_slot, nn = (size_t)n, no = (size_t)q->n_orf, ne = (size_t)n_ex, ng = (size_t)q->n_gene;
-    RT_CUDA(ctx, S.prof.reserve(prof.size()));
-    RT_CUDA(ctx, S.prof_base.reserve(nn + 1));
-    RT_CUDA(ctx, S.slot_base.reserve(nn + 1));
-    RT_CUDA(ctx, S.row.reserve(nn));
-    RT_CUDA(ctx, S.gene.reserve(nn));
-    RT_CUDA(ctx, S.ex_ptr.reserve(no + 1));
-    RT_CUDA(ctx, S.ex_start.reserve(ne));
-    RT_CUDA(ctx, S.ex_end.reserve(ne));
-    RT_CUDA(ctx, S.strand.reserve(no));
+    const size_t ns = (size_t)n_slot, ng = (size_t)q->n_gene;
+    if (int rc = R.reserve(ctx)) return rc;
     RT_CUDA(ctx, S.key.reserve(ns));
     RT_CUDA(ctx, S.key2.reserve(ns));
     RT_CUDA(ctx, S.val.reserve(ns));
     RT_CUDA(ctx, S.val2.reserve(ns));
     RT_CUDA(ctx, S.counters.reserve(2));
-    RT_CUDA(ctx, S.flag.reserve(nn));
-    RT_CUDA(ctx, S.claim.reserve(1));
     RT_CUDA(ctx, S.total.reserve(ng));
     RT_CUDA(ctx, S.length.reserve(ng));
     // the sort looks at the key bits in use: 32 of coordinate and those of the largest gene id, n_gene - 1.  A dropped
@@ -2271,30 +2317,17 @@ int rt_count_orfs(rt_ctx* ctx, const rt_count_query* q, uint64_t* total, uint64_
                                                  key_bits, S.st.s));
     RT_CUDA(ctx, S.temp.reserve(temp_bytes));
     RT_CUDA(ctx, cudaEventRecord(S.ev[0], S.st));
-    RT_CUDA(ctx, S.prof.upload(prof.p, prof.size(), S.st));
-    RT_CUDA(ctx, S.prof_base.upload(prof_base.data(), nn + 1, S.st));
-    RT_CUDA(ctx, S.slot_base.upload(slot_base.data(), nn + 1, S.st));
-    RT_CUDA(ctx, S.row.upload(q->row, nn, S.st));
-    RT_CUDA(ctx, S.gene.upload(q->gene, nn, S.st));
-    if (n) {
-        RT_CUDA(ctx, S.ex_ptr.upload(q->exon_ptr, no + 1, S.st));
-        RT_CUDA(ctx, S.ex_start.upload(q->exon_start, ne, S.st));
-        RT_CUDA(ctx, S.ex_end.upload(q->exon_end, ne, S.st));
-        RT_CUDA(ctx, S.strand.upload(q->orf_strand, no, S.st));
-    }
+    if (int rc = R.upload(ctx, S.st)) return rc;
     const unsigned long long counters0[2] = {0, ~0ull};
     RT_CUDA(ctx, S.counters.upload(counters0, 2, S.st));
-    RT_CUDA(ctx, cudaMemsetAsync(S.claim.p, 0, sizeof(unsigned), S.st));
     RT_CUDA(ctx, cudaMemsetAsync(S.total.p, 0, sizeof(unsigned long long) * ng, S.st));
     RT_CUDA(ctx, cudaMemsetAsync(S.length.p, 0, sizeof(unsigned long long) * ng, S.st));
     RT_CUDA(ctx, cudaEventRecord(S.ev[1], S.st));
     // 3. count_emit_kernel
-    const rt::CountArgs A{S.prof.p, S.prof_base.p, S.slot_base.p, S.row.p, S.ex_ptr.p, S.ex_start.p, S.ex_end.p,
-                          S.strand.p, S.gene.p, S.key.p, S.val.p, S.counters.p, S.flag.p, (long long)n, S.claim.p};
+    const rt::CountArgs A{R.args(), S.key.p, S.val.p, S.counters.p};
     const int64_t big = std::max(1, ctx->n_sm * 8);
     if (n) {
-        const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((n + rt::kCodonWarps - 1) / rt::kCodonWarps, big));
-        rt::count_emit_kernel<<<grid, rt::kCodonWarps * 32, 0, S.st>>>(A);
+        rt::count_emit_kernel<<<R.emit_grid(big), rt::kCodonWarps * 32, 0, S.st>>>(A);
         ctx->launches++;
         RT_CUDA(ctx, cudaGetLastError());
     }
@@ -2304,12 +2337,8 @@ int rt_count_orfs(rt_ctx* ctx, const rt_count_query* q, uint64_t* total, uint64_
     RT_CUDA(ctx, cudaStreamSynchronize(S.st));
     summary[0] = (int64_t)h_counters[0];
     if (h_counters[1] != ~0ull) {                      // a refused profile: no counts
-        uint8_t f = 0;
-        RT_CUDA(ctx, cudaMemcpyAsync(&f, S.flag.p + h_counters[1], 1, cudaMemcpyDeviceToHost, S.st));
-        RT_CUDA(ctx, cudaStreamSynchronize(S.st));
-        summary[2] = (int64_t)h_counters[1];
-        summary[3] = f;
-        if (stage_ms) RT_CUDA(ctx, cudaEventElapsedTime(&stage_ms[1], S.ev[0], S.ev[1]));
+        if (int rc = R.read_refusal(ctx, S.st, h_counters[1], summary + 2)) return rc;
+        if (stage_ms) RT_CUDA(ctx, stage_times(S.ev, 1, stage_ms + 1));
         return RT_OK;
     }
     // 4. stable sort by key: slots are in (line, oriented nt) order, so the first slot of every key is the first pair
@@ -2335,8 +2364,7 @@ int rt_count_orfs(rt_ctx* ctx, const rt_count_query* q, uint64_t* total, uint64_
     uint64_t kept = 0;
     for (size_t g = 0; g < ng; ++g) kept += length[g];
     summary[1] = (int64_t)kept;
-    if (stage_ms)
-        for (int k = 1; k < RT_COUNT_STAGES; ++k) RT_CUDA(ctx, cudaEventElapsedTime(&stage_ms[k], S.ev[k - 1], S.ev[k]));
+    if (stage_ms) RT_CUDA(ctx, stage_times(S.ev, RT_COUNT_STAGES - 1, stage_ms + 1));
     return RT_OK;
 }
 

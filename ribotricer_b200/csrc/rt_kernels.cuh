@@ -2594,6 +2594,14 @@ struct SeqArgs {
     unsigned* claim;                  // work counter, zeroed before every launch
 };
 
+// The warp's next item t < n from a work counter (lane 0 claims it, the warp shares it); false when none is left.
+__device__ __forceinline__ bool warp_claim(unsigned* counter, long long n, unsigned& t) {
+    t = 0;
+    if ((threadIdx.x & 31) == 0) t = atomicAdd(counter, 1u);
+    t = __shfl_sync(kFull, t, 0);
+    return (long long)t < n;
+}
+
 constexpr int kSeqWarps = 8;
 constexpr int kSeqWindow = 3 * 32 * 8;
 
@@ -2610,11 +2618,7 @@ __global__ void __launch_bounds__(kSeqWarps * 32) orf_seq_kernel(SeqArgs A, long
     }
     uint8_t* win = window[Protein ? threadIdx.x >> 5 : 0];
     const long long base = A.line_off[row_lo];
-    for (;;) {
-        unsigned t = 0;
-        if (lane == 0) t = atomicAdd(A.claim, 1u);
-        t = __shfl_sync(kFull, t, 0);
-        if ((long long)t >= n_rows) return;
+    for (unsigned t; warp_claim(A.claim, n_rows, t);) {
         const long long r = row_lo + t;
         char* o = out + (A.line_off[r] - base);
         const long long i0 = A.id_off[r], n_id = A.id_off[r + 1] - i0;
@@ -2686,6 +2690,58 @@ __global__ void __launch_bounds__(kSeqWarps * 32) orf_seq_kernel(SeqArgs A, long
     }
 }
 
+// ---------------------------------------------------------------------------------- selected detected-ORF rows
+// The selected rows of a detected-ORFs TSV as codon_emit_kernel and count_emit_kernel read them: one warp per row,
+// claimed dynamically (profiles run from "[]" to more than 100 knt).
+struct RowArgs {
+    const char* prof;                 // profile text of the selected rows, back to back
+    const long long* prof_base;       // n_sel + 1
+    const long long* len_base;        // n_sel + 1: row lengths in nt, scanned
+    const long long* row;             // index row of each selected row
+    const long long* exon_ptr;
+    const int* ex_start;
+    const int* ex_end;
+    const uint8_t* strand;            // per index row, 1: reverse
+    const int* gene;
+    uint8_t* flag;                    // per selected row: its refusal bits (1 malformed, 2 value above 2^31 - 1, ...)
+    long long n_sel;
+    unsigned* claim;                  // work counter, zeroed before the launch
+};
+
+// Refuses selected row t with `bits`: sets its flag and takes part in the atomicMin of the first refused row, *first.
+__device__ __forceinline__ void refuse_row(uint8_t* flag, unsigned long long* first, unsigned t, unsigned bits) {
+    flag[t] = (uint8_t)bits;
+    atomicMin(first, (unsigned long long)t);
+}
+
+// Per lane: the genomic coordinate of oriented nt k of a row of L nt, through the row's intervals.  The cursor keeps
+// interval e and the nt of the intervals left of it, `before` (ascending order); '-' rows walk the intervals from the
+// right.  A lane asks for ascending k.
+struct IntervalCursor {
+    const int* ex_start;
+    const int* ex_end;
+    long long L, e, before;
+    bool rev;
+    __device__ __forceinline__ IntervalCursor(const RowArgs& A, long long r, long long L_)
+        : ex_start(A.ex_start), ex_end(A.ex_end), L(L_) {
+        const long long e0 = A.exon_ptr[r], e1 = A.exon_ptr[r + 1];
+        rev = A.strand[r] == 1;
+        e = rev ? e1 - 1 : e0;
+        before = 0;
+        if (rev)
+            for (long long x = e0; x < e1 - 1; ++x) before += ex_end[x] - ex_start[x] + 1;
+    }
+    __device__ __forceinline__ int coord(long long k) {
+        const long long a = rev ? L - 1 - k : k;       // ascending index of oriented nt k
+        if (rev) {
+            while (a < before) { --e; before -= ex_end[e] - ex_start[e] + 1; }
+        } else {
+            while (a >= before + (ex_end[e] - ex_start[e] + 1)) { before += ex_end[e] - ex_start[e] + 1; ++e; }
+        }
+        return ex_start[e] + (int)(a - before);
+    }
+};
+
 // ---------------------------------------------------------------------------------------------- count-orfs-codon
 // codon_emit_kernel: one warp per selected TSV row, claimed dynamically (profiles run from "[]" to more than 100 knt).
 // The warp reads the profile text in 32-byte windows: every byte is checked against the grammar "[" (D(", "D)*)? "]"
@@ -2696,25 +2752,14 @@ __global__ void __launch_bounds__(kSeqWarps * 32) orf_seq_kernel(SeqArgs A, long
 // gseq << 32 | first nt and the value (gene * 64 + code) << 32 | count; a codon with N, or past the profile, gets the key
 // ~0 (dropped).
 struct CodonArgs {
-    const char* prof;                 // profile text of the selected rows, back to back
-    const long long* prof_base;       // n_sel + 1
-    const char* seq;                  // their letters, back to back
-    const long long* seq_base;        // n_sel + 1: row lengths
+    RowArgs rows;                     // flag 4: a codon count above 2^32 - 1
+    const char* seq;                  // the rows' letters, back to back (at len_base)
     const long long* slot_base;       // n_sel + 1: floor(length / 3) slots per row
-    const long long* row;             // index row of each selected row
-    const long long* exon_ptr;
-    const int* ex_start;
-    const int* ex_end;
-    const uint8_t* strand;            // per index row, 1: reverse
-    const int* gene;
     const int* gseq;
     unsigned long long* cnt;          // per slot: codon count, zeroed before the launch
     unsigned long long* pos_key;      // per slot: place key
     unsigned long long* val;          // per slot: (gene * 64 + codon) << 32 | count
     unsigned long long* counters;     // [0] codons named, [1] with N, [2] first refused row (atomicMin), zeroed / ~0
-    uint8_t* flag;                    // per selected row: 1 malformed, 2 value above 2^31 - 1, 4 codon count above 2^32 - 1
-    long long n_sel;
-    unsigned* claim;                  // work counter, zeroed before the launch
 };
 
 constexpr int kCodonWarps = 8;
@@ -2764,15 +2809,12 @@ __device__ __forceinline__ unsigned profile_walk(const char* s, long long n, int
 }
 
 __global__ void __launch_bounds__(kCodonWarps * 32) codon_emit_kernel(const CodonArgs A) {
+    const RowArgs& R = A.rows;
     const int lane = threadIdx.x & 31;
-    for (;;) {
-        unsigned t = 0;
-        if (lane == 0) t = atomicAdd(A.claim, 1u);
-        t = __shfl_sync(kFull, t, 0);
-        if ((long long)t >= A.n_sel) return;
-        const char* s = A.prof + A.prof_base[t];
-        const long long n = A.prof_base[t + 1] - A.prof_base[t];
-        const long long L = A.seq_base[t + 1] - A.seq_base[t];
+    for (unsigned t; warp_claim(R.claim, R.n_sel, t);) {
+        const char* s = R.prof + R.prof_base[t];
+        const long long n = R.prof_base[t + 1] - R.prof_base[t];
+        const long long L = R.len_base[t + 1] - R.len_base[t];
         const long long s0 = A.slot_base[t], n_slot = A.slot_base[t + 1] - s0;
         long long P;                                       // values parsed
         unsigned bad = profile_walk(s, n, lane, P, [&](long long j, unsigned long long v) {
@@ -2781,25 +2823,14 @@ __global__ void __launch_bounds__(kCodonWarps * 32) codon_emit_kernel(const Codo
         bad = __reduce_or_sync(kFull, bad);
         __syncwarp();                                      // the counts of this row are in place (read through L2 below)
         if (bad) {
-            if (lane == 0) {
-                A.flag[t] = (uint8_t)bad;
-                atomicMin(A.counters + 2, (unsigned long long)t);
-            }
+            if (lane == 0) refuse_row(R.flag, A.counters + 2, t, bad);
             continue;
         }
         const long long n_cod = min(P, L) / 3;
-        const long long r = A.row[t], e0 = A.exon_ptr[r], e1 = A.exon_ptr[r + 1];
-        const bool rev = A.strand[r] == 1;
-        const char* letters = A.seq + A.seq_base[t];
-        const unsigned long long hi_gene = (unsigned long long)A.gene[t] * 64ull;
+        IntervalCursor cur(R, R.row[t], L);
+        const char* letters = A.seq + R.len_base[t];
+        const unsigned long long hi_gene = (unsigned long long)R.gene[t] * 64ull;
         const unsigned long long hi_place = (unsigned long long)(unsigned)A.gseq[t] << 32;
-        // per lane: interval cursor `e` and the nt of the intervals left of it, `before` (ascending order)
-        long long e = rev ? e1 - 1 : e0, before = 0;
-        if (rev) {
-            long long tail = 0;
-            for (long long x = e0; x < e1 - 1; ++x) tail += A.ex_end[x] - A.ex_start[x] + 1;
-            before = tail;
-        }
         unsigned named = 0, with_n = 0, over = 0;
         for (long long k = lane; k < n_slot; k += 32) {
             unsigned long long key = ~0ull, value = 0;
@@ -2819,14 +2850,7 @@ __global__ void __launch_bounds__(kCodonWarps * 32) codon_emit_kernel(const Codo
                 if (has_n) {
                     ++with_n;
                 } else {
-                    const long long a = rev ? L - 1 - 3 * k : 3 * k;      // ascending index of the first oriented nt
-                    if (rev) {
-                        while (a < before) { --e; before -= A.ex_end[e] - A.ex_start[e] + 1; }
-                    } else {
-                        while (a >= before + (A.ex_end[e] - A.ex_start[e] + 1)) { before += A.ex_end[e] - A.ex_start[e] + 1; ++e; }
-                    }
-                    const int pos = A.ex_start[e] + (int)(a - before);
-                    key = hi_place | (unsigned)pos;
+                    key = hi_place | (unsigned)cur.coord(3 * k);
                     value = (hi_gene + (unsigned long long)code) << 32 | (c & 0xffffffffull);
                 }
             }
@@ -2839,10 +2863,7 @@ __global__ void __launch_bounds__(kCodonWarps * 32) codon_emit_kernel(const Codo
         if (lane == 0) {
             if (named) atomicAdd(A.counters + 0, (unsigned long long)named);
             if (with_n) atomicAdd(A.counters + 1, (unsigned long long)with_n);
-            if (over) {
-                A.flag[t] = 4;
-                atomicMin(A.counters + 2, (unsigned long long)t);
-            }
+            if (over) refuse_row(R.flag, A.counters + 2, t, 4);
         }
     }
 }
@@ -2929,65 +2950,32 @@ __global__ void __launch_bounds__(256) codon_stats_kernel(const unsigned long lo
 // per-lane cursor ('-' rows walk them from the right); slots k in [m, L) get the key ~0 (dropped).  A refused line sets
 // its flag and takes part in an atomicMin of the first refused line.
 struct CountArgs {
-    const char* prof;                 // profile text of the selected lines, back to back
-    const long long* prof_base;       // n_sel + 1
-    const long long* slot_base;       // n_sel + 1: row lengths, scanned
-    const long long* row;             // index row of each selected line
-    const long long* exon_ptr;
-    const int* ex_start;
-    const int* ex_end;
-    const uint8_t* strand;            // per index row, 1: reverse
-    const int* gene;
-    unsigned long long* key;          // per slot
+    RowArgs rows;                     // flag: 1 malformed, 2 value above 2^31 - 1
+    unsigned long long* key;          // per slot (len_base)
     unsigned* val;                    // per slot
     unsigned long long* counters;     // [0] positions named (sum of m), [1] first refused line (atomicMin), zeroed / ~0
-    uint8_t* flag;                    // per selected line: 1 malformed, 2 value above 2^31 - 1
-    long long n_sel;
-    unsigned* claim;                  // work counter, zeroed before the launch
 };
 
 __global__ void __launch_bounds__(kCodonWarps * 32) count_emit_kernel(const CountArgs A) {
+    const RowArgs& R = A.rows;
     const int lane = threadIdx.x & 31;
-    for (;;) {
-        unsigned t = 0;
-        if (lane == 0) t = atomicAdd(A.claim, 1u);
-        t = __shfl_sync(kFull, t, 0);
-        if ((long long)t >= A.n_sel) return;
-        const long long s0 = A.slot_base[t], L = A.slot_base[t + 1] - s0;
+    for (unsigned t; warp_claim(R.claim, R.n_sel, t);) {
+        const long long s0 = R.len_base[t], L = R.len_base[t + 1] - s0;
         long long P;
-        unsigned bad = profile_walk(A.prof + A.prof_base[t], A.prof_base[t + 1] - A.prof_base[t], lane, P,
+        unsigned bad = profile_walk(R.prof + R.prof_base[t], R.prof_base[t + 1] - R.prof_base[t], lane, P,
                                     [&](long long j, unsigned long long v) {
             if (j < L) A.val[s0 + j] = (unsigned)v;
         });
         bad = __reduce_or_sync(kFull, bad);
         if (bad) {
-            if (lane == 0) {
-                A.flag[t] = (uint8_t)bad;
-                atomicMin(A.counters + 1, (unsigned long long)t);
-            }
+            if (lane == 0) refuse_row(R.flag, A.counters + 1, t, bad);
             continue;
         }
         const long long m = min(P, L);
-        const long long r = A.row[t], e0 = A.exon_ptr[r], e1 = A.exon_ptr[r + 1];
-        const bool rev = A.strand[r] == 1;
-        const unsigned long long hi = (unsigned long long)(unsigned)A.gene[t] << 32;
-        // per lane: interval cursor `e` and the nt of the intervals left of it, `before` (ascending order)
-        long long e = rev ? e1 - 1 : e0, before = 0;
-        if (rev)
-            for (long long x = e0; x < e1 - 1; ++x) before += A.ex_end[x] - A.ex_start[x] + 1;
-        for (long long k = lane; k < L; k += 32) {
-            unsigned long long key = ~0ull;
-            if (k < m) {
-                const long long a = rev ? L - 1 - k : k;   // ascending index of oriented nt k
-                if (rev) {
-                    while (a < before) { --e; before -= A.ex_end[e] - A.ex_start[e] + 1; }
-                } else {
-                    while (a >= before + (A.ex_end[e] - A.ex_start[e] + 1)) { before += A.ex_end[e] - A.ex_start[e] + 1; ++e; }
-                }
-                key = hi | (unsigned)(A.ex_start[e] + (int)(a - before));
-            }
-            A.key[s0 + k] = key;
-        }
+        IntervalCursor cur(R, R.row[t], L);
+        const unsigned long long hi = (unsigned long long)(unsigned)R.gene[t] << 32;
+        for (long long k = lane; k < L; k += 32)
+            A.key[s0 + k] = k < m ? hi | (unsigned)cur.coord(k) : ~0ull;
         if (lane == 0 && m) atomicAdd(A.counters + 0, (unsigned long long)m);
     }
 }

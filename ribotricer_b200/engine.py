@@ -107,6 +107,34 @@ class Engine:
     def _check(self, rc):
         _lib.check(rc, self.ctx)
 
+    def _command(self, fn, n_stages: int, stage_ms: np.ndarray | None, *args):
+        """``fn(ctx, *args, stage times)`` for a native command that checks its input: RT_EINVAL (a refused input)
+        raises ValueError with the command's message, any other error RtError.  ``stage_ms``, when given, receives the
+        ``n_stages`` stage times."""
+        ms = np.zeros(n_stages, np.float32)
+        rc = fn(self.ctx, *args, _np_ptr(ms))
+        if rc == _lib.RT_EINVAL:
+            raise ValueError(self.lib.rt_last_error(self.ctx).decode())
+        self._check(rc)
+        if stage_ms is not None:
+            stage_ms[:] = ms
+
+    _ROW_TYPES = dict(row=np.int64, gene=np.int32, gseq=np.int32, prof_off=np.int64, prof_len=np.int64, tsv=np.uint8,
+                      seq_off=np.int64, seq=np.uint8, exon_ptr=np.int64, exon_start=np.int32, exon_end=np.int32,
+                      orf_strand=np.uint8)
+
+    @classmethod
+    def _rows_query(cls, query_type, sel: dict, exon_ptr, exon_start, exon_end, orf_strand, texts: dict, **sizes):
+        """A ``query_type`` (``CodonQuery`` or ``CountQuery``) of the selected TSV rows: the columns of ``sel``, the
+        index intervals and the file ``texts`` that it names, contiguous in their C types (kept alive by the query as
+        ``arrays``), and the table ``sizes``."""
+        src = dict(sel, exon_ptr=exon_ptr, exon_start=exon_start, exon_end=exon_end, orf_strand=orf_strand, **texts)
+        arrays = {k: np.ascontiguousarray(src[k], cls._ROW_TYPES[k]) for k, _ in query_type._fields_ if k in cls._ROW_TYPES}
+        q = query_type(n_sel=len(arrays["row"]), n_orf=len(arrays["exon_ptr"]) - 1,
+                       **{k: int(v) for k, v in sizes.items()}, **{k: _np_ptr(a) for k, a in arrays.items()})
+        q.arrays = arrays
+        return q
+
     @property
     def launches(self) -> int:
         return int(self.lib.rt_launch_count(self.ctx))
@@ -493,13 +521,7 @@ class Engine:
                           _np_ptr(orf_contig), _np_ptr(orf_strand), len(contig_base), _np_ptr(contig_base),
                           _np_ptr(contig_len), _np_ptr(codes), len(codes), _np_ptr(id_off), _np_ptr(ids),
                           int(bool(protein)), int(chunk_bytes))
-        ms = np.zeros(_lib.RT_SEQ_STAGES, np.float32)
-        rc = self.lib.rt_orf_seq_write(self.ctx, C.byref(q), str(path).encode(), _np_ptr(ms))
-        if rc == _lib.RT_EINVAL:
-            raise ValueError(self.lib.rt_last_error(self.ctx).decode())
-        self._check(rc)
-        if stage_ms is not None:
-            stage_ms[:] = ms
+        self._command(self.lib.rt_orf_seq_write, _lib.RT_SEQ_STAGES, stage_ms, C.byref(q), str(path).encode())
 
     # --------------------------------------------------------------- count-orfs-codon
     def codon_counts(self, sel: dict, tsv, seq, exon_ptr, exon_start, exon_end, orf_strand, n_gene: int, n_gseq: int,
@@ -508,25 +530,13 @@ class Engine:
         TSV rows (``row``, ``gene``, ``gseq``, ``prof_off``, ``prof_len``) and ``seq_off`` per index row; ``tsv`` and
         ``seq`` are the two file texts (uint8).  Returns (gene table [n_gene * 64, 5], pooled table [64, 5], summary[6])
         as uint64 / int64 arrays: see ``rt_codon_counts`` in the header."""
-        arr = lambda a, dt: np.ascontiguousarray(a, dt)  # noqa: E731
-        row, gene, gseq = arr(sel["row"], np.int64), arr(sel["gene"], np.int32), arr(sel["gseq"], np.int32)
-        prof_off, prof_len, seq_off = arr(sel["prof_off"], np.int64), arr(sel["prof_len"], np.int64), arr(sel["seq_off"], np.int64)
-        exon_ptr, exon_start, exon_end = arr(exon_ptr, np.int64), arr(exon_start, np.int32), arr(exon_end, np.int32)
-        orf_strand = arr(orf_strand, np.uint8)
-        q = _lib.CodonQuery(len(row), _np_ptr(row), _np_ptr(gene), _np_ptr(gseq), _np_ptr(prof_off), _np_ptr(prof_len),
-                            _np_ptr(tsv), _np_ptr(seq_off), _np_ptr(seq), len(exon_ptr) - 1, _np_ptr(exon_ptr),
-                            _np_ptr(exon_start), _np_ptr(exon_end), _np_ptr(orf_strand), int(n_gene), int(n_gseq))
+        q = self._rows_query(_lib.CodonQuery, sel, exon_ptr, exon_start, exon_end, orf_strand, dict(tsv=tsv, seq=seq),
+                             n_gene=n_gene, n_gseq=n_gseq)
         gene_tab = np.zeros((64 * int(n_gene), _lib.RT_CODON_CELL), np.uint64)
         pooled_tab = np.zeros((64, _lib.RT_CODON_CELL), np.uint64)
         summary = np.zeros(6, np.int64)
-        ms = np.zeros(_lib.RT_CODON_STAGES, np.float32)
-        rc = self.lib.rt_codon_counts(self.ctx, C.byref(q), _np_ptr(gene_tab), _np_ptr(pooled_tab), _np_ptr(summary),
-                                      _np_ptr(ms))
-        if rc == _lib.RT_EINVAL:
-            raise ValueError(self.lib.rt_last_error(self.ctx).decode())
-        self._check(rc)
-        if stage_ms is not None:
-            stage_ms[:] = ms
+        self._command(self.lib.rt_codon_counts, _lib.RT_CODON_STAGES, stage_ms, C.byref(q), _np_ptr(gene_tab),
+                      _np_ptr(pooled_tab), _np_ptr(summary))
         return gene_tab, pooled_tab, summary
 
     # --------------------------------------------------------------- count-orfs
@@ -535,23 +545,12 @@ class Engine:
         """Per-gene read counts of DESIGN.md section 13 (``rt_count_orfs``).  ``sel`` holds the columns of the selected
         TSV lines (``row``, ``gene``, ``prof_off``, ``prof_len``); ``tsv`` is the file text (uint8).  Returns (total
         [n_gene], length [n_gene], summary[4]) as uint64 / int64 arrays: see ``rt_count_orfs`` in the header."""
-        arr = lambda a, dt: np.ascontiguousarray(a, dt)  # noqa: E731
-        row, gene = arr(sel["row"], np.int64), arr(sel["gene"], np.int32)
-        prof_off, prof_len = arr(sel["prof_off"], np.int64), arr(sel["prof_len"], np.int64)
-        exon_ptr, exon_start, exon_end = arr(exon_ptr, np.int64), arr(exon_start, np.int32), arr(exon_end, np.int32)
-        orf_strand = arr(orf_strand, np.uint8)
-        q = _lib.CountQuery(len(row), _np_ptr(row), _np_ptr(gene), _np_ptr(prof_off), _np_ptr(prof_len), _np_ptr(tsv),
-                            len(exon_ptr) - 1, _np_ptr(exon_ptr), _np_ptr(exon_start), _np_ptr(exon_end),
-                            _np_ptr(orf_strand), int(n_gene))
+        q = self._rows_query(_lib.CountQuery, sel, exon_ptr, exon_start, exon_end, orf_strand, dict(tsv=tsv),
+                             n_gene=n_gene)
         total, length = np.zeros(int(n_gene), np.uint64), np.zeros(int(n_gene), np.uint64)
         summary = np.zeros(4, np.int64)
-        ms = np.zeros(_lib.RT_COUNT_STAGES, np.float32)
-        rc = self.lib.rt_count_orfs(self.ctx, C.byref(q), _np_ptr(total), _np_ptr(length), _np_ptr(summary), _np_ptr(ms))
-        if rc == _lib.RT_EINVAL:
-            raise ValueError(self.lib.rt_last_error(self.ctx).decode())
-        self._check(rc)
-        if stage_ms is not None:
-            stage_ms[:] = ms
+        self._command(self.lib.rt_count_orfs, _lib.RT_COUNT_STAGES, stage_ms, C.byref(q), _np_ptr(total),
+                      _np_ptr(length), _np_ptr(summary))
         return total, length, summary
 
     # --------------------------------------------------------------- BGZF text inputs
@@ -566,13 +565,10 @@ class Engine:
 
         h = C.c_void_p()
         sm = np.zeros(4, np.int64)
-        ms = np.zeros(_lib.RT_BGZF_STAGES, np.float32)
-        rc = self.lib.rt_bgzf_inflate(self.ctx, str(path).encode(), C.byref(h), _np_ptr(sm), _np_ptr(ms))
-        if summary is not None:
-            summary[:] = sm
-        if rc == _lib.RT_EINVAL:
-            raise ValueError(self.lib.rt_last_error(self.ctx).decode())
-        self._check(rc)
-        if stage_ms is not None:
-            stage_ms[:] = ms
+        try:
+            self._command(self.lib.rt_bgzf_inflate, _lib.RT_BGZF_STAGES, stage_ms, str(path).encode(), C.byref(h),
+                          _np_ptr(sm))
+        finally:
+            if summary is not None:
+                summary[:] = sm
         return NativeText(h, str(path))

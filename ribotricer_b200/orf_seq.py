@@ -13,12 +13,11 @@ from __future__ import annotations
 
 import os
 import pathlib
-import time
 
 import numpy as np
 
 from . import _lib
-from .bgzf import open_texts
+from .bgzf import StageClock, open_texts
 from .index import load_native_index
 from .prepare_orfs import Genome
 
@@ -29,22 +28,14 @@ def orf_seq(ribotricer_index, genome_fasta, saveto, translate=False, chunk_bytes
     protein instead of the nucleotides.  ``stage_ms``, when given, receives the time of every stage in milliseconds."""
     from .detect_orfs import get_engine
 
-    times = {} if stage_ms is None else stage_ms
-    clock = time.perf_counter()
-
-    def lap(name):
-        nonlocal clock
-        now = time.perf_counter()
-        times[name] = (now - clock) * 1e3
-        clock = now
-
+    clock = StageClock(stage_ms)
     index_src, fasta_src = open_texts([ribotricer_index, genome_fasta], "orfs-seq")
-    lap("inflate")
+    clock.lap("inflate")
     idx = load_native_index(index_src)
     id_off, ids = idx.ids()
-    lap("index_load")
+    clock.lap("index_load")
     genome = Genome(fasta_src)
-    lap("fasta_load")
+    clock.lap("fasta_load")
     lut = {name: i for i, name in enumerate(genome.names)}
     table = np.array([lut.get(c, -1) for c in idx.chrom_names], np.int64)
     for k in np.flatnonzero(table < 0).tolist():
@@ -57,15 +48,14 @@ def orf_seq(ribotricer_index, genome_fasta, saveto, translate=False, chunk_bytes
     contig_base = np.cumsum(contig_len) - contig_len
     orf_contig = np.searchsorted(used, table)[idx.orf_chrom_id] if idx.n_orf else np.zeros(0, np.int64)
     genome.close()
-    lap("codes")
+    clock.lap("codes")
     pathlib.Path(os.path.dirname(os.path.abspath(saveto))).mkdir(parents=True, exist_ok=True)
     dev_ms = np.zeros(_lib.RT_SEQ_STAGES, np.float32)
     get_engine().orf_seq_write(saveto, idx.exon_ptr, idx.exon_start, idx.exon_end, orf_contig,
                                idx.orf_strand_code == 1, contig_base, contig_len, codes, id_off, ids, bool(translate),
                                chunk_bytes, stage_ms=dev_ms)
-    lap("write")
-    for name, ms in zip(("upload", "orf_seq_kernel", "copy_back"), dev_ms.tolist()):
-        times["device:" + name] = ms
+    clock.lap("write")
+    clock.device(("upload", "orf_seq_kernel", "copy_back"), dev_ms)
     n_orf = idx.n_orf
     residues = os.path.getsize(saveto) - len("ORF_ID\tsequence\n") - int(id_off[-1]) - 2 * n_orf
     unit = "aa" if translate else "nt"

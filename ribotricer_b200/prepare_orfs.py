@@ -19,7 +19,7 @@ import pathlib
 import numpy as np
 
 from . import _lib
-from .bgzf import NativeText, open_text, open_texts
+from .bgzf import NativeText, StageClock, open_text, open_texts
 
 TYPES = ("annotated", "uORF", "overlap_uORF", "super_uORF", "overlap_dORF", "dORF", "novel", "internal")
 BASES = "ACGT"
@@ -275,8 +275,6 @@ def prepare_orfs(gtf, fasta, prefix, min_orf_length=60, start_codons={"ATG"}, st
                  longest=False, stage_ms: dict | None = None):
     """Write ``{prefix}_candidate_orfs.tsv`` (DESIGN.md section 9).  ``stage_ms``, when given, receives the time of
     every stage in milliseconds."""
-    import time
-
     from .detect_orfs import get_engine
 
     if min_orf_length < 0:
@@ -285,38 +283,29 @@ def prepare_orfs(gtf, fasta, prefix, min_orf_length=60, start_codons={"ATG"}, st
         raise ValueError("the start and stop codon lists must not be empty")
     start_mask, stop_mask = codon_mask(start_codons), codon_mask(stop_codons)
     pathlib.Path(os.path.dirname(prefix) or ".").mkdir(parents=True, exist_ok=True)
-    times = {} if stage_ms is None else stage_ms
-    clock = time.perf_counter()
-
-    def lap(name):
-        nonlocal clock
-        now = time.perf_counter()
-        times[name] = (now - clock) * 1e3
-        clock = now
-
+    clock = StageClock(stage_ms)
     fasta_src, gtf_src = open_texts([fasta, gtf], "prepare-orfs")
-    lap("inflate")
+    clock.lap("inflate")
     genome = Genome(fasta_src)
-    lap("fasta_load")
+    clock.lap("fasta_load")
     g = load_gtf(gtf_src)
-    lap("gtf_load")
+    clock.lap("gtf_load")
     tx = build_transcripts(g, genome)
     used = np.unique(tx["contig"]).astype(np.int32)
     codes = genome.codes(used)
     base = np.zeros(len(genome.names), np.int64)
     base[used] = np.concatenate([[0], np.cumsum(genome.lengths[used])[:-1]]) if len(used) else 0
     tx_base = base[tx["contig"]] if tx["n"] else np.zeros(0, np.int64)
-    lap("transcripts")
+    clock.lap("transcripts")
     ann = _annotated(tx, codes, tx_base, start_mask)
-    lap("annotated")
+    clock.lap("annotated")
     dev_ms = np.zeros(_lib.RT_ORF_STAGES, np.float32)
     cand = get_engine().orf_search(codes, tx_base, tx["exon_ptr"], tx["exon_start"], tx["exon_end"], tx["strand"],
                                    tx["cds_bounds"], start_mask, stop_mask, int(min_orf_length), bool(longest),
                                    stage_ms=dev_ms)
-    lap("orf_search")
-    for name, ms in zip(("upload", "orf_splice_kernel", "orf_walk_kernel<count>", "row_scan", "orf_walk_kernel<fill>",
-                         "orf_interval_kernel<count>+scan", "orf_interval_kernel<fill>"), dev_ms.tolist()):
-        times["device:" + name] = ms
+    clock.lap("orf_search")
+    clock.device(("upload", "orf_splice_kernel", "orf_walk_kernel<count>", "row_scan", "orf_walk_kernel<fill>",
+                  "orf_interval_kernel<count>+scan", "orf_interval_kernel<fill>"), dev_ms)
     text, text_off, id_len = _tx_text(tx, g["strings"])
     n_ann = len(ann["row_tx"])
     rows = {k: np.concatenate([ann[k], cand[k]]) for k in ("row_tx", "row_type", "row_codon", "iv_start", "iv_end")}
@@ -328,7 +317,7 @@ def prepare_orfs(gtf, fasta, prefix, min_orf_length=60, start_codons={"ATG"}, st
                                                             "iv_end")])
     if rc != 0:
         raise _io_error("cannot write the index")
-    lap("write")
+    clock.lap("write")
     genome.close()
     print(f"prepare-orfs: {tx['n']} transcripts ({tx['n_skipped']} skipped), {n_ann} annotated and "
           f"{n_rows - n_ann} candidate ORFs written to {prefix}_candidate_orfs.tsv")

@@ -271,6 +271,7 @@ def test_closed_engines_give_their_device_memory_back(case, tmp_path):
     many = {k: np.repeat(v, 80) for k, v in reads.items()}        # stays coordinate-sorted
     rng = np.random.default_rng(5)
     orf_q, seq_q, codon_q = _orf_query(rng, 3000), _seq_query(rng, 3000), _codon_query(rng, 2000, 2500)
+    count_q = {k: v for k, v in codon_q.items() if k not in ("seq", "n_gseq")}
     scores = rng.random(50_000)
     boot = rng.integers(0, len(scores), (30_000, 6)).astype(np.int64)   # 240 KB of keys per replicate: global scratch
     free = []
@@ -292,20 +293,24 @@ def test_closed_engines_give_their_device_memory_back(case, tmp_path):
         for protein in (False, True):
             eng.orf_seq_write(tmp_path / f"seq{cycle}.tsv", **seq_q, protein=protein, chunk_bytes=1 << 16)
         tabs = eng.codon_counts(**codon_q)
+        counts = eng.orf_counts(**count_q)
         med = learn_cutoff._bootstrap_medians(eng, scores, boot)
         if cycle == 0:
-            first = (cols, rows, tabs, med)
+            first = (cols, rows, tabs, med, counts)
         else:
             _same(cols, first[0])
             _same(rows, first[1])
             for x, y in zip(tabs, first[2]):
                 assert np.array_equal(x, y)
             assert np.array_equal(med, first[3])
+            for x, y in zip(counts, first[4]):
+                assert np.array_equal(x, y)
         eng.close()
         del cov
         torch.cuda.synchronize()
         torch.cuda.empty_cache()
         free.append(torch.cuda.mem_get_info()[0])
     assert first[2][2][4] == -1, "a profile of the codon query was refused"
+    assert first[4][2][2] == -1, "a profile of the count query was refused"
     drift = [f - free[0] for f in free[1:]]
     assert all(abs(d) <= 4 << 20 for d in drift), drift
